@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--backend auto|ffma|tc]
                     [--config 1..5] [--rows R] [--scaling weak|strong] [--global-rows G] [--mode nadp|mpg] [--env pt|ip|idp]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -22,8 +23,14 @@ The other BASELINE.json configs (parity-test cases and the config matrix of prof
   --config 5 : PathTracking MPG-v2 + prioritized replay at B = 262,144: sum-tree sample -> compute_gradient ->
                update_priorities on the device, reported as updates/s (e2e) next to the policy-gradient value
 One JSON line is printed by rank 0.
+--dump-outputs DIR : after the timed steps, rank 0 writes what the last timed step returned, so that two builds can be
+          compared output for output on the same seeded inputs:
+            DIR/policy_grad.npy       flat policy gradient of the last device step (fp32; all-reduced when N > 1)
+            DIR/compute_gradient.npy  the arrays of the last e2e compute_gradient, flattened and concatenated in the
+                                      order it returns them (clipped [Q1 | Q2 | policy]; --impl reference: the oracle's)
 """
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -65,6 +72,13 @@ def flop_per_state_step(env_id, full_bptt):
     else:
         traj = (n + 1) * f_pi + n * f_pi + (2 * f_pi - 2 * d_o * HID) + 4 * f_q
     return traj / n
+
+
+def dump_outputs(out_dir, arrays):
+    """{name: array} -> out_dir/<name>.npy; fp32 is kept, every other dtype is written as fp64."""
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if isinstance(a, torch.Tensor) else np.asarray(a)
+        np.save(os.path.join(out_dir, name + '.npy'), a if a.dtype == np.float32 else a.astype(np.float64))
 
 
 def make_inputs(env_id, rows, seed=1234):
@@ -151,6 +165,7 @@ class ClockSampler:
         try:
             self.p = subprocess.Popen(['nvidia-smi', f'--query-gpu={self.Q}', '--format=csv,noheader,nounits',
                                        '-lms', '100', '-i', str(gpu_index)], stdout=self.f, stderr=subprocess.DEVNULL)
+            atexit.register(self.p.kill)    # a run that fails before stop() must not leave the sampler behind
         except Exception:
             self.p = None
 
@@ -213,16 +228,17 @@ def run_reference(opts, c, rank):
 
     def step():
         if c['alg'] == 'NADP':
-            O.nadp_compute_gradient(args, weights, batch, nq, npol, torch.float32)
-        else:
-            O.mpg_compute_gradient(args, weights, batch, npol, 4000, torch.float32)
+            return O.nadp_compute_gradient(args, weights, batch, nq, npol, torch.float32)
+        return O.mpg_compute_gradient(args, weights, batch, npol, 4000, torch.float32)
     for _ in range(opts.warmup):
         step()
     ts = []
     for _ in range(opts.steps):
         t0 = time.perf_counter()
-        step()
+        out = step()
         ts.append(time.perf_counter() - t0)
+    if opts.dump_outputs:
+        dump_outputs(opts.dump_outputs, {'compute_gradient': out['compute_gradient']})
     dt = float(np.mean(ts))
     value = rows * N_STEPS / dt
     sample = (f'all {rows} rows of one GPU\'s shard per step, full {c["alg"]} compute_gradient (Q side + policy rollout '
@@ -275,8 +291,14 @@ def main():
     ap.add_argument('--mode', default='', choices=['', 'nadp', 'mpg'])
     ap.add_argument('--env', default='', choices=['', 'pt', 'ip', 'idp'])
     ap.add_argument('--no-cpu-baseline', action='store_true')
+    ap.add_argument('--dump-outputs', default='', metavar='DIR',
+                    help='write the outputs of the last timed step as DIR/<name>.npy (see the module docstring)')
     opts = ap.parse_args()
     opts.warmup = max(opts.warmup, 3) if opts.impl == 'ours' else opts.warmup
+    if opts.steps < 1:
+        raise SystemExit('--steps must be at least 1')
+    if opts.dump_outputs:
+        os.makedirs(opts.dump_outputs, exist_ok=True)
 
     rank = int(os.environ.get('RANK', '0'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))
@@ -352,19 +374,13 @@ def main():
     for a, b in ev:
         flush.zero_()                       # evict L2 between timed iterations
         a.record()
-        device_step()
+        g_last = device_step()
         b.record()
     barrier()
     step_ms = [a.elapsed_time(b) for a, b in ev]
     launches = e.launch_count - l0
-    # dominant-kernel duration (events recorded inside the library right around the rollout kernel)
-    kernel_ms = []
-    for _ in range(3):
-        flush.zero_()
-        device_step()
-        torch.cuda.synchronize()
-        kernel_ms.append(e.kernel_ms())
-    kernel_ms = [k for k in kernel_ms if k is not None and k > 0]
+    # dominant-kernel duration of the last timed step (events recorded inside the library right around the rollout kernel)
+    kernel_ms = e.kernel_ms()
     e.set_timing(False)
     total_ms = torch.tensor([sum(step_ms)], dtype=torch.float64, device='cuda')
     if world > 1:
@@ -393,7 +409,7 @@ def main():
 
     for it in range(2):
         update(it)
-    e2e_steps = max(3, min(opts.steps, 10))
+    e2e_steps = opts.steps
     block_s = []
     for _ in range(3):            # three blocks of K updates; the MEDIAN block is reported
         barrier()
@@ -409,6 +425,9 @@ def main():
     d2h = int(sum(g.nbytes for g in grads)) + 4 * 8
     e2e_value = rows * world * N_STEPS / e2e_s
     clocks = sampler.stop() if sampler else None
+    if opts.dump_outputs and rank == 0:
+        dump_outputs(opts.dump_outputs, {'policy_grad': g_last,
+                                         'compute_gradient': np.concatenate([x.ravel() for x in grads])})
 
     if rank != 0:
         if world > 1:
@@ -421,7 +440,7 @@ def main():
     except Exception:
         pass
     flop = flop_per_state_step(env_id, full_bptt)
-    k_ms = float(np.mean(kernel_ms)) if kernel_ms else ms_per_step
+    k_ms = kernel_ms if kernel_ms > 0 else ms_per_step
     if full_bptt and backend == 'tc' and rows > e.MAX_TC_FULL_BPTT_ROWS:
         k_ms = ms_per_step      # the call is split into row chunks (several launches): the whole step is the denominator
     achieved_tf = rows * N_STEPS * flop / (k_ms * 1e-3) / 1e12
