@@ -59,7 +59,7 @@ typedef struct {
   int32_t num_future_data;   /* PathTracking only (path_tracking_env.py:265-271) */
   int32_t obs_dim;           /* 6+nfd | 4 | 11 */
   int32_t act_dim;           /* 2 | 1 | 1 */
-  int32_t hidden;            /* *_num_hidden_units; this build supports 256 with 2 hidden layers */
+  int32_t hidden;            /* *_num_hidden_units of every net of the handle: 64, 128 or 256 (2 hidden layers) */
   int32_t policy_out_tanh;   /* policy_out_activation == 'tanh' */
   float action_range;        /* policy.py:197; <= 0 means None */
   float obs_scale[MPG_MAX_OBS]; /* preprocessor.py:134-145, 'scale' mode */
@@ -207,9 +207,10 @@ int mpg_philox_noise(mpg_ctx* ctx, const mpg_rollout_params* p, float* out, void
 
 /* Kernel family used by mpg_policy_grad / mpg_rollout_forward:
  *   MPG_BACKEND_FFMA  fp32 CUDA-core contractions (every env / shape this build supports)
- *   MPG_BACKEND_TC    tcgen05 tensor-core contractions with split-bf16 operands (fp32-accurate);
+ *   MPG_BACKEND_TC    tcgen05 tensor-core contractions with split-bf16 operands (fp32-accurate), hidden = 256 only;
  *                     returns MPG_ERR_UNSUPPORTED for configurations it does not cover
- * mpg_create selects MPG_BACKEND_TC whenever it covers the configuration (obs_dim + act_dim + 1 <= 16), else
+ * mpg_create selects MPG_BACKEND_TC whenever it covers the configuration (hidden = 256 and
+ * obs_dim + act_dim + 1 <= 16), else
  * MPG_BACKEND_FFMA; the environment variable MPG_B200_BACKEND=ffma forces the fp32 path at creation. */
 enum { MPG_BACKEND_FFMA = 0, MPG_BACKEND_TC = 1 };
 int mpg_set_backend(mpg_ctx* ctx, int backend);

@@ -3,6 +3,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <new>
+#include <type_traits>
 #include <vector>
 
 #include "rollout_kernels.cuh"
@@ -80,9 +81,23 @@ int fail(mpg_ctx* ctx, int code, const char* fmt, const char* detail = "") {
     if (e__ != cudaSuccess) return fail(ctx, MPG_ERR_CUDA, #expr ": %s", cudaGetErrorString(e__)); \
   } while (0)
 
+// flat parameter layout of one net of this handle
+GradLayout layout(const mpg_ctx* c, const NetStore& n) { return GradLayout(n.in_dim, n.out_dim, c->cfg.hidden); }
+
+// The one place the handle's hidden width becomes the template argument of the FFMA kernels: f(integral_constant<H>).
+// mpg_create admits 64, 128 and 256 only.
+template <typename F>
+int with_hidden(const mpg_ctx* c, F&& f) {
+  switch (c->cfg.hidden) {
+    case 64: return f(std::integral_constant<int, 64>());
+    case 128: return f(std::integral_constant<int, 128>());
+    default: return f(std::integral_constant<int, 256>());
+  }
+}
+
 NetDev net_dev(const mpg_ctx* c, int net) {
   const NetStore& n = c->nets[net];
-  GradLayout L(n.in_dim, n.out_dim);
+  const GradLayout L = layout(c, n);
   NetDev d;
   d.W1p = n.W1p; d.b1 = n.flat + L.ob1; d.W2p = n.W2p; d.b2 = n.flat + L.ob2; d.W2Tp = n.W2Tp;
   d.W3 = n.flat + L.oW3; d.b3 = n.flat + L.ob3; d.W1 = n.flat + L.oW1;
@@ -90,16 +105,17 @@ NetDev net_dev(const mpg_ctx* c, int net) {
   return d;
 }
 
+template <int H>
 __global__ void pack_kernel(const float* __restrict__ flat, int in_dim, int out_dim, float* __restrict__ W1p,
                             float* __restrict__ W2p, float* __restrict__ W2Tp) {
-  const GradLayout L(in_dim, out_dim);
+  const GradLayout L(in_dim, out_dim, H);
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= H * H) return;
-  // packed column pc = 128 (j >> 2) + 4 l + (j & 3)  <->  natural column c = l + 32 j (mlp_tile.cuh: rowgemm)
-  const int k = idx / H, pc = idx % H, l = (pc & 127) >> 2, j = (pc >> 7) * 4 + (pc & 3), c = l + 32 * j;
-  W2p[idx] = flat[L.oW2 + k * H + c];
-  W2Tp[idx] = flat[L.oW2 + c * H + k];   // W2T[n=k][col c] = W2[c][k]
-  if (k < in_dim) W1p[idx] = flat[L.oW1 + k * H + c];
+  // natural column c of row k -> packed column packed_col<H>(c) (mlp_tile.cuh: rowgemm reads through the same map)
+  const int k = idx / H, c = idx % H, o = k * H + packed_col<H>(c);
+  W2p[o] = flat[L.oW2 + k * H + c];
+  W2Tp[o] = flat[L.oW2 + c * H + k];   // W2T[n=k][col c] = W2[c][k]
+  if (k < in_dim) W1p[o] = flat[L.oW1 + k * H + c];
 }
 
 __global__ void adam_kernel(float* __restrict__ w, float* __restrict__ m, float* __restrict__ v, const float* __restrict__ g,
@@ -226,9 +242,9 @@ __global__ void philox_noise_kernel(unsigned long long seed, long long global_ro
   out[idx] = philox_normal(seed, nr, (uint32_t)t);
 }
 
-template <typename K>
+template <int H, typename K>
 int set_smem(mpg_ctx* ctx, K kernel) {
-  CUDA_OK(ctx, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, Smem::FLOATS * 4));
+  CUDA_OK(ctx, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, Smem<H>::FLOATS * 4));
   return MPG_OK;
 }
 
@@ -291,17 +307,21 @@ int rec_hi_only(const mpg_ctx* ctx, long long contraction_rows) {
 
 template <bool BWD>
 int launch_rollout(mpg_ctx* ctx, const RolloutArgs& a, int grid, cudaStream_t st, int env) {
-  const size_t smem = Smem::FLOATS * 4;
+  if (BWD && env == MPG_ENV_PATH_TRACKING_REAL) return fail(ctx, MPG_ERR_UNSUPPORTED, "the real environment is forward only%s");
   if (ctx->timing) cudaEventRecord(ctx->ev0, st);
-  if (env == MPG_ENV_PATH_TRACKING_REAL) {
-    if (BWD) return fail(ctx, MPG_ERR_UNSUPPORTED, "the real environment is forward only%s");
-    rollout_kernel<MPG_ENV_PATH_TRACKING_REAL, false><<<grid, NT, smem, st>>>(a);
-  } else
-  switch (env) {
-    case MPG_ENV_PATH_TRACKING: rollout_kernel<MPG_ENV_PATH_TRACKING, BWD><<<grid, NT, smem, st>>>(a); break;
-    case MPG_ENV_INVERTED_PENDULUM: rollout_kernel<MPG_ENV_INVERTED_PENDULUM, BWD><<<grid, NT, smem, st>>>(a); break;
-    default: rollout_kernel<MPG_ENV_INVERTED_DOUBLE_PENDULUM, BWD><<<grid, NT, smem, st>>>(a); break;
-  }
+  with_hidden(ctx, [&](auto hc) {
+    constexpr int HW = decltype(hc)::value;
+    const size_t smem = Smem<HW>::FLOATS * 4;
+    if (env == MPG_ENV_PATH_TRACKING_REAL) {
+      rollout_kernel<HW, MPG_ENV_PATH_TRACKING_REAL, false><<<grid, NT, smem, st>>>(a);
+    } else
+    switch (env) {
+      case MPG_ENV_PATH_TRACKING: rollout_kernel<HW, MPG_ENV_PATH_TRACKING, BWD><<<grid, NT, smem, st>>>(a); break;
+      case MPG_ENV_INVERTED_PENDULUM: rollout_kernel<HW, MPG_ENV_INVERTED_PENDULUM, BWD><<<grid, NT, smem, st>>>(a); break;
+      default: rollout_kernel<HW, MPG_ENV_INVERTED_DOUBLE_PENDULUM, BWD><<<grid, NT, smem, st>>>(a); break;
+    }
+    return MPG_OK;
+  });
   if (ctx->timing) { cudaEventRecord(ctx->ev1, st); ctx->timed = 1; }
   ctx->launches++;
   CUDA_OK(ctx, cudaGetLastError());
@@ -322,7 +342,8 @@ int mpg_get_backend(const mpg_ctx* ctx) { return ctx->backend; }
 int mpg_set_backend(mpg_ctx* ctx, int backend) {
   if (!ctx || (backend != MPG_BACKEND_FFMA && backend != MPG_BACKEND_TC)) return fail(ctx, MPG_ERR_ARG, "bad backend%s");
   if (backend == MPG_BACKEND_TC && !ctx->tc.ready)
-    return fail(ctx, MPG_ERR_UNSUPPORTED, "tensor-core backend does not cover this configuration%s");
+    return fail(ctx, MPG_ERR_UNSUPPORTED,
+                "tensor-core backend does not cover this configuration (it needs hidden = 256 and obs_dim + act_dim <= 15)%s");
   ctx->backend = backend;
   return MPG_OK;
 }
@@ -369,7 +390,7 @@ int mpg_tc_selftest(mpg_ctx* ctx, int kind, const float* X, const float* W, floa
 
 int mpg_param_count(const mpg_ctx* ctx, int net) {
   if (net < 0 || net >= MPG_NUM_NETS) return -1;
-  return GradLayout(ctx->nets[net].in_dim, ctx->nets[net].out_dim).total;
+  return layout(ctx, ctx->nets[net]).total;
 }
 
 int mpg_create(const mpg_config* cfg, mpg_ctx** out) {
@@ -378,7 +399,8 @@ int mpg_create(const mpg_config* cfg, mpg_ctx** out) {
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
     return fail(nullptr, MPG_ERR_CUDA, "no CUDA device: mpg_b200 has no CPU fallback%s");
-  if (cfg->hidden != H) return fail(nullptr, MPG_ERR_UNSUPPORTED, "only hidden = 256 (2 hidden layers) is built%s");
+  if (cfg->hidden != 64 && cfg->hidden != 128 && cfg->hidden != 256)
+    return fail(nullptr, MPG_ERR_UNSUPPORTED, "hidden must be 64, 128 or 256 (2 hidden layers); other widths are not built%s");
   if (cfg->env < 0 || cfg->env > 3) return fail(nullptr, MPG_ERR_ARG, "unknown env%s");
   static const int SD[4] = {6, 4, 6, 8}, AD[4] = {2, 1, 1, 2};
   if (cfg->act_dim != AD[cfg->env]) return fail(nullptr, MPG_ERR_ARG, "act_dim does not match env%s");
@@ -412,10 +434,10 @@ int mpg_create(const mpg_config* cfg, mpg_ctx** out) {
     const bool is_pol = (n == MPG_NET_POLICY || n == MPG_NET_POLICY_TARGET);
     ns.in_dim = is_pol ? cfg->obs_dim : cfg->obs_dim + cfg->act_dim;
     ns.out_dim = is_pol ? 2 * cfg->act_dim : 1;
-    GradLayout L(ns.in_dim, ns.out_dim);
+    const GradLayout L = layout(c, ns);
+    const size_t hw = (size_t)cfg->hidden;
     maxP = L.total > (int)maxP ? L.total : maxP;
-    ok = ok && alloc(&ns.flat, L.total) && alloc(&ns.W1p, (size_t)MAX_IN * H) && alloc(&ns.W2p, (size_t)H * H)
-         && alloc(&ns.W2Tp, (size_t)H * H);
+    ok = ok && alloc(&ns.flat, L.total) && alloc(&ns.W1p, MAX_IN * hw) && alloc(&ns.W2p, hw * hw) && alloc(&ns.W2Tp, hw * hw);
   }
   c->partial_stride = (maxP + 3) & ~size_t(3);
   ok = ok && alloc(&c->ckpt, (size_t)(cfg->max_horizon + 1) * cfg->max_rows * c->S)
@@ -428,17 +450,21 @@ int mpg_create(const mpg_config* cfg, mpg_ctx** out) {
     mpg_destroy(c);
     return MPG_ERR_CUDA;
   }
-  int rc = 0;
-  rc |= set_smem(c, rollout_kernel<MPG_ENV_PATH_TRACKING, true>);
-  rc |= set_smem(c, rollout_kernel<MPG_ENV_PATH_TRACKING, false>);
-  rc |= set_smem(c, rollout_kernel<MPG_ENV_INVERTED_PENDULUM, true>);
-  rc |= set_smem(c, rollout_kernel<MPG_ENV_INVERTED_PENDULUM, false>);
-  rc |= set_smem(c, rollout_kernel<MPG_ENV_INVERTED_DOUBLE_PENDULUM, true>);
-  rc |= set_smem(c, rollout_kernel<MPG_ENV_INVERTED_DOUBLE_PENDULUM, false>);
-  rc |= set_smem(c, rollout_kernel<MPG_ENV_PATH_TRACKING_REAL, false>);
-  rc |= set_smem(c, q_grad_kernel);
-  rc |= set_smem(c, eval_kernel);
-  rc |= set_smem(c, env_sample_kernel);
+  const int rc = with_hidden(c, [&](auto hc) {   // the instantiations this handle launches
+    constexpr int HW = decltype(hc)::value;
+    int r = 0;
+    r |= set_smem<HW>(c, rollout_kernel<HW, MPG_ENV_PATH_TRACKING, true>);
+    r |= set_smem<HW>(c, rollout_kernel<HW, MPG_ENV_PATH_TRACKING, false>);
+    r |= set_smem<HW>(c, rollout_kernel<HW, MPG_ENV_INVERTED_PENDULUM, true>);
+    r |= set_smem<HW>(c, rollout_kernel<HW, MPG_ENV_INVERTED_PENDULUM, false>);
+    r |= set_smem<HW>(c, rollout_kernel<HW, MPG_ENV_INVERTED_DOUBLE_PENDULUM, true>);
+    r |= set_smem<HW>(c, rollout_kernel<HW, MPG_ENV_INVERTED_DOUBLE_PENDULUM, false>);
+    r |= set_smem<HW>(c, rollout_kernel<HW, MPG_ENV_PATH_TRACKING_REAL, false>);
+    r |= set_smem<HW>(c, q_grad_kernel<HW>);
+    r |= set_smem<HW>(c, eval_kernel<HW>);
+    r |= set_smem<HW>(c, env_sample_kernel<HW>);
+    return r;
+  });
   if (rc) {
     strncpy(g_create_err, c->err, 512);
     mpg_destroy(c);
@@ -476,19 +502,29 @@ void mpg_destroy(mpg_ctx* c) {
   delete c;
 }
 
+// FFMA weight images (W1p, W2p, W2Tp) of one net from its flat natural weights
+static void launch_pack(mpg_ctx* ctx, const NetStore& ns, cudaStream_t st) {
+  with_hidden(ctx, [&](auto hc) {
+    constexpr int HW = decltype(hc)::value;
+    pack_kernel<HW><<<(HW * HW + 255) / 256, 256, 0, st>>>(ns.flat, ns.in_dim, ns.out_dim, ns.W1p, ns.W2p, ns.W2Tp);
+    return MPG_OK;
+  });
+  ctx->launches++;
+}
+
 int mpg_set_weights(mpg_ctx* ctx, int net, const float* const w[6], void* stream) {
   if (!ctx || net < 0 || net >= MPG_NUM_NETS || !w) return fail(ctx, MPG_ERR_ARG, "bad argument to mpg_set_weights%s");
   cudaStream_t st = (cudaStream_t)stream;
   NetStore& ns = ctx->nets[net];
-  GradLayout L(ns.in_dim, ns.out_dim);
+  const GradLayout L = layout(ctx, ns);
+  const int hw = ctx->cfg.hidden;
   const int off[6] = {L.oW1, L.ob1, L.oW2, L.ob2, L.oW3, L.ob3};
-  const int cnt[6] = {ns.in_dim * H, H, H * H, H, H * ns.out_dim, ns.out_dim};
+  const int cnt[6] = {ns.in_dim * hw, hw, hw * hw, hw, hw * ns.out_dim, ns.out_dim};
   for (int i = 0; i < 6; ++i) {
     if (!w[i]) return fail(ctx, MPG_ERR_ARG, "null weight pointer%s");
     CUDA_OK(ctx, cudaMemcpyAsync(ns.flat + off[i], w[i], cnt[i] * sizeof(float), cudaMemcpyDefault, st));
   }
-  pack_kernel<<<(H * H + 255) / 256, 256, 0, st>>>(ns.flat, ns.in_dim, ns.out_dim, ns.W1p, ns.W2p, ns.W2Tp);
-  ctx->launches++;
+  launch_pack(ctx, ns, st);
   CUDA_OK(ctx, cudaGetLastError());
   ns.set = true;
   return tc_pack_weights(ctx->tc, net, ns.flat, ns.in_dim, ns.out_dim, st) ? MPG_OK
@@ -497,8 +533,7 @@ int mpg_set_weights(mpg_ctx* ctx, int net, const float* const w[6], void* stream
 
 static int repack(mpg_ctx* ctx, int net, cudaStream_t st) {
   NetStore& ns = ctx->nets[net];
-  pack_kernel<<<(H * H + 255) / 256, 256, 0, st>>>(ns.flat, ns.in_dim, ns.out_dim, ns.W1p, ns.W2p, ns.W2Tp);
-  ctx->launches++;
+  launch_pack(ctx, ns, st);
   CUDA_OK(ctx, cudaGetLastError());
   return tc_pack_weights(ctx->tc, net, ns.flat, ns.in_dim, ns.out_dim, st) ? MPG_OK
                                                                            : fail(ctx, MPG_ERR_CUDA, "tc weight pack failed%s");
@@ -520,7 +555,7 @@ int mpg_adam_step(mpg_ctx* ctx, int net, const float* grad, float lr, int64_t st
   if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   NetStore& ns = ctx->nets[net];
-  const int n = GradLayout(ns.in_dim, ns.out_dim).total;
+  const int n = layout(ctx, ns).total;
   if ((rc = adam_alloc(ctx, ns, n, st))) return rc;
   const double t = (double)step;
   const float lr_t = (float)((double)lr * sqrt(1.0 - pow((double)beta2, t)) / (1.0 - pow((double)beta1, t)));
@@ -536,7 +571,7 @@ int mpg_get_adam_state(mpg_ctx* ctx, int net, float* m, float* v, void* stream) 
   if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   NetStore& ns = ctx->nets[net];
-  const int n = GradLayout(ns.in_dim, ns.out_dim).total;
+  const int n = layout(ctx, ns).total;
   if ((rc = adam_alloc(ctx, ns, n, st))) return rc;
   CUDA_OK(ctx, cudaMemcpyAsync(m, ns.adam_m, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
   CUDA_OK(ctx, cudaMemcpyAsync(v, ns.adam_v, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
@@ -549,7 +584,7 @@ int mpg_set_adam_state(mpg_ctx* ctx, int net, const float* m, const float* v, vo
   if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   NetStore& ns = ctx->nets[net];
-  const int n = GradLayout(ns.in_dim, ns.out_dim).total;
+  const int n = layout(ctx, ns).total;
   if ((rc = adam_alloc(ctx, ns, n, st))) return rc;
   CUDA_OK(ctx, cudaMemcpyAsync(ns.adam_m, m, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
   CUDA_OK(ctx, cudaMemcpyAsync(ns.adam_v, v, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
@@ -563,7 +598,7 @@ int mpg_polyak_update(mpg_ctx* ctx, int src_net, int dst_net, float tau, void* s
   NetStore &a = ctx->nets[src_net], &d = ctx->nets[dst_net];
   if (a.in_dim != d.in_dim || a.out_dim != d.out_dim) return fail(ctx, MPG_ERR_ARG, "polyak: nets differ in shape%s");
   cudaStream_t st = (cudaStream_t)stream;
-  const int n = GradLayout(a.in_dim, a.out_dim).total;
+  const int n = layout(ctx, a).total;
   polyak_kernel<<<(n + 255) / 256, 256, 0, st>>>(d.flat, a.flat, n, tau);
   ctx->launches++;
   CUDA_OK(ctx, cudaGetLastError());
@@ -575,9 +610,10 @@ int mpg_get_weights(mpg_ctx* ctx, int net, float* const w[6], void* stream) {
   if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   NetStore& ns = ctx->nets[net];
-  GradLayout L(ns.in_dim, ns.out_dim);
+  const GradLayout L = layout(ctx, ns);
+  const int hw = ctx->cfg.hidden;
   const int off[6] = {L.oW1, L.ob1, L.oW2, L.ob2, L.oW3, L.ob3};
-  const int cnt[6] = {ns.in_dim * H, H, H * H, H, H * ns.out_dim, ns.out_dim};
+  const int cnt[6] = {ns.in_dim * hw, hw, hw * hw, hw, hw * ns.out_dim, ns.out_dim};
   for (int i = 0; i < 6; ++i)
     CUDA_OK(ctx, cudaMemcpyAsync(w[i], ns.flat + off[i], cnt[i] * sizeof(float), cudaMemcpyDefault, st));
   return MPG_OK;
@@ -594,7 +630,7 @@ int mpg_policy_grad(mpg_ctx* ctx, const mpg_rollout_params* p, const float* obs,
   a.obs = obs; a.noise = noise; a.returns_out = returns_out;
   a.noise_mode = noise ? 1 : (p->use_philox ? 2 : 0);
   const int MB = p->rows * p->M;
-  const GradLayout L(a.pol.in_dim, a.pol.out_dim);
+  const GradLayout L = layout(ctx, ctx->nets[p->policy_net]);
   if (ctx->backend == MPG_BACKEND_TC) {
     // tensor-core path: fused rollout + BPTT (dX chain), then the split-K weight-gradient GEMMs
     const int ntiles = (MB + tc::ACT_ROWS - 1) / tc::ACT_ROWS;
@@ -781,7 +817,7 @@ int mpg_q_grad(mpg_ctx* ctx, int net, int rows, int64_t global_rows, const float
     da.hi_only = ta.rec_hi_only;
     const int dgrid = 2 * da.nrecords < ctx->sms ? 2 * da.nrecords : (ctx->sms & ~1);
     tc::tc_dw_kernel<<<dgrid, tc::DW_THREADS, tc::DW_SMEM, st>>>(da);
-    const GradLayout L(qin, 1);
+    const GradLayout L(qin, 1, tc::H);
     reduce_partials_kernel<<<(L.total + 255) / 256, 256, 0, st>>>(ctx->partial, ctx->partial_stride, ctx->sms, L.total,
                                                                   grad_out, nullptr, nullptr);
     if (loss_sum_out) {
@@ -802,9 +838,13 @@ int mpg_q_grad(mpg_ctx* ctx, int net, int rows, int64_t global_rows, const float
   a.q = net_dev(ctx, net);
   const int ntiles = (rows + TILE_R - 1) / TILE_R;
   const int grid = ntiles < ctx->sms ? ntiles : ctx->sms;
-  const GradLayout L(a.q.in_dim, a.q.out_dim);
+  const GradLayout L = layout(ctx, ctx->nets[net]);
   CUDA_OK(ctx, cudaMemsetAsync(ctx->partial, 0, (size_t)grid * ctx->partial_stride * sizeof(float), st));
-  q_grad_kernel<<<grid, NT, Smem::FLOATS * 4, st>>>(a);
+  with_hidden(ctx, [&](auto hc) {
+    constexpr int HW = decltype(hc)::value;
+    q_grad_kernel<HW><<<grid, NT, Smem<HW>::FLOATS * 4, st>>>(a);
+    return MPG_OK;
+  });
   reduce_partials_kernel<<<(L.total + 255) / 256, 256, 0, st>>>(ctx->partial, ctx->partial_stride, grid, L.total,
                                                                 grad_out, ctx->loss_partial, loss_sum_out);
   ctx->launches += 2;
@@ -820,7 +860,11 @@ static int launch_eval(mpg_ctx* ctx, EvalArgs& a, void* stream) {
   for (int i = 0; i < MPG_MAX_OBS; ++i) a.obs_scale[i] = c.obs_scale[i];
   const int ntiles = (a.rows + TILE_R - 1) / TILE_R;
   const int grid = ntiles < ctx->sms ? ntiles : ctx->sms;
-  eval_kernel<<<grid, NT, Smem::FLOATS * 4, (cudaStream_t)stream>>>(a);
+  with_hidden(ctx, [&](auto hc) {
+    constexpr int HW = decltype(hc)::value;
+    eval_kernel<HW><<<grid, NT, Smem<HW>::FLOATS * 4, (cudaStream_t)stream>>>(a);
+    return MPG_OK;
+  });
   ctx->launches++;
   CUDA_OK(ctx, cudaGetLastError());
   return MPG_OK;
@@ -1023,7 +1067,11 @@ int mpg_env_sample(mpg_ctx* ctx, int policy_net, int agents, int steps, float ex
   a.explore_noise = explore_noise; a.reset_obs = reset_obs; a.state = state; a.obs = obs;
   a.out_obs = out_obs; a.out_act = out_act; a.out_rew = out_rew; a.out_obs_tp1 = out_obs_tp1; a.out_done = out_done;
   a.net = net_dev(ctx, policy_net);
-  env_sample_kernel<<<(agents + TILE_R - 1) / TILE_R, NT, Smem::FLOATS * 4, (cudaStream_t)stream>>>(a);
+  with_hidden(ctx, [&](auto hc) {
+    constexpr int HW = decltype(hc)::value;
+    env_sample_kernel<HW><<<(agents + TILE_R - 1) / TILE_R, NT, Smem<HW>::FLOATS * 4, (cudaStream_t)stream>>>(a);
+    return MPG_OK;
+  });
   ctx->launches++;
   CUDA_OK(ctx, cudaGetLastError());
   return MPG_OK;

@@ -8,7 +8,8 @@
 
 namespace mpg {
 
-constexpr int H = 256;        // hidden width (model.py: *_num_hidden_units default)
+// The hidden width H (64, 128 or 256) is a template parameter of the FFMA tile engine (mlp_tile.cuh); the tensor-core
+// path has its own tc::H = 256 (tc_common.cuh).
 constexpr int TILE_R = 64;    // rows (trajectories) per CTA tile
 constexpr int RP = 68;        // row pitch of [feature][row] activation tiles in shared memory
 constexpr int NT = 256;       // threads per CTA

@@ -5,14 +5,25 @@
 //   * the "row GEMM" (out[r][n] = sum_k in[k][r] W[k][n]) reads its A operand as warp-broadcast
 //     float4s and its B operand (a weight slab staged by cp.async) as conflict-free float4s;
 //   * the "dW GEMM" (dW[k][n] += sum_r X[k][r] Y[n][r]) reads both operands as float4s along rows.
-// Thread mapping of the row GEMM: warp w owns rows 8w..8w+7, lane l owns columns l + 32 j (j<8).
-// Weights are re-packed once per set_weights so that those 8 columns are two float4s, each at a 16-byte lane stride
-// (a 32-byte lane stride made every weight read a 2-way bank conflict and the loop shared-memory bound in round 1):
+// The hidden width H (64, 128 or 256) is a template parameter; NT = 256 threads and TILE_R = 64 rows for every width.
+// Thread mapping of the row GEMM: warp w owns rows 8w..8w+7, lane l owns columns l + 32 j (j < H/32).
+// Weights are re-packed once per set_weights so that those columns are read as vectors of G = min(4, H/32) floats at a
+// 4G-byte lane stride (a 32-byte lane stride made every weight read a 2-way bank conflict and the loop shared-memory
+// bound in round 1); packed_col<H> below is that map.  At H = 256:
 //   Wp[k][4 l + j] = W[k][l + 32 j] (j < 4),  Wp[k][128 + 4 l + j - 4] = W[k][l + 32 j] (j >= 4).
+// Where a step gives thread tid feature tid, at H < NT the P = NT/H threads tid = f + H p of feature f split the rows
+// into P equal slices; their partial sums are combined in the order p = 0, 1, .. when the accumulators are flushed.
 #pragma once
 #include "common.cuh"
 
 namespace mpg {
+
+// packed column (within a row of W1p / W2p / W2Tp) of natural column c = l + 32 j: vector j / G of lane l, element j % G
+template <int H>
+__host__ __device__ __forceinline__ constexpr int packed_col(int c) {
+  constexpr int G = H / 32 < 4 ? H / 32 : 4;
+  return ((c >> 5) / G) * (32 * G) + G * (c & 31) + (c >> 5) % G;
+}
 
 struct NetDev {
   const float* W1p;   // [in_dim][H] packed columns
@@ -29,14 +40,17 @@ struct NetDev {
 // flat gradient layout (Keras order W1|b1|W2|b2|W3|b3)
 struct GradLayout {
   int oW1, ob1, oW2, ob2, oW3, ob3, total;
-  __host__ __device__ GradLayout(int in_dim, int out_dim) {
+  __host__ __device__ GradLayout(int in_dim, int out_dim, int H) {
     oW1 = 0; ob1 = oW1 + in_dim * H; oW2 = ob1 + H; ob2 = oW2 + H * H; oW3 = ob2 + H; ob3 = oW3 + H * out_dim;
     total = ob3 + out_dim;
   }
 };
 
 // shared memory carve-up (floats)
+template <int H>
 struct Smem {
+  // the slab doubles as scratch of the input-gradient partials, [4][MAX_IN][RP]: at H < 256 that is the larger of the two
+  static constexpr int SLAB = 2 * KS * H > 4 * MAX_IN * RP ? 2 * KS * H : 4 * MAX_IN * RP;
   float* bufA;   // [H][RP]
   float* bufB;   // [H][RP]
   float* slab;   // [2][KS*H]  (also scratch for the input-gradient partials)
@@ -45,23 +59,26 @@ struct Smem {
   float* d3;     // [4][RP]       output-layer deltas
   float* y3;     // [4][RP]       output-layer pre-activations / outputs
   __device__ explicit Smem(float* base) {
-    bufA = base; bufB = bufA + H * RP; slab = bufB + H * RP; xin = slab + 2 * KS * H; gx = xin + MAX_IN * RP;
+    bufA = base; bufB = bufA + H * RP; slab = bufB + H * RP; xin = slab + SLAB; gx = xin + MAX_IN * RP;
     d3 = gx + MAX_IN * RP; y3 = d3 + 4 * RP;
   }
-  static constexpr int FLOATS = 2 * H * RP + 2 * KS * H + 2 * MAX_IN * RP + 8 * RP;
+  static constexpr int FLOATS = 2 * H * RP + SLAB + 2 * MAX_IN * RP + 8 * RP;
 };
+static_assert(Smem<256>::SLAB == 2 * KS * 256, "the H = 256 carve-up is unchanged");
 
 // ---------------------------------------------------------------------------------------------
 // row GEMM: acc[i][j] = sum_k in_s[k][8w+i] * W[k][l+32j]; weight slabs double-buffered via cp.async.
 // Contains __syncthreads(): on entry-side (before first read of in_s) and after the last read.
 // ---------------------------------------------------------------------------------------------
+template <int H>
 __device__ __forceinline__ void rowgemm(const float* __restrict__ in_s, int K, const float* __restrict__ Wp_g,
-                                        float* __restrict__ slab, float (&acc)[8][8]) {
+                                        float* __restrict__ slab, float (&acc)[8][H / 32]) {
+  constexpr int NJ = H / 32, G = NJ < 4 ? NJ : 4;
   const int tid = threadIdx.x, w = tid >> 5, l = tid & 31;
 #pragma unroll
   for (int i = 0; i < 8; ++i)
 #pragma unroll
-    for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
+    for (int j = 0; j < NJ; ++j) acc[i][j] = 0.f;
   const int nslab = (K + KS - 1) / KS;
   auto issue = [&](int s) {
     const int k0 = s * KS, kn = min(KS, K - k0);
@@ -74,32 +91,42 @@ __device__ __forceinline__ void rowgemm(const float* __restrict__ in_s, int K, c
   for (int s = 0; s < nslab; ++s) {
     if (s + 1 < nslab) { issue(s + 1); cp_async_wait<1>(); } else { cp_async_wait<0>(); }
     __syncthreads();
-    const float* sb = slab + (s & 1) * KS * H + l * 4;
+    const float* sb = slab + (s & 1) * KS * H;
     const int k0 = s * KS, kn = min(KS, K - k0);
     const float* ap = in_s + (size_t)k0 * RP + w * 8;
 #pragma unroll 4
     for (int kk = 0; kk < kn; ++kk) {
       const float4 a0 = *reinterpret_cast<const float4*>(ap + kk * RP);
       const float4 a1 = *reinterpret_cast<const float4*>(ap + kk * RP + 4);
-      const float4 b0 = *reinterpret_cast<const float4*>(sb + kk * H);
-      const float4 b1 = *reinterpret_cast<const float4*>(sb + kk * H + 128);
       const float a[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
-      const float b[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
+      float b[NJ];
+#pragma unroll
+      for (int v = 0; v < NJ / G; ++v) {   // vector v holds columns l + 32 (G v + e), e < G
+        const float* bp = sb + kk * H + packed_col<H>(l + 32 * G * v);
+        if constexpr (G == 4) {
+          const float4 t = *reinterpret_cast<const float4*>(bp);
+          b[4 * v] = t.x; b[4 * v + 1] = t.y; b[4 * v + 2] = t.z; b[4 * v + 3] = t.w;
+        } else {
+          const float2 t = *reinterpret_cast<const float2*>(bp);
+          b[2 * v] = t.x; b[2 * v + 1] = t.y;
+        }
+      }
 #pragma unroll
       for (int i = 0; i < 8; ++i)
 #pragma unroll
-        for (int j = 0; j < 8; ++j) acc[i][j] = fmaf(a[i], b[j], acc[i][j]);
+        for (int j = 0; j < NJ; ++j) acc[i][j] = fmaf(a[i], b[j], acc[i][j]);
     }
     __syncthreads();
   }
 }
 
 // epilogue: out[c][rows] = elu(acc + bias[c])
-__device__ __forceinline__ void store_bias_elu(const float (&acc)[8][8], const float* __restrict__ bias,
+template <int H>
+__device__ __forceinline__ void store_bias_elu(const float (&acc)[8][H / 32], const float* __restrict__ bias,
                                                float* __restrict__ out_s) {
   const int tid = threadIdx.x, w = tid >> 5, l = tid & 31;
 #pragma unroll
-  for (int j = 0; j < 8; ++j) {
+  for (int j = 0; j < H / 32; ++j) {
     const int c = l + 32 * j;
     const float bv = __ldg(bias + c);
     float4 v0, v1;
@@ -111,10 +138,11 @@ __device__ __forceinline__ void store_bias_elu(const float (&acc)[8][8], const f
 }
 
 // epilogue: act_s[c][rows] <- acc * elu'(act_s[c][rows])   (in place: activation -> delta)
-__device__ __forceinline__ void store_times_elugrad(const float (&acc)[8][8], float* __restrict__ act_s) {
+template <int H>
+__device__ __forceinline__ void store_times_elugrad(const float (&acc)[8][H / 32], float* __restrict__ act_s) {
   const int tid = threadIdx.x, w = tid >> 5, l = tid & 31;
 #pragma unroll
-  for (int j = 0; j < 8; ++j) {
+  for (int j = 0; j < H / 32; ++j) {
     const int c = l + 32 * j;
     float4* p0 = reinterpret_cast<float4*>(act_s + c * RP + w * 8);
     float4 h0 = p0[0], h1 = p0[1];
@@ -130,12 +158,13 @@ __device__ __forceinline__ void store_times_elugrad(const float (&acc)[8][8], fl
 // forward: xin[0..in_dim) -> h1 (bufA) -> h2 (bufB) -> y3[j][r] = h2 W3 + b3 for j < n_out
 // (n_out = number of output columns actually consumed: act_dim for the policy mean, 1 for Q)
 // ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ void mlp_forward_tile(const NetDev& net, Smem& sm, int n_out) {
-  float acc[8][8];
-  rowgemm(sm.xin, net.in_dim, net.W1p, sm.slab, acc);
-  store_bias_elu(acc, net.b1, sm.bufA);
-  rowgemm(sm.bufA, H, net.W2p, sm.slab, acc);   // first internal barrier publishes bufA
-  store_bias_elu(acc, net.b2, sm.bufB);
+template <int H>
+__device__ __forceinline__ void mlp_forward_tile(const NetDev& net, Smem<H>& sm, int n_out) {
+  float acc[8][H / 32];
+  rowgemm<H>(sm.xin, net.in_dim, net.W1p, sm.slab, acc);
+  store_bias_elu<H>(acc, net.b1, sm.bufA);
+  rowgemm<H>(sm.bufA, H, net.W2p, sm.slab, acc);   // first internal barrier publishes bufA
+  store_bias_elu<H>(acc, net.b2, sm.bufB);
   __syncthreads();
   // output layer: thread (r, q) sums features k = q, q+4, ... for every consumed column, then the
   // four partial sums are combined in a fixed order through shared memory (deterministic)
@@ -161,11 +190,12 @@ __device__ __forceinline__ void mlp_forward_tile(const NetDev& net, Smem& sm, in
   __syncthreads();
 }
 
-// persistent per-thread gradient accumulators (thread tid owns feature tid)
+// persistent per-thread gradient accumulators: thread tid owns feature tid % H, rows slice tid / H (see the top)
+template <int H>
 struct GradAcc {
-  float dW1[MAX_IN];  // dW1[i][tid]
+  float dW1[MAX_IN];  // dW1[i][tid % H]
   float db1, db2;
-  float dW3[MAX_A];   // dW3[tid][j]
+  float dW3[MAX_A];   // dW3[tid % H][j]
   float db3;          // db3[tid] for tid < n_out
   __device__ void zero() {
     db3 = 0.f;
@@ -177,27 +207,30 @@ struct GradAcc {
   }
 };
 
-// dW2[k][n] += sum_r X[k][r] Y[n][r] into this CTA's private global partial (natural (k,n) layout)
+// dW2[k][n] += sum_r X[k][r] Y[n][r] into this CTA's private global partial (natural (k,n) layout).
+// H/64 chunks of 64 columns n (warp w: n = 64 chunk + 8 w + j, j < 8); lane l owns the rows k = l + 32 i, i < H/32.
+template <int H>
 __device__ __forceinline__ void dw2_accumulate(const float* __restrict__ X, const float* __restrict__ Y,
                                                float* __restrict__ dW2g) {
+  constexpr int NI = H / 32;
   const int tid = threadIdx.x, w = tid >> 5, l = tid & 31;
-  for (int chunk = 0; chunk < 4; ++chunk) {
-    float acc[8][8];
+  for (int chunk = 0; chunk < H / 64; ++chunk) {
+    float acc[NI][8];
 #pragma unroll
-    for (int i = 0; i < 8; ++i)
+    for (int i = 0; i < NI; ++i)
 #pragma unroll
       for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
     const float* yb = Y + (chunk * 64 + w * 8) * RP;
 #pragma unroll 2
     for (int r4 = 0; r4 < TILE_R; r4 += 4) {
-      float4 x[8];
+      float4 x[NI];
 #pragma unroll
-      for (int i = 0; i < 8; ++i) x[i] = *reinterpret_cast<const float4*>(X + (l + 32 * i) * RP + r4);
+      for (int i = 0; i < NI; ++i) x[i] = *reinterpret_cast<const float4*>(X + (l + 32 * i) * RP + r4);
 #pragma unroll
       for (int j = 0; j < 8; ++j) {
         const float4 y = *reinterpret_cast<const float4*>(yb + j * RP + r4);
 #pragma unroll
-        for (int i = 0; i < 8; ++i) {
+        for (int i = 0; i < NI; ++i) {
           acc[i][j] = fmaf(x[i].x, y.x, acc[i][j]);
           acc[i][j] = fmaf(x[i].y, y.y, acc[i][j]);
           acc[i][j] = fmaf(x[i].z, y.z, acc[i][j]);
@@ -206,7 +239,7 @@ __device__ __forceinline__ void dw2_accumulate(const float* __restrict__ X, cons
       }
     }
 #pragma unroll
-    for (int i = 0; i < 8; ++i) {
+    for (int i = 0; i < NI; ++i) {
       float4* g = reinterpret_cast<float4*>(dW2g + (size_t)(l + 32 * i) * H + chunk * 64 + w * 8);
       float4 g0 = g[0], g1 = g[1];
       g0.x += acc[i][0]; g0.y += acc[i][1]; g0.z += acc[i][2]; g0.w += acc[i][3];
@@ -222,17 +255,21 @@ __device__ __forceinline__ void dw2_accumulate(const float* __restrict__ X, cons
 // gx[i][r] = dL/d xin[i][r].  With want_dw the parameter gradients are accumulated into `ga`
 // (registers) and dW2g (global partial).
 // ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ void mlp_backward_tile(const NetDev& net, Smem& sm, int n_out, bool want_dw, bool want_gin,
-                                                  GradAcc& ga, float* __restrict__ dW2g) {
+template <int H>
+__device__ __forceinline__ void mlp_backward_tile(const NetDev& net, Smem<H>& sm, int n_out, bool want_dw, bool want_gin,
+                                                  GradAcc<H>& ga, float* __restrict__ dW2g) {
   const int tid = threadIdx.x;
-  // (1) thread k=tid walks its feature row: dW3 += h2 d3, delta2 = (d3 W3^T) elu'(h2) in place, db2
+  // feature f of this thread and its slice [r0, r0 + RS) of the tile rows (P = 1: all rows)
+  constexpr int P = NT / H, RS = TILE_R / P;
+  const int f = P == 1 ? tid : tid % H, r0 = P == 1 ? 0 : (tid / H) * RS;
+  // (1) thread (f, slice) walks its feature row: dW3 += h2 d3, delta2 = (d3 W3^T) elu'(h2) in place, db2
   {
     float w3[MAX_A];
 #pragma unroll
-    for (int j = 0; j < MAX_A; ++j) w3[j] = (j < n_out) ? __ldg(net.W3 + tid * net.out_dim + j) : 0.f;
-    float* hrow = sm.bufB + tid * RP;
+    for (int j = 0; j < MAX_A; ++j) w3[j] = (j < n_out) ? __ldg(net.W3 + f * net.out_dim + j) : 0.f;
+    float* hrow = sm.bufB + f * RP;
     float s_db2 = 0.f, s_dw3[MAX_A] = {0.f, 0.f};
-    for (int r4 = 0; r4 < TILE_R; r4 += 4) {
+    for (int r4 = r0; r4 < r0 + RS; r4 += 4) {
       float4 h = *reinterpret_cast<float4*>(hrow + r4);
       float hv[4] = {h.x, h.y, h.z, h.w}, dv[4];
 #pragma unroll
@@ -263,19 +300,19 @@ __device__ __forceinline__ void mlp_backward_tile(const NetDev& net, Smem& sm, i
   }
   __syncthreads();
   // (2) dW2 += h1^T delta2
-  if (want_dw) dw2_accumulate(sm.bufA, sm.bufB, dW2g);
+  if (want_dw) dw2_accumulate<H>(sm.bufA, sm.bufB, dW2g);
   // (3) delta1 = (delta2 W2^T) elu'(h1), in place over h1
   {
-    float acc[8][8];
-    rowgemm(sm.bufB, H, net.W2Tp, sm.slab, acc);
-    store_times_elugrad(acc, sm.bufA);
+    float acc[8][H / 32];
+    rowgemm<H>(sm.bufB, H, net.W2Tp, sm.slab, acc);
+    store_times_elugrad<H>(acc, sm.bufA);
   }
   __syncthreads();
-  // (4) dW1 += xin^T delta1, db1
+  // (4) dW1 += xin^T delta1, db1 (thread (f, slice) as in (1))
   if (want_dw) {
-    const float* drow = sm.bufA + tid * RP;
+    const float* drow = sm.bufA + f * RP;
     float s_db1 = 0.f;
-    for (int r4 = 0; r4 < TILE_R; r4 += 4) {
+    for (int r4 = r0; r4 < r0 + RS; r4 += 4) {
       const float4 d = *reinterpret_cast<const float4*>(drow + r4);
       s_db1 += (d.x + d.y) + (d.z + d.w);
 #pragma unroll
@@ -287,20 +324,20 @@ __device__ __forceinline__ void mlp_backward_tile(const NetDev& net, Smem& sm, i
     }
     ga.db1 += s_db1;
   }
-  // (5) gx[i][r] = sum_n delta1[n][r] W1[i][n]: thread (r, q) covers n in [64q, 64q+64), partials
+  // (5) gx[i][r] = sum_n delta1[n][r] W1[i][n]: thread (r, q) covers n in [q H/4, (q+1) H/4), partials
   //     combined in fixed order
   if (want_gin) {
     const int r = tid & 63, q = tid >> 6;
     float part[MAX_IN];
 #pragma unroll
     for (int i = 0; i < MAX_IN; ++i) part[i] = 0.f;
-    for (int n = q * 64; n < q * 64 + 64; ++n) {
+    for (int n = q * (H / 4); n < (q + 1) * (H / 4); ++n) {
       const float d = sm.bufA[n * RP + r];
 #pragma unroll
       for (int i = 0; i < MAX_IN; ++i)
         if (i < net.in_dim) part[i] = fmaf(d, __ldg(net.W1 + i * H + n), part[i]);
     }
-    float* scratch = sm.slab;  // [4][MAX_IN][RP] = 5440 floats <= 2*KS*H
+    float* scratch = sm.slab;  // [4][MAX_IN][RP] = 5440 floats <= Smem<H>::SLAB
 #pragma unroll
     for (int i = 0; i < MAX_IN; ++i)
       if (i < net.in_dim) scratch[(q * MAX_IN + i) * RP + r] = part[i];
@@ -314,18 +351,27 @@ __device__ __forceinline__ void mlp_backward_tile(const NetDev& net, Smem& sm, i
   __syncthreads();
 }
 
-// write the register-resident accumulators of this CTA into its private partial buffer
-__device__ __forceinline__ void flush_grad_acc(const NetDev& net, const GradAcc& ga, float* __restrict__ partial) {
-  const GradLayout L(net.in_dim, net.out_dim);
-  const int tid = threadIdx.x;
+// write the register-resident accumulators of this CTA into its private partial buffer.  At H < NT the row slices of a
+// feature are added in the order slice 0, 1, .. (one barrier between slices): bit-reproducible, no atomics.
+// Every thread of the CTA must call it.
+template <int H>
+__device__ __forceinline__ void flush_grad_acc(const NetDev& net, const GradAcc<H>& ga, float* __restrict__ partial) {
+  const GradLayout L(net.in_dim, net.out_dim, H);
+  constexpr int P = NT / H;
+  const int tid = threadIdx.x, f = P == 1 ? tid : tid % H, slice = P == 1 ? 0 : tid / H;
+  for (int p = 0; p < P; ++p) {
+    if (p > 0) __syncthreads();   // the previous slice's sums are in place
+    if (slice != p) continue;
+    auto put = [&](int idx, float v) { partial[idx] = p == 0 ? v : partial[idx] + v; };
 #pragma unroll
-  for (int i = 0; i < MAX_IN; ++i)
-    if (i < net.in_dim) partial[L.oW1 + i * H + tid] = ga.dW1[i];
-  partial[L.ob1 + tid] = ga.db1;
-  partial[L.ob2 + tid] = ga.db2;
+    for (int i = 0; i < MAX_IN; ++i)
+      if (i < net.in_dim) put(L.oW1 + i * H + f, ga.dW1[i]);
+    put(L.ob1 + f, ga.db1);
+    put(L.ob2 + f, ga.db2);
 #pragma unroll
-  for (int j = 0; j < MAX_A; ++j)
-    if (j < net.out_dim) partial[L.oW3 + tid * net.out_dim + j] = ga.dW3[j];
+    for (int j = 0; j < MAX_A; ++j)
+      if (j < net.out_dim) put(L.oW3 + f * net.out_dim + j, ga.dW3[j]);
+  }
   if (tid < MAX_A && tid < net.out_dim) partial[L.ob3 + tid] = ga.db3;
   // columns j >= MAX_A (the unused log-std half of the policy head, policy.py:198) keep their zeros
 }

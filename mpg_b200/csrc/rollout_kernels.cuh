@@ -56,19 +56,19 @@ __device__ __forceinline__ void head_fwd_grad(float z, int out_tanh, float range
   if (range > 0.f) { const float th = tanhf(m); g *= range * (1.f - th * th); act = range * th; }
 }
 
-template <int ENV, bool BWD>
+template <int H, int ENV, bool BWD>
 __global__ void __launch_bounds__(NT, 1) rollout_kernel(const __grid_constant__ RolloutArgs a) {
   extern __shared__ float4 smem_raw[];
-  Smem sm(reinterpret_cast<float*>(smem_raw));
+  Smem<H> sm(reinterpret_cast<float*>(smem_raw));
   using E = Env<ENV>;
   constexpr int S = E::S, A = E::A;
   const int tid = threadIdx.x;
   const int MB = a.rows * a.M;
   const int ntiles = (MB + TILE_R - 1) / TILE_R;
   const bool rowthread = tid < TILE_R;
-  const GradLayout L(a.pol.in_dim, a.pol.out_dim);
+  const GradLayout L(a.pol.in_dim, a.pol.out_dim, H);
   float* partial = a.partial + (size_t)blockIdx.x * a.partial_stride;
-  GradAcc ga;
+  GradAcc<H> ga;
   ga.zero();
   const float cscale = -1.f / ((float)a.M * (float)a.global_rows);
 
@@ -248,15 +248,16 @@ struct QGradArgs {
   NetDev q;
 };
 
+template <int H>
 __global__ void __launch_bounds__(NT, 1) q_grad_kernel(const __grid_constant__ QGradArgs a) {
   extern __shared__ float4 smem_raw[];
-  Smem sm(reinterpret_cast<float*>(smem_raw));
+  Smem<H> sm(reinterpret_cast<float*>(smem_raw));
   __shared__ float red[TILE_R];
   const int tid = threadIdx.x;
   const int ntiles = (a.rows + TILE_R - 1) / TILE_R;
-  const GradLayout L(a.q.in_dim, a.q.out_dim);
+  const GradLayout L(a.q.in_dim, a.q.out_dim, H);
   float* partial = a.partial + (size_t)blockIdx.x * a.partial_stride;
-  GradAcc ga;
+  GradAcc<H> ga;
   ga.zero();
   float loss = 0.f;
   for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
@@ -310,9 +311,10 @@ struct EvalArgs {
   NetDev net0, net1, net2;
 };
 
+template <int H>
 __global__ void __launch_bounds__(NT, 1) eval_kernel(const __grid_constant__ EvalArgs a) {
   extern __shared__ float4 smem_raw[];
-  Smem sm(reinterpret_cast<float*>(smem_raw));
+  Smem<H> sm(reinterpret_cast<float*>(smem_raw));
   const int tid = threadIdx.x;
   const int ntiles = (a.rows + TILE_R - 1) / TILE_R;
   for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
@@ -395,10 +397,11 @@ struct SampleArgs {
   NetDev net;
 };
 
+template <int H>
 __global__ void __launch_bounds__(NT, 1) env_sample_kernel(const __grid_constant__ SampleArgs a) {
   using E = Env<MPG_ENV_PT_REAL>;
   extern __shared__ float4 smem_raw[];
-  Smem sm(reinterpret_cast<float*>(smem_raw));
+  Smem<H> sm(reinterpret_cast<float*>(smem_raw));
   const int tid = threadIdx.x, row = blockIdx.x * TILE_R + tid;
   const bool rt = tid < TILE_R, valid = rt && row < a.agents;
   float s[E::S], o[MPG_MAX_OBS];

@@ -20,6 +20,10 @@
 namespace mpg {
 namespace tc {
 
+// hidden width of the tensor-core path: the weight ring, the TMEM column map, the epilogue warp <-> 64-column quarter
+// map and the image sizes are all laid out for 256 (the handle offers this backend at hidden = 256 only)
+constexpr int H = 256;
+
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
 // ---- mbarrier --------------------------------------------------------------------------------

@@ -850,7 +850,7 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
     if (lane == 0) { mf->wsum[(warp & 3) * 2] = s0; mf->wsum[(warp & 3) * 2 + 1] = s1; }
     bar_sync(BAR_ROW, ROW_THREADS);
     if (tid == EPI_THREADS) {
-      const GradLayout L(A.pol.in_dim, A.pol.out_dim);
+      const GradLayout L(A.pol.in_dim, A.pol.out_dim, H);
       float* partial = a.partial + (size_t)blockIdx.x * a.partial_stride;
       partial[L.ob3 + 0] = (mf->wsum[0] + mf->wsum[2]) + (mf->wsum[4] + mf->wsum[6]);
       if (NA > 1) partial[L.ob3 + 1] = (mf->wsum[1] + mf->wsum[3]) + (mf->wsum[5] + mf->wsum[7]);
@@ -861,7 +861,7 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
     tc_fence_before();
     if (elected) bulk_wait_all();
     if (BWD) {
-      const GradLayout L(A.pol.in_dim, A.pol.out_dim);
+      const GradLayout L(A.pol.in_dim, A.pol.out_dim, H);
       float* partial = a.partial + (size_t)blockIdx.x * a.partial_stride;
       if (any_dw && hc == 0) {
         // D1 / D3: TMEM lane = feature inside the 128-feature half, columns = input index (BIAS_K: bias) / action
@@ -1093,7 +1093,7 @@ __global__ void __launch_bounds__(DW_THREADS, 1) tc_dw_kernel(const __grid_const
       }
     }
     // ------------------------------- epilogue: TMEM -> this CTA's partial gradient -------------------------------
-    const GradLayout L(A.in_dim, A.out_dim);
+    const GradLayout L(A.in_dim, A.out_dim, H);
     float* partial = A.partial + (size_t)blockIdx.x * A.partial_stride;
     const int f = mh * 128 + warp * 32 + lane;                   // feature owned by this thread (TMEM lane)
     const uint32_t lane_off = (uint32_t)(warp * 32) << 16;

@@ -35,6 +35,7 @@ inline bool tc_set_smem(K kernel, int bytes) {
 }
 
 inline bool tc_init(TcState& t, const mpg_config& cfg, int /*sms*/, size_t& ws_bytes) {
+  if (cfg.hidden != tc::H) return true;                  // every layout of this path is built for 256; stay on FFMA
   if (cfg.obs_dim + cfg.act_dim + 1 > 16) return true;   // first-layer K must fit one UMMA k-step; stay on FFMA
   auto alloc = [&](void** p, size_t n) {
     if (cudaMalloc(p, n) != cudaSuccess) return false;
@@ -76,9 +77,9 @@ inline void tc_destroy(TcState& t) {
 // flat: Keras-order natural weights W1|b1|W2|b2|W3|b3 on the device
 inline bool tc_pack_weights(TcState& t, int net, const float* flat, int in_dim, int out_dim, cudaStream_t st) {
   if (!t.nets[net].big_fwd) return true;   // tensor-core path not configured for this handle
-  const GradLayout L(in_dim, out_dim);
-  tc::pack_big_image<true><<<32, 256, 0, st>>>(flat + L.oW2, 1, H, t.nets[net].big_fwd);     // value(n,k) = W2[k][n]
-  tc::pack_big_image<false><<<32, 256, 0, st>>>(flat + L.oW2, H, 1, t.nets[net].big_dx);      // value(k,n) = W2[k][n]
+  const GradLayout L(in_dim, out_dim, tc::H);
+  tc::pack_big_image<true><<<32, 256, 0, st>>>(flat + L.oW2, 1, tc::H, t.nets[net].big_fwd);     // value(n,k) = W2[k][n]
+  tc::pack_big_image<false><<<32, 256, 0, st>>>(flat + L.oW2, tc::H, 1, t.nets[net].big_dx);      // value(k,n) = W2[k][n]
   tc::pack_l1_image<true><<<2, 256, 0, st>>>(flat + L.oW1, flat + L.ob1, in_dim, tc::BIAS_K, t.nets[net].l1);
   tc::pack_l1_image<false><<<2, 256, 0, st>>>(flat + L.oW1, flat + L.ob1, in_dim, tc::BIAS_K, t.nets[net].l1b, 1.4426950408889634f);   // z1 log2(e), see epi_delta1_blocks
   tc::pack_in_image<<<2, 256, 0, st>>>(flat + L.oW1, in_dim, t.nets[net].in);
@@ -86,7 +87,7 @@ inline bool tc_pack_weights(TcState& t, int net, const float* flat, int in_dim, 
 }
 
 inline tc::TcNet tc_net(const TcState& t, int net, const float* flat, int in_dim, int out_dim) {
-  const GradLayout L(in_dim, out_dim);
+  const GradLayout L(in_dim, out_dim, tc::H);
   tc::TcNet n;
   n.big_fwd = t.nets[net].big_fwd; n.big_dx = t.nets[net].big_dx; n.l1 = t.nets[net].l1; n.l1b = t.nets[net].l1b; n.in = t.nets[net].in;
   n.W3 = flat + L.oW3; n.b2 = flat + L.ob2; n.b3 = flat + L.ob3;
@@ -129,7 +130,7 @@ inline cudaError_t tc_selftest(TcState& t, int kind, const float* X, const float
     const char* g = getenv("MPG_SELFTEST_GRID");
     int grid = g ? atoi(g) & ~1 : 2;
     if (grid < 2) grid = 2;
-    tc::pack_pair_image<<<32, 256, 0, st>>>(W, H, 1, t.scratch_img);
+    tc::pack_pair_image<<<32, 256, 0, st>>>(W, tc::H, 1, t.scratch_img);
     tc::pair_probe_kernel<<<grid, 192, tc::PAIR_SMEM, st>>>(X, t.scratch_img, Z, repeats);
     return cudaGetLastError();
   }
@@ -138,7 +139,7 @@ inline cudaError_t tc_selftest(TcState& t, int kind, const float* X, const float
     tc::selftest_kernel<<<g ? atoi(g) : 1, tc::CTA_THREADS, tc::SmemMap::TOTAL + 1024, st>>>(kind, X, t.scratch_img, Z, repeats);
     return cudaGetLastError();
   }
-  if (kind == 0) tc::pack_big_image<false><<<32, 256, 0, st>>>(W, H, 1, t.scratch_img);
+  if (kind == 0) tc::pack_big_image<false><<<32, 256, 0, st>>>(W, tc::H, 1, t.scratch_img);
   else if (kind == 1) tc::pack_l1_image<true><<<2, 256, 0, st>>>(W, W, 16, -1, t.scratch_img);
   else tc::pack_in_image<<<2, 256, 0, st>>>(W, 16, t.scratch_img);
   tc::selftest_kernel<<<1, tc::CTA_THREADS, tc::SmemMap::TOTAL + 1024, st>>>(kind, X, t.scratch_img, Z, repeats);

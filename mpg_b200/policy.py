@@ -17,6 +17,9 @@ from .engine import Engine
 from .synthetic import make_mlp_weights
 
 
+HIDDEN_WIDTHS = (64, 128, 256)   # hidden widths the fp32 (FFMA) kernels are built for; tensor cores: 256 only
+
+
 class PolicyWithQs(object):
     def __init__(self, obs_dim, act_dim, value_num_hidden_layers=2, value_num_hidden_units=256,
                  value_hidden_activation='elu', policy_num_hidden_layers=2, policy_num_hidden_units=256,
@@ -25,13 +28,17 @@ class PolicyWithQs(object):
                  **kwargs):
         if value_num_hidden_layers != 2 or policy_num_hidden_layers != 2:
             raise NotImplementedError('the sm_100a kernels are built for 2 hidden layers (reference default)')
-        if value_num_hidden_units != 256 or policy_num_hidden_units != 256:
-            raise NotImplementedError('the sm_100a kernels are built for 256 hidden units (reference default)')
+        if value_num_hidden_units != policy_num_hidden_units:
+            raise NotImplementedError('value_num_hidden_units and policy_num_hidden_units must be equal: one hidden '
+                                      'width per handle (got %r and %r)' % (value_num_hidden_units, policy_num_hidden_units))
+        if policy_num_hidden_units not in HIDDEN_WIDTHS:
+            raise NotImplementedError('the sm_100a kernels are built for %s hidden units (got %r)'
+                                      % (' / '.join(map(str, HIDDEN_WIDTHS)), policy_num_hidden_units))
         if value_hidden_activation != 'elu' or policy_hidden_activation != 'elu':
             raise NotImplementedError("hidden activation must be 'elu' (reference default)")
         if not deterministic_policy:
             raise NotImplementedError('the model-based learners use deterministic_policy=True (train_script.py:273)')
-        self.obs_dim, self.act_dim = obs_dim, act_dim
+        self.obs_dim, self.act_dim, self.hidden = obs_dim, act_dim, int(policy_num_hidden_units)
         self.policy_only, self.double_Q, self.target = policy_only, double_Q, target
         self.tau, self.delay_update, self.action_range = tau, delay_update, action_range
         self.deterministic_policy = True
@@ -45,7 +52,7 @@ class PolicyWithQs(object):
                              obs_scale=kwargs.get('obs_scale'), rew_scale=kwargs.get('rew_scale', 1.0),
                              rew_shift=kwargs.get('rew_shift', 0.0), gamma=kwargs.get('gamma', 0.99),
                              policy_out_activation=policy_out_activation, action_range=action_range,
-                             num_future_data=kwargs.get('num_future_data', 0), max_rows=max(rows, 64),
+                             num_future_data=kwargs.get('num_future_data', 0), hidden=self.hidden, max_rows=max(rows, 64),
                              max_horizon=max(lists + [1]), device=kwargs.get('device'), debug_lib=kwargs.get('debug_lib', False))
         # slot order == get_weights() order (policy.py:72-89)
         if policy_only:
@@ -66,8 +73,8 @@ class PolicyWithQs(object):
 
     def _init(self, rng, slot):
         if slot in (_lib.NET_POLICY, _lib.NET_POLICY_TARGET):
-            return make_mlp_weights(rng, self.obs_dim, 256, 2 * self.act_dim, bias_scale=0.0)
-        return make_mlp_weights(rng, self.obs_dim + self.act_dim, 256, 1, bias_scale=0.0)
+            return make_mlp_weights(rng, self.obs_dim, self.hidden, 2 * self.act_dim, bias_scale=0.0)
+        return make_mlp_weights(rng, self.obs_dim + self.act_dim, self.hidden, 1, bias_scale=0.0)
 
     # -- weights --------------------------------------------------------------------------------
     def get_weights(self):
