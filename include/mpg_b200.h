@@ -216,6 +216,14 @@ enum { MPG_BACKEND_FFMA = 0, MPG_BACKEND_TC = 1 };
 int mpg_set_backend(mpg_ctx* ctx, int backend);
 int mpg_get_backend(const mpg_ctx* ctx);
 
+/* Hidden activation of every net of the handle (value_hidden_activation == policy_hidden_activation, model.py
+ * Dense(activation=...)): applies to every call that evaluates an MLP, on both backends and at every width.
+ * A new handle uses MPG_ACT_ELU; an unknown value returns MPG_ERR_ARG.  The weight images do not depend on it, so the
+ * activation may change between calls on one handle. */
+enum { MPG_ACT_ELU = 0, MPG_ACT_RELU = 1, MPG_ACT_TANH = 2 };
+int mpg_set_activation(mpg_ctx* ctx, int act);
+int mpg_get_activation(const mpg_ctx* ctx);
+
 /* Optional device timing of the dominant (rollout) kernel: when enabled, CUDA events are recorded on
  * the caller's stream immediately around that launch; mpg_kernel_ms() waits for the last pair and
  * returns its duration in milliseconds (<0: nothing recorded). Used by bench.py for the roofline. */

@@ -12,6 +12,7 @@ MAX_OBS, MAX_LIST = 16, 8
 ENV_IDS = {'PathTracking-v0': 0, 'InvertedPendulumConti-v0': 1, 'InvertedDoublePendulum-v2': 2,
            'PathTracking-v0-real': 3}   # the ground-truth PathTrackingEnv (forward only)
 NET_Q1, NET_Q2, NET_POLICY, NET_Q1_TARGET, NET_Q2_TARGET, NET_POLICY_TARGET = range(6)
+ACTIVATIONS = {'elu': 0, 'relu': 1, 'tanh': 2}   # MPG_ACT_*: hidden activation of every net of a handle
 
 # every symbol include/mpg_b200.h declares (tests check that the library exports all of them)
 SYMBOLS = [
@@ -24,6 +25,7 @@ SYMBOLS = [
     'mpg_set_adam_state', 'mpg_env_sample',
     'mpg_replay_create', 'mpg_replay_destroy', 'mpg_replay_last_error', 'mpg_replay_size', 'mpg_replay_add',
     'mpg_replay_sample', 'mpg_replay_update_priorities', 'mpg_replay_tree_stats', 'mpg_q_bootstrap', 'mpg_env_step',
+    'mpg_set_activation', 'mpg_get_activation',
 ]
 # exported by libmpg_b200_dbg.so only (include/mpg_b200.h, #ifdef MPG_DEBUG_PROBES)
 DEBUG_SYMBOLS = ['mpg_tc_selftest', 'mpg_set_profile_buffer']
@@ -92,6 +94,8 @@ def load(debug=False):
         'mpg_launch_count': (u64, [vp]),
         'mpg_set_backend': (i32, [vp, i32]),
         'mpg_get_backend': (i32, [vp]),
+        'mpg_set_activation': (i32, [vp, i32]),
+        'mpg_get_activation': (i32, [vp]),
         'mpg_set_timing': (i32, [vp, i32]),
         'mpg_kernel_ms': (f32, [vp]),
         'mpg_tc_selftest': (i32, [vp, i32, vp, vp, vp, i32, vp]),

@@ -8,9 +8,16 @@
 
 #include "rollout_kernels.cuh"
 #include "tc_rollout.cuh"
+#include "act_instances.cuh"
 #include "replay.cuh"
 
 using namespace mpg;
+
+// the relu and tanh kernels are compiled in act_relu.cu / act_tanh.cu
+namespace mpg {
+MPG_ACT_INSTANCES(extern, MPG_ACT_RELU)
+MPG_ACT_INSTANCES(extern, MPG_ACT_TANH)
+}  // namespace mpg
 
 namespace {
 
@@ -35,7 +42,8 @@ bool wait_dbg_init() {
   if (cudaHostAlloc((void**)&h, 256, cudaHostAllocMapped) != cudaSuccess) { cudaGetLastError(); return false; }
   memset(h, 0, 256);
   if (cudaHostGetDevicePointer((void**)&d, h, 0) != cudaSuccess
-      || cudaMemcpyToSymbol(mpg::tc::g_wait_dbg, &d, sizeof(d)) != cudaSuccess) {
+      || cudaMemcpyToSymbol(mpg::tc::g_wait_dbg, &d, sizeof(d)) != cudaSuccess || !mpg::wait_dbg_attach_relu(d)
+      || !mpg::wait_dbg_attach_tanh(d)) {
     cudaGetLastError(); cudaFreeHost(h); return false;
   }
   g_wait_host = h;
@@ -57,6 +65,7 @@ struct mpg_ctx {
   size_t ws_bytes = 0;
   uint64_t launches = 0;
   int backend = MPG_BACKEND_FFMA;
+  int act = MPG_ACT_ELU;                  // hidden activation of every net (MPG_ACT_*)
   int timing = 0, timed = 0;
   long long* prof = nullptr;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
@@ -84,14 +93,22 @@ int fail(mpg_ctx* ctx, int code, const char* fmt, const char* detail = "") {
 // flat parameter layout of one net of this handle
 GradLayout layout(const mpg_ctx* c, const NetStore& n) { return GradLayout(n.in_dim, n.out_dim, c->cfg.hidden); }
 
-// The one place the handle's hidden width becomes the template argument of the FFMA kernels: f(integral_constant<H>).
-// mpg_create admits 64, 128 and 256 only.
+// The one place the handle's hidden width and activation become the template arguments of the FFMA kernels:
+// f(integral_constant<H>, integral_constant<ACT>).  mpg_create admits widths 64, 128 and 256 only, mpg_set_activation
+// the three MPG_ACT_* values.
 template <typename F>
-int with_hidden(const mpg_ctx* c, F&& f) {
+int with_mlp(const mpg_ctx* c, F&& f) {
+  auto with_act = [&](auto hc) {
+    switch (c->act) {
+      case MPG_ACT_RELU: return f(hc, std::integral_constant<int, MPG_ACT_RELU>());
+      case MPG_ACT_TANH: return f(hc, std::integral_constant<int, MPG_ACT_TANH>());
+      default: return f(hc, std::integral_constant<int, MPG_ACT_ELU>());
+    }
+  };
   switch (c->cfg.hidden) {
-    case 64: return f(std::integral_constant<int, 64>());
-    case 128: return f(std::integral_constant<int, 128>());
-    default: return f(std::integral_constant<int, 256>());
+    case 64: return with_act(std::integral_constant<int, 64>());
+    case 128: return with_act(std::integral_constant<int, 128>());
+    default: return with_act(std::integral_constant<int, 256>());
   }
 }
 
@@ -309,16 +326,16 @@ template <bool BWD>
 int launch_rollout(mpg_ctx* ctx, const RolloutArgs& a, int grid, cudaStream_t st, int env) {
   if (BWD && env == MPG_ENV_PATH_TRACKING_REAL) return fail(ctx, MPG_ERR_UNSUPPORTED, "the real environment is forward only%s");
   if (ctx->timing) cudaEventRecord(ctx->ev0, st);
-  with_hidden(ctx, [&](auto hc) {
-    constexpr int HW = decltype(hc)::value;
+  with_mlp(ctx, [&](auto hc, auto ac) {
+    constexpr int HW = decltype(hc)::value, ACT = decltype(ac)::value;
     const size_t smem = Smem<HW>::FLOATS * 4;
     if (env == MPG_ENV_PATH_TRACKING_REAL) {
-      rollout_kernel<HW, MPG_ENV_PATH_TRACKING_REAL, false><<<grid, NT, smem, st>>>(a);
+      rollout_kernel<HW, ACT, MPG_ENV_PATH_TRACKING_REAL, false><<<grid, NT, smem, st>>>(a);
     } else
     switch (env) {
-      case MPG_ENV_PATH_TRACKING: rollout_kernel<HW, MPG_ENV_PATH_TRACKING, BWD><<<grid, NT, smem, st>>>(a); break;
-      case MPG_ENV_INVERTED_PENDULUM: rollout_kernel<HW, MPG_ENV_INVERTED_PENDULUM, BWD><<<grid, NT, smem, st>>>(a); break;
-      default: rollout_kernel<HW, MPG_ENV_INVERTED_DOUBLE_PENDULUM, BWD><<<grid, NT, smem, st>>>(a); break;
+      case MPG_ENV_PATH_TRACKING: rollout_kernel<HW, ACT, MPG_ENV_PATH_TRACKING, BWD><<<grid, NT, smem, st>>>(a); break;
+      case MPG_ENV_INVERTED_PENDULUM: rollout_kernel<HW, ACT, MPG_ENV_INVERTED_PENDULUM, BWD><<<grid, NT, smem, st>>>(a); break;
+      default: rollout_kernel<HW, ACT, MPG_ENV_INVERTED_DOUBLE_PENDULUM, BWD><<<grid, NT, smem, st>>>(a); break;
     }
     return MPG_OK;
   });
@@ -345,6 +362,13 @@ int mpg_set_backend(mpg_ctx* ctx, int backend) {
     return fail(ctx, MPG_ERR_UNSUPPORTED,
                 "tensor-core backend does not cover this configuration (it needs hidden = 256 and obs_dim + act_dim <= 15)%s");
   ctx->backend = backend;
+  return MPG_OK;
+}
+
+int mpg_get_activation(const mpg_ctx* ctx) { return ctx->act; }
+int mpg_set_activation(mpg_ctx* ctx, int act) {
+  if (!ctx || (act != MPG_ACT_ELU && act != MPG_ACT_RELU && act != MPG_ACT_TANH)) return fail(ctx, MPG_ERR_ARG, "bad activation%s");
+  ctx->act = act;
   return MPG_OK;
 }
 
@@ -450,21 +474,26 @@ int mpg_create(const mpg_config* cfg, mpg_ctx** out) {
     mpg_destroy(c);
     return MPG_ERR_CUDA;
   }
-  const int rc = with_hidden(c, [&](auto hc) {   // the instantiations this handle launches
-    constexpr int HW = decltype(hc)::value;
-    int r = 0;
-    r |= set_smem<HW>(c, rollout_kernel<HW, MPG_ENV_PATH_TRACKING, true>);
-    r |= set_smem<HW>(c, rollout_kernel<HW, MPG_ENV_PATH_TRACKING, false>);
-    r |= set_smem<HW>(c, rollout_kernel<HW, MPG_ENV_INVERTED_PENDULUM, true>);
-    r |= set_smem<HW>(c, rollout_kernel<HW, MPG_ENV_INVERTED_PENDULUM, false>);
-    r |= set_smem<HW>(c, rollout_kernel<HW, MPG_ENV_INVERTED_DOUBLE_PENDULUM, true>);
-    r |= set_smem<HW>(c, rollout_kernel<HW, MPG_ENV_INVERTED_DOUBLE_PENDULUM, false>);
-    r |= set_smem<HW>(c, rollout_kernel<HW, MPG_ENV_PATH_TRACKING_REAL, false>);
-    r |= set_smem<HW>(c, q_grad_kernel<HW>);
-    r |= set_smem<HW>(c, eval_kernel<HW>);
-    r |= set_smem<HW>(c, env_sample_kernel<HW>);
-    return r;
-  });
+  int rc = 0;
+  for (const int act : {MPG_ACT_ELU, MPG_ACT_RELU, MPG_ACT_TANH}) {   // the instantiations this handle may launch
+    c->act = act;
+    rc |= with_mlp(c, [&](auto hc, auto ac) {
+      constexpr int HW = decltype(hc)::value, ACT = decltype(ac)::value;
+      int r = 0;
+      r |= set_smem<HW>(c, rollout_kernel<HW, ACT, MPG_ENV_PATH_TRACKING, true>);
+      r |= set_smem<HW>(c, rollout_kernel<HW, ACT, MPG_ENV_PATH_TRACKING, false>);
+      r |= set_smem<HW>(c, rollout_kernel<HW, ACT, MPG_ENV_INVERTED_PENDULUM, true>);
+      r |= set_smem<HW>(c, rollout_kernel<HW, ACT, MPG_ENV_INVERTED_PENDULUM, false>);
+      r |= set_smem<HW>(c, rollout_kernel<HW, ACT, MPG_ENV_INVERTED_DOUBLE_PENDULUM, true>);
+      r |= set_smem<HW>(c, rollout_kernel<HW, ACT, MPG_ENV_INVERTED_DOUBLE_PENDULUM, false>);
+      r |= set_smem<HW>(c, rollout_kernel<HW, ACT, MPG_ENV_PATH_TRACKING_REAL, false>);
+      r |= set_smem<HW>(c, q_grad_kernel<HW, ACT>);
+      r |= set_smem<HW>(c, eval_kernel<HW, ACT>);
+      r |= set_smem<HW>(c, env_sample_kernel<HW, ACT>);
+      return r;
+    });
+  }
+  c->act = MPG_ACT_ELU;
   if (rc) {
     strncpy(g_create_err, c->err, 512);
     mpg_destroy(c);
@@ -504,7 +533,7 @@ void mpg_destroy(mpg_ctx* c) {
 
 // FFMA weight images (W1p, W2p, W2Tp) of one net from its flat natural weights
 static void launch_pack(mpg_ctx* ctx, const NetStore& ns, cudaStream_t st) {
-  with_hidden(ctx, [&](auto hc) {
+  with_mlp(ctx, [&](auto hc, auto) {   // the packing does not depend on the activation
     constexpr int HW = decltype(hc)::value;
     pack_kernel<HW><<<(HW * HW + 255) / 256, 256, 0, st>>>(ns.flat, ns.in_dim, ns.out_dim, ns.W1p, ns.W2p, ns.W2Tp);
     return MPG_OK;
@@ -673,7 +702,7 @@ int mpg_policy_grad(mpg_ctx* ctx, const mpg_rollout_params* p, const float* obs,
     CUDA_OK(ctx, cudaMemsetAsync(ctx->partial, 0, (size_t)(split ? 2 : 1) * ctx->sms * ctx->partial_stride * sizeof(float), st));
     if (ctx->timing) cudaEventRecord(ctx->ev0, st);
     if (!split) {
-      CUDA_OK(ctx, tc_launch_rollout<true>(ctx->cfg.env, ta, grid, st));
+      CUDA_OK(ctx, tc_launch_rollout<true>(ctx->cfg.env, ctx->act, ta, grid, st));
       if (ctx->timing) { cudaEventRecord(ctx->ev1, st); ctx->timed = 1; }
       tc::DwArgs da = dw_args(0, ntiles, 0);
       int dgrid = 2 * da.nrecords < ctx->sms ? 2 * da.nrecords : (ctx->sms & ~1);
@@ -683,12 +712,12 @@ int mpg_policy_grad(mpg_ctx* ctx, const mpg_rollout_params* p, const float* obs,
       ctx->launches += 3;
     } else {
       ta.tile0 = 0; ta.tile1 = full;
-      CUDA_OK(ctx, tc_launch_rollout<true>(ctx->cfg.env, ta, ctx->sms, st));
+      CUDA_OK(ctx, tc_launch_rollout<true>(ctx->cfg.env, ctx->act, ta, ctx->sms, st));
       CUDA_OK(ctx, cudaEventRecord(ctx->ev_wave, st));
       tc::TcArgs tb = ta;
       tb.tile0 = full; tb.tile1 = ntiles;
       tb.r.partial = ctx->partial + (size_t)ctx->sms * ctx->partial_stride;
-      CUDA_OK(ctx, tc_launch_rollout<true>(ctx->cfg.env, tb, tail, st));
+      CUDA_OK(ctx, tc_launch_rollout<true>(ctx->cfg.env, ctx->act, tb, tail, st));
       if (ctx->timing) { cudaEventRecord(ctx->ev1, st); ctx->timed = 1; }
       CUDA_OK(ctx, cudaStreamWaitEvent(ctx->aux, ctx->ev_wave, 0));
       tc::tc_dw_kernel<<<(ctx->sms - tail) & ~1, tc::DW_THREADS, dw_smem, ctx->aux>>>(dw_args(0, full, 0));
@@ -745,7 +774,7 @@ int mpg_rollout_forward(mpg_ctx* ctx, const mpg_rollout_params* p, const float* 
     if (a.has_q) ta.q = tc_net(ctx->tc, p->q_net, ctx->nets[p->q_net].flat, a.q.in_dim, a.q.out_dim);
     ta.act_ckpt = ctx->tc.act_ckpt;
     if (ctx->timing) cudaEventRecord(ctx->ev0, st);
-    CUDA_OK(ctx, tc_launch_rollout<false>(env, ta, grid, st));
+    CUDA_OK(ctx, tc_launch_rollout<false>(env, ctx->act, ta, grid, st));
     if (ctx->timing) { cudaEventRecord(ctx->ev1, st); ctx->timed = 1; }
     ctx->launches++;
     return MPG_OK;
@@ -809,7 +838,7 @@ int mpg_q_grad(mpg_ctx* ctx, int net, int rows, int64_t global_rows, const float
     // to it (measured 1.4e-3 at 262,144 rows); this GEMM is 0.04 ms, there is nothing to gain
     ta.rec_hi_only = 0;
     CUDA_OK(ctx, cudaMemsetAsync(ctx->partial, 0, (size_t)ctx->sms * ctx->partial_stride * sizeof(float), st));
-    CUDA_OK(ctx, tc_launch_rollout<true>(c.env, ta, grid, st));
+    CUDA_OK(ctx, tc_launch_rollout<true>(c.env, ctx->act, ta, grid, st));
     tc::DwArgs da;
     da.store = ctx->tc.store; da.nrecords = ntiles;
     da.in_dim = qin; da.out_dim = 1;
@@ -840,9 +869,9 @@ int mpg_q_grad(mpg_ctx* ctx, int net, int rows, int64_t global_rows, const float
   const int grid = ntiles < ctx->sms ? ntiles : ctx->sms;
   const GradLayout L = layout(ctx, ctx->nets[net]);
   CUDA_OK(ctx, cudaMemsetAsync(ctx->partial, 0, (size_t)grid * ctx->partial_stride * sizeof(float), st));
-  with_hidden(ctx, [&](auto hc) {
-    constexpr int HW = decltype(hc)::value;
-    q_grad_kernel<HW><<<grid, NT, Smem<HW>::FLOATS * 4, st>>>(a);
+  with_mlp(ctx, [&](auto hc, auto ac) {
+    constexpr int HW = decltype(hc)::value, ACT = decltype(ac)::value;
+    q_grad_kernel<HW, ACT><<<grid, NT, Smem<HW>::FLOATS * 4, st>>>(a);
     return MPG_OK;
   });
   reduce_partials_kernel<<<(L.total + 255) / 256, 256, 0, st>>>(ctx->partial, ctx->partial_stride, grid, L.total,
@@ -860,9 +889,9 @@ static int launch_eval(mpg_ctx* ctx, EvalArgs& a, void* stream) {
   for (int i = 0; i < MPG_MAX_OBS; ++i) a.obs_scale[i] = c.obs_scale[i];
   const int ntiles = (a.rows + TILE_R - 1) / TILE_R;
   const int grid = ntiles < ctx->sms ? ntiles : ctx->sms;
-  with_hidden(ctx, [&](auto hc) {
-    constexpr int HW = decltype(hc)::value;
-    eval_kernel<HW><<<grid, NT, Smem<HW>::FLOATS * 4, (cudaStream_t)stream>>>(a);
+  with_mlp(ctx, [&](auto hc, auto ac) {
+    constexpr int HW = decltype(hc)::value, ACT = decltype(ac)::value;
+    eval_kernel<HW, ACT><<<grid, NT, Smem<HW>::FLOATS * 4, (cudaStream_t)stream>>>(a);
     return MPG_OK;
   });
   ctx->launches++;
@@ -1067,9 +1096,9 @@ int mpg_env_sample(mpg_ctx* ctx, int policy_net, int agents, int steps, float ex
   a.explore_noise = explore_noise; a.reset_obs = reset_obs; a.state = state; a.obs = obs;
   a.out_obs = out_obs; a.out_act = out_act; a.out_rew = out_rew; a.out_obs_tp1 = out_obs_tp1; a.out_done = out_done;
   a.net = net_dev(ctx, policy_net);
-  with_hidden(ctx, [&](auto hc) {
-    constexpr int HW = decltype(hc)::value;
-    env_sample_kernel<HW><<<(agents + TILE_R - 1) / TILE_R, NT, Smem<HW>::FLOATS * 4, (cudaStream_t)stream>>>(a);
+  with_mlp(ctx, [&](auto hc, auto ac) {
+    constexpr int HW = decltype(hc)::value, ACT = decltype(ac)::value;
+    env_sample_kernel<HW, ACT><<<(agents + TILE_R - 1) / TILE_R, NT, Smem<HW>::FLOATS * 4, (cudaStream_t)stream>>>(a);
     return MPG_OK;
   });
   ctx->launches++;

@@ -18,10 +18,27 @@ constexpr int MAX_IN = 20;    // max MLP input width (obs 16 + act 2, padded)
 constexpr int MAX_S = 6;      // max env state dim
 constexpr int MAX_A = 2;      // max action dim
 
-// ELU (model.py hidden_activation='elu'): x>0 ? x : exp(x)-1.
+// Hidden activations (model.py Dense(activation=...)): ACT is MPG_ACT_ELU / MPG_ACT_RELU / MPG_ACT_TANH.  Each derivative is
+// expressed through the layer's OUTPUT y, so the backward pass needs only the stored activations (TF's EluGrad, ReluGrad,
+// TanhGrad).
+// ELU: x>0 ? x : exp(x)-1.
 __device__ __forceinline__ float elu(float x) { return x > 0.f ? x : expm1f(x); }
 // derivative expressed through the OUTPUT y (TF EluGrad): y>0 ? 1 : y+1
 __device__ __forceinline__ float elu_grad_from_out(float y) { return y > 0.f ? 1.f : y + 1.f; }
+// forward: tanhf is the fp32-accurate library function (a few ulp), never tanh.approx
+template <int ACT>
+__device__ __forceinline__ float act_fwd(float x) {
+  if constexpr (ACT == MPG_ACT_RELU) return x > 0.f ? x : 0.f;
+  else if constexpr (ACT == MPG_ACT_TANH) return tanhf(x);
+  else return elu(x);
+}
+// relu: 0 at the kink (TF ReluGrad); tanh: 1 - y^2
+template <int ACT>
+__device__ __forceinline__ float act_grad_from_out(float y) {
+  if constexpr (ACT == MPG_ACT_RELU) return y > 0.f ? 1.f : 0.f;
+  else if constexpr (ACT == MPG_ACT_TANH) return fmaf(-y, y, 1.f);
+  else return elu_grad_from_out(y);
+}
 
 __device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
   unsigned s = (unsigned)__cvta_generic_to_shared(smem);

@@ -1,5 +1,6 @@
 // CTA-tile MLP engine (fp32 FFMA path): forward and backward of the reference's MLPNet
-// (model.py:20-43: Dense(H,elu) -> Dense(H,elu) -> Dense(out)) on a tile of TILE_R rows.
+// (model.py:20-43: Dense(H,act) -> Dense(H,act) -> Dense(out)) on a tile of TILE_R rows.
+// The hidden activation ACT (common.cuh: act_fwd / act_grad_from_out) is a template parameter beside H.
 //
 // Shared-memory activation tiles are stored [feature][row] with row pitch RP (68 floats) so that
 //   * the "row GEMM" (out[r][n] = sum_k in[k][r] W[k][n]) reads its A operand as warp-broadcast
@@ -120,9 +121,9 @@ __device__ __forceinline__ void rowgemm(const float* __restrict__ in_s, int K, c
   }
 }
 
-// epilogue: out[c][rows] = elu(acc + bias[c])
-template <int H>
-__device__ __forceinline__ void store_bias_elu(const float (&acc)[8][H / 32], const float* __restrict__ bias,
+// epilogue: out[c][rows] = act(acc + bias[c])
+template <int H, int ACT>
+__device__ __forceinline__ void store_bias_act(const float (&acc)[8][H / 32], const float* __restrict__ bias,
                                                float* __restrict__ out_s) {
   const int tid = threadIdx.x, w = tid >> 5, l = tid & 31;
 #pragma unroll
@@ -130,26 +131,28 @@ __device__ __forceinline__ void store_bias_elu(const float (&acc)[8][H / 32], co
     const int c = l + 32 * j;
     const float bv = __ldg(bias + c);
     float4 v0, v1;
-    v0.x = elu(acc[0][j] + bv); v0.y = elu(acc[1][j] + bv); v0.z = elu(acc[2][j] + bv); v0.w = elu(acc[3][j] + bv);
-    v1.x = elu(acc[4][j] + bv); v1.y = elu(acc[5][j] + bv); v1.z = elu(acc[6][j] + bv); v1.w = elu(acc[7][j] + bv);
+    v0.x = act_fwd<ACT>(acc[0][j] + bv); v0.y = act_fwd<ACT>(acc[1][j] + bv);
+    v0.z = act_fwd<ACT>(acc[2][j] + bv); v0.w = act_fwd<ACT>(acc[3][j] + bv);
+    v1.x = act_fwd<ACT>(acc[4][j] + bv); v1.y = act_fwd<ACT>(acc[5][j] + bv);
+    v1.z = act_fwd<ACT>(acc[6][j] + bv); v1.w = act_fwd<ACT>(acc[7][j] + bv);
     *reinterpret_cast<float4*>(out_s + c * RP + w * 8) = v0;
     *reinterpret_cast<float4*>(out_s + c * RP + w * 8 + 4) = v1;
   }
 }
 
-// epilogue: act_s[c][rows] <- acc * elu'(act_s[c][rows])   (in place: activation -> delta)
-template <int H>
-__device__ __forceinline__ void store_times_elugrad(const float (&acc)[8][H / 32], float* __restrict__ act_s) {
+// epilogue: act_s[c][rows] <- acc * act'(act_s[c][rows])   (in place: activation -> delta)
+template <int H, int ACT>
+__device__ __forceinline__ void store_times_actgrad(const float (&acc)[8][H / 32], float* __restrict__ act_s) {
   const int tid = threadIdx.x, w = tid >> 5, l = tid & 31;
 #pragma unroll
   for (int j = 0; j < H / 32; ++j) {
     const int c = l + 32 * j;
     float4* p0 = reinterpret_cast<float4*>(act_s + c * RP + w * 8);
     float4 h0 = p0[0], h1 = p0[1];
-    h0.x = acc[0][j] * elu_grad_from_out(h0.x); h0.y = acc[1][j] * elu_grad_from_out(h0.y);
-    h0.z = acc[2][j] * elu_grad_from_out(h0.z); h0.w = acc[3][j] * elu_grad_from_out(h0.w);
-    h1.x = acc[4][j] * elu_grad_from_out(h1.x); h1.y = acc[5][j] * elu_grad_from_out(h1.y);
-    h1.z = acc[6][j] * elu_grad_from_out(h1.z); h1.w = acc[7][j] * elu_grad_from_out(h1.w);
+    h0.x = acc[0][j] * act_grad_from_out<ACT>(h0.x); h0.y = acc[1][j] * act_grad_from_out<ACT>(h0.y);
+    h0.z = acc[2][j] * act_grad_from_out<ACT>(h0.z); h0.w = acc[3][j] * act_grad_from_out<ACT>(h0.w);
+    h1.x = acc[4][j] * act_grad_from_out<ACT>(h1.x); h1.y = acc[5][j] * act_grad_from_out<ACT>(h1.y);
+    h1.z = acc[6][j] * act_grad_from_out<ACT>(h1.z); h1.w = acc[7][j] * act_grad_from_out<ACT>(h1.w);
     p0[0] = h0; p0[1] = h1;
   }
 }
@@ -158,13 +161,13 @@ __device__ __forceinline__ void store_times_elugrad(const float (&acc)[8][H / 32
 // forward: xin[0..in_dim) -> h1 (bufA) -> h2 (bufB) -> y3[j][r] = h2 W3 + b3 for j < n_out
 // (n_out = number of output columns actually consumed: act_dim for the policy mean, 1 for Q)
 // ---------------------------------------------------------------------------------------------
-template <int H>
+template <int H, int ACT>
 __device__ __forceinline__ void mlp_forward_tile(const NetDev& net, Smem<H>& sm, int n_out) {
   float acc[8][H / 32];
   rowgemm<H>(sm.xin, net.in_dim, net.W1p, sm.slab, acc);
-  store_bias_elu<H>(acc, net.b1, sm.bufA);
+  store_bias_act<H, ACT>(acc, net.b1, sm.bufA);
   rowgemm<H>(sm.bufA, H, net.W2p, sm.slab, acc);   // first internal barrier publishes bufA
-  store_bias_elu<H>(acc, net.b2, sm.bufB);
+  store_bias_act<H, ACT>(acc, net.b2, sm.bufB);
   __syncthreads();
   // output layer: thread (r, q) sums features k = q, q+4, ... for every consumed column, then the
   // four partial sums are combined in a fixed order through shared memory (deterministic)
@@ -255,14 +258,14 @@ __device__ __forceinline__ void dw2_accumulate(const float* __restrict__ X, cons
 // gx[i][r] = dL/d xin[i][r].  With want_dw the parameter gradients are accumulated into `ga`
 // (registers) and dW2g (global partial).
 // ---------------------------------------------------------------------------------------------
-template <int H>
+template <int H, int ACT>
 __device__ __forceinline__ void mlp_backward_tile(const NetDev& net, Smem<H>& sm, int n_out, bool want_dw, bool want_gin,
                                                   GradAcc<H>& ga, float* __restrict__ dW2g) {
   const int tid = threadIdx.x;
   // feature f of this thread and its slice [r0, r0 + RS) of the tile rows (P = 1: all rows)
   constexpr int P = NT / H, RS = TILE_R / P;
   const int f = P == 1 ? tid : tid % H, r0 = P == 1 ? 0 : (tid / H) * RS;
-  // (1) thread (f, slice) walks its feature row: dW3 += h2 d3, delta2 = (d3 W3^T) elu'(h2) in place, db2
+  // (1) thread (f, slice) walks its feature row: dW3 += h2 d3, delta2 = (d3 W3^T) act'(h2) in place, db2
   {
     float w3[MAX_A];
 #pragma unroll
@@ -282,7 +285,7 @@ __device__ __forceinline__ void mlp_backward_tile(const NetDev& net, Smem<H>& sm
             g = fmaf(d, w3[j], g);
             s_dw3[j] = fmaf(hv[e], d, s_dw3[j]);
           }
-        dv[e] = g * elu_grad_from_out(hv[e]);
+        dv[e] = g * act_grad_from_out<ACT>(hv[e]);
         s_db2 += dv[e];
       }
       *reinterpret_cast<float4*>(hrow + r4) = make_float4(dv[0], dv[1], dv[2], dv[3]);
@@ -301,11 +304,11 @@ __device__ __forceinline__ void mlp_backward_tile(const NetDev& net, Smem<H>& sm
   __syncthreads();
   // (2) dW2 += h1^T delta2
   if (want_dw) dw2_accumulate<H>(sm.bufA, sm.bufB, dW2g);
-  // (3) delta1 = (delta2 W2^T) elu'(h1), in place over h1
+  // (3) delta1 = (delta2 W2^T) act'(h1), in place over h1
   {
     float acc[8][H / 32];
     rowgemm<H>(sm.bufB, H, net.W2Tp, sm.slab, acc);
-    store_times_elugrad<H>(acc, sm.bufA);
+    store_times_actgrad<H, ACT>(acc, sm.bufA);
   }
   __syncthreads();
   // (4) dW1 += xin^T delta1, db1 (thread (f, slice) as in (1))

@@ -56,7 +56,7 @@ __device__ __forceinline__ void head_fwd_grad(float z, int out_tanh, float range
   if (range > 0.f) { const float th = tanhf(m); g *= range * (1.f - th * th); act = range * th; }
 }
 
-template <int H, int ENV, bool BWD>
+template <int H, int ACT, int ENV, bool BWD>
 __global__ void __launch_bounds__(NT, 1) rollout_kernel(const __grid_constant__ RolloutArgs a) {
   extern __shared__ float4 smem_raw[];
   Smem<H> sm(reinterpret_cast<float*>(smem_raw));
@@ -105,7 +105,7 @@ __global__ void __launch_bounds__(NT, 1) rollout_kernel(const __grid_constant__ 
       const bool given = (t == 0 && a.use_start_actions);
       if (!given) {
         __syncthreads();
-        mlp_forward_tile(a.pol, sm, A);
+        mlp_forward_tile<H, ACT>(a.pol, sm, A);
       }
       if (rowthread) {
 #pragma unroll
@@ -122,7 +122,7 @@ __global__ void __launch_bounds__(NT, 1) rollout_kernel(const __grid_constant__ 
         float qv = 0.f;
         if (a.has_q) {
           __syncthreads();
-          mlp_forward_tile(a.q, sm, 1);
+          mlp_forward_tile<H, ACT>(a.q, sm, 1);
           if (rowthread) qv = sm.y3[tid];
         }
         if (valid && a.returns_out) a.returns_out[(size_t)kidx * MB + grow] = rsum + gpow * qv;
@@ -165,7 +165,7 @@ __global__ void __launch_bounds__(NT, 1) rollout_kernel(const __grid_constant__ 
           for (int i = 0; i < a.obs_dim; ++i) sm.xin[i * RP + tid] = valid ? o[i] * a.obs_scale[i] : 0.f;
         }
         __syncthreads();
-        mlp_forward_tile(a.pol, sm, A);
+        mlp_forward_tile<H, ACT>(a.pol, sm, A);
         float act[A], g_a[A], g_s[S], zpre[A];
 #pragma unroll
         for (int j = 0; j < A; ++j) { act[j] = 0.f; g_a[j] = 0.f; zpre[j] = 0.f; }
@@ -187,10 +187,10 @@ __global__ void __launch_bounds__(NT, 1) rollout_kernel(const __grid_constant__ 
             for (int j = 0; j < A; ++j) sm.xin[(a.obs_dim + j) * RP + tid] = act[j];
           }
           __syncthreads();
-          mlp_forward_tile(a.q, sm, 1);
+          mlp_forward_tile<H, ACT>(a.q, sm, 1);
           if (rowthread) sm.d3[tid] = valid ? cscale * a.list_w[kidx] * gp : 0.f;
           __syncthreads();
-          mlp_backward_tile(a.q, sm, 1, false, true, ga, nullptr);
+          mlp_backward_tile<H, ACT>(a.q, sm, 1, false, true, ga, nullptr);
           if (rowthread && valid) {
             float go[MPG_MAX_OBS];
             for (int i = 0; i < a.obs_dim; ++i) go[i] = sm.gx[i * RP + tid] * a.obs_scale[i];
@@ -199,7 +199,7 @@ __global__ void __launch_bounds__(NT, 1) rollout_kernel(const __grid_constant__ 
             for (int j = 0; j < A; ++j) g_a[j] += sm.gx[(a.obs_dim + j) * RP + tid];
           }
           __syncthreads();
-          mlp_forward_tile(a.pol, sm, A);   // the Q pass reused bufA/bufB: recompute h1, h2 of the policy
+          mlp_forward_tile<H, ACT>(a.pol, sm, A);   // the Q pass reused bufA/bufB: recompute h1, h2 of the policy
         }
         if (t < a.horizon && rowthread && valid) {
           float Wt = 0.f;
@@ -215,7 +215,7 @@ __global__ void __launch_bounds__(NT, 1) rollout_kernel(const __grid_constant__ 
         __syncthreads();
         const bool want_dw = a.full_bptt || t == 0;
         const bool want_gin = t > 0;
-        mlp_backward_tile(a.pol, sm, A, want_dw, want_gin, ga, partial + L.oW2);
+        mlp_backward_tile<H, ACT>(a.pol, sm, A, want_dw, want_gin, ga, partial + L.oW2);
         if (rowthread && valid) {
 #pragma unroll
           for (int j = 0; j < S; ++j) { lam[j] = g_s[j]; snext[j] = s[j]; }
@@ -248,7 +248,7 @@ struct QGradArgs {
   NetDev q;
 };
 
-template <int H>
+template <int H, int ACT>
 __global__ void __launch_bounds__(NT, 1) q_grad_kernel(const __grid_constant__ QGradArgs a) {
   extern __shared__ float4 smem_raw[];
   Smem<H> sm(reinterpret_cast<float*>(smem_raw));
@@ -270,14 +270,14 @@ __global__ void __launch_bounds__(NT, 1) q_grad_kernel(const __grid_constant__ Q
         sm.xin[(a.obs_dim + j) * RP + tid] = valid ? a.act[(size_t)row * a.act_dim + j] : 0.f;
     }
     __syncthreads();
-    mlp_forward_tile(a.q, sm, 1);
+    mlp_forward_tile<H, ACT>(a.q, sm, 1);
     if (tid < TILE_R) {
       float diff = valid ? sm.y3[tid] - a.target[row] : 0.f;
       loss += 0.5f * diff * diff;
       sm.d3[tid] = diff * a.inv_global_rows;
     }
     __syncthreads();
-    mlp_backward_tile(a.q, sm, 1, true, false, ga, partial + L.oW2);
+    mlp_backward_tile<H, ACT>(a.q, sm, 1, true, false, ga, partial + L.oW2);
   }
   flush_grad_acc(a.q, ga, partial);
   if (tid < TILE_R) red[tid] = loss;
@@ -311,7 +311,7 @@ struct EvalArgs {
   NetDev net0, net1, net2;
 };
 
-template <int H>
+template <int H, int ACT>
 __global__ void __launch_bounds__(NT, 1) eval_kernel(const __grid_constant__ EvalArgs a) {
   extern __shared__ float4 smem_raw[];
   Smem<H> sm(reinterpret_cast<float*>(smem_raw));
@@ -332,14 +332,14 @@ __global__ void __launch_bounds__(NT, 1) eval_kernel(const __grid_constant__ Eva
     };
     auto policy_to_xin = [&](const NetDev& net) {   // a = pi(xin obs rows) -> xin action rows
       __syncthreads();
-      mlp_forward_tile(net, sm, a.act_dim);
+      mlp_forward_tile<H, ACT>(net, sm, a.act_dim);
       if (rt)
         for (int j = 0; j < a.act_dim; ++j)
           sm.xin[(a.obs_dim + j) * RP + tid] = head_fwd(sm.y3[j * RP + tid], a.policy_out_tanh, a.action_range);
     };
     auto q_eval = [&](const NetDev& net) -> float {
       __syncthreads();
-      mlp_forward_tile(net, sm, 1);
+      mlp_forward_tile<H, ACT>(net, sm, 1);
       return rt ? sm.y3[tid] : 0.f;
     };
     if (a.mode == 0) {
@@ -397,7 +397,7 @@ struct SampleArgs {
   NetDev net;
 };
 
-template <int H>
+template <int H, int ACT>
 __global__ void __launch_bounds__(NT, 1) env_sample_kernel(const __grid_constant__ SampleArgs a) {
   using E = Env<MPG_ENV_PT_REAL>;
   extern __shared__ float4 smem_raw[];
@@ -412,7 +412,7 @@ __global__ void __launch_bounds__(NT, 1) env_sample_kernel(const __grid_constant
     if (rt)
       for (int i = 0; i < a.obs_dim; ++i) sm.xin[i * RP + tid] = o[i] * a.obs_scale[i];
     __syncthreads();
-    mlp_forward_tile(a.net, sm, a.act_dim);
+    mlp_forward_tile<H, ACT>(a.net, sm, a.act_dim);
     if (valid) {
       const size_t tr = (size_t)t * a.agents + row;
       float act[E::A], o1[MPG_MAX_OBS];
@@ -480,6 +480,7 @@ __global__ void model_step_kernel(int rows, int obs_dim, int nfd, const float* _
   if (rew_out) rew_out[r] = rew;
 }
 
+#ifndef MPG_ACT_UNIT   // non-template kernels are defined in api.cu's unit only (act_instances.cuh)
 // real PathTracking environment step with the done flag
 __global__ void env_step_kernel(int rows, int obs_dim, int nfd, const float* __restrict__ state_in,
                                 const float* __restrict__ action, float* __restrict__ state_out,
@@ -500,6 +501,7 @@ __global__ void env_step_kernel(int rows, int obs_dim, int nfd, const float* __r
   if (rew_out) rew_out[r] = rew;
   if (done_out) done_out[r] = done;
 }
+#endif
 
 // g_state_in = J_s^T (E^T g_obs_out + g_state_out) + g_rew dr/ds ; g_action likewise
 template <int ENV>

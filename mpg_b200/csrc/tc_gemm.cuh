@@ -352,7 +352,7 @@ __device__ __forceinline__ void fwd_pair_issue(Bars* b, uint8_t* smem, Sync& s, 
     ++s.k_cnt;
   }
 }
-// Tail of a backward step: the first-layer pre-activations are recomputed chunk by chunk for elu'(z1) (the [p|a|1]
+// Tail of a backward step: the first-layer pre-activations are recomputed chunk by chunk for act'(z1) (the [p|a|1]
 // image of this step is still in place), then the input-gradient GEMM (do_gp) follows the delta1 blocks, then the
 // delta1 / [p|1] images are contracted over the rows into the persistent D1 accumulator (do_d1).
 template <int ROLE>
@@ -492,7 +492,7 @@ __global__ void pack_big_image(const float* __restrict__ src, int rs, int cs, ui
   *reinterpret_cast<uint4*>(img + stage + 2 * STAGE_BYTES + off) = l;
 }
 // first-layer image: value(n, k) = scale * (k < in_dim ? W1[k][n] : (k == bias_k ? b1[n] : 0)); 256 rows x 16 k,
-// (scale = log2(e) for the bf16 image of the BPTT recompute, whose z1 only feeds elu'(z1) = 2^(min(z1, 0) log2 e))
+// (scale = log2(e) for the bf16 image of the BPTT recompute, whose z1 only feeds act'(z1), e.g. elu'(z1) = 2^(min(z1, 0) log2 e))
 // INTERLEAVE K-major: [hi 8 KB | lo 8 KB]
 template <bool F16>
 __global__ void pack_l1_image(const float* __restrict__ W1, const float* __restrict__ b1, int in_dim, int bias_k,
@@ -512,6 +512,7 @@ __global__ void pack_l1_image(const float* __restrict__ W1, const float* __restr
   *reinterpret_cast<uint4*>(img + off) = h;
   *reinterpret_cast<uint4*>(img + 8192 + off) = l;
 }
+#ifndef MPG_ACT_UNIT   // non-template kernels are defined in api.cu's unit only (act_instances.cuh)
 // input-gradient image: value(i, n) = i < in_dim ? W1[i][n] : 0; per 64-k block 32 rows (hi of rows 0..15, then lo of rows
 // 0..15) x 128 B, SW128 K-major: 4 x 4 KB
 __global__ void pack_in_image(const float* __restrict__ W1, int in_dim, uint8_t* __restrict__ img) {
@@ -528,8 +529,9 @@ __global__ void pack_in_image(const float* __restrict__ W1, int in_dim, uint8_t*
   *reinterpret_cast<uint4*>(img + off(i)) = h;
   *reinterpret_cast<uint4*>(img + off(16 + i)) = l;
 }
+#endif
 
-#ifdef MPG_DEBUG_PROBES
+#if defined(MPG_DEBUG_PROBES) && !defined(MPG_ACT_UNIT)
 // ---- self test: the three GEMM kinds against caller-provided fp32 data ---------------------------------------
 //   kind 0: Z[128 x 256] = X[128 x 256] . (image of Wt[256 x 256])^T
 //   kind 1: Z[128 x 256] = X16[128 x 16] . (first-layer image)^T

@@ -1,6 +1,6 @@
 // Tensor-core (tcgen05) model-rollout kernels.
 //
-// tc_rollout_kernel<ENV,BWD>: one persistent CTA per SM owns a tile of 128 trajectories and walks the
+// tc_rollout_kernel<ENV,BWD,ACT>: one persistent CTA per SM owns a tile of 128 trajectories and walks the
 // horizon.  All 256x256 (and 16x256 / 256x16) contractions of the policy / Q MLPs run on the 5th-gen
 // tensor cores with split-bf16 operands (3 products, fp32 accumulation in TMEM); weights are streamed from
 // L2 through a shared-memory ring by the TMA engine; the per-row vehicle / pendulum dynamics, rewards,
@@ -8,7 +8,7 @@
 // Backward = BPTT from the 24-byte state checkpoints.  The forward pass of the gradient kernel leaves the second
 // hidden activation of every step behind as a ready-made operand image (1 KB per row and step, written straight
 // from the epilogue registers); BPTT pulls it back with one bulk copy per step instead of re-running layer 1 + layer 2
-// (one third of the contraction work and two of the five epilogues of a backward step).  elu'(z1) still comes from
+// (one third of the contraction work and two of the five epilogues of a backward step).  act'(z1) still comes from
 // the cheap K = 16 first-layer recompute.  The dX chain (what the recurrence needs) is fully fused.  The weight-gradient contractions (K = rows) cannot be accumulated in place: the
 // fp32 accumulator of dW2 alone is 256 KB = all of TMEM.  Their operand tiles (h1, h2, delta1, delta2 as
 // split-bf16 images, written to shared memory anyway as UMMA operands) are bulk-stored once and consumed
@@ -79,6 +79,36 @@ constexpr int SM_TOTAL = SM_D3IMG + 8192;
 
 __device__ __forceinline__ void epi_bar() { asm volatile("bar.sync 1, %0;" ::"n"(EPI_THREADS) : "memory"); }
 __device__ __forceinline__ float elu_fast(float x) { return x > 0.f ? x : exp_fast(x) - 1.f; }
+// hidden activation of the E1 / E2 epilogues.  tanh: the fp32 library tanhf (a few ulp); tanh.approx (MUFU.TANH, relative
+// error ~2^-11) would break the 1e-5 closed-loop bar the fp16-pair forward meets.  tanh values lie in [-1, 1]: the fp16 pair
+// of h1 does not saturate.
+template <int ACT>
+__device__ __forceinline__ float act_fast(float x) {
+  if constexpr (ACT == MPG_ACT_RELU) return x > 0.f ? x : 0.f;
+  else if constexpr (ACT == MPG_ACT_TANH) return tanhf(x);
+  else return elu_fast(x);
+}
+// g act'(z2) through the output h2 (bf16 pair read back from the h2 image): elu' = 1 + min(h2, 0), relu' = [h2 > 0],
+// tanh' = 1 - h2^2
+template <int ACT>
+__device__ __forceinline__ float times_act_grad_out(float g, float h) {
+  if constexpr (ACT == MPG_ACT_RELU) return h > 0.f ? g : 0.f;
+  else if constexpr (ACT == MPG_ACT_TANH) return g * fmaf(-h, h, 1.f);
+  else return fmaf(g, fminf(h, 0.f), g);
+}
+// act'(z1) from z = z1 log2(e) (the pre-scaled bf16 first-layer image): elu' = 2^min(z, 0), exactly 1 for z >= 0;
+// relu' = [z > 0]; tanh' = 1 - tanh^2(z1) = 4 e / (1 + e)^2 with e = 2^(-2|z|) = exp(-2|z1|) (no cancellation)
+template <int ACT>
+__device__ __forceinline__ float act_grad_log2e(float z) {
+  if constexpr (ACT == MPG_ACT_RELU) {
+    return z > 0.f ? 1.f : 0.f;
+  } else if constexpr (ACT == MPG_ACT_TANH) {
+    const float e = ex2_ftz(-2.f * fabsf(z)), d = 1.f + e;
+    return __fdividef(4.f * e, d * d);
+  } else {
+    return ex2_ftz(fminf(z, 0.f));
+  }
+}
 
 // load 8 consecutive features of row r back from a split-bf16 image (hi + lo)
 __device__ __forceinline__ void act_load8(const uint8_t* act_hi, const uint8_t* act_lo, int r, int cc, float* x) {
@@ -135,6 +165,7 @@ __device__ __forceinline__ void store_wait(bool elected) {
 // the activation image is complete (and published to the MMA warp) after 1/4 of the epilogue.
 
 // z1 (streamed through the two TMEM chunk buffers, bias folded in) -> h1 image
+template <int ACT>
 __device__ MPG_EPI_INLINE void epi_hidden1_blocks(Bars* b, uint32_t tm_zc_lane, uint8_t* act, int row, int hc) {
   // (reading the two chunk buffers out in pairs, to release chunk 1 early and get chunk 3 out of the layer-2 GEMM's way, was
   // slower: a first-layer chunk takes ~500 cycles in the tensor pipe, so block 0 started that much later)
@@ -145,13 +176,14 @@ __device__ MPG_EPI_INLINE void epi_hidden1_blocks(Bars* b, uint32_t tm_zc_lane, 
     tmem_ld16(tm_zc_lane + (kb & 1) * 64 + hc * 16, v);
     epi_release_chunk(b, kb);
 #pragma unroll
-    for (int i = 0; i < 16; ++i) v[i] = elu_fast(v[i]);
+    for (int i = 0; i < 16; ++i) v[i] = act_fast<ACT>(v[i]);
     act_store8<true>(act, act + ACT_SPLIT, row, c0 >> 3, v);
     act_store8<true>(act, act + ACT_SPLIT, row, (c0 >> 3) + 1, v + 8);
     epi_block_done(b, kb);
   }
 }
 // z2 (TMEM) + b2 -> h2 -> partial output-layer dot products (forward pass: no image needed)
+template <int ACT>
 __device__ MPG_EPI_INLINE void epi_hidden2(uint32_t tm_lane, const float* b2, const float* W3, int hc, float& p0, float& p1) {
   p0 = 0.f; p1 = 0.f;
   for (int c0 = hc * COLS_PER_WARP; c0 < (hc + 1) * COLS_PER_WARP; c0 += 32) {
@@ -159,7 +191,7 @@ __device__ MPG_EPI_INLINE void epi_hidden2(uint32_t tm_lane, const float* b2, co
     tmem_ld32(tm_lane + c0, v);
 #pragma unroll
     for (int i = 0; i < 32; ++i) {
-      const float h = elu_fast(v[i] + b2[c0 + i]);
+      const float h = act_fast<ACT>(v[i] + b2[c0 + i]);
       const float2 w = *reinterpret_cast<const float2*>(W3 + 2 * (c0 + i));
       p0 = fmaf(h, w.x, p0);
       p1 = fmaf(h, w.y, p1);
@@ -171,6 +203,7 @@ __device__ MPG_EPI_INLINE void epi_hidden2(uint32_t tm_lane, const float* b2, co
 // (the canonical no-swizzle UMMA layout: K-major with LBO = 2048, SBO = 128, and MN-major with LBO = 128, SBO = 2048).
 // A warp (32 consecutive rows, one chunk) writes 512 contiguous bytes per store instruction.
 __device__ __forceinline__ uint32_t lin_chunk_off(int r, int cc) { return (uint32_t)(cc * (ACT_ROWS * 16) + r * 16); }
+template <int ACT>
 __device__ MPG_EPI_INLINE void epi_hidden2_gstore(uint32_t tm_lane, const float* b2, const float* W3, uint8_t* gimg, int row,
                                                   int hc, float& p0, float& p1) {
   p0 = 0.f; p1 = 0.f;
@@ -179,7 +212,7 @@ __device__ MPG_EPI_INLINE void epi_hidden2_gstore(uint32_t tm_lane, const float*
     tmem_ld16(tm_lane + c0, v);
 #pragma unroll
     for (int i = 0; i < 16; ++i) {
-      v[i] = elu_fast(v[i] + b2[c0 + i]);
+      v[i] = act_fast<ACT>(v[i] + b2[c0 + i]);
       const float2 w = *reinterpret_cast<const float2*>(W3 + 2 * (c0 + i));
       p0 = fmaf(v[i], w.x, p0);
       p1 = fmaf(v[i], w.y, p1);
@@ -198,6 +231,7 @@ __device__ MPG_EPI_INLINE void epi_hidden2_gstore(uint32_t tm_lane, const float*
   }
 }
 // same, and keep h2 as an image (Q part of the backward pass: delta2 and the dW3 operand are derived from it)
+template <int ACT>
 __device__ MPG_EPI_INLINE void epi_hidden2_img(uint32_t tm_lane, const float* b2, const float* W3, uint8_t* act, int row,
                                                int hc, float& p0, float& p1, bool draining = false, bool elected = false) {
   p0 = 0.f; p1 = 0.f;
@@ -208,7 +242,7 @@ __device__ MPG_EPI_INLINE void epi_hidden2_img(uint32_t tm_lane, const float* b2
     if (draining) store_wait_block(elected, kb);             // block kb of the old image has been read out
 #pragma unroll
     for (int i = 0; i < 16; ++i) {
-      v[i] = elu_fast(v[i] + b2[c0 + i]);
+      v[i] = act_fast<ACT>(v[i] + b2[c0 + i]);
       const float2 w = *reinterpret_cast<const float2*>(W3 + 2 * (c0 + i));
       p0 = fmaf(v[i], w.x, p0);
       p1 = fmaf(v[i], w.y, p1);
@@ -217,7 +251,8 @@ __device__ MPG_EPI_INLINE void epi_hidden2_img(uint32_t tm_lane, const float* b2
     act_store8(act, act + ACT_SPLIT, row, (c0 >> 3) + 1, v + 8);
   }
 }
-// delta2 = (delta3 W3^T) * elu'(h2), h2 read back from its image and overwritten in place by delta2
+// delta2 = (delta3 W3^T) * act'(h2), h2 read back from its image and overwritten in place by delta2
+template <int ACT>
 __device__ MPG_EPI_INLINE void epi_delta2_blocks(Bars* b, const float* W3, float d30, float d31, uint8_t* act, int row, int hc,
                                                  Sync* wait_half1 = nullptr) {
   for (int kb = 0; kb < 4; ++kb) {
@@ -230,7 +265,7 @@ __device__ MPG_EPI_INLINE void epi_delta2_blocks(Bars* b, const float* W3, float
     for (int i = 0; i < 16; ++i) {
       const float2 w = *reinterpret_cast<const float2*>(W3 + 2 * (c0 + i));
       const float g = fmaf(d30, w.x, d31 * w.y);
-      v[i] = fmaf(g, fminf(v[i], 0.f), g);            // g elu'(z), elu'(z) = 1 + min(h2, 0) expressed through the output h2
+      v[i] = times_act_grad_out<ACT>(g, v[i]);        // g act'(z2), expressed through the output h2
     }
     act_store8(act, act + ACT_SPLIT, row, c0 >> 3, v);
     act_store8(act, act + ACT_SPLIT, row, (c0 >> 3) + 1, v + 8);
@@ -244,6 +279,7 @@ __device__ MPG_EPI_INLINE void epi_delta2_blocks(Bars* b, const float* W3, float
 // their first half has completed (d_full), blocks 2, 3 after the second (d_half).  Only the WRITES wait for that: the
 // reads and the arithmetic of blocks 0 and 2 run underneath those UMMAs (16 per half, ~190 cycles each from the
 // no-swizzle image).
+template <int ACT>
 __device__ MPG_EPI_INLINE void epi_delta2_from_h2(Bars* b, const float* W3, float d30, float d31, uint8_t* act, int row, int hc,
                                                   uint32_t img_parity, Sync* wait_d3 = nullptr) {
   for (int kb = 0; kb < 4; ++kb) {
@@ -266,7 +302,7 @@ __device__ MPG_EPI_INLINE void epi_delta2_from_h2(Bars* b, const float* W3, floa
     for (int i = 0; i < 16; ++i) {
       const float2 w = *reinterpret_cast<const float2*>(W3 + 2 * (c0 + i));
       const float g = fmaf(d30, w.x, d31 * w.y);
-      v[i] = fmaf(g, fminf(v[i], 0.f), g);            // g elu'(z), elu'(z) = 1 + min(h2, 0) expressed through the output h2
+      v[i] = times_act_grad_out<ACT>(g, v[i]);        // g act'(z2), expressed through the output h2
     }
     if (wait_d3 && kb == 0) epi_wait_d(b, *wait_d3);         // the D3 UMMAs have read blocks 0, 1 of the h2 image
     if (wait_d3 && kb == 2) epi_wait_half(b, *wait_d3);      // ... and blocks 2, 3
@@ -276,8 +312,9 @@ __device__ MPG_EPI_INLINE void epi_delta2_from_h2(Bars* b, const float* W3, floa
     epi_block_done(b, kb);
   }
 }
-// delta1 = g_h1 (TMEM work) * elu'(z1) (z1 log2(e) recomputed with the pre-scaled bf16 first-layer image, streamed through the
+// delta1 = g_h1 (TMEM work) * act'(z1) (z1 log2(e) recomputed with the pre-scaled bf16 first-layer image, streamed through the
 // chunk buffers) -> delta1 image
+template <int ACT>
 __device__ MPG_EPI_INLINE void epi_delta1_blocks(Bars* b, uint32_t tm_work_lane, uint32_t tm_zc_lane, uint8_t* act, int row,
                                                  int hc, bool draining = false, bool elected = false, bool release_img = false) {
   for (int kb = 0; kb < 4; ++kb) {
@@ -289,7 +326,7 @@ __device__ MPG_EPI_INLINE void epi_delta1_blocks(Bars* b, uint32_t tm_work_lane,
     epi_release_chunk(b, kb);
     if (draining) store_wait_block(elected, kb);             // block kb of the old image has been read out
 #pragma unroll
-    for (int i = 0; i < 16; ++i) g[i] *= ex2_ftz(fminf(z[i], 0.f));     // z = z1 log2(e) (l1b image): elu'(z1) = 2^min(z, 0), exactly 1 for z >= 0
+    for (int i = 0; i < 16; ++i) g[i] *= act_grad_log2e<ACT>(z[i]);     // z = z1 log2(e) (l1b image)
     act_store8(act, act + ACT_SPLIT, row, c0 >> 3, g);
     act_store8(act, act + ACT_SPLIT, row, (c0 >> 3) + 1, g + 8);
     epi_block_done(b, kb);
@@ -328,7 +365,7 @@ constexpr int XCHG_THREADS = EPI_THREADS + ROW_THREADS;
 // ROLE_ROW: 4 warps, thread = trajectory: environment step and adjoint, output head, [p|a|1] / delta3 images,
 // checkpoints, returns -- the scalar recurrence lives in registers of threads that hold nothing else.
 // ROLE_PRODUCER / ROLE_MMA: one thread each.
-template <int ENV, bool BWD, int ROLE>
+template <int ENV, bool BWD, int ACT, int ROLE>
 __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars* b) {
   using E = Env<ENV>;
   constexpr int S = E::S, NA = E::A;
@@ -466,14 +503,14 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
       if (ROLE == ROLE_EPI) {
         stamp(17);
         if (store_pending) { store_wait(elected); store_pending = false; }   // the previous step's h1 record has left long ago
-        epi_hidden1_blocks(b, tm_z1c + lane_off, act_img, row, hc);          // follows the z1 chunk stream
+        epi_hidden1_blocks<ACT>(b, tm_z1c + lane_off, act_img, row, hc);          // follows the z1 chunk stream
         stamp(18);
         if (slot) { store_image_follow(elected, b, sy, slot + SLOT_H1, act_img, A.rec_hi_only != 0); store_pending = true; }
         epi_wait_d(b, sy);                                   // z2 (all layer-2 UMMAs done)
         stamp(19);
         float p0, p1;
-        if (BWD) epi_hidden2_gstore(tm_work + lane_off, mf->b2p, mf->W3p, h2slot, row, hc, p0, p1);
-        else epi_hidden2(tm_work + lane_off, mf->b2p, mf->W3p, hc, p0, p1);
+        if (BWD) epi_hidden2_gstore<ACT>(tm_work + lane_off, mf->b2p, mf->W3p, h2slot, row, hc, p0, p1);
+        else epi_hidden2<ACT>(tm_work + lane_off, mf->b2p, mf->W3p, hc, p0, p1);
         stamp(20);
         mf->part[(hc * 2 + 0) * ACT_ROWS + row] = p0;
         mf->part[(hc * 2 + 1) * ACT_ROWS + row] = p1;
@@ -493,15 +530,15 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
       fwd_pair_issue<ROLE>(b, smem, sy, A.q.l1, A.q.big_fwd, tm_z1c, tm_work);
       if (ROLE == ROLE_EPI) {
         if (store_pending) { store_wait(elected); store_pending = false; }
-        epi_hidden1_blocks(b, tm_z1c + lane_off, act_img, row, hc);
+        epi_hidden1_blocks<ACT>(b, tm_z1c + lane_off, act_img, row, hc);
         if (qslot) store_image(elected, qslot + SLOT_H1, act_img, A.rec_hi_only ? ACT_SPLIT : 2 * ACT_SPLIT);
         epi_wait_d(b, sy);
         float p0, p1;
         if (with_img) {
           if (qslot) store_wait(elected);
-          epi_hidden2_img(tm_work + lane_off, mf->b2q, mf->W3q, act_img, row, hc, p0, p1);
+          epi_hidden2_img<ACT>(tm_work + lane_off, mf->b2q, mf->W3q, act_img, row, hc, p0, p1);
         } else {
-          epi_hidden2(tm_work + lane_off, mf->b2q, mf->W3q, hc, p0, p1);
+          epi_hidden2<ACT>(tm_work + lane_off, mf->b2q, mf->W3q, hc, p0, p1);
         }
         mf->part[(hc * 2 + 0) * ACT_ROWS + row] = p0;
         bar_arrive(BAR_PART, XCHG_THREADS);
@@ -709,14 +746,14 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
           }
           gemm_issue<ROLE>(0, b, smem, sy, A.q.big_dx, tm_work);  // g_h1q, K-blocks issued as delta2 blocks appear
           if (ROLE == ROLE_EPI) {
-            epi_delta2_blocks(b, mf->W3q, mf->d3s[row], 0.f, act_img, row, hc, reg ? &sy : nullptr);
+            epi_delta2_blocks<ACT>(b, mf->W3q, mf->d3s[row], 0.f, act_img, row, hc, reg ? &sy : nullptr);
             if (qslot) store_image(elected, qslot + SLOT_D2, act_img, A.rec_hi_only ? ACT_SPLIT : 2 * ACT_SPLIT);
             epi_wait_d(b, sy);
           }
           bwd_tail_issue<ROLE>(b, smem, sy, A.q.l1b, A.q.in, !reg, reg, d1_started, tm_z1c, tm_gp, tm_d1, true);
           if (ROLE == ROLE_EPI) {
             if (qslot) store_wait(elected);                // delta2 image read out before it is overwritten
-            epi_delta1_blocks(b, tm_work + lane_off, tm_z1c + lane_off, act_img, row, hc);
+            epi_delta1_blocks<ACT>(b, tm_work + lane_off, tm_z1c + lane_off, act_img, row, hc);
             if (!reg) epi_wait_d(b, sy);
           }
           if (reg) { d1_pending = true; ++acc_issued; }
@@ -786,7 +823,7 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
         if (ROLE == ROLE_MMA) stamp(5);
         if (want_dw) d3_issue<ROLE>(b, smem, sy, SM_D3IMG, d3_started, tm_d3, true, A.rec_hi_only != 0);   // dW3 += h2^T delta3
         if (ROLE == ROLE_MMA) stamp(6);
-        // ---- [p|1] image of step t (first-layer recompute for elu'(z1), D1 operand, db2 record); the D1 UMMAs of the
+        // ---- [p|1] image of step t (first-layer recompute for act'(z1), D1 operand, db2 record); the D1 UMMAs of the
         // previous step still read the old one ----
         if (rowthread) {
           acc_wait();
@@ -805,7 +842,7 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
         if (ROLE == ROLE_MMA) stamp(4);
         if (ROLE == ROLE_EPI) {
           stamp(6);
-          epi_delta2_from_h2(b, mf->W3p, mf->d3s[row], mf->d3s[ACT_ROWS + row], act_img, row, hc, (sy.i_cnt - 1) & 1,
+          epi_delta2_from_h2<ACT>(b, mf->W3p, mf->d3s[row], mf->d3s[ACT_ROWS + row], act_img, row, hc, (sy.i_cnt - 1) & 1,
                              want_dw ? &sy : nullptr);
           stamp(7);
           if (rec) store_image_follow(elected, b, sy, slot + SLOT_D2, act_img, A.rec_hi_only != 0);   // delta2 blocks leave behind their K-blocks
@@ -816,7 +853,7 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
         bwd_tail_issue<ROLE>(b, smem, sy, A.pol.l1b, A.pol.in, t > 0, want_dw, d1_started, tm_z1c, tm_gp, tm_d1, true, early_next);
         if (ROLE == ROLE_PRODUCER && early_next) load_h2(t - 1);
         if (ROLE == ROLE_EPI) {
-          epi_delta1_blocks(b, tm_work + lane_off, tm_z1c + lane_off, act_img, row, hc, rec, elected, early_next);
+          epi_delta1_blocks<ACT>(b, tm_work + lane_off, tm_z1c + lane_off, act_img, row, hc, rec, elected, early_next);
           stamp(9);
           if (t > 0) epi_wait_d(b, sy);
           stamp(10);
@@ -899,7 +936,7 @@ constexpr int LAUNCH_REGS = 80, EPI_REGS = 80, ROW_REGS = 96, AUX_REGS = 64;
 static_assert(EPI_THREADS * EPI_REGS + ROW_THREADS * ROW_REGS + 128 * AUX_REGS <= ROLLOUT_THREADS * LAUNCH_REGS,
               "setmaxnreg only redistributes the register pool of the CTA");
 
-template <int ENV, bool BWD>
+template <int ENV, bool BWD, int ACT>
 __global__ void __launch_bounds__(ROLLOUT_THREADS, 1) tc_rollout_kernel(const __grid_constant__ TcArgs A) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -923,14 +960,14 @@ __global__ void __launch_bounds__(ROLLOUT_THREADS, 1) tc_rollout_kernel(const __
   Bars* b = cta_setup(smem, XCHG_THREADS, MMA_WARP);   // contains __syncthreads()
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (warp < EPI_WARPS) {
-    run_rollout<ENV, BWD, ROLE_EPI>(A, smem, b);
+    run_rollout<ENV, BWD, ACT, ROLE_EPI>(A, smem, b);
   } else if (warp < PRODUCER_WARP) {
     asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(ROW_REGS));
-    run_rollout<ENV, BWD, ROLE_ROW>(A, smem, b);
+    run_rollout<ENV, BWD, ACT, ROLE_ROW>(A, smem, b);
   } else {
     asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(AUX_REGS));
-    if (warp == PRODUCER_WARP) { if (elect_one()) run_rollout<ENV, BWD, ROLE_PRODUCER>(A, smem, b); }
-    else if (warp == MMA_WARP) { if (elect_one()) run_rollout<ENV, BWD, ROLE_MMA>(A, smem, b); }
+    if (warp == PRODUCER_WARP) { if (elect_one()) run_rollout<ENV, BWD, ACT, ROLE_PRODUCER>(A, smem, b); }
+    else if (warp == MMA_WARP) { if (elect_one()) run_rollout<ENV, BWD, ACT, ROLE_MMA>(A, smem, b); }
   }
   cta_teardown(b, MMA_WARP);
 }
@@ -977,6 +1014,7 @@ struct DwBars {
 
 constexpr int DW_CONV_WARPS = 8;                                // warps 0..7 convert h1 (0..3 also read the accumulators out)
 constexpr int DW_THREADS = (DW_CONV_WARPS + 2) * 32;           // + producer warp + mma warp
+#ifndef MPG_ACT_UNIT   // non-template kernels are defined in api.cu's unit only (act_instances.cuh)
 __global__ void __launch_bounds__(DW_THREADS, 1) tc_dw_kernel(const __grid_constant__ DwArgs A) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -1117,6 +1155,7 @@ __global__ void __launch_bounds__(DW_THREADS, 1) tc_dw_kernel(const __grid_const
   __syncthreads();
   if (warp == DW_CONV_WARPS + 1) tmem_dealloc(tmem, TMEM_COLS);
 }
+#endif
 
 }  // namespace tc
 }  // namespace mpg

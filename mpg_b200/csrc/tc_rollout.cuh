@@ -1,5 +1,7 @@
 // Tensor-core (tcgen05) path: state owned by the handle, weight-image packing, launchers.
 #pragma once
+#include <type_traits>
+
 #include "tc_kernels.cuh"
 #ifdef MPG_DEBUG_PROBES
 #include "tc_pair_probe.cuh"
@@ -52,14 +54,18 @@ inline bool tc_init(TcState& t, const mpg_config& cfg, int /*sms*/, size_t& ws_b
          && alloc((void**)&t.nets[n].l1, 16384) && alloc((void**)&t.nets[n].l1b, 16384) && alloc((void**)&t.nets[n].in, 16384);
   if (!ok) return false;
   const int sm = tc::SM_TOTAL + 1024;
-  ok = tc_set_smem(tc::tc_rollout_kernel<MPG_ENV_PATH_TRACKING, true>, sm)
-       && tc_set_smem(tc::tc_rollout_kernel<MPG_ENV_PATH_TRACKING, false>, sm)
-       && tc_set_smem(tc::tc_rollout_kernel<MPG_ENV_INVERTED_PENDULUM, true>, sm)
-       && tc_set_smem(tc::tc_rollout_kernel<MPG_ENV_INVERTED_PENDULUM, false>, sm)
-       && tc_set_smem(tc::tc_rollout_kernel<MPG_ENV_INVERTED_DOUBLE_PENDULUM, true>, sm)
-       && tc_set_smem(tc::tc_rollout_kernel<MPG_ENV_INVERTED_DOUBLE_PENDULUM, false>, sm)
-       && tc_set_smem(tc::tc_rollout_kernel<MPG_ENV_PATH_TRACKING_REAL, false>, sm)
-       && tc_set_smem(tc::tc_dw_kernel, tc::DW_SMEM);
+  auto set_act = [&](auto ac) {
+    constexpr int ACT = decltype(ac)::value;
+    return tc_set_smem(tc::tc_rollout_kernel<MPG_ENV_PATH_TRACKING, true, ACT>, sm)
+           && tc_set_smem(tc::tc_rollout_kernel<MPG_ENV_PATH_TRACKING, false, ACT>, sm)
+           && tc_set_smem(tc::tc_rollout_kernel<MPG_ENV_INVERTED_PENDULUM, true, ACT>, sm)
+           && tc_set_smem(tc::tc_rollout_kernel<MPG_ENV_INVERTED_PENDULUM, false, ACT>, sm)
+           && tc_set_smem(tc::tc_rollout_kernel<MPG_ENV_INVERTED_DOUBLE_PENDULUM, true, ACT>, sm)
+           && tc_set_smem(tc::tc_rollout_kernel<MPG_ENV_INVERTED_DOUBLE_PENDULUM, false, ACT>, sm)
+           && tc_set_smem(tc::tc_rollout_kernel<MPG_ENV_PATH_TRACKING_REAL, false, ACT>, sm);
+  };
+  ok = set_act(std::integral_constant<int, MPG_ACT_ELU>()) && set_act(std::integral_constant<int, MPG_ACT_RELU>())
+       && set_act(std::integral_constant<int, MPG_ACT_TANH>()) && tc_set_smem(tc::tc_dw_kernel, tc::DW_SMEM);
 #ifdef MPG_DEBUG_PROBES
   ok = ok && tc_set_smem(tc::selftest_kernel, tc::SmemMap::TOTAL + 1024) && tc_set_smem(tc::pair_probe_kernel, tc::PAIR_SMEM);
 #endif
@@ -81,7 +87,7 @@ inline bool tc_pack_weights(TcState& t, int net, const float* flat, int in_dim, 
   tc::pack_big_image<true><<<32, 256, 0, st>>>(flat + L.oW2, 1, tc::H, t.nets[net].big_fwd);     // value(n,k) = W2[k][n]
   tc::pack_big_image<false><<<32, 256, 0, st>>>(flat + L.oW2, tc::H, 1, t.nets[net].big_dx);      // value(k,n) = W2[k][n]
   tc::pack_l1_image<true><<<2, 256, 0, st>>>(flat + L.oW1, flat + L.ob1, in_dim, tc::BIAS_K, t.nets[net].l1);
-  tc::pack_l1_image<false><<<2, 256, 0, st>>>(flat + L.oW1, flat + L.ob1, in_dim, tc::BIAS_K, t.nets[net].l1b, 1.4426950408889634f);   // z1 log2(e), see epi_delta1_blocks
+  tc::pack_l1_image<false><<<2, 256, 0, st>>>(flat + L.oW1, flat + L.ob1, in_dim, tc::BIAS_K, t.nets[net].l1b, 1.4426950408889634f);   // z1 log2(e) for every activation, see act_grad_log2e
   tc::pack_in_image<<<2, 256, 0, st>>>(flat + L.oW1, in_dim, t.nets[net].in);
   return cudaGetLastError() == cudaSuccess;
 }
@@ -106,20 +112,29 @@ inline bool tc_ensure_buf(uint8_t*& buf, size_t& have, size_t bytes) {
 inline bool tc_ensure_store(TcState& t, size_t bytes) { return tc_ensure_buf(t.store, t.store_bytes, bytes); }
 inline bool tc_ensure_h2store(TcState& t, size_t bytes) { return tc_ensure_buf(t.h2store, t.h2store_bytes, bytes); }
 
+// act: MPG_ACT_* of the handle
 template <bool BWD>
-inline cudaError_t tc_launch_rollout(int env, const tc::TcArgs& a, int grid, cudaStream_t st) {
+inline cudaError_t tc_launch_rollout(int env, int act, const tc::TcArgs& a, int grid, cudaStream_t st) {
   const size_t smem = tc::SM_TOTAL + 1024;
-  if (env == MPG_ENV_PATH_TRACKING_REAL) {
-    if (BWD) return cudaErrorNotSupported;
-    tc::tc_rollout_kernel<MPG_ENV_PATH_TRACKING_REAL, false><<<grid, tc::ROLLOUT_THREADS, smem, st>>>(a);
+  auto launch = [&](auto ac) {
+    constexpr int ACT = decltype(ac)::value;
+    if (env == MPG_ENV_PATH_TRACKING_REAL) {
+      if (BWD) return cudaErrorNotSupported;
+      tc::tc_rollout_kernel<MPG_ENV_PATH_TRACKING_REAL, false, ACT><<<grid, tc::ROLLOUT_THREADS, smem, st>>>(a);
+      return cudaGetLastError();
+    }
+    switch (env) {
+      case MPG_ENV_PATH_TRACKING: tc::tc_rollout_kernel<MPG_ENV_PATH_TRACKING, BWD, ACT><<<grid, tc::ROLLOUT_THREADS, smem, st>>>(a); break;
+      case MPG_ENV_INVERTED_PENDULUM: tc::tc_rollout_kernel<MPG_ENV_INVERTED_PENDULUM, BWD, ACT><<<grid, tc::ROLLOUT_THREADS, smem, st>>>(a); break;
+      default: tc::tc_rollout_kernel<MPG_ENV_INVERTED_DOUBLE_PENDULUM, BWD, ACT><<<grid, tc::ROLLOUT_THREADS, smem, st>>>(a); break;
+    }
     return cudaGetLastError();
+  };
+  switch (act) {
+    case MPG_ACT_RELU: return launch(std::integral_constant<int, MPG_ACT_RELU>());
+    case MPG_ACT_TANH: return launch(std::integral_constant<int, MPG_ACT_TANH>());
+    default: return launch(std::integral_constant<int, MPG_ACT_ELU>());
   }
-  switch (env) {
-    case MPG_ENV_PATH_TRACKING: tc::tc_rollout_kernel<MPG_ENV_PATH_TRACKING, BWD><<<grid, tc::ROLLOUT_THREADS, smem, st>>>(a); break;
-    case MPG_ENV_INVERTED_PENDULUM: tc::tc_rollout_kernel<MPG_ENV_INVERTED_PENDULUM, BWD><<<grid, tc::ROLLOUT_THREADS, smem, st>>>(a); break;
-    default: tc::tc_rollout_kernel<MPG_ENV_INVERTED_DOUBLE_PENDULUM, BWD><<<grid, tc::ROLLOUT_THREADS, smem, st>>>(a); break;
-  }
-  return cudaGetLastError();
 }
 
 #ifdef MPG_DEBUG_PROBES

@@ -26,13 +26,16 @@ class Engine:
 
     def __init__(self, env_id, obs_dim, act_dim, obs_scale, rew_scale, rew_shift, gamma,
                  policy_out_activation='tanh', action_range=None, num_future_data=0, hidden=256,
-                 max_rows=4096, max_horizon=25, device=None, debug_lib=False, **_unused):
+                 max_rows=4096, max_horizon=25, device=None, debug_lib=False, hidden_activation='elu', **_unused):
         self.lib = _lib.load(debug=bool(debug_lib))   # debug_lib: the library with the development probes (tests / tools)
         if not torch.cuda.is_available():
             raise RuntimeError('mpg_b200 needs a CUDA device (B200, sm_100a); there is no CPU fallback')
         self.device = torch.device('cuda', torch.cuda.current_device()) if device is None else torch.device(device)
         if env_id not in ENV_IDS:
             raise ValueError(f'unknown env_id {env_id!r}')
+        if hidden_activation not in _lib.ACTIVATIONS:
+            raise ValueError(f'hidden_activation must be one of {sorted(_lib.ACTIVATIONS)} (got {hidden_activation!r})')
+        self.hidden_activation = hidden_activation
         self.env_id, self.obs_dim, self.act_dim = env_id, int(obs_dim), int(act_dim)
         cfg = MpgConfig()
         cfg.env = ENV_IDS[env_id]
@@ -56,6 +59,7 @@ class Engine:
             rc = self.lib.mpg_create(ctypes.byref(cfg), ctypes.byref(self.h))
         if rc != 0:
             raise RuntimeError('mpg_create failed: ' + self.lib.mpg_last_error(None).decode())
+        self._check(self.lib.mpg_set_activation(self.h, _lib.ACTIVATIONS[hidden_activation]))
         self.state_dim = self.lib.mpg_state_dim(self.h)
         self.num_sms = self.lib.mpg_num_sms(self.h)
 
@@ -84,6 +88,7 @@ class Engine:
             rc = self.lib.mpg_create(ctypes.byref(self.cfg), ctypes.byref(self.h))
         if rc != 0:
             raise RuntimeError('mpg_create failed: ' + self.lib.mpg_last_error(None).decode())
+        self._check(self.lib.mpg_set_activation(self.h, _lib.ACTIVATIONS[self.hidden_activation]))
         for net, w in saved.items():
             self.set_net_weights(net, w)
             m, v = moments[net]

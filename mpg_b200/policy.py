@@ -18,6 +18,7 @@ from .synthetic import make_mlp_weights
 
 
 HIDDEN_WIDTHS = (64, 128, 256)   # hidden widths the fp32 (FFMA) kernels are built for; tensor cores: 256 only
+HIDDEN_ACTIVATIONS = ('elu', 'relu', 'tanh')   # hidden activations both backends are built for
 
 
 class PolicyWithQs(object):
@@ -34,11 +35,17 @@ class PolicyWithQs(object):
         if policy_num_hidden_units not in HIDDEN_WIDTHS:
             raise NotImplementedError('the sm_100a kernels are built for %s hidden units (got %r)'
                                       % (' / '.join(map(str, HIDDEN_WIDTHS)), policy_num_hidden_units))
-        if value_hidden_activation != 'elu' or policy_hidden_activation != 'elu':
-            raise NotImplementedError("hidden activation must be 'elu' (reference default)")
+        if value_hidden_activation != policy_hidden_activation:
+            raise NotImplementedError('value_hidden_activation and policy_hidden_activation must be equal: one hidden '
+                                      'activation per handle (got %r and %r)' % (value_hidden_activation,
+                                                                                 policy_hidden_activation))
+        if policy_hidden_activation not in HIDDEN_ACTIVATIONS:
+            raise NotImplementedError('the sm_100a kernels are built for the hidden activations %s (got %r)'
+                                      % (' / '.join(HIDDEN_ACTIVATIONS), policy_hidden_activation))
         if not deterministic_policy:
             raise NotImplementedError('the model-based learners use deterministic_policy=True (train_script.py:273)')
         self.obs_dim, self.act_dim, self.hidden = obs_dim, act_dim, int(policy_num_hidden_units)
+        self.hidden_activation = policy_hidden_activation
         self.policy_only, self.double_Q, self.target = policy_only, double_Q, target
         self.tau, self.delay_update, self.action_range = tau, delay_update, action_range
         self.deterministic_policy = True
@@ -52,7 +59,8 @@ class PolicyWithQs(object):
                              obs_scale=kwargs.get('obs_scale'), rew_scale=kwargs.get('rew_scale', 1.0),
                              rew_shift=kwargs.get('rew_shift', 0.0), gamma=kwargs.get('gamma', 0.99),
                              policy_out_activation=policy_out_activation, action_range=action_range,
-                             num_future_data=kwargs.get('num_future_data', 0), hidden=self.hidden, max_rows=max(rows, 64),
+                             num_future_data=kwargs.get('num_future_data', 0), hidden=self.hidden,
+                             hidden_activation=self.hidden_activation, max_rows=max(rows, 64),
                              max_horizon=max(lists + [1]), device=kwargs.get('device'), debug_lib=kwargs.get('debug_lib', False))
         # slot order == get_weights() order (policy.py:72-89)
         if policy_only:

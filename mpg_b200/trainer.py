@@ -1,6 +1,6 @@
 """Trainer (trainer.py:18-80) for the single-process topology: one worker, one replay buffer, one learner and one
 evaluator on one GPU, sharing ONE PolicyWithQs so that no weight ever crosses the host.
-    python -m mpg_b200.trainer --alg MPG-v2 --iters 2000 [--hidden 64|128|256]"""
+    python -m mpg_b200.trainer --alg MPG-v2 --iters 2000 [--hidden 64|128|256] [--activation elu|relu|tanh]"""
 import argparse
 import json
 import logging
@@ -47,6 +47,8 @@ def main():
     ap.add_argument('--iters', type=int, default=2000)
     ap.add_argument('--batch', type=int, default=256)
     ap.add_argument('--hidden', type=int, default=256, help='hidden units of the policy and Q nets: 64, 128 or 256')
+    ap.add_argument('--activation', default='elu', choices=('elu', 'relu', 'tanh'),
+                    help='hidden activation of the policy and Q nets')
     ap.add_argument('--log_dir', default=None)
     o = ap.parse_args()
     logging.basicConfig(level=logging.INFO)
@@ -54,7 +56,8 @@ def main():
                         max_buffer_size=500000, replay_starts=3000, buffer_log_interval=10 ** 9, num_eval_agent=64,
                         num_eval_episode=1, fixed_steps=100, eval_interval=max(o.iters // 10, 1), log_interval=100,
                         max_iter=o.iters, log_dir=o.log_dir, value_num_hidden_units=o.hidden,
-                        policy_num_hidden_units=o.hidden)
+                        policy_num_hidden_units=o.hidden, value_hidden_activation=o.activation,
+                        policy_hidden_activation=o.activation)
     import time
     trainer = Trainer(args)
     t0 = time.perf_counter()

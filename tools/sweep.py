@@ -5,6 +5,8 @@ Prints one JSON line per case (device time by CUDA events, 3 warm-ups, median of
     python tools/sweep.py > profiles/rNN_sweep.jsonl
 --hidden H (64, 128, 256; default 256) sets the width of the policy and Q nets; the lines of H != 256 carry `hidden`
 and `flop_per_state_step`.  The algorithmic FLOP per state-step at that width (SURVEY.md 8(a)) is printed to stderr.
+--activation (elu, relu, tanh; default elu) sets the hidden activation of the policy and Q nets; the lines of a
+non-default activation carry `activation`.
 --env / --mode / --rows / --backend restrict the sweep to the matching cases."""
 import argparse
 import json
@@ -35,9 +37,10 @@ def flop_per_state_step(mode, H, d_o, d_a, n=N):
     return total / n
 
 
-def run(env_id, mode, B, backend, H=256):
+def run(env_id, mode, B, backend, H=256, act='elu'):
     args = default_args('NADP' if mode == 'nadp' else 'MPG-v2', env_id, replay_batch_size=B,
-                        value_num_hidden_units=H, policy_num_hidden_units=H)
+                        value_num_hidden_units=H, policy_num_hidden_units=H,
+                        value_hidden_activation=act, policy_hidden_activation=act)
     pol = PolicyWithQs(**vars(args))
     pol.set_weights(synthetic.make_policy_with_qs_weights(1, args.obs_dim, args.act_dim, H, double_q=(mode != 'nadp')))
     e = pol.engine
@@ -62,12 +65,15 @@ def run(env_id, mode, B, backend, H=256):
     r = dict(env=env_id, mode=mode, rows=B, backend=backend, ms=ms, state_steps_per_s=B * N / (ms * 1e-3))
     if H != 256:
         r.update(hidden=H, flop_per_state_step=flop_per_state_step(mode, H, args.obs_dim, args.act_dim))
+    if act != 'elu':
+        r.update(activation=act)
     return r
 
 
 if __name__ == '__main__':
     ap = argparse.ArgumentParser()
     ap.add_argument('--hidden', type=int, default=256, choices=(64, 128, 256))
+    ap.add_argument('--activation', default='elu', choices=('elu', 'relu', 'tanh'))
     ap.add_argument('--env', default=None)
     ap.add_argument('--mode', default=None, choices=('nadp', 'mpg'))
     ap.add_argument('--rows', type=int, default=None)
@@ -91,7 +97,7 @@ if __name__ == '__main__':
                 continue  # full-BPTT dW2 operand store is 53 KB per row: call in <= 256K-row chunks
             if backend == 'ffma' and B > 262144:
                 continue
-            r = run(env, mode, B, backend, o.hidden)
+            r = run(env, mode, B, backend, o.hidden, o.activation)
             if r:
                 print(json.dumps(r), flush=True)
             torch.cuda.empty_cache()
