@@ -1,10 +1,8 @@
-// relu instantiations of the MLP kernels (see act_instances.cuh)
-#define MPG_ACT_UNIT
-#include "act_instances.cuh"
+// relu instantiations of the MLP kernels (mlp_kernels.cuh)
+#include "mlp_kernels.cuh"
 
 namespace mpg {
-MPG_ACT_INSTANCES(, MPG_ACT_RELU)
-bool wait_dbg_attach_relu(unsigned long long* dev_ptr) {
-  return cudaMemcpyToSymbol(tc::g_wait_dbg, &dev_ptr, sizeof(dev_ptr)) == cudaSuccess;
-}
+static constexpr MlpKernels relu64 = MlpLaunch<64, MPG_ACT_RELU>::table(), relu128 = MlpLaunch<128, MPG_ACT_RELU>::table(),
+                            relu256 = MlpLaunch<256, MPG_ACT_RELU>::table();
+const MlpKernels& relu_kernels(int hidden) { return hidden == 64 ? relu64 : hidden == 128 ? relu128 : relu256; }
 }  // namespace mpg

@@ -1,10 +1,8 @@
-// tanh instantiations of the MLP kernels (see act_instances.cuh)
-#define MPG_ACT_UNIT
-#include "act_instances.cuh"
+// tanh instantiations of the MLP kernels (mlp_kernels.cuh)
+#include "mlp_kernels.cuh"
 
 namespace mpg {
-MPG_ACT_INSTANCES(, MPG_ACT_TANH)
-bool wait_dbg_attach_tanh(unsigned long long* dev_ptr) {
-  return cudaMemcpyToSymbol(tc::g_wait_dbg, &dev_ptr, sizeof(dev_ptr)) == cudaSuccess;
-}
+static constexpr MlpKernels tanh64 = MlpLaunch<64, MPG_ACT_TANH>::table(), tanh128 = MlpLaunch<128, MPG_ACT_TANH>::table(),
+                            tanh256 = MlpLaunch<256, MPG_ACT_TANH>::table();
+const MlpKernels& tanh_kernels(int hidden) { return hidden == 64 ? tanh64 : hidden == 128 ? tanh128 : tanh256; }
 }  // namespace mpg

@@ -3,21 +3,14 @@
 #include <cstdlib>
 #include <cstring>
 #include <new>
-#include <type_traits>
 #include <vector>
 
-#include "rollout_kernels.cuh"
+#include "mlp_kernels.cuh"
+#include "model_kernels.cuh"
 #include "tc_rollout.cuh"
-#include "act_instances.cuh"
 #include "replay.cuh"
 
 using namespace mpg;
-
-// the relu and tanh kernels are compiled in act_relu.cu / act_tanh.cu
-namespace mpg {
-MPG_ACT_INSTANCES(extern, MPG_ACT_RELU)
-MPG_ACT_INSTANCES(extern, MPG_ACT_TANH)
-}  // namespace mpg
 
 namespace {
 
@@ -41,9 +34,10 @@ bool wait_dbg_init() {
   unsigned long long* h = nullptr; unsigned long long* d = nullptr;
   if (cudaHostAlloc((void**)&h, 256, cudaHostAllocMapped) != cudaSuccess) { cudaGetLastError(); return false; }
   memset(h, 0, 256);
-  if (cudaHostGetDevicePointer((void**)&d, h, 0) != cudaSuccess
-      || cudaMemcpyToSymbol(mpg::tc::g_wait_dbg, &d, sizeof(d)) != cudaSuccess || !mpg::wait_dbg_attach_relu(d)
-      || !mpg::wait_dbg_attach_tanh(d)) {
+  // this unit's copy (the dW kernel) and that of each activation's unit (the rollout kernels)
+  if (cudaHostGetDevicePointer((void**)&d, h, 0) != cudaSuccess || !tc::wait_dbg_attach(d)
+      || !mlp_kernels(tc::H, MPG_ACT_ELU).attach_watchdog(d) || !mlp_kernels(tc::H, MPG_ACT_RELU).attach_watchdog(d)
+      || !mlp_kernels(tc::H, MPG_ACT_TANH).attach_watchdog(d)) {
     cudaGetLastError(); cudaFreeHost(h); return false;
   }
   g_wait_host = h;
@@ -92,25 +86,6 @@ int fail(mpg_ctx* ctx, int code, const char* fmt, const char* detail = "") {
 
 // flat parameter layout of one net of this handle
 GradLayout layout(const mpg_ctx* c, const NetStore& n) { return GradLayout(n.in_dim, n.out_dim, c->cfg.hidden); }
-
-// The one place the handle's hidden width and activation become the template arguments of the FFMA kernels:
-// f(integral_constant<H>, integral_constant<ACT>).  mpg_create admits widths 64, 128 and 256 only, mpg_set_activation
-// the three MPG_ACT_* values.
-template <typename F>
-int with_mlp(const mpg_ctx* c, F&& f) {
-  auto with_act = [&](auto hc) {
-    switch (c->act) {
-      case MPG_ACT_RELU: return f(hc, std::integral_constant<int, MPG_ACT_RELU>());
-      case MPG_ACT_TANH: return f(hc, std::integral_constant<int, MPG_ACT_TANH>());
-      default: return f(hc, std::integral_constant<int, MPG_ACT_ELU>());
-    }
-  };
-  switch (c->cfg.hidden) {
-    case 64: return with_act(std::integral_constant<int, 64>());
-    case 128: return with_act(std::integral_constant<int, 128>());
-    default: return with_act(std::integral_constant<int, 256>());
-  }
-}
 
 NetDev net_dev(const mpg_ctx* c, int net) {
   const NetStore& n = c->nets[net];
@@ -259,12 +234,6 @@ __global__ void philox_noise_kernel(unsigned long long seed, long long global_ro
   out[idx] = philox_normal(seed, nr, (uint32_t)t);
 }
 
-template <int H, typename K>
-int set_smem(mpg_ctx* ctx, K kernel) {
-  CUDA_OK(ctx, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, Smem<H>::FLOATS * 4));
-  return MPG_OK;
-}
-
 int check_net(mpg_ctx* ctx, int net) {
   if (net < 0 || net >= MPG_NUM_NETS) return fail(ctx, MPG_ERR_ARG, "bad net id%s");
   if (!ctx->nets[net].set) return fail(ctx, MPG_ERR_STATE, "weights of a required net were never set%s");
@@ -322,23 +291,49 @@ int rec_hi_only(const mpg_ctx* ctx, long long contraction_rows) {
   return contraction_rows >= 262144 ? 1 : 0;
 }
 
+// grad_out = the sum of the first nparts partial gradients of net (and *loss_out = that of the partial losses, when given)
+void launch_reduce(const mpg_ctx* ctx, int net, int nparts, float* grad_out, float* loss_out, cudaStream_t st) {
+  const int n = layout(ctx, ctx->nets[net]).total;
+  reduce_partials_kernel<<<(n + 255) / 256, 256, 0, st>>>(ctx->partial, ctx->partial_stride, nparts, n, grad_out,
+                                                          ctx->loss_partial, loss_out);
+}
+
+// tensor-core rollout kernel of the handle's activation; cudaErrorNotSupported: there is none (backward on the real env)
+template <bool BWD>
+cudaError_t tc_launch_rollout(int env, int act, const tc::TcArgs& a, int grid, cudaStream_t st) {
+  if (!mlp_kernels(tc::H, act).tc_rollout(env, BWD, a, grid, st)) return cudaErrorNotSupported;
+  return cudaGetLastError();
+}
+
+// the arguments of the tensor-core rollout kernel that every launch shares: the rollout and the nets' weight images
+tc::TcArgs tc_args(const mpg_ctx* ctx, const RolloutArgs& a, int policy_net, int q_net) {
+  tc::TcArgs ta;
+  memset(&ta, 0, sizeof(ta));
+  ta.r = a;
+  ta.pol = tc_net(ctx->tc, policy_net, ctx->nets[policy_net].flat, a.pol.in_dim, a.pol.out_dim);
+  if (a.has_q) ta.q = tc_net(ctx->tc, q_net, ctx->nets[q_net].flat, a.q.in_dim, a.q.out_dim);
+  ta.act_ckpt = ctx->tc.act_ckpt;
+  return ta;
+}
+
+// weight gradient of the dW operand store records of tiles [tile0, tile0 + tiles) into the partial gradients from row
+// part_row on: tc_dw_kernel, two CTAs per record, at most the even number of the `sms` SMs it may use
+void launch_dw(const mpg_ctx* ctx, const tc::TcArgs& ta, int tile0, int tiles, int part_row, int sms, cudaStream_t st) {
+  tc::DwArgs da;
+  da.store = ctx->tc.store + (size_t)tile0 * ta.store_steps * tc::SLOT_BYTES;
+  da.nrecords = tiles * ta.store_steps;
+  da.in_dim = ta.pol.in_dim; da.out_dim = ta.pol.out_dim;
+  da.partial = ctx->partial + (size_t)part_row * ctx->partial_stride; da.partial_stride = (long long)ctx->partial_stride;
+  da.hi_only = ta.rec_hi_only;
+  const int grid = 2 * da.nrecords < sms ? 2 * da.nrecords : (sms & ~1);
+  tc::tc_dw_kernel<<<grid, tc::DW_THREADS, tc::DW_SMEM, st>>>(da);
+}
+
 template <bool BWD>
 int launch_rollout(mpg_ctx* ctx, const RolloutArgs& a, int grid, cudaStream_t st, int env) {
-  if (BWD && env == MPG_ENV_PATH_TRACKING_REAL) return fail(ctx, MPG_ERR_UNSUPPORTED, "the real environment is forward only%s");
   if (ctx->timing) cudaEventRecord(ctx->ev0, st);
-  with_mlp(ctx, [&](auto hc, auto ac) {
-    constexpr int HW = decltype(hc)::value, ACT = decltype(ac)::value;
-    const size_t smem = Smem<HW>::FLOATS * 4;
-    if (env == MPG_ENV_PATH_TRACKING_REAL) {
-      rollout_kernel<HW, ACT, MPG_ENV_PATH_TRACKING_REAL, false><<<grid, NT, smem, st>>>(a);
-    } else
-    switch (env) {
-      case MPG_ENV_PATH_TRACKING: rollout_kernel<HW, ACT, MPG_ENV_PATH_TRACKING, BWD><<<grid, NT, smem, st>>>(a); break;
-      case MPG_ENV_INVERTED_PENDULUM: rollout_kernel<HW, ACT, MPG_ENV_INVERTED_PENDULUM, BWD><<<grid, NT, smem, st>>>(a); break;
-      default: rollout_kernel<HW, ACT, MPG_ENV_INVERTED_DOUBLE_PENDULUM, BWD><<<grid, NT, smem, st>>>(a); break;
-    }
-    return MPG_OK;
-  });
+  if (!mlp_kernels(ctx->cfg.hidden, ctx->act).rollout(env, BWD, a, grid, st))
+    return fail(ctx, MPG_ERR_UNSUPPORTED, "the real environment is forward only%s");
   if (ctx->timing) { cudaEventRecord(ctx->ev1, st); ctx->timed = 1; }
   ctx->launches++;
   CUDA_OK(ctx, cudaGetLastError());
@@ -474,28 +469,11 @@ int mpg_create(const mpg_config* cfg, mpg_ctx** out) {
     mpg_destroy(c);
     return MPG_ERR_CUDA;
   }
-  int rc = 0;
-  for (const int act : {MPG_ACT_ELU, MPG_ACT_RELU, MPG_ACT_TANH}) {   // the instantiations this handle may launch
-    c->act = act;
-    rc |= with_mlp(c, [&](auto hc, auto ac) {
-      constexpr int HW = decltype(hc)::value, ACT = decltype(ac)::value;
-      int r = 0;
-      r |= set_smem<HW>(c, rollout_kernel<HW, ACT, MPG_ENV_PATH_TRACKING, true>);
-      r |= set_smem<HW>(c, rollout_kernel<HW, ACT, MPG_ENV_PATH_TRACKING, false>);
-      r |= set_smem<HW>(c, rollout_kernel<HW, ACT, MPG_ENV_INVERTED_PENDULUM, true>);
-      r |= set_smem<HW>(c, rollout_kernel<HW, ACT, MPG_ENV_INVERTED_PENDULUM, false>);
-      r |= set_smem<HW>(c, rollout_kernel<HW, ACT, MPG_ENV_INVERTED_DOUBLE_PENDULUM, true>);
-      r |= set_smem<HW>(c, rollout_kernel<HW, ACT, MPG_ENV_INVERTED_DOUBLE_PENDULUM, false>);
-      r |= set_smem<HW>(c, rollout_kernel<HW, ACT, MPG_ENV_PATH_TRACKING_REAL, false>);
-      r |= set_smem<HW>(c, q_grad_kernel<HW, ACT>);
-      r |= set_smem<HW>(c, eval_kernel<HW, ACT>);
-      r |= set_smem<HW>(c, env_sample_kernel<HW, ACT>);
-      return r;
-    });
-  }
-  c->act = MPG_ACT_ELU;
-  if (rc) {
-    strncpy(g_create_err, c->err, 512);
+  cudaError_t e = cudaSuccess;
+  for (const int act : {MPG_ACT_ELU, MPG_ACT_RELU, MPG_ACT_TANH})   // the activation can change on the handle later
+    if (e == cudaSuccess) e = mlp_kernels(cfg->hidden, act).set_smem();
+  if (e != cudaSuccess) {
+    snprintf(g_create_err, 512, "cudaFuncSetAttribute (max dynamic shared memory of the MLP kernels): %s", cudaGetErrorString(e));
     mpg_destroy(c);
     return MPG_ERR_CUDA;
   }
@@ -533,11 +511,12 @@ void mpg_destroy(mpg_ctx* c) {
 
 // FFMA weight images (W1p, W2p, W2Tp) of one net from its flat natural weights
 static void launch_pack(mpg_ctx* ctx, const NetStore& ns, cudaStream_t st) {
-  with_mlp(ctx, [&](auto hc, auto) {   // the packing does not depend on the activation
-    constexpr int HW = decltype(hc)::value;
-    pack_kernel<HW><<<(HW * HW + 255) / 256, 256, 0, st>>>(ns.flat, ns.in_dim, ns.out_dim, ns.W1p, ns.W2p, ns.W2Tp);
-    return MPG_OK;
-  });
+  const int hw = ctx->cfg.hidden, grid = (hw * hw + 255) / 256;   // mpg_create admits 64, 128 and 256
+  switch (hw) {
+    case 64: pack_kernel<64><<<grid, 256, 0, st>>>(ns.flat, ns.in_dim, ns.out_dim, ns.W1p, ns.W2p, ns.W2Tp); break;
+    case 128: pack_kernel<128><<<grid, 256, 0, st>>>(ns.flat, ns.in_dim, ns.out_dim, ns.W1p, ns.W2p, ns.W2Tp); break;
+    default: pack_kernel<256><<<grid, 256, 0, st>>>(ns.flat, ns.in_dim, ns.out_dim, ns.W1p, ns.W2p, ns.W2Tp); break;
+  }
   ctx->launches++;
 }
 
@@ -659,17 +638,11 @@ int mpg_policy_grad(mpg_ctx* ctx, const mpg_rollout_params* p, const float* obs,
   a.obs = obs; a.noise = noise; a.returns_out = returns_out;
   a.noise_mode = noise ? 1 : (p->use_philox ? 2 : 0);
   const int MB = p->rows * p->M;
-  const GradLayout L = layout(ctx, ctx->nets[p->policy_net]);
   if (ctx->backend == MPG_BACKEND_TC) {
     // tensor-core path: fused rollout + BPTT (dX chain), then the split-K weight-gradient GEMMs
     const int ntiles = (MB + tc::ACT_ROWS - 1) / tc::ACT_ROWS;
     const int grid = ntiles < ctx->sms ? ntiles : ctx->sms;
-    tc::TcArgs ta;
-    memset(&ta, 0, sizeof(ta));
-    ta.r = a;
-    ta.pol = tc_net(ctx->tc, p->policy_net, ctx->nets[p->policy_net].flat, a.pol.in_dim, a.pol.out_dim);
-    if (a.has_q) ta.q = tc_net(ctx->tc, p->q_net, ctx->nets[p->q_net].flat, a.q.in_dim, a.q.out_dim);
-    ta.act_ckpt = ctx->tc.act_ckpt;
+    tc::TcArgs ta = tc_args(ctx, a, p->policy_net, p->q_net);
     ta.store_steps = p->full_bptt ? p->horizon + 1 : 1;
     const size_t need = (size_t)ntiles * ta.store_steps * tc::SLOT_BYTES;
     if (!tc_ensure_store(ctx->tc, need)) return fail(ctx, MPG_ERR_CUDA, "cudaMalloc of the dW operand store failed%s");
@@ -680,16 +653,6 @@ int mpg_policy_grad(mpg_ctx* ctx, const mpg_rollout_params* p, const float* obs,
     ta.h2store = ctx->tc.h2store;
     ta.z_ckpt = ctx->tc.z_ckpt;
     ta.prof = ctx->prof;
-    const size_t dw_smem = tc::DW_SMEM;
-    auto dw_args = [&](int tile0, int tiles, int part_row) {
-      tc::DwArgs da;
-      da.store = ctx->tc.store + (size_t)tile0 * ta.store_steps * tc::SLOT_BYTES;
-      da.nrecords = tiles * ta.store_steps;
-      da.in_dim = a.pol.in_dim; da.out_dim = a.pol.out_dim;
-      da.partial = ctx->partial + (size_t)part_row * ctx->partial_stride; da.partial_stride = (long long)ctx->partial_stride;
-      da.hi_only = ta.rec_hi_only;
-      return da;
-    };
     // Wave-tail overlap: with ntiles = w * sms + tail the last wave leaves sms - tail SMs idle.  The full waves and
     // the tail wave are two launches; the weight-gradient GEMMs of the full waves (HBM-bound) run on the side
     // stream on exactly the SMs the tail wave does not use.  Partial rows [0, sms): full waves, [sms, 2 sms): tail.
@@ -704,11 +667,8 @@ int mpg_policy_grad(mpg_ctx* ctx, const mpg_rollout_params* p, const float* obs,
     if (!split) {
       CUDA_OK(ctx, tc_launch_rollout<true>(ctx->cfg.env, ctx->act, ta, grid, st));
       if (ctx->timing) { cudaEventRecord(ctx->ev1, st); ctx->timed = 1; }
-      tc::DwArgs da = dw_args(0, ntiles, 0);
-      int dgrid = 2 * da.nrecords < ctx->sms ? 2 * da.nrecords : (ctx->sms & ~1);
-      tc::tc_dw_kernel<<<dgrid, tc::DW_THREADS, dw_smem, st>>>(da);
-      reduce_partials_kernel<<<(L.total + 255) / 256, 256, 0, st>>>(ctx->partial, ctx->partial_stride, ctx->sms, L.total,
-                                                                    grad_out, nullptr, nullptr);
+      launch_dw(ctx, ta, 0, ntiles, 0, ctx->sms, st);
+      launch_reduce(ctx, p->policy_net, ctx->sms, grad_out, nullptr, st);
       ctx->launches += 3;
     } else {
       ta.tile0 = 0; ta.tile1 = full;
@@ -720,14 +680,11 @@ int mpg_policy_grad(mpg_ctx* ctx, const mpg_rollout_params* p, const float* obs,
       CUDA_OK(ctx, tc_launch_rollout<true>(ctx->cfg.env, ctx->act, tb, tail, st));
       if (ctx->timing) { cudaEventRecord(ctx->ev1, st); ctx->timed = 1; }
       CUDA_OK(ctx, cudaStreamWaitEvent(ctx->aux, ctx->ev_wave, 0));
-      tc::tc_dw_kernel<<<(ctx->sms - tail) & ~1, tc::DW_THREADS, dw_smem, ctx->aux>>>(dw_args(0, full, 0));
+      launch_dw(ctx, ta, 0, full, 0, ctx->sms - tail, ctx->aux);   // full waves: >= sms records, all of the idle SMs
       CUDA_OK(ctx, cudaEventRecord(ctx->ev_aux, ctx->aux));
-      tc::DwArgs db = dw_args(full, tail, ctx->sms);
-      int dgrid = 2 * db.nrecords < ctx->sms ? 2 * db.nrecords : (ctx->sms & ~1);
-      tc::tc_dw_kernel<<<dgrid, tc::DW_THREADS, dw_smem, st>>>(db);
+      launch_dw(ctx, ta, full, tail, ctx->sms, ctx->sms, st);
       CUDA_OK(ctx, cudaStreamWaitEvent(st, ctx->ev_aux, 0));
-      reduce_partials_kernel<<<(L.total + 255) / 256, 256, 0, st>>>(ctx->partial, ctx->partial_stride, 2 * ctx->sms, L.total,
-                                                                    grad_out, nullptr, nullptr);
+      launch_reduce(ctx, p->policy_net, 2 * ctx->sms, grad_out, nullptr, st);
       ctx->launches += 5;
     }
     CUDA_OK(ctx, cudaGetLastError());
@@ -738,8 +695,7 @@ int mpg_policy_grad(mpg_ctx* ctx, const mpg_rollout_params* p, const float* obs,
   CUDA_OK(ctx, cudaMemsetAsync(ctx->partial, 0, (size_t)grid * ctx->partial_stride * sizeof(float), st));
   rc = launch_rollout<true>(ctx, a, grid, st, ctx->cfg.env);
   if (rc) return rc;
-  reduce_partials_kernel<<<(L.total + 255) / 256, 256, 0, st>>>(ctx->partial, ctx->partial_stride, grid, L.total,
-                                                                grad_out, nullptr, nullptr);
+  launch_reduce(ctx, p->policy_net, grid, grad_out, nullptr, st);
   ctx->launches++;
   CUDA_OK(ctx, cudaGetLastError());
   return MPG_OK;
@@ -767,12 +723,7 @@ int mpg_rollout_forward(mpg_ctx* ctx, const mpg_rollout_params* p, const float* 
   if (ctx->backend == MPG_BACKEND_TC) {
     const int ntiles = (MB + tc::ACT_ROWS - 1) / tc::ACT_ROWS;
     const int grid = ntiles < ctx->sms ? ntiles : ctx->sms;
-    tc::TcArgs ta;
-    memset(&ta, 0, sizeof(ta));
-    ta.r = a;
-    ta.pol = tc_net(ctx->tc, p->policy_net, ctx->nets[p->policy_net].flat, a.pol.in_dim, a.pol.out_dim);
-    if (a.has_q) ta.q = tc_net(ctx->tc, p->q_net, ctx->nets[p->q_net].flat, a.q.in_dim, a.q.out_dim);
-    ta.act_ckpt = ctx->tc.act_ckpt;
+    const tc::TcArgs ta = tc_args(ctx, a, p->policy_net, p->q_net);
     if (ctx->timing) cudaEventRecord(ctx->ev0, st);
     CUDA_OK(ctx, tc_launch_rollout<false>(env, ctx->act, ta, grid, st));
     if (ctx->timing) { cudaEventRecord(ctx->ev1, st); ctx->timed = 1; }
@@ -811,23 +762,17 @@ int mpg_q_grad(mpg_ctx* ctx, int net, int rows, int64_t global_rows, const float
   if (ctx->backend == MPG_BACKEND_TC && rows <= ctx->cfg.max_rows) {
     // tensor-core path: the rollout kernel in regression mode (horizon 0, given actions) + the dW kernel
     const mpg_config& c = ctx->cfg;
-    const int qin = c.obs_dim + c.act_dim;
-    tc::TcArgs ta;
-    memset(&ta, 0, sizeof(ta));
-    RolloutArgs& r = ta.r;
-    r.obs_dim = c.obs_dim; r.act_dim = c.act_dim; r.nfd = c.num_future_data; r.policy_out_tanh = c.policy_out_tanh;
-    r.action_range = c.action_range;
-    for (int i = 0; i < MPG_MAX_OBS; ++i) r.obs_scale[i] = c.obs_scale[i];
-    r.rew_scale = c.rew_scale; r.rew_shift = c.rew_shift; r.gamma = c.gamma;
-    r.rows = rows; r.M = 1; r.horizon = 0; r.n_list = 1; r.list[0] = 0; r.list_w[0] = 1.f;
-    r.full_bptt = 1; r.has_q = 1; r.use_start_actions = 1; r.noise_mode = 0;
-    r.global_rows = global_rows > 0 ? global_rows : rows;
-    r.obs = obs; r.start_actions = act; r.returns_out = ctx->tc.qtmp; r.ckpt = ctx->ckpt;
-    r.partial = ctx->partial; r.partial_stride = (long long)ctx->partial_stride;
-    ta.q = tc_net(ctx->tc, net, ctx->nets[net].flat, qin, 1);
-    ta.pol = ta.q;   // unused in regression mode (actions are given, the policy part is skipped); fixes the gradient layout
-    ta.act_ckpt = ctx->tc.act_ckpt;
-    ta.q_regress = 1; ta.q_target = target; ta.q_inv_rows = 1.f / (float)r.global_rows;
+    mpg_rollout_params p;
+    memset(&p, 0, sizeof(p));
+    p.rows = rows; p.M = 1; p.horizon = 0; p.n_list = 1; p.list[0] = 0; p.list_w[0] = 1.f; p.full_bptt = 1;
+    p.global_rows = global_rows;
+    p.q_net = net;
+    p.policy_net = net;   // unused in regression mode (actions are given, the policy part is skipped); fixes the gradient layout
+    RolloutArgs a;
+    if ((rc = fill_rollout_args(ctx, &p, a))) return rc;
+    a.use_start_actions = 1; a.start_actions = act; a.obs = obs; a.returns_out = ctx->tc.qtmp;
+    tc::TcArgs ta = tc_args(ctx, a, net, net);
+    ta.q_regress = 1; ta.q_target = target; ta.q_inv_rows = 1.f / (float)a.global_rows;
     const int ntiles = (rows + tc::ACT_ROWS - 1) / tc::ACT_ROWS;
     const int grid = ntiles < ctx->sms ? ntiles : ctx->sms;
     ta.store_steps = 1;
@@ -839,16 +784,8 @@ int mpg_q_grad(mpg_ctx* ctx, int net, int rows, int64_t global_rows, const float
     ta.rec_hi_only = 0;
     CUDA_OK(ctx, cudaMemsetAsync(ctx->partial, 0, (size_t)ctx->sms * ctx->partial_stride * sizeof(float), st));
     CUDA_OK(ctx, tc_launch_rollout<true>(c.env, ctx->act, ta, grid, st));
-    tc::DwArgs da;
-    da.store = ctx->tc.store; da.nrecords = ntiles;
-    da.in_dim = qin; da.out_dim = 1;
-    da.partial = ctx->partial; da.partial_stride = (long long)ctx->partial_stride;
-    da.hi_only = ta.rec_hi_only;
-    const int dgrid = 2 * da.nrecords < ctx->sms ? 2 * da.nrecords : (ctx->sms & ~1);
-    tc::tc_dw_kernel<<<dgrid, tc::DW_THREADS, tc::DW_SMEM, st>>>(da);
-    const GradLayout L(qin, 1, tc::H);
-    reduce_partials_kernel<<<(L.total + 255) / 256, 256, 0, st>>>(ctx->partial, ctx->partial_stride, ctx->sms, L.total,
-                                                                  grad_out, nullptr, nullptr);
+    launch_dw(ctx, ta, 0, ntiles, 0, ctx->sms, st);
+    launch_reduce(ctx, net, ctx->sms, grad_out, nullptr, st);
     if (loss_sum_out) {
       sq_err_partial_kernel<<<64, 256, 0, st>>>(ctx->tc.qtmp, target, rows, ctx->red_part);
       sum_partials64_kernel<<<1, 1, 0, st>>>(ctx->red_part, loss_sum_out);
@@ -867,15 +804,9 @@ int mpg_q_grad(mpg_ctx* ctx, int net, int rows, int64_t global_rows, const float
   a.q = net_dev(ctx, net);
   const int ntiles = (rows + TILE_R - 1) / TILE_R;
   const int grid = ntiles < ctx->sms ? ntiles : ctx->sms;
-  const GradLayout L = layout(ctx, ctx->nets[net]);
   CUDA_OK(ctx, cudaMemsetAsync(ctx->partial, 0, (size_t)grid * ctx->partial_stride * sizeof(float), st));
-  with_mlp(ctx, [&](auto hc, auto ac) {
-    constexpr int HW = decltype(hc)::value, ACT = decltype(ac)::value;
-    q_grad_kernel<HW, ACT><<<grid, NT, Smem<HW>::FLOATS * 4, st>>>(a);
-    return MPG_OK;
-  });
-  reduce_partials_kernel<<<(L.total + 255) / 256, 256, 0, st>>>(ctx->partial, ctx->partial_stride, grid, L.total,
-                                                                grad_out, ctx->loss_partial, loss_sum_out);
+  mlp_kernels(ctx->cfg.hidden, ctx->act).q_grad(a, grid, st);
+  launch_reduce(ctx, net, grid, grad_out, loss_sum_out, st);
   ctx->launches += 2;
   CUDA_OK(ctx, cudaGetLastError());
   return MPG_OK;
@@ -889,11 +820,7 @@ static int launch_eval(mpg_ctx* ctx, EvalArgs& a, void* stream) {
   for (int i = 0; i < MPG_MAX_OBS; ++i) a.obs_scale[i] = c.obs_scale[i];
   const int ntiles = (a.rows + TILE_R - 1) / TILE_R;
   const int grid = ntiles < ctx->sms ? ntiles : ctx->sms;
-  with_mlp(ctx, [&](auto hc, auto ac) {
-    constexpr int HW = decltype(hc)::value, ACT = decltype(ac)::value;
-    eval_kernel<HW, ACT><<<grid, NT, Smem<HW>::FLOATS * 4, (cudaStream_t)stream>>>(a);
-    return MPG_OK;
-  });
+  mlp_kernels(c.hidden, ctx->act).eval(a, grid, (cudaStream_t)stream);
   ctx->launches++;
   CUDA_OK(ctx, cudaGetLastError());
   return MPG_OK;
@@ -1023,18 +950,12 @@ int mpg_td_error(mpg_ctx* ctx, int rows, const float* obs, const float* act, con
   return launch_eval(ctx, a, stream);
 }
 
-#define ENV_SWITCH(ctx, CALL)                                             \
-  switch ((ctx)->cfg.env) {                                               \
-    case MPG_ENV_PATH_TRACKING: { constexpr int EV = MPG_ENV_PATH_TRACKING; CALL; } break; \
-    case MPG_ENV_INVERTED_PENDULUM: { constexpr int EV = MPG_ENV_INVERTED_PENDULUM; CALL; } break; \
-    case MPG_ENV_PATH_TRACKING_REAL: { constexpr int EV = MPG_ENV_PATH_TRACKING_REAL; CALL; } break; \
-    default: { constexpr int EV = MPG_ENV_INVERTED_DOUBLE_PENDULUM; CALL; } break; \
-  }
-
 int mpg_model_reset(mpg_ctx* ctx, int rows, const float* obs, float* state_out, void* stream) {
   if (!ctx || !obs || !state_out || rows <= 0) return fail(ctx, MPG_ERR_ARG, "bad argument to mpg_model_reset%s");
   cudaStream_t st = (cudaStream_t)stream;
-  ENV_SWITCH(ctx, (model_reset_kernel<EV><<<(rows + 127) / 128, 128, 0, st>>>(rows, ctx->cfg.obs_dim, obs, state_out)));
+  with_env(ctx->cfg.env, false, [&](auto env, auto) {
+    model_reset_kernel<decltype(env)::value><<<(rows + 127) / 128, 128, 0, st>>>(rows, ctx->cfg.obs_dim, obs, state_out);
+  });
   ctx->launches++;
   CUDA_OK(ctx, cudaGetLastError());
   return MPG_OK;
@@ -1044,8 +965,10 @@ int mpg_model_step(mpg_ctx* ctx, int rows, const float* state_in, const float* a
                    float* state_out, float* obs_out, float* rew_out, void* stream) {
   if (!ctx || !state_in || !action || !state_out || rows <= 0) return fail(ctx, MPG_ERR_ARG, "bad argument to mpg_model_step%s");
   cudaStream_t st = (cudaStream_t)stream;
-  ENV_SWITCH(ctx, (model_step_kernel<EV><<<(rows + 127) / 128, 128, 0, st>>>(
-                      rows, ctx->cfg.obs_dim, ctx->cfg.num_future_data, state_in, action, eps, state_out, obs_out, rew_out)));
+  with_env(ctx->cfg.env, false, [&](auto env, auto) {
+    model_step_kernel<decltype(env)::value><<<(rows + 127) / 128, 128, 0, st>>>(
+        rows, ctx->cfg.obs_dim, ctx->cfg.num_future_data, state_in, action, eps, state_out, obs_out, rew_out);
+  });
   ctx->launches++;
   CUDA_OK(ctx, cudaGetLastError());
   return MPG_OK;
@@ -1056,11 +979,13 @@ int mpg_model_step_bwd(mpg_ctx* ctx, int rows, const float* state_in, const floa
                        float* g_action, void* stream) {
   if (!ctx || !state_in || !action || !g_state_in || !g_action || rows <= 0)
     return fail(ctx, MPG_ERR_ARG, "bad argument to mpg_model_step_bwd%s");
-  if (ctx->cfg.env == MPG_ENV_PATH_TRACKING_REAL) return fail(ctx, MPG_ERR_UNSUPPORTED, "the real environment is forward only%s");
   cudaStream_t st = (cudaStream_t)stream;
-  ENV_SWITCH(ctx, (model_step_bwd_kernel<EV><<<(rows + 127) / 128, 128, 0, st>>>(
-                      rows, ctx->cfg.obs_dim, ctx->cfg.num_future_data, state_in, action, eps, g_obs_out, g_rew_out,
-                      g_state_out, g_state_in, g_action)));
+  if (!with_env(ctx->cfg.env, true, [&](auto env, auto) {
+        model_step_bwd_kernel<decltype(env)::value><<<(rows + 127) / 128, 128, 0, st>>>(
+            rows, ctx->cfg.obs_dim, ctx->cfg.num_future_data, state_in, action, eps, g_obs_out, g_rew_out, g_state_out,
+            g_state_in, g_action);
+      }))
+    return fail(ctx, MPG_ERR_UNSUPPORTED, "the real environment is forward only%s");
   ctx->launches++;
   CUDA_OK(ctx, cudaGetLastError());
   return MPG_OK;
@@ -1096,11 +1021,7 @@ int mpg_env_sample(mpg_ctx* ctx, int policy_net, int agents, int steps, float ex
   a.explore_noise = explore_noise; a.reset_obs = reset_obs; a.state = state; a.obs = obs;
   a.out_obs = out_obs; a.out_act = out_act; a.out_rew = out_rew; a.out_obs_tp1 = out_obs_tp1; a.out_done = out_done;
   a.net = net_dev(ctx, policy_net);
-  with_mlp(ctx, [&](auto hc, auto ac) {
-    constexpr int HW = decltype(hc)::value, ACT = decltype(ac)::value;
-    env_sample_kernel<HW, ACT><<<(agents + TILE_R - 1) / TILE_R, NT, Smem<HW>::FLOATS * 4, (cudaStream_t)stream>>>(a);
-    return MPG_OK;
-  });
+  mlp_kernels(ctx->cfg.hidden, ctx->act).env_sample(a, (agents + TILE_R - 1) / TILE_R, (cudaStream_t)stream);
   ctx->launches++;
   CUDA_OK(ctx, cudaGetLastError());
   return MPG_OK;
@@ -1112,7 +1033,9 @@ int mpg_compute_rewards(mpg_ctx* ctx, int rows, const float* state, const float*
   if ((ctx->cfg.env == MPG_ENV_PATH_TRACKING || ctx->cfg.env == MPG_ENV_PATH_TRACKING_REAL) && !scaled_action)
     return fail(ctx, MPG_ERR_ARG, "PathTracking rewards need actions%s");
   cudaStream_t st = (cudaStream_t)stream;
-  ENV_SWITCH(ctx, (rewards_kernel<EV><<<(rows + 127) / 128, 128, 0, st>>>(rows, state, scaled_action, rew_out)));
+  with_env(ctx->cfg.env, false, [&](auto env, auto) {
+    rewards_kernel<decltype(env)::value><<<(rows + 127) / 128, 128, 0, st>>>(rows, state, scaled_action, rew_out);
+  });
   ctx->launches++;
   CUDA_OK(ctx, cudaGetLastError());
   return MPG_OK;

@@ -4,6 +4,8 @@
 //   InvertedDoublePendulum envs_and_models/inverted_double_pendulum_model.py:14-53,89-144
 // Adjoint derivations: SURVEY.md 8(a) "Adjoint the kernel must implement" + Appendix A.
 #pragma once
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace mpg {
@@ -428,6 +430,34 @@ __device__ __forceinline__ void env_step_bwd(const float* s, const float* act, c
   else if constexpr (ENV == MPG_ENV_PT_REAL) { }   // the real environment is never differentiated
   else if constexpr (ENV == MPG_ENV_INVERTED_PENDULUM) Env<ENV>::template step_bwd<FAST>(s, act, lam, rc, gs, ga, s1);
   else Env<ENV>::step_bwd(s, act, lam, rc, gs, ga, s1);
+}
+
+// The one place a runtime environment id (MPG_ENV_*) and backward flag become the template arguments of a kernel: calls
+// f(integral_constant<int, ENV>, integral_constant<bool, BWD>) and returns true.  The real environment is forward only: with
+// bwd set it has no kernel, and with_env calls nothing and returns false.
+template <typename F>
+bool with_env(int env, bool bwd, F&& f) {
+  auto fwd_or_bwd = [&](auto e) {
+    if (bwd) f(e, std::true_type()); else f(e, std::false_type());
+    return true;
+  };
+  switch (env) {
+    case MPG_ENV_PATH_TRACKING: return fwd_or_bwd(std::integral_constant<int, MPG_ENV_PATH_TRACKING>());
+    case MPG_ENV_INVERTED_PENDULUM: return fwd_or_bwd(std::integral_constant<int, MPG_ENV_INVERTED_PENDULUM>());
+    case MPG_ENV_PATH_TRACKING_REAL:
+      if (bwd) return false;
+      f(std::integral_constant<int, MPG_ENV_PATH_TRACKING_REAL>(), std::false_type());
+      return true;
+    default: return fwd_or_bwd(std::integral_constant<int, MPG_ENV_INVERTED_DOUBLE_PENDULUM>());
+  }
+}
+// f(ENV, BWD) for every variant with_env selects
+template <typename F>
+void for_each_env(F&& f) {
+  for (int env = MPG_ENV_PATH_TRACKING; env <= MPG_ENV_PATH_TRACKING_REAL; ++env) {
+    with_env(env, false, f);
+    with_env(env, true, f);
+  }
 }
 
 }  // namespace mpg

@@ -47,17 +47,16 @@ __device__ __forceinline__ bool mbar_try(uint64_t* bar, uint32_t parity) {
 // Watchdog of the mbarrier waits: a protocol error must not hang the GPU.  g_wait_dbg points to pinned, mapped host
 // memory (set once per process by the library); a wait that does not complete within MPG_WAIT_LIMIT_CYCLES records
 // {site (source line), block, thread, parity} there and traps, so that the launch fails with an error the host can report.
-// The relu / tanh translation units keep their own copies of the record pointer and of mbar_timeout (act_instances.cuh).
-#ifdef MPG_ACT_UNIT
-#define MPG_UNIT_LOCAL static
-#else
-#define MPG_UNIT_LOCAL
-#endif
-MPG_UNIT_LOCAL __device__ unsigned long long* g_wait_dbg = nullptr;
+// Every translation unit has its own copy of the record pointer and of mbar_timeout: the library attaches each unit's
+// copy with wait_dbg_attach (api.cu: wait_dbg_init, MlpKernels::attach_watchdog).
+static __device__ unsigned long long* g_wait_dbg = nullptr;
 #ifndef MPG_WAIT_LIMIT_CYCLES
 #define MPG_WAIT_LIMIT_CYCLES 4000000000ll    /* ~2 s at 1.965 GHz; the longest legitimate wait is a few hundred microseconds */
 #endif
-MPG_UNIT_LOCAL __device__ __noinline__ void mbar_timeout(int site, uint32_t parity) {
+static inline bool wait_dbg_attach(unsigned long long* dev_ptr) {
+  return cudaMemcpyToSymbol(g_wait_dbg, &dev_ptr, sizeof(dev_ptr)) == cudaSuccess;
+}
+static __device__ __noinline__ void mbar_timeout(int site, uint32_t parity) {
   if (g_wait_dbg) {
     // records {site, block, thread, parity} at g_wait_dbg[4 + 4 k], k = warpgroup of the thread (0..3 epilogue, 4 row warps,
     // 5/6 producer / mma warp), g_wait_dbg[0] = flag.  The first thread to give up lingers a little before it traps, so that

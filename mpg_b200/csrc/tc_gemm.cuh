@@ -472,155 +472,5 @@ __device__ __forceinline__ void cta_teardown(Bars* b, int mma_warp = EPI_WARPS +
   if ((threadIdx.x >> 5) == mma_warp) tmem_dealloc(b->tmem_base, TMEM_COLS);
 }
 
-// ---- global weight-image packing (run once per set_weights) ------------------------------------------------
-// big image: value(row, k) = src[row * rs + k * cs], 256 rows x 256 k -> 16 stages (kb, split, kh) of 256 rows x 64 B,
-// SW64 K-major (8-row groups of 512 B, 16-byte chunk index ^ ((row >> 1) & 3))
-template <bool F16>
-__global__ void pack_big_image(const float* __restrict__ src, int rs, int cs, uint8_t* __restrict__ img) {
-  const int idx = blockIdx.x * blockDim.x + threadIdx.x;   // one thread per (row, 8-element chunk): 256 x 32
-  if (idx >= 256 * 32) return;
-  const int row = idx >> 5, cc = idx & 31;
-  float x[8];
-#pragma unroll
-  for (int e = 0; e < 8; ++e) x[e] = src[(size_t)row * rs + (size_t)(cc * 8 + e) * cs];
-  uint4 h, l;
-  split2x<F16>(x[0], x[1], h.x, l.x); split2x<F16>(x[2], x[3], h.y, l.y); split2x<F16>(x[4], x[5], h.z, l.z); split2x<F16>(x[6], x[7], h.w, l.w);
-  const int kb = cc >> 3, kh = (cc >> 2) & 1, c = cc & 3;
-  const size_t stage = (size_t)(kb * 4 + kh) * STAGE_BYTES;   // streamed in (k-block, split, k-half) order
-  const uint32_t off = (row >> 3) * 512 + (row & 7) * 64 + ((c ^ ((row >> 1) & 3)) << 4);
-  *reinterpret_cast<uint4*>(img + stage + off) = h;
-  *reinterpret_cast<uint4*>(img + stage + 2 * STAGE_BYTES + off) = l;
-}
-// first-layer image: value(n, k) = scale * (k < in_dim ? W1[k][n] : (k == bias_k ? b1[n] : 0)); 256 rows x 16 k,
-// (scale = log2(e) for the bf16 image of the BPTT recompute, whose z1 only feeds act'(z1), e.g. elu'(z1) = 2^(min(z1, 0) log2 e))
-// INTERLEAVE K-major: [hi 8 KB | lo 8 KB]
-template <bool F16>
-__global__ void pack_l1_image(const float* __restrict__ W1, const float* __restrict__ b1, int in_dim, int bias_k,
-                              uint8_t* __restrict__ img, float scale = 1.f) {
-  const int idx = blockIdx.x * blockDim.x + threadIdx.x;   // (n, k-half): 256 x 2
-  if (idx >= 512) return;
-  const int n = idx >> 1, kh = idx & 1;
-  float x[8];
-#pragma unroll
-  for (int e = 0; e < 8; ++e) {
-    const int k = kh * 8 + e;
-    x[e] = scale * (k < in_dim ? W1[(size_t)k * H + n] : (k == bias_k ? b1[n] : 0.f));
-  }
-  uint4 h, l;
-  split2x<F16>(x[0], x[1], h.x, l.x); split2x<F16>(x[2], x[3], h.y, l.y); split2x<F16>(x[4], x[5], h.z, l.z); split2x<F16>(x[6], x[7], h.w, l.w);
-  const uint32_t off = il_chunk_off(n, kh);
-  *reinterpret_cast<uint4*>(img + off) = h;
-  *reinterpret_cast<uint4*>(img + 8192 + off) = l;
-}
-#ifndef MPG_ACT_UNIT   // non-template kernels are defined in api.cu's unit only (act_instances.cuh)
-// input-gradient image: value(i, n) = i < in_dim ? W1[i][n] : 0; per 64-k block 32 rows (hi of rows 0..15, then lo of rows
-// 0..15) x 128 B, SW128 K-major: 4 x 4 KB
-__global__ void pack_in_image(const float* __restrict__ W1, int in_dim, uint8_t* __restrict__ img) {
-  const int idx = blockIdx.x * blockDim.x + threadIdx.x;   // (i, chunk): 16 x 32
-  if (idx >= 512) return;
-  const int i = idx >> 5, cc = idx & 31;
-  float x[8];
-#pragma unroll
-  for (int e = 0; e < 8; ++e) x[e] = i < in_dim ? W1[(size_t)i * H + cc * 8 + e] : 0.f;
-  uint4 h, l;
-  split2(x[0], x[1], h.x, l.x); split2(x[2], x[3], h.y, l.y); split2(x[4], x[5], h.z, l.z); split2(x[6], x[7], h.w, l.w);
-  const int kb = cc >> 3, c = cc & 7;
-  auto off = [&](int row) { return (uint32_t)(kb * 4096 + (row >> 3) * 1024 + (row & 7) * 128 + ((c ^ (row & 7)) << 4)); };
-  *reinterpret_cast<uint4*>(img + off(i)) = h;
-  *reinterpret_cast<uint4*>(img + off(16 + i)) = l;
-}
-#endif
-
-#if defined(MPG_DEBUG_PROBES) && !defined(MPG_ACT_UNIT)
-// ---- self test: the three GEMM kinds against caller-provided fp32 data ---------------------------------------
-//   kind 0: Z[128 x 256] = X[128 x 256] . (image of Wt[256 x 256])^T
-//   kind 1: Z[128 x 256] = X16[128 x 16] . (first-layer image)^T
-//   kind 2: Z[128 x 16]  = X[128 x 256] . (input-gradient image)^T
-__global__ void __launch_bounds__(CTA_THREADS, 1) selftest_kernel(int kind, const float* __restrict__ X,
-                                                                 const uint8_t* __restrict__ img, float* __restrict__ Z,
-                                                                 int repeats) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);   // SW128 needs 1024-byte alignment
-  Bars* b = cta_setup(smem);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t tmem = b->tmem_base;
-  Sync s;
-  if (warp < EPI_WARPS) {
-    const int row = (warp & 3) * 32 + lane, hc = warp >> 2;
-    constexpr int CW = COLS_PER_WARP;
-    for (int rep = 0; rep < repeats; ++rep) {
-      if (kind >= 3) {          // timing probes: back-to-back big GEMMs on whatever the images hold, one wait at the end
-        if (rep == repeats - 1) epi_wait_d(b, s);
-        continue;
-      }
-      if (kind == 1) {
-        if (hc == 0) {
-          for (int kh = 0; kh < 2; ++kh) {
-            float x[8];
-            for (int e = 0; e < 8; ++e) x[e] = X[row * 16 + kh * 8 + e];
-            uint4 h, l;
-            split2h(x[0], x[1], h.x, l.x); split2h(x[2], x[3], h.y, l.y); split2h(x[4], x[5], h.z, l.z); split2h(x[6], x[7], h.w, l.w);
-            *reinterpret_cast<uint4*>(smem + SmemMap::PIMG + p_chunk_off(row, kh)) = h;
-            *reinterpret_cast<uint4*>(smem + SmemMap::PIMG + p_chunk_off(row, 2 + kh)) = l;
-          }
-        }
-      } else {
-        for (int cc = hc * (CW / 8); cc < (hc + 1) * (CW / 8); ++cc) {
-          float x[8];
-          for (int e = 0; e < 8; ++e) x[e] = X[row * 256 + cc * 8 + e];
-          act_store8(smem + SmemMap::ACT, smem + SmemMap::ACT + ACT_SPLIT, row, cc, x);
-        }
-      }
-      gemm<ROLE_EPI>(kind, b, smem, s, img, tmem + TM_WORK);
-      const uint32_t lane_base = tmem + TM_WORK + ((uint32_t)((warp & 3) * 32) << 16);
-      if (kind == 2) {
-        if (hc == 0) {
-          float v[16], v2[16];
-          tmem_ld16(lane_base, v);
-          tmem_ld16(lane_base + 16, v2);
-          for (int j = 0; j < 16; ++j) Z[row * 16 + j] = v[j] + v2[j];
-        }
-      } else {
-        for (int c0 = hc * CW; c0 < (hc + 1) * CW; c0 += 32) {
-          float v[32];
-          tmem_ld32(lane_base + c0, v);
-          for (int j = 0; j < 32; ++j) Z[row * 256 + c0 + j] = v[j];
-        }
-      }
-    }
-    tc_fence_before();
-  } else if (warp == EPI_WARPS) {
-    if (lane == 0)
-      for (int rep = 0; rep < repeats; ++rep)
-        if (kind != 4) gemm<ROLE_PRODUCER>(kind == 3 ? 0 : kind, b, smem, s, img, 0);
-  } else {
-    if (lane == 0)
-      for (int rep = 0; rep < repeats; ++rep) {
-        if (kind == 3) {          // weights streamed through the ring, no epilogue in the loop
-          mma_big<FMT_BF16>(b, smem_u32(smem) + SmemMap::ACT, smem_u32(smem) + SmemMap::RING, s, tmem + TM_WORK, false);
-          if (rep == repeats - 1) mma_publish_d(b);
-        } else if (kind == 4) {   // operands resident, no streaming: the tensor pipe's own rate for this shape
-          constexpr uint32_t idesc = make_idesc(128, 256, 0, 0);
-          const uint32_t act = smem_u32(smem) + SmemMap::ACT, ring = smem_u32(smem) + SmemMap::RING;
-          for (int k = 0; k < 16; ++k) {
-            const uint64_t ko = (uint64_t)((k & 3) * 2);
-            const uint64_t dah = make_desc(act + (k >> 2) * ACT_BLOCK, 16, 1024, LAYOUT_SW128) + ko;
-            const uint64_t dal = make_desc(act + ACT_SPLIT + (k >> 2) * ACT_BLOCK, 16, 1024, LAYOUT_SW128) + ko;
-            const uint64_t dbh = make_desc(ring, 16, 1024, LAYOUT_SW128) + ko;
-            const uint64_t dbl = make_desc(ring + 32768, 16, 1024, LAYOUT_SW128) + ko;
-            umma_bf16(tmem + TM_WORK, dah, dbh, idesc, 1u);
-            umma_bf16(tmem + TM_WORK, dal, dbh, idesc, 1u);
-            umma_bf16(tmem + TM_WORK, dah, dbl, idesc, 1u);
-          }
-          if (rep == repeats - 1) mma_publish_d(b);
-        } else {
-          gemm<ROLE_MMA>(kind, b, smem, s, img, tmem + TM_WORK);
-        }
-      }
-  }
-  cta_teardown(b);
-}
-#endif
-
 }  // namespace tc
 }  // namespace mpg
