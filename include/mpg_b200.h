@@ -76,8 +76,10 @@ typedef struct {
   int32_t M;                 /* args.M: tf.tile factor */
   int32_t horizon;           /* n = max(rollout list) */
   int32_t n_list;            /* len(num_rollout_list_*) <= MPG_MAX_LIST */
-  int32_t list[MPG_MAX_LIST];   /* rollout indices k (each <= horizon) */
-  float list_w[MPG_MAX_LIST];   /* loss weights w_k (rule_based_weights; 1 for NADP) */
+  int32_t list[MPG_MAX_LIST];   /* rollout indices k (each <= horizon), in any order; an index may repeat */
+  float list_w[MPG_MAX_LIST];   /* loss weights w_k (rule_based_weights; 1 for NADP), any sign, zero allowed.  Entries
+                                 * are independent terms of the loss, like the reference's tf.stack over the list:
+                                 * repeated indices each get their own returns row, and their weights add up */
   int32_t full_bptt;         /* 1: dW at every step (NADP, deriv_interval_policy); 0: a_0 only (default MPG) */
   int32_t q_net;             /* bootstrap net: MPG_NET_Q1 / MPG_NET_Q1_TARGET, or -1 for none (AMPC) */
   int32_t policy_net;        /* MPG_NET_POLICY (a_t = pi(p_t)) */

@@ -116,16 +116,19 @@ __global__ void __launch_bounds__(NT, 1) rollout_kernel(const __grid_constant__ 
           if (a.traj_act && valid) a.traj_act[((size_t)t * MB + grow) * A + j] = act[j];
         }
       }
-      int kidx = -1;
-      for (int k = 0; k < a.n_list; ++k) if (a.list[k] == t) kidx = k;
-      if (kidx >= 0) {
+      bool listed = false;
+      for (int k = 0; k < a.n_list; ++k) if (a.list[k] == t) listed = true;
+      if (listed) {
         float qv = 0.f;
         if (a.has_q) {
           __syncthreads();
           mlp_forward_tile<H, ACT>(a.q, sm, 1);
           if (rowthread) qv = sm.y3[tid];
         }
-        if (valid && a.returns_out) a.returns_out[(size_t)kidx * MB + grow] = rsum + gpow * qv;
+        // every entry of step t gets its row, repeated entries included
+        if (valid && a.returns_out)
+          for (int k = 0; k < a.n_list; ++k)
+            if (a.list[k] == t) a.returns_out[(size_t)k * MB + grow] = rsum + gpow * qv;
       }
       if (t < a.horizon && rowthread && valid) {
         float eps = 0.f;
@@ -178,17 +181,20 @@ __global__ void __launch_bounds__(NT, 1) rollout_kernel(const __grid_constant__ 
             act[j] = head_fwd(zpre[j], a.policy_out_tanh, a.action_range);
           }
         }
-        int kidx = -1;
-        for (int k = 0; k < a.n_list; ++k) if (a.list[k] == t) kidx = k;
-        if (kidx >= 0 && a.has_q && a.list_w[kidx] != 0.f) {   // zero-weight entries are stats only
-          // Q input-gradient: upstream c w_k gamma^t on Q1(p_t, a_t)
+        // Q part of step t: the summed weight of every entry at t; entries that all weigh zero are stats only
+        float w_t = 0.f;
+        bool q_part = false;
+        for (int k = 0; k < a.n_list; ++k)
+          if (a.list[k] == t) { w_t += a.list_w[k]; q_part = q_part || a.list_w[k] != 0.f; }
+        if (q_part && a.has_q) {
+          // Q input-gradient: upstream c w_t gamma^t on Q1(p_t, a_t)
           if (rowthread) {
 #pragma unroll
             for (int j = 0; j < A; ++j) sm.xin[(a.obs_dim + j) * RP + tid] = act[j];
           }
           __syncthreads();
           mlp_forward_tile<H, ACT>(a.q, sm, 1);
-          if (rowthread) sm.d3[tid] = valid ? cscale * a.list_w[kidx] * gp : 0.f;
+          if (rowthread) sm.d3[tid] = valid ? cscale * w_t * gp : 0.f;
           __syncthreads();
           mlp_backward_tile<H, ACT>(a.q, sm, 1, false, true, ga, nullptr);
           if (rowthread && valid) {

@@ -608,7 +608,11 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
           if (rowthread) write_pimg(s, act, true);
           qv = q_forward(false, nullptr);
         }
-        if (valid && a.returns_out) a.returns_out[(size_t)kidx * MB + grow] = rsum + gpow * qv;
+        // every entry of step t gets its row, repeated entries included (kidx is the last of them)
+        if (valid && a.returns_out)
+#pragma unroll
+          for (int k = 0; k < MPG_MAX_LIST; ++k)
+            if (k < a.n_list && a.list[k] == t) a.returns_out[(size_t)k * MB + grow] = rsum + gpow * qv;
       }
       if (t < a.horizon && valid) {
         float eps = 0.f;
@@ -673,13 +677,15 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
         if (ROLE == ROLE_ROW) stamp(4);
         const int kidx = list_index(t);
         if (want_dw) any_dw = true;
-        // ---- Q input gradient at the list steps: upstream c w_k gamma^t on Q1(p_t, a_t) ----
+        // ---- Q input gradient at the list steps: upstream c w_t gamma^t on Q1(p_t, a_t), w_t = the summed weight of
+        // every entry at step t ----
         float w_k = 0.f;
         if (kidx >= 0) {
 #pragma unroll
-          for (int k = 0; k < MPG_MAX_LIST; ++k) if (k == kidx) w_k = a.list_w[k];
+          for (int k = 0; k < MPG_MAX_LIST; ++k) if (k < a.n_list && a.list[k] == t) w_k += a.list_w[k];
         }
-        // does step tt start with a Q part (which uses the activation image before the policy part does)?
+        // does step tt start with a Q part (which uses the activation image before the policy part does)?  Yes when some
+        // entry at tt has a non-zero weight: the h2 prefetch schedule below and the gate of the Q part both ask this
         auto q_part_at = [&](int tt) {
           bool q = false;
           if (tt < 64) {
@@ -708,7 +714,7 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
               }
           }
         };
-        if (kidx >= 0 && a.has_q && (w_k != 0.f || A.q_regress)) {
+        if (kidx >= 0 && a.has_q && (q_part_at(t) || A.q_regress)) {
           const bool reg = A.q_regress != 0;      // regression: weight gradients of the Q net, no input gradient
           uint8_t* qslot = (reg && store_dw) ? A.store + (size_t)tile * SLOT_BYTES : nullptr;
           if (rowthread) {
