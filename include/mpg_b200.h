@@ -11,8 +11,8 @@
  * Conventions
  *   - all tensors fp32, row-major, DEVICE pointers unless the name ends in _host;
  *   - network weights use the Keras layout of the reference: kernels (in, out), list order
- *     [W1, b1, W2, b2, W3, b3] (model.py:20-43); gradients are written in the same order into one
- *     flat buffer (W1|b1|W2|b2|W3|b3);
+ *     [W1, b1, W2, b2, W3, b3] (model.py:20-43; [W1, b1, .., WL, bL, Wout, bout] for L hidden layers);
+ *     gradients are written in the same order into one flat buffer (W1|b1|W2|b2|W3|b3);
  *   - every function returns 0 on success, <0 on error; mpg_last_error() gives the message;
  *   - nothing is freed or retained from caller memory; workspace belongs to the handle;
  *   - all work is enqueued on `stream`; no hidden synchronisation.
@@ -59,7 +59,7 @@ typedef struct {
   int32_t num_future_data;   /* PathTracking only (path_tracking_env.py:265-271) */
   int32_t obs_dim;           /* 6+nfd | 4 | 11 */
   int32_t act_dim;           /* 2 | 1 | 1 */
-  int32_t hidden;            /* *_num_hidden_units of every net of the handle: 64, 128 or 256 (2 hidden layers) */
+  int32_t hidden;            /* *_num_hidden_units of every net of the handle: 64, 128 or 256 */
   int32_t policy_out_tanh;   /* policy_out_activation == 'tanh' */
   float action_range;        /* policy.py:197; <= 0 means None */
   float obs_scale[MPG_MAX_OBS]; /* preprocessor.py:134-145, 'scale' mode */
@@ -91,7 +91,12 @@ typedef struct {
 } mpg_rollout_params;
 
 /* ---- lifetime ---------------------------------------------------------------------------- */
+/* A handle whose six nets have 2 hidden layers (the reference default): mpg_create_layers(cfg, 2, out). */
 int mpg_create(const mpg_config* cfg, mpg_ctx** out);
+/* A handle whose six nets have `hidden_layers` hidden layers (*_num_hidden_layers, model.py:20-43): 1, 2 or 3; any
+ * other depth returns MPG_ERR_UNSUPPORTED.  Every backend covers 1..3 except MPG_BACKEND_TC, which needs 2. */
+int mpg_create_layers(const mpg_config* cfg, int hidden_layers, mpg_ctx** out);
+int mpg_hidden_layers(const mpg_ctx* ctx);
 void mpg_destroy(mpg_ctx* ctx);
 const char* mpg_last_error(const mpg_ctx* ctx);   /* ctx may be NULL: last create() error */
 size_t mpg_workspace_bytes(const mpg_ctx* ctx);
@@ -99,10 +104,11 @@ int mpg_num_sms(const mpg_ctx* ctx);
 int mpg_param_count(const mpg_ctx* ctx, int net); /* floats in one net's flat gradient */
 
 /* ---- weights: PolicyWithQs.set_weights (policy.py:116-121) -------------------------------- */
-/* w[0..5] = W1,b1,W2,b2,W3,b3 device pointers in Keras layout; repacked into the kernel layouts. */
-int mpg_set_weights(mpg_ctx* ctx, int net, const float* const w[6], void* stream);
-/* copy back in Keras layout (PolicyWithQs.get_weights, policy.py:112-114) */
-int mpg_get_weights(mpg_ctx* ctx, int net, float* const w[6], void* stream);
+/* w[0 .. 2(L+1)) = W1,b1,W2,b2,..,WL,bL,Wout,bout pointers in Keras layout, L = mpg_hidden_layers (six at L = 2);
+ * repacked into the kernel layouts. */
+int mpg_set_weights(mpg_ctx* ctx, int net, const float* const w[], void* stream);
+/* copy back in Keras layout (PolicyWithQs.get_weights, policy.py:112-114), the same 2(L+1) pointers */
+int mpg_get_weights(mpg_ctx* ctx, int net, float* const w[], void* stream);
 
 /* ---- policy gradient through the model rollout ------------------------------------------- */
 /* MPGLearner.policy_forward_and_backward (mpg_learner.py:356-365) /
@@ -211,7 +217,7 @@ int mpg_philox_noise(mpg_ctx* ctx, const mpg_rollout_params* p, float* out, void
  *   MPG_BACKEND_FFMA  fp32 CUDA-core contractions (every env / shape this build supports)
  *   MPG_BACKEND_TC    tcgen05 tensor-core contractions with split-bf16 operands (fp32-accurate), hidden = 256 only;
  *                     returns MPG_ERR_UNSUPPORTED for configurations it does not cover
- * mpg_create selects MPG_BACKEND_TC whenever it covers the configuration (hidden = 256 and
+ * mpg_create selects MPG_BACKEND_TC whenever it covers the configuration (hidden = 256, 2 hidden layers and
  * obs_dim + act_dim + 1 <= 16), else
  * MPG_BACKEND_FFMA; the environment variable MPG_B200_BACKEND=ffma forces the fp32 path at creation. */
 enum { MPG_BACKEND_FFMA = 0, MPG_BACKEND_TC = 1 };

@@ -13,6 +13,7 @@ ENV_IDS = {'PathTracking-v0': 0, 'InvertedPendulumConti-v0': 1, 'InvertedDoubleP
            'PathTracking-v0-real': 3}   # the ground-truth PathTrackingEnv (forward only)
 NET_Q1, NET_Q2, NET_POLICY, NET_Q1_TARGET, NET_Q2_TARGET, NET_POLICY_TARGET = range(6)
 ACTIVATIONS = {'elu': 0, 'relu': 1, 'tanh': 2}   # MPG_ACT_*: hidden activation of every net of a handle
+HIDDEN_LAYERS = (1, 2, 3)   # mpg_create_layers: hidden layers of every net of a handle
 
 # every symbol include/mpg_b200.h declares (tests check that the library exports all of them)
 SYMBOLS = [
@@ -25,7 +26,7 @@ SYMBOLS = [
     'mpg_set_adam_state', 'mpg_env_sample',
     'mpg_replay_create', 'mpg_replay_destroy', 'mpg_replay_last_error', 'mpg_replay_size', 'mpg_replay_add',
     'mpg_replay_sample', 'mpg_replay_update_priorities', 'mpg_replay_tree_stats', 'mpg_q_bootstrap', 'mpg_env_step',
-    'mpg_set_activation', 'mpg_get_activation',
+    'mpg_set_activation', 'mpg_get_activation', 'mpg_create_layers', 'mpg_hidden_layers',
 ]
 # exported by libmpg_b200_dbg.so only (include/mpg_b200.h, #ifdef MPG_DEBUG_PROBES)
 DEBUG_SYMBOLS = ['mpg_tc_selftest', 'mpg_set_profile_buffer']
@@ -68,6 +69,8 @@ def load(debug=False):
     P = ctypes.POINTER
     sig = {
         'mpg_create': (i32, [P(MpgConfig), P(vp)]),
+        'mpg_create_layers': (i32, [P(MpgConfig), i32, P(vp)]),
+        'mpg_hidden_layers': (i32, [vp]),
         'mpg_destroy': (None, [vp]),
         'mpg_last_error': (ctypes.c_char_p, [vp]),
         'mpg_workspace_bytes': (ctypes.c_size_t, [vp]),

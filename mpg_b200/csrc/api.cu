@@ -15,10 +15,10 @@ using namespace mpg;
 namespace {
 
 struct NetStore {
-  float* flat = nullptr;   // Keras order W1|b1|W2|b2|W3|b3 (natural layouts)
+  float* flat = nullptr;   // Keras order W1|b1|W2|b2|..|WL|bL|Wout|bout (natural layouts)
   float* W1p = nullptr;
-  float* W2p = nullptr;
-  float* W2Tp = nullptr;
+  float* Wp = nullptr;     // [L - 1][H][H]: the hidden -> hidden kernels W2..WL, packed columns (none at L = 1)
+  float* WTp = nullptr;    // [L - 1][H][H]: their transposes, packed columns
   float* adam_m = nullptr;   // Adam moments (allocated on the first optimiser step)
   float* adam_v = nullptr;
   int in_dim = 0, out_dim = 0;
@@ -60,6 +60,7 @@ struct mpg_ctx {
   uint64_t launches = 0;
   int backend = MPG_BACKEND_FFMA;
   int act = MPG_ACT_ELU;                  // hidden activation of every net (MPG_ACT_*)
+  int layers = 2;                         // hidden layers of every net (1..MAX_LAYERS)
   int timing = 0, timed = 0;
   long long* prof = nullptr;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
@@ -85,28 +86,36 @@ int fail(mpg_ctx* ctx, int code, const char* fmt, const char* detail = "") {
   } while (0)
 
 // flat parameter layout of one net of this handle
-GradLayout layout(const mpg_ctx* c, const NetStore& n) { return GradLayout(n.in_dim, n.out_dim, c->cfg.hidden); }
+GradLayout layout(const mpg_ctx* c, const NetStore& n) { return GradLayout(n.in_dim, n.out_dim, c->cfg.hidden, c->layers); }
 
 NetDev net_dev(const mpg_ctx* c, int net) {
   const NetStore& n = c->nets[net];
   const GradLayout L = layout(c, n);
+  const size_t hh = (size_t)c->cfg.hidden * c->cfg.hidden;
   NetDev d;
-  d.W1p = n.W1p; d.b1 = n.flat + L.ob1; d.W2p = n.W2p; d.b2 = n.flat + L.ob2; d.W2Tp = n.W2Tp;
-  d.W3 = n.flat + L.oW3; d.b3 = n.flat + L.ob3; d.W1 = n.flat + L.oW1;
-  d.in_dim = n.in_dim; d.out_dim = n.out_dim;
+  memset(&d, 0, sizeof(d));
+  d.W1p = n.W1p; d.b1 = n.flat + L.ob1;
+  for (int l = 2; l <= c->layers; ++l) {
+    d.Wp[l - 2] = n.Wp + (l - 2) * hh; d.WTp[l - 2] = n.WTp + (l - 2) * hh; d.b[l - 2] = n.flat + L.ob(l);
+  }
+  d.Wout = n.flat + L.oWout; d.bout = n.flat + L.obout; d.W1 = n.flat + L.oW1;
+  d.in_dim = n.in_dim; d.out_dim = n.out_dim; d.layers = c->layers;
   return d;
 }
 
 template <int H>
-__global__ void pack_kernel(const float* __restrict__ flat, int in_dim, int out_dim, float* __restrict__ W1p,
-                            float* __restrict__ W2p, float* __restrict__ W2Tp) {
-  const GradLayout L(in_dim, out_dim, H);
+__global__ void pack_kernel(const float* __restrict__ flat, int in_dim, int out_dim, int layers, float* __restrict__ W1p,
+                            float* __restrict__ Wp, float* __restrict__ WTp) {
+  const GradLayout L(in_dim, out_dim, H, layers);
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= H * H) return;
   // natural column c of row k -> packed column packed_col<H>(c) (mlp_tile.cuh: rowgemm reads through the same map)
   const int k = idx / H, c = idx % H, o = k * H + packed_col<H>(c);
-  W2p[o] = flat[L.oW2 + k * H + c];
-  W2Tp[o] = flat[L.oW2 + c * H + k];   // W2T[n=k][col c] = W2[c][k]
+  for (int l = 2; l <= layers; ++l) {
+    const size_t img = (size_t)(l - 2) * H * H;
+    Wp[img + o] = flat[L.oW(l) + k * H + c];
+    WTp[img + o] = flat[L.oW(l) + c * H + k];   // WT[n=k][col c] = W[c][k]
+  }
   if (k < in_dim) W1p[o] = flat[L.oW1 + k * H + c];
 }
 
@@ -353,9 +362,17 @@ uint64_t mpg_launch_count(const mpg_ctx* ctx) { return ctx->launches; }
 int mpg_get_backend(const mpg_ctx* ctx) { return ctx->backend; }
 int mpg_set_backend(mpg_ctx* ctx, int backend) {
   if (!ctx || (backend != MPG_BACKEND_FFMA && backend != MPG_BACKEND_TC)) return fail(ctx, MPG_ERR_ARG, "bad backend%s");
-  if (backend == MPG_BACKEND_TC && !ctx->tc.ready)
+  if (backend == MPG_BACKEND_TC && !ctx->tc.ready) {
+    if (ctx->layers != 2) {
+      char n[16];
+      snprintf(n, sizeof(n), "%d", ctx->layers);
+      return fail(ctx, MPG_ERR_UNSUPPORTED,
+                  "tensor-core backend does not cover this configuration (it needs hidden = 256 and 2 hidden layers; "
+                  "this handle has %s)", n);
+    }
     return fail(ctx, MPG_ERR_UNSUPPORTED,
                 "tensor-core backend does not cover this configuration (it needs hidden = 256 and obs_dim + act_dim <= 15)%s");
+  }
   ctx->backend = backend;
   return MPG_OK;
 }
@@ -412,14 +429,20 @@ int mpg_param_count(const mpg_ctx* ctx, int net) {
   return layout(ctx, ctx->nets[net]).total;
 }
 
-int mpg_create(const mpg_config* cfg, mpg_ctx** out) {
+int mpg_hidden_layers(const mpg_ctx* ctx) { return ctx->layers; }
+
+int mpg_create(const mpg_config* cfg, mpg_ctx** out) { return mpg_create_layers(cfg, 2, out); }
+
+int mpg_create_layers(const mpg_config* cfg, int hidden_layers, mpg_ctx** out) {
   if (!cfg || !out) return fail(nullptr, MPG_ERR_ARG, "null argument%s");
   *out = nullptr;
+  if (hidden_layers < 1 || hidden_layers > MAX_LAYERS)
+    return fail(nullptr, MPG_ERR_UNSUPPORTED, "hidden_layers must be 1, 2 or 3; deeper nets are not supported%s");
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
     return fail(nullptr, MPG_ERR_CUDA, "no CUDA device: mpg_b200 has no CPU fallback%s");
   if (cfg->hidden != 64 && cfg->hidden != 128 && cfg->hidden != 256)
-    return fail(nullptr, MPG_ERR_UNSUPPORTED, "hidden must be 64, 128 or 256 (2 hidden layers); other widths are not built%s");
+    return fail(nullptr, MPG_ERR_UNSUPPORTED, "hidden must be 64, 128 or 256; other widths are not built%s");
   if (cfg->env < 0 || cfg->env > 3) return fail(nullptr, MPG_ERR_ARG, "unknown env%s");
   static const int SD[4] = {6, 4, 6, 8}, AD[4] = {2, 1, 1, 2};
   if (cfg->act_dim != AD[cfg->env]) return fail(nullptr, MPG_ERR_ARG, "act_dim does not match env%s");
@@ -429,6 +452,7 @@ int mpg_create(const mpg_config* cfg, mpg_ctx** out) {
   mpg_ctx* c = new (std::nothrow) mpg_ctx();
   if (!c) return fail(nullptr, MPG_ERR_ARG, "out of host memory%s");
   c->cfg = *cfg;
+  c->layers = hidden_layers;
   c->err[0] = 0;
   c->S = SD[cfg->env];
   cudaDeviceProp prop;
@@ -456,13 +480,15 @@ int mpg_create(const mpg_config* cfg, mpg_ctx** out) {
     const GradLayout L = layout(c, ns);
     const size_t hw = (size_t)cfg->hidden;
     maxP = L.total > (int)maxP ? L.total : maxP;
-    ok = ok && alloc(&ns.flat, L.total) && alloc(&ns.W1p, MAX_IN * hw) && alloc(&ns.W2p, hw * hw) && alloc(&ns.W2Tp, hw * hw);
+    const size_t himg = (size_t)(hidden_layers - 1) * hw * hw;
+    ok = ok && alloc(&ns.flat, L.total) && alloc(&ns.W1p, MAX_IN * hw)
+         && (himg == 0 || (alloc(&ns.Wp, himg) && alloc(&ns.WTp, himg)));
   }
   c->partial_stride = (maxP + 3) & ~size_t(3);
   ok = ok && alloc(&c->ckpt, (size_t)(cfg->max_horizon + 1) * cfg->max_rows * c->S)
        && alloc(&c->partial, (size_t)2 * c->sms * c->partial_stride) && alloc(&c->loss_partial, c->sms)
        && alloc(&c->stats_part, (size_t)MPG_MAX_LIST * 64 * 2) && alloc(&c->red_part, 128);
-  if (ok) ok = tc_init(c->tc, c->cfg, c->sms, c->ws_bytes);
+  if (ok) ok = tc_init(c->tc, c->cfg, hidden_layers, c->sms, c->ws_bytes);
   wait_dbg_init();   // best effort: without it a timed-out wait still traps, only the record is missing
   if (!ok) {
     snprintf(g_create_err, 512, "cudaMalloc of the workspace failed: %s", cudaGetErrorString(cudaGetLastError()));
@@ -497,7 +523,7 @@ int mpg_create(const mpg_config* cfg, mpg_ctx** out) {
 void mpg_destroy(mpg_ctx* c) {
   if (!c) return;
   for (int n = 0; n < MPG_NUM_NETS; ++n) {
-    cudaFree(c->nets[n].flat); cudaFree(c->nets[n].W1p); cudaFree(c->nets[n].W2p); cudaFree(c->nets[n].W2Tp);
+    cudaFree(c->nets[n].flat); cudaFree(c->nets[n].W1p); cudaFree(c->nets[n].Wp); cudaFree(c->nets[n].WTp);
     cudaFree(c->nets[n].adam_m); cudaFree(c->nets[n].adam_v);
   }
   cudaFree(c->ckpt); cudaFree(c->partial); cudaFree(c->loss_partial); cudaFree(c->stats_part); cudaFree(c->red_part);
@@ -509,28 +535,36 @@ void mpg_destroy(mpg_ctx* c) {
   delete c;
 }
 
-// FFMA weight images (W1p, W2p, W2Tp) of one net from its flat natural weights
+// FFMA weight images (W1p, Wp, WTp) of one net from its flat natural weights
 static void launch_pack(mpg_ctx* ctx, const NetStore& ns, cudaStream_t st) {
   const int hw = ctx->cfg.hidden, grid = (hw * hw + 255) / 256;   // mpg_create admits 64, 128 and 256
+  const int L = ctx->layers;
   switch (hw) {
-    case 64: pack_kernel<64><<<grid, 256, 0, st>>>(ns.flat, ns.in_dim, ns.out_dim, ns.W1p, ns.W2p, ns.W2Tp); break;
-    case 128: pack_kernel<128><<<grid, 256, 0, st>>>(ns.flat, ns.in_dim, ns.out_dim, ns.W1p, ns.W2p, ns.W2Tp); break;
-    default: pack_kernel<256><<<grid, 256, 0, st>>>(ns.flat, ns.in_dim, ns.out_dim, ns.W1p, ns.W2p, ns.W2Tp); break;
+    case 64: pack_kernel<64><<<grid, 256, 0, st>>>(ns.flat, ns.in_dim, ns.out_dim, L, ns.W1p, ns.Wp, ns.WTp); break;
+    case 128: pack_kernel<128><<<grid, 256, 0, st>>>(ns.flat, ns.in_dim, ns.out_dim, L, ns.W1p, ns.Wp, ns.WTp); break;
+    default: pack_kernel<256><<<grid, 256, 0, st>>>(ns.flat, ns.in_dim, ns.out_dim, L, ns.W1p, ns.Wp, ns.WTp); break;
   }
   ctx->launches++;
 }
 
-int mpg_set_weights(mpg_ctx* ctx, int net, const float* const w[6], void* stream) {
+// flat offset and size of the i-th of the 2 (L + 1) weight arrays W1, b1, W2, b2, .., WL, bL, Wout, bout of a net
+static void weight_array(const mpg_ctx* ctx, const NetStore& ns, int i, int& off, int& cnt) {
+  const GradLayout L = layout(ctx, ns);
+  const int hw = ctx->cfg.hidden, l = i / 2 + 1;
+  if (l == 1) { off = i ? L.ob1 : L.oW1; cnt = i ? hw : ns.in_dim * hw; }
+  else if (l <= ctx->layers) { off = i & 1 ? L.ob(l) : L.oW(l); cnt = i & 1 ? hw : hw * hw; }
+  else { off = i & 1 ? L.obout : L.oWout; cnt = i & 1 ? ns.out_dim : hw * ns.out_dim; }
+}
+
+int mpg_set_weights(mpg_ctx* ctx, int net, const float* const w[], void* stream) {
   if (!ctx || net < 0 || net >= MPG_NUM_NETS || !w) return fail(ctx, MPG_ERR_ARG, "bad argument to mpg_set_weights%s");
   cudaStream_t st = (cudaStream_t)stream;
   NetStore& ns = ctx->nets[net];
-  const GradLayout L = layout(ctx, ns);
-  const int hw = ctx->cfg.hidden;
-  const int off[6] = {L.oW1, L.ob1, L.oW2, L.ob2, L.oW3, L.ob3};
-  const int cnt[6] = {ns.in_dim * hw, hw, hw * hw, hw, hw * ns.out_dim, ns.out_dim};
-  for (int i = 0; i < 6; ++i) {
+  for (int i = 0; i < 2 * (ctx->layers + 1); ++i) {
     if (!w[i]) return fail(ctx, MPG_ERR_ARG, "null weight pointer%s");
-    CUDA_OK(ctx, cudaMemcpyAsync(ns.flat + off[i], w[i], cnt[i] * sizeof(float), cudaMemcpyDefault, st));
+    int off, cnt;
+    weight_array(ctx, ns, i, off, cnt);
+    CUDA_OK(ctx, cudaMemcpyAsync(ns.flat + off, w[i], cnt * sizeof(float), cudaMemcpyDefault, st));
   }
   launch_pack(ctx, ns, st);
   CUDA_OK(ctx, cudaGetLastError());
@@ -613,17 +647,16 @@ int mpg_polyak_update(mpg_ctx* ctx, int src_net, int dst_net, float tau, void* s
   return repack(ctx, dst_net, st);
 }
 
-int mpg_get_weights(mpg_ctx* ctx, int net, float* const w[6], void* stream) {
+int mpg_get_weights(mpg_ctx* ctx, int net, float* const w[], void* stream) {
   int rc = check_net(ctx, net);
   if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   NetStore& ns = ctx->nets[net];
-  const GradLayout L = layout(ctx, ns);
-  const int hw = ctx->cfg.hidden;
-  const int off[6] = {L.oW1, L.ob1, L.oW2, L.ob2, L.oW3, L.ob3};
-  const int cnt[6] = {ns.in_dim * hw, hw, hw * hw, hw, hw * ns.out_dim, ns.out_dim};
-  for (int i = 0; i < 6; ++i)
-    CUDA_OK(ctx, cudaMemcpyAsync(w[i], ns.flat + off[i], cnt[i] * sizeof(float), cudaMemcpyDefault, st));
+  for (int i = 0; i < 2 * (ctx->layers + 1); ++i) {
+    int off, cnt;
+    weight_array(ctx, ns, i, off, cnt);
+    CUDA_OK(ctx, cudaMemcpyAsync(w[i], ns.flat + off, cnt * sizeof(float), cudaMemcpyDefault, st));
+  }
   return MPG_OK;
 }
 

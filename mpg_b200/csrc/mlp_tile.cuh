@@ -1,5 +1,5 @@
 // CTA-tile MLP engine (fp32 FFMA path): forward and backward of the reference's MLPNet
-// (model.py:20-43: Dense(H,act) -> Dense(H,act) -> Dense(out)) on a tile of TILE_R rows.
+// (model.py:20-43: L x Dense(H,act) -> Dense(out), L = 1..MAX_LAYERS) on a tile of TILE_R rows.
 // The hidden activation ACT (common.cuh: act_fwd / act_grad_from_out) is a template parameter beside H.
 //
 // Shared-memory activation tiles are stored [feature][row] with row pitch RP (68 floats) so that
@@ -19,32 +19,40 @@
 
 namespace mpg {
 
-// packed column (within a row of W1p / W2p / W2Tp) of natural column c = l + 32 j: vector j / G of lane l, element j % G
+// packed column (within a row of W1p / Wp / WTp) of natural column c = l + 32 j: vector j / G of lane l, element j % G
 template <int H>
 __host__ __device__ __forceinline__ constexpr int packed_col(int c) {
   constexpr int G = H / 32 < 4 ? H / 32 : 4;
   return ((c >> 5) / G) * (32 * G) + G * (c & 31) + (c >> 5) % G;
 }
 
+// hidden layers of a net: the backward pass keeps every activation in the two tiles bufA / bufB, recomputing h1 at
+// L = 3 (mlp_backward_tile); L = 4 would need a third tile, which does not fit beside the H = 256 carve-up
+constexpr int MAX_LAYERS = 3;
+
 struct NetDev {
   const float* W1p;   // [in_dim][H] packed columns
   const float* b1;    // [H]
-  const float* W2p;   // [H][H] packed columns
-  const float* b2;    // [H]
-  const float* W2Tp;  // [H(n)][H(k)] = W2^T, packed columns
-  const float* W3;    // [H][out_dim] natural
-  const float* b3;    // [out_dim]
+  // hidden -> hidden layer l = 2..layers at index l - 2
+  const float* Wp[MAX_LAYERS - 1];    // [H][H] packed columns
+  const float* WTp[MAX_LAYERS - 1];   // [H(n)][H(k)] = W_l^T, packed columns
+  const float* b[MAX_LAYERS - 1];     // [H]
+  const float* Wout;  // [H][out_dim] natural
+  const float* bout;  // [out_dim]
   const float* W1;    // [in_dim][H] natural (for the input gradient)
-  int in_dim, out_dim;
+  int in_dim, out_dim, layers;
 };
 
-// flat gradient layout (Keras order W1|b1|W2|b2|W3|b3)
+// flat gradient layout (Keras order W1|b1|W2|b2|..|WL|bL|Wout|bout); every offset is a multiple of 4 (H is)
 struct GradLayout {
-  int oW1, ob1, oW2, ob2, oW3, ob3, total;
-  __host__ __device__ GradLayout(int in_dim, int out_dim, int H) {
-    oW1 = 0; ob1 = oW1 + in_dim * H; oW2 = ob1 + H; ob2 = oW2 + H * H; oW3 = ob2 + H; ob3 = oW3 + H * out_dim;
-    total = ob3 + out_dim;
+  int h, oW1, ob1, oWout, obout, total;
+  __host__ __device__ GradLayout(int in_dim, int out_dim, int H, int layers) {
+    h = H; oW1 = 0; ob1 = oW1 + in_dim * H; oWout = ob1 + H + (layers - 1) * (H * H + H); obout = oWout + H * out_dim;
+    total = obout + out_dim;
   }
+  // kernel and bias of hidden -> hidden layer l = 2..layers
+  __host__ __device__ int oW(int l) const { return ob1 + h + (l - 2) * (h * h + h); }
+  __host__ __device__ int ob(int l) const { return oW(l) + h * h; }
 };
 
 // shared memory carve-up (floats)
@@ -158,26 +166,32 @@ __device__ __forceinline__ void store_times_actgrad(const float (&acc)[8][H / 32
 }
 
 // ---------------------------------------------------------------------------------------------
-// forward: xin[0..in_dim) -> h1 (bufA) -> h2 (bufB) -> y3[j][r] = h2 W3 + b3 for j < n_out
-// (n_out = number of output columns actually consumed: act_dim for the policy mean, 1 for Q)
+// forward: xin[0..in_dim) -> h1 (bufA) -> h2 (bufB) -> h3 (bufA) .. -> y3[j][r] = hL Wout + bout for j < n_out
+// (n_out = number of output columns actually consumed: act_dim for the policy mean, 1 for Q).
+// h_l is in bufA for odd l, in bufB for even l.
 // ---------------------------------------------------------------------------------------------
 template <int H, int ACT>
 __device__ __forceinline__ void mlp_forward_tile(const NetDev& net, Smem<H>& sm, int n_out) {
   float acc[8][H / 32];
   rowgemm<H>(sm.xin, net.in_dim, net.W1p, sm.slab, acc);
   store_bias_act<H, ACT>(acc, net.b1, sm.bufA);
-  rowgemm<H>(sm.bufA, H, net.W2p, sm.slab, acc);   // first internal barrier publishes bufA
-  store_bias_act<H, ACT>(acc, net.b2, sm.bufB);
+  float *hin = sm.bufA, *hout = sm.bufB;
+  for (int l = 2; l <= net.layers; ++l) {
+    rowgemm<H>(hin, H, net.Wp[l - 2], sm.slab, acc);   // first internal barrier publishes hin, the last ends its reads
+    store_bias_act<H, ACT>(acc, net.b[l - 2], hout);
+    float* t = hin; hin = hout; hout = t;
+  }
+  const float* hL = hin;
   __syncthreads();
   // output layer: thread (r, q) sums features k = q, q+4, ... for every consumed column, then the
   // four partial sums are combined in a fixed order through shared memory (deterministic)
   const int tid = threadIdx.x, r = tid & 63, q = tid >> 6;
   float part[MAX_A] = {0.f, 0.f};
   for (int k = q; k < H; k += 4) {
-    const float h = sm.bufB[k * RP + r];
+    const float h = hL[k * RP + r];
 #pragma unroll
     for (int j = 0; j < MAX_A; ++j)
-      if (j < n_out) part[j] = fmaf(h, __ldg(net.W3 + k * net.out_dim + j), part[j]);
+      if (j < n_out) part[j] = fmaf(h, __ldg(net.Wout + k * net.out_dim + j), part[j]);
   }
   float* scratch = sm.slab;  // [4][MAX_A][RP]
 #pragma unroll
@@ -186,31 +200,34 @@ __device__ __forceinline__ void mlp_forward_tile(const NetDev& net, Smem<H>& sm,
   __syncthreads();
   if (tid < 64 * n_out) {
     const int j = tid >> 6;
-    float v = __ldg(net.b3 + j);
+    float v = __ldg(net.bout + j);
     for (int qq = 0; qq < 4; ++qq) v += scratch[(qq * MAX_A + j) * RP + r];
     sm.y3[j * RP + r] = v;
   }
   __syncthreads();
 }
 
-// persistent per-thread gradient accumulators: thread tid owns feature tid % H, rows slice tid / H (see the top)
+// persistent per-thread gradient accumulators: thread tid owns feature tid % H, rows slice tid / H (see the top).
+// Bias l lives in db[l - 1], always indexed by a compile-time constant so that the array stays in registers.
 template <int H>
 struct GradAcc {
-  float dW1[MAX_IN];  // dW1[i][tid % H]
-  float db1, db2;
-  float dW3[MAX_A];   // dW3[tid % H][j]
-  float db3;          // db3[tid] for tid < n_out
+  float dW1[MAX_IN];     // dW1[i][tid % H]
+  float db[MAX_LAYERS];  // db_l[tid % H]
+  float dWout[MAX_A];    // dWout[tid % H][j]
+  float dbout;           // dbout[tid] for tid < n_out
   __device__ void zero() {
-    db3 = 0.f;
+    dbout = 0.f;
 #pragma unroll
     for (int i = 0; i < MAX_IN; ++i) dW1[i] = 0.f;
-    db1 = db2 = 0.f;
 #pragma unroll
-    for (int j = 0; j < MAX_A; ++j) dW3[j] = 0.f;
+    for (int l = 0; l < MAX_LAYERS; ++l) db[l] = 0.f;
+#pragma unroll
+    for (int j = 0; j < MAX_A; ++j) dWout[j] = 0.f;
   }
 };
 
-// dW2[k][n] += sum_r X[k][r] Y[n][r] into this CTA's private global partial (natural (k,n) layout).
+// dW_l[k][n] += sum_r X[k][r] Y[n][r] (hidden -> hidden layer l) into this CTA's private global partial (natural (k,n)
+// layout).
 // H/64 chunks of 64 columns n (warp w: n = 64 chunk + 8 w + j, j < 8); lane l owns the rows k = l + 32 i, i < H/32.
 template <int H>
 __device__ __forceinline__ void dw2_accumulate(const float* __restrict__ X, const float* __restrict__ Y,
@@ -253,79 +270,107 @@ __device__ __forceinline__ void dw2_accumulate(const float* __restrict__ X, cons
 }
 
 // ---------------------------------------------------------------------------------------------
-// backward. On entry: xin = layer input, bufA = h1, bufB = h2 (from mlp_forward_tile) and
-// d3[j][r] = dL/d y3[j][r] for j < n_out (rows >= valid must hold 0). On exit (want_gin):
-// gx[i][r] = dL/d xin[i][r].  With want_dw the parameter gradients are accumulated into `ga`
-// (registers) and dW2g (global partial).
+// backward. On entry: xin = layer input, the tiles as mlp_forward_tile left them (h_L in bufA for odd L, bufB for
+// even L; at L = 2 h1 is still in bufA) and d3[j][r] = dL/d y3[j][r] for j < n_out (rows >= valid must hold 0).
+// On exit (want_gin): gx[i][r] = dL/d xin[i][r].  With want_dw the parameter gradients are accumulated into `ga`
+// (registers) and `partial` (this CTA's global partial, GradLayout order: the dW_l of the hidden -> hidden layers).
+// Every delta is formed in place over its activation, so the pass needs no tile beyond bufA / bufB.  At L = 3 h1 was
+// overwritten by h3; it is recomputed from xin (same code and inputs as the forward: bit-identical) once delta3 is
+// consumed.
 // ---------------------------------------------------------------------------------------------
 template <int H, int ACT>
 __device__ __forceinline__ void mlp_backward_tile(const NetDev& net, Smem<H>& sm, int n_out, bool want_dw, bool want_gin,
-                                                  GradAcc<H>& ga, float* __restrict__ dW2g) {
+                                                  GradAcc<H>& ga, float* __restrict__ partial) {
   const int tid = threadIdx.x;
   // feature f of this thread and its slice [r0, r0 + RS) of the tile rows (P = 1: all rows)
   constexpr int P = NT / H, RS = TILE_R / P;
   const int f = P == 1 ? tid : tid % H, r0 = P == 1 ? 0 : (tid / H) * RS;
-  // (1) thread (f, slice) walks its feature row: dW3 += h2 d3, delta2 = (d3 W3^T) act'(h2) in place, db2
+  const int layers = net.layers;
+  // delta_l is formed over the tile of h_l; h_{l-1} is in the other one
+  float* d = (layers & 1) ? sm.bufA : sm.bufB;
+  float* h = (layers & 1) ? sm.bufB : sm.bufA;
+  // (1) thread (f, slice) walks its feature row: dWout += hL d3, deltaL = (d3 Wout^T) act'(hL) in place, dbL
   {
-    float w3[MAX_A];
+    float wo[MAX_A];
 #pragma unroll
-    for (int j = 0; j < MAX_A; ++j) w3[j] = (j < n_out) ? __ldg(net.W3 + f * net.out_dim + j) : 0.f;
-    float* hrow = sm.bufB + f * RP;
-    float s_db2 = 0.f, s_dw3[MAX_A] = {0.f, 0.f};
+    for (int j = 0; j < MAX_A; ++j) wo[j] = (j < n_out) ? __ldg(net.Wout + f * net.out_dim + j) : 0.f;
+    float* hrow = d + f * RP;
+    float s_db = 0.f, s_dwo[MAX_A] = {0.f, 0.f};
     for (int r4 = r0; r4 < r0 + RS; r4 += 4) {
-      float4 h = *reinterpret_cast<float4*>(hrow + r4);
-      float hv[4] = {h.x, h.y, h.z, h.w}, dv[4];
+      float4 hv4 = *reinterpret_cast<float4*>(hrow + r4);
+      float hv[4] = {hv4.x, hv4.y, hv4.z, hv4.w}, dv[4];
 #pragma unroll
       for (int e = 0; e < 4; ++e) {
         float g = 0.f;
 #pragma unroll
         for (int j = 0; j < MAX_A; ++j)
           if (j < n_out) {
-            const float d = sm.d3[j * RP + r4 + e];
-            g = fmaf(d, w3[j], g);
-            s_dw3[j] = fmaf(hv[e], d, s_dw3[j]);
+            const float dd = sm.d3[j * RP + r4 + e];
+            g = fmaf(dd, wo[j], g);
+            s_dwo[j] = fmaf(hv[e], dd, s_dwo[j]);
           }
         dv[e] = g * act_grad_from_out<ACT>(hv[e]);
-        s_db2 += dv[e];
+        s_db += dv[e];
       }
       *reinterpret_cast<float4*>(hrow + r4) = make_float4(dv[0], dv[1], dv[2], dv[3]);
     }
     if (want_dw) {
-      ga.db2 += s_db2;
+      // dbL for L = 2, 3 (at L = 1 this is db1, summed with dW1 in (4)).  A select, not a branch: a conditional
+      // store is merged into one store through a runtime index, which moves the accumulators to local memory.
+      ga.db[1] += layers == 2 ? s_db : 0.f;
+      ga.db[2] += layers == 3 ? s_db : 0.f;
 #pragma unroll
-      for (int j = 0; j < MAX_A; ++j) ga.dW3[j] += s_dw3[j];
+      for (int j = 0; j < MAX_A; ++j) ga.dWout[j] += s_dwo[j];
     }
   }
   if (want_dw && tid < n_out) {
-    float s_db3 = 0.f;
-    for (int r = 0; r < TILE_R; ++r) s_db3 += sm.d3[tid * RP + r];
-    ga.db3 += s_db3;
+    float s_dbo = 0.f;
+    for (int r = 0; r < TILE_R; ++r) s_dbo += sm.d3[tid * RP + r];
+    ga.dbout += s_dbo;
   }
   __syncthreads();
-  // (2) dW2 += h1^T delta2
-  if (want_dw) dw2_accumulate<H>(sm.bufA, sm.bufB, dW2g);
-  // (3) delta1 = (delta2 W2^T) act'(h1), in place over h1
-  {
-    float acc[8][H / 32];
-    rowgemm<H>(sm.bufB, H, net.W2Tp, sm.slab, acc);
-    store_times_actgrad<H, ACT>(acc, sm.bufA);
+  const GradLayout L(net.in_dim, net.out_dim, H, layers);
+  for (int l = layers; l >= 2; --l) {
+    // (2) dW_l += h_{l-1}^T delta_l
+    if (want_dw) dw2_accumulate<H>(h, d, partial + L.oW(l));
+    // (3) delta_{l-1} = (delta_l W_l^T) act'(h_{l-1}), in place over h_{l-1}
+    {
+      float acc[8][H / 32];
+      rowgemm<H>(d, H, net.WTp[l - 2], sm.slab, acc);
+      store_times_actgrad<H, ACT>(acc, h);
+      if (l == 3) {   // delta3 is consumed: recompute h1 (overwritten by h3) into its tile
+        rowgemm<H>(sm.xin, net.in_dim, net.W1p, sm.slab, acc);
+        store_bias_act<H, ACT>(acc, net.b1, d);
+      }
+    }
+    __syncthreads();
+    float* t = d; d = h; h = t;
+    if (want_dw && l == 3) {   // db2 of the middle layer at L = 3 (thread (f, slice) as in (1)); db1 is summed in (4)
+      const float* drow = d + f * RP;
+      float s_db = 0.f;
+      for (int r4 = r0; r4 < r0 + RS; r4 += 4) {
+        const float4 dd = *reinterpret_cast<const float4*>(drow + r4);
+        s_db += (dd.x + dd.y) + (dd.z + dd.w);
+      }
+      ga.db[1] += s_db;
+    }
   }
-  __syncthreads();
+  // delta1 is in bufA
   // (4) dW1 += xin^T delta1, db1 (thread (f, slice) as in (1))
   if (want_dw) {
     const float* drow = sm.bufA + f * RP;
     float s_db1 = 0.f;
     for (int r4 = r0; r4 < r0 + RS; r4 += 4) {
-      const float4 d = *reinterpret_cast<const float4*>(drow + r4);
-      s_db1 += (d.x + d.y) + (d.z + d.w);
+      const float4 dd = *reinterpret_cast<const float4*>(drow + r4);
+      s_db1 += (dd.x + dd.y) + (dd.z + dd.w);
 #pragma unroll
       for (int i = 0; i < MAX_IN; ++i)
         if (i < net.in_dim) {
           const float4 x = *reinterpret_cast<const float4*>(sm.xin + i * RP + r4);
-          ga.dW1[i] = fmaf(x.x, d.x, fmaf(x.y, d.y, fmaf(x.z, d.z, fmaf(x.w, d.w, ga.dW1[i]))));
+          ga.dW1[i] = fmaf(x.x, dd.x, fmaf(x.y, dd.y, fmaf(x.z, dd.z, fmaf(x.w, dd.w, ga.dW1[i]))));
         }
     }
-    ga.db1 += s_db1;
+    ga.db[0] += s_db1;
   }
   // (5) gx[i][r] = sum_n delta1[n][r] W1[i][n]: thread (r, q) covers n in [q H/4, (q+1) H/4), partials
   //     combined in fixed order
@@ -359,7 +404,7 @@ __device__ __forceinline__ void mlp_backward_tile(const NetDev& net, Smem<H>& sm
 // Every thread of the CTA must call it.
 template <int H>
 __device__ __forceinline__ void flush_grad_acc(const NetDev& net, const GradAcc<H>& ga, float* __restrict__ partial) {
-  const GradLayout L(net.in_dim, net.out_dim, H);
+  const GradLayout L(net.in_dim, net.out_dim, H, net.layers);
   constexpr int P = NT / H;
   const int tid = threadIdx.x, f = P == 1 ? tid : tid % H, slice = P == 1 ? 0 : tid / H;
   for (int p = 0; p < P; ++p) {
@@ -369,13 +414,15 @@ __device__ __forceinline__ void flush_grad_acc(const NetDev& net, const GradAcc<
 #pragma unroll
     for (int i = 0; i < MAX_IN; ++i)
       if (i < net.in_dim) put(L.oW1 + i * H + f, ga.dW1[i]);
-    put(L.ob1 + f, ga.db1);
-    put(L.ob2 + f, ga.db2);
+    put(L.ob1 + f, ga.db[0]);
+#pragma unroll
+    for (int l = 2; l <= MAX_LAYERS; ++l)
+      if (l <= net.layers) put(L.ob(l) + f, ga.db[l - 1]);
 #pragma unroll
     for (int j = 0; j < MAX_A; ++j)
-      if (j < net.out_dim) put(L.oW3 + f * net.out_dim + j, ga.dW3[j]);
+      if (j < net.out_dim) put(L.oWout + f * net.out_dim + j, ga.dWout[j]);
   }
-  if (tid < MAX_A && tid < net.out_dim) partial[L.ob3 + tid] = ga.db3;
+  if (tid < MAX_A && tid < net.out_dim) partial[L.obout + tid] = ga.dbout;
   // columns j >= MAX_A (the unused log-std half of the policy head, policy.py:198) keep their zeros
 }
 

@@ -32,7 +32,7 @@ struct RolloutArgs {
   float* traj_act;
   float* ckpt;      // [horizon+1][M*rows][S]
   float* partial;   // [grid][partial_stride]
-  long long partial_stride;   // floats, multiple of 4 (float4 accesses into the dW2 region)
+  long long partial_stride;   // floats, multiple of 4 (float4 accesses into the hidden -> hidden dW regions)
   NetDev pol, q;
 };
 
@@ -66,7 +66,6 @@ __global__ void __launch_bounds__(NT, 1) rollout_kernel(const __grid_constant__ 
   const int MB = a.rows * a.M;
   const int ntiles = (MB + TILE_R - 1) / TILE_R;
   const bool rowthread = tid < TILE_R;
-  const GradLayout L(a.pol.in_dim, a.pol.out_dim, H);
   float* partial = a.partial + (size_t)blockIdx.x * a.partial_stride;
   GradAcc<H> ga;
   ga.zero();
@@ -205,7 +204,7 @@ __global__ void __launch_bounds__(NT, 1) rollout_kernel(const __grid_constant__ 
             for (int j = 0; j < A; ++j) g_a[j] += sm.gx[(a.obs_dim + j) * RP + tid];
           }
           __syncthreads();
-          mlp_forward_tile<H, ACT>(a.pol, sm, A);   // the Q pass reused bufA/bufB: recompute h1, h2 of the policy
+          mlp_forward_tile<H, ACT>(a.pol, sm, A);   // the Q pass reused bufA/bufB: recompute every layer of the policy
         }
         if (t < a.horizon && rowthread && valid) {
           float Wt = 0.f;
@@ -221,7 +220,7 @@ __global__ void __launch_bounds__(NT, 1) rollout_kernel(const __grid_constant__ 
         __syncthreads();
         const bool want_dw = a.full_bptt || t == 0;
         const bool want_gin = t > 0;
-        mlp_backward_tile<H, ACT>(a.pol, sm, A, want_dw, want_gin, ga, partial + L.oW2);
+        mlp_backward_tile<H, ACT>(a.pol, sm, A, want_dw, want_gin, ga, partial);
         if (rowthread && valid) {
 #pragma unroll
           for (int j = 0; j < S; ++j) { lam[j] = g_s[j]; snext[j] = s[j]; }
@@ -261,7 +260,6 @@ __global__ void __launch_bounds__(NT, 1) q_grad_kernel(const __grid_constant__ Q
   __shared__ float red[TILE_R];
   const int tid = threadIdx.x;
   const int ntiles = (a.rows + TILE_R - 1) / TILE_R;
-  const GradLayout L(a.q.in_dim, a.q.out_dim, H);
   float* partial = a.partial + (size_t)blockIdx.x * a.partial_stride;
   GradAcc<H> ga;
   ga.zero();
@@ -283,7 +281,7 @@ __global__ void __launch_bounds__(NT, 1) q_grad_kernel(const __grid_constant__ Q
       sm.d3[tid] = diff * a.inv_global_rows;
     }
     __syncthreads();
-    mlp_backward_tile<H, ACT>(a.q, sm, 1, true, false, ga, partial + L.oW2);
+    mlp_backward_tile<H, ACT>(a.q, sm, 1, true, false, ga, partial);
   }
   flush_grad_acc(a.q, ga, partial);
   if (tid < TILE_R) red[tid] = loss;

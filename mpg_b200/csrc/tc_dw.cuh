@@ -164,7 +164,7 @@ __global__ void __launch_bounds__(DW_THREADS, 1) tc_dw_kernel(const __grid_const
       }
     }
     // ------------------------------- epilogue: TMEM -> this CTA's partial gradient -------------------------------
-    const GradLayout L(A.in_dim, A.out_dim, H);
+    const GradLayout L(A.in_dim, A.out_dim, H, 2);
     float* partial = A.partial + (size_t)blockIdx.x * A.partial_stride;
     const int f = mh * 128 + warp * 32 + lane;                   // feature owned by this thread (TMEM lane)
     const uint32_t lane_off = (uint32_t)(warp * 32) << 16;
@@ -174,13 +174,13 @@ __global__ void __launch_bounds__(DW_THREADS, 1) tc_dw_kernel(const __grid_const
       for (int c0 = 0; c0 < 256; c0 += 32) {
         float v[32];
         tmem_ld32(tmem + DW_TM_D2 + lane_off + c0, v);
-        float4* dst = reinterpret_cast<float4*>(partial + L.oW2 + (size_t)f * H + c0);
+        float4* dst = reinterpret_cast<float4*>(partial + L.oW(2) + (size_t)f * H + c0);
 #pragma unroll
         for (int i = 0; i < 8; ++i) dst[i] = make_float4(v[4 * i], v[4 * i + 1], v[4 * i + 2], v[4 * i + 3]);
       }
       float v[16];
       tmem_ld16(tmem + DW_TM_DB2 + lane_off, v);
-      partial[L.ob2 + f] = v[BIAS_K];
+      partial[L.ob(2) + f] = v[BIAS_K];
     }
     tc_fence_before();
   }

@@ -893,10 +893,10 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
     if (lane == 0) { mf->wsum[(warp & 3) * 2] = s0; mf->wsum[(warp & 3) * 2 + 1] = s1; }
     bar_sync(BAR_ROW, ROW_THREADS);
     if (tid == EPI_THREADS) {
-      const GradLayout L(A.pol.in_dim, A.pol.out_dim, H);
+      const GradLayout L(A.pol.in_dim, A.pol.out_dim, H, 2);
       float* partial = a.partial + (size_t)blockIdx.x * a.partial_stride;
-      partial[L.ob3 + 0] = (mf->wsum[0] + mf->wsum[2]) + (mf->wsum[4] + mf->wsum[6]);
-      if (NA > 1) partial[L.ob3 + 1] = (mf->wsum[1] + mf->wsum[3]) + (mf->wsum[5] + mf->wsum[7]);
+      partial[L.obout + 0] = (mf->wsum[0] + mf->wsum[2]) + (mf->wsum[4] + mf->wsum[6]);
+      if (NA > 1) partial[L.obout + 1] = (mf->wsum[1] + mf->wsum[3]) + (mf->wsum[5] + mf->wsum[7]);
     }
   }
   if (ROLE == ROLE_EPI && acc_issued > 0) mbar_wait(&b->acc_done, (acc_issued - 1) & 1, 20000 + __LINE__);   // last D1 accumulation complete
@@ -904,7 +904,7 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
     tc_fence_before();
     if (elected) bulk_wait_all();
     if (BWD) {
-      const GradLayout L(A.pol.in_dim, A.pol.out_dim, H);
+      const GradLayout L(A.pol.in_dim, A.pol.out_dim, H, 2);
       float* partial = a.partial + (size_t)blockIdx.x * a.partial_stride;
       if (any_dw && hc == 0) {
         // D1 / D3: TMEM lane = feature inside the 128-feature half, columns = input index (BIAS_K: bias) / action
@@ -923,7 +923,7 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
           tmem_ld16(tm_d3 + half * 16 + lane_off, v);
 #pragma unroll
           for (int j = 0; j < 2; ++j)
-            if (j < ncol3) partial[L.oW3 + (size_t)f * A.pol.out_dim + j] = v[j] + v[2 + j];
+            if (j < ncol3) partial[L.oWout + (size_t)f * A.pol.out_dim + j] = v[j] + v[2 + j];
         }
       }
     }

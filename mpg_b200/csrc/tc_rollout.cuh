@@ -186,8 +186,9 @@ inline bool tc_set_smem(K kernel, int bytes) {
   return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes) == cudaSuccess;
 }
 
-inline bool tc_init(TcState& t, const mpg_config& cfg, int /*sms*/, size_t& ws_bytes) {
+inline bool tc_init(TcState& t, const mpg_config& cfg, int hidden_layers, int /*sms*/, size_t& ws_bytes) {
   if (cfg.hidden != tc::H) return true;                  // every layout of this path is built for 256; stay on FFMA
+  if (hidden_layers != 2) return true;                   // and for two hidden layers; stay on FFMA
   if (cfg.obs_dim + cfg.act_dim + 1 > 16) return true;   // first-layer K must fit one UMMA k-step; stay on FFMA
   auto alloc = [&](void** p, size_t n) {
     if (cudaMalloc(p, n) != cudaSuccess) return false;
@@ -222,9 +223,9 @@ inline void tc_destroy(TcState& t) {
 // flat: Keras-order natural weights W1|b1|W2|b2|W3|b3 on the device
 inline bool tc_pack_weights(TcState& t, int net, const float* flat, int in_dim, int out_dim, cudaStream_t st) {
   if (!t.nets[net].big_fwd) return true;   // tensor-core path not configured for this handle
-  const GradLayout L(in_dim, out_dim, tc::H);
-  tc::pack_big_image<true><<<32, 256, 0, st>>>(flat + L.oW2, 1, tc::H, t.nets[net].big_fwd);     // value(n,k) = W2[k][n]
-  tc::pack_big_image<false><<<32, 256, 0, st>>>(flat + L.oW2, tc::H, 1, t.nets[net].big_dx);      // value(k,n) = W2[k][n]
+  const GradLayout L(in_dim, out_dim, tc::H, 2);
+  tc::pack_big_image<true><<<32, 256, 0, st>>>(flat + L.oW(2), 1, tc::H, t.nets[net].big_fwd);     // value(n,k) = W2[k][n]
+  tc::pack_big_image<false><<<32, 256, 0, st>>>(flat + L.oW(2), tc::H, 1, t.nets[net].big_dx);      // value(k,n) = W2[k][n]
   tc::pack_l1_image<true><<<2, 256, 0, st>>>(flat + L.oW1, flat + L.ob1, in_dim, tc::BIAS_K, t.nets[net].l1);
   tc::pack_l1_image<false><<<2, 256, 0, st>>>(flat + L.oW1, flat + L.ob1, in_dim, tc::BIAS_K, t.nets[net].l1b, 1.4426950408889634f);   // z1 log2(e) for every activation, see act_grad_log2e
   tc::pack_in_image<<<2, 256, 0, st>>>(flat + L.oW1, in_dim, t.nets[net].in);
@@ -232,10 +233,10 @@ inline bool tc_pack_weights(TcState& t, int net, const float* flat, int in_dim, 
 }
 
 inline tc::TcNet tc_net(const TcState& t, int net, const float* flat, int in_dim, int out_dim) {
-  const GradLayout L(in_dim, out_dim, tc::H);
+  const GradLayout L(in_dim, out_dim, tc::H, 2);
   tc::TcNet n;
   n.big_fwd = t.nets[net].big_fwd; n.big_dx = t.nets[net].big_dx; n.l1 = t.nets[net].l1; n.l1b = t.nets[net].l1b; n.in = t.nets[net].in;
-  n.W3 = flat + L.oW3; n.b2 = flat + L.ob2; n.b3 = flat + L.ob3;
+  n.W3 = flat + L.oWout; n.b2 = flat + L.ob(2); n.b3 = flat + L.obout;
   n.in_dim = in_dim; n.out_dim = out_dim;
   return n;
 }

@@ -14,6 +14,14 @@ from ._lib import MpgConfig, RolloutParams, ENV_IDS
 BACKEND_FFMA, BACKEND_TC = 0, 1
 
 
+def mlp_shapes(in_dim, hidden, out_dim, layers=2):
+    """Keras shapes [W1,b1,W2,b2,..,WL,bL,Wout,bout] of an MLPNet with `layers` hidden layers (model.py:20-43)."""
+    shapes = [(in_dim, hidden), (hidden,)]
+    for _ in range(layers - 1):
+        shapes += [(hidden, hidden), (hidden,)]
+    return shapes + [(hidden, out_dim), (out_dim,)]
+
+
 def _ptr(t):
     if t is None:
         return None
@@ -26,7 +34,11 @@ class Engine:
 
     def __init__(self, env_id, obs_dim, act_dim, obs_scale, rew_scale, rew_shift, gamma,
                  policy_out_activation='tanh', action_range=None, num_future_data=0, hidden=256,
-                 max_rows=4096, max_horizon=25, device=None, debug_lib=False, hidden_activation='elu', **_unused):
+                 max_rows=4096, max_horizon=25, device=None, debug_lib=False, hidden_activation='elu', hidden_layers=2,
+                 **_unused):
+        if int(hidden_layers) not in _lib.HIDDEN_LAYERS:
+            raise ValueError(f'hidden_layers must be one of {_lib.HIDDEN_LAYERS} (got {hidden_layers!r})')
+        self.hidden_layers = int(hidden_layers)
         self.lib = _lib.load(debug=bool(debug_lib))   # debug_lib: the library with the development probes (tests / tools)
         if not torch.cuda.is_available():
             raise RuntimeError('mpg_b200 needs a CUDA device (B200, sm_100a); there is no CPU fallback')
@@ -56,9 +68,9 @@ class Engine:
         self._weights = {}
         self.h = ctypes.c_void_p()
         with torch.cuda.device(self.device):
-            rc = self.lib.mpg_create(ctypes.byref(cfg), ctypes.byref(self.h))
+            rc = self.lib.mpg_create_layers(ctypes.byref(cfg), self.hidden_layers, ctypes.byref(self.h))
         if rc != 0:
-            raise RuntimeError('mpg_create failed: ' + self.lib.mpg_last_error(None).decode())
+            raise RuntimeError('mpg_create_layers failed: ' + self.lib.mpg_last_error(None).decode())
         self._check(self.lib.mpg_set_activation(self.h, _lib.ACTIVATIONS[hidden_activation]))
         self.state_dim = self.lib.mpg_state_dim(self.h)
         self.num_sms = self.lib.mpg_num_sms(self.h)
@@ -85,9 +97,9 @@ class Engine:
         self.cfg.max_rows = max(int(rows), self.cfg.max_rows)
         self.cfg.max_horizon = max(int(horizon), self.cfg.max_horizon)
         with torch.cuda.device(self.device):
-            rc = self.lib.mpg_create(ctypes.byref(self.cfg), ctypes.byref(self.h))
+            rc = self.lib.mpg_create_layers(ctypes.byref(self.cfg), self.hidden_layers, ctypes.byref(self.h))
         if rc != 0:
-            raise RuntimeError('mpg_create failed: ' + self.lib.mpg_last_error(None).decode())
+            raise RuntimeError('mpg_create_layers failed: ' + self.lib.mpg_last_error(None).decode())
         self._check(self.lib.mpg_set_activation(self.h, _lib.ACTIVATIONS[self.hidden_activation]))
         for net, w in saved.items():
             self.set_net_weights(net, w)
@@ -148,30 +160,31 @@ class Engine:
 
     # ------------------------------------------------------------------ weights
     def net_shapes(self, net):
-        """Keras shapes [W1,b1,W2,b2,W3,b3] of slot `net` (model.py:20-43: kernels are (in, out))."""
+        """Keras shapes [W1,b1,W2,b2,..,WL,bL,Wout,bout] of slot `net` (model.py:20-43: kernels are (in, out))."""
         is_pol = net in (_lib.NET_POLICY, _lib.NET_POLICY_TARGET)
-        i, o, h = (self.obs_dim, 2 * self.act_dim, self.cfg.hidden) if is_pol else (self.obs_dim + self.act_dim, 1, self.cfg.hidden)
-        return [(i, h), (h,), (h, h), (h,), (h, o), (o,)]
+        i, o = (self.obs_dim, 2 * self.act_dim) if is_pol else (self.obs_dim + self.act_dim, 1)
+        return mlp_shapes(i, self.cfg.hidden, o, self.hidden_layers)
 
     def set_net_weights(self, net, weights):
-        """weights: [W1,b1,W2,b2,W3,b3] numpy arrays or tensors in Keras layout (model.py:20-43).
+        """weights: [W1,b1,..,WL,bL,Wout,bout] (2 (L+1) arrays) numpy arrays or tensors in Keras layout (model.py:20-43).
         Like Keras' set_weights, a wrong count or shape raises ValueError (the C side copies fixed sizes)."""
         weights = list(weights)
         want = self.net_shapes(net)
-        if len(weights) != 6:
-            raise ValueError(f'net {net}: expected 6 weight arrays [W1,b1,W2,b2,W3,b3], got {len(weights)}')
+        if len(weights) != len(want):
+            raise ValueError(f'net {net}: expected {len(want)} weight arrays [W1,b1,..,Wout,bout] '
+                             f'({self.hidden_layers} hidden layers), got {len(weights)}')
         for k, (w, shp) in enumerate(zip(weights, want)):
             if tuple(np.shape(w)) != shp:
                 raise ValueError(f'net {net}: weight {k} has shape {tuple(np.shape(w))}, expected {shp}')
         ts = [self.dev(w) for w in weights]
-        arr = (ctypes.c_void_p * 6)(*[t.data_ptr() for t in ts])
+        arr = (ctypes.c_void_p * len(ts))(*[t.data_ptr() for t in ts])
         self._check(self.lib.mpg_set_weights(self.h, net, arr, self.stream))
         self._weights[net] = ts
 
     def get_net_weights(self, net):
         """Current weights of `net` read back from the handle (they change under mpg_adam_step / polyak)."""
         ts = [torch.empty_like(t) for t in self._weights[net]]
-        arr = (ctypes.c_void_p * 6)(*[t.data_ptr() for t in ts])
+        arr = (ctypes.c_void_p * len(ts))(*[t.data_ptr() for t in ts])
         self._check(self.lib.mpg_get_weights(self.h, net, arr, self.stream))
         return [t.cpu().numpy() for t in ts]
 

@@ -160,4 +160,5 @@ class LearnerBase(object):
         return pin[:n].numpy().copy()
 
     def _split_to_numpy(self, flat_host, nets):
-        return parallel.split_flat(flat_host, self.args.obs_dim, self.args.act_dim, nets, self.engine.cfg.hidden)
+        return parallel.split_flat(flat_host, self.args.obs_dim, self.args.act_dim, nets, self.engine.cfg.hidden,
+                                   self.engine.hidden_layers)

@@ -8,6 +8,8 @@ the hot path lives here."""
 import numpy as np
 import torch
 
+from .engine import mlp_shapes
+
 
 def dist_info():
     """(world_size, rank) of the default process group, (1, 0) when not initialised."""
@@ -28,18 +30,18 @@ def allreduce_flat(flat, world_size):
     return flat
 
 
-def net_shapes(obs_dim, act_dim, kind, hidden=256):
-    """Shapes of one net's [W1,b1,W2,b2,W3,b3] (Keras (in,out) kernels); kind 'q' or 'pi'."""
+def net_shapes(obs_dim, act_dim, kind, hidden=256, layers=2):
+    """Shapes of one net's [W1,b1,..,WL,bL,Wout,bout] (Keras (in,out) kernels, L = layers); kind 'q' or 'pi'."""
     in_dim = obs_dim + (act_dim if kind == 'q' else 0)
     out_dim = 1 if kind == 'q' else 2 * act_dim
-    return [(in_dim, hidden), (hidden,), (hidden, hidden), (hidden,), (hidden, out_dim), (out_dim,)]
+    return mlp_shapes(in_dim, hidden, out_dim, layers)
 
 
-def split_flat(flat_host, obs_dim, act_dim, nets, hidden=256):
+def split_flat(flat_host, obs_dim, act_dim, nets, hidden=256, layers=2):
     """flat fp32 host vector (concatenated nets) -> list of arrays in the reference's gradient-list order."""
     out, pos = [], 0
     for kind in nets:
-        for shape in net_shapes(obs_dim, act_dim, kind, hidden):
+        for shape in net_shapes(obs_dim, act_dim, kind, hidden, layers):
             n = int(np.prod(shape))
             out.append(flat_host[pos:pos + n].reshape(shape))
             pos += n

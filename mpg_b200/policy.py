@@ -2,7 +2,8 @@
 weights inside a libmpg_b200 handle.
 
 Kept: constructor keywords, get_weights / set_weights nested-list format
-(models + target_models, each [W1,b1,W2,b2,W3,b3] with Keras (in,out) kernels, policy.py:112-121),
+(models + target_models, each [W1,b1,W2,b2,W3,b3] with Keras (in,out) kernels, policy.py:112-121; 2 (L+1) arrays at
+L hidden layers),
 compute_action / compute_mode / compute_target_action / compute_Q1 / compute_Q2 / compute_Q1_target /
 compute_Q2_target on RAW-scaled ("processed") observations exactly like the reference.
 apply_gradients (policy.py:123-171) runs on the device-resident weights: Keras-Adam with PolynomialDecay
@@ -19,6 +20,7 @@ from .synthetic import make_mlp_weights
 
 HIDDEN_WIDTHS = (64, 128, 256)   # hidden widths the fp32 (FFMA) kernels are built for; tensor cores: 256 only
 HIDDEN_ACTIVATIONS = ('elu', 'relu', 'tanh')   # hidden activations both backends are built for
+HIDDEN_LAYERS = (1, 2, 3)   # hidden layers the fp32 (FFMA) kernels are built for; tensor cores: 2 only
 
 
 class PolicyWithQs(object):
@@ -27,8 +29,12 @@ class PolicyWithQs(object):
                  policy_hidden_activation='elu', policy_out_activation='tanh', policy_only=False, double_Q=False,
                  target=True, tau=0.005, delay_update=1, deterministic_policy=True, action_range=None, seed=0,
                  **kwargs):
-        if value_num_hidden_layers != 2 or policy_num_hidden_layers != 2:
-            raise NotImplementedError('the sm_100a kernels are built for 2 hidden layers (reference default)')
+        if value_num_hidden_layers != policy_num_hidden_layers:
+            raise NotImplementedError('value_num_hidden_layers and policy_num_hidden_layers must be equal: one depth per '
+                                      'handle (got %r and %r)' % (value_num_hidden_layers, policy_num_hidden_layers))
+        if policy_num_hidden_layers not in HIDDEN_LAYERS:
+            raise NotImplementedError('the sm_100a kernels are built for %s hidden layers (got %r)'
+                                      % (' / '.join(map(str, HIDDEN_LAYERS)), policy_num_hidden_layers))
         if value_num_hidden_units != policy_num_hidden_units:
             raise NotImplementedError('value_num_hidden_units and policy_num_hidden_units must be equal: one hidden '
                                       'width per handle (got %r and %r)' % (value_num_hidden_units, policy_num_hidden_units))
@@ -45,6 +51,7 @@ class PolicyWithQs(object):
         if not deterministic_policy:
             raise NotImplementedError('the model-based learners use deterministic_policy=True (train_script.py:273)')
         self.obs_dim, self.act_dim, self.hidden = obs_dim, act_dim, int(policy_num_hidden_units)
+        self.hidden_layers = int(policy_num_hidden_layers)
         self.hidden_activation = policy_hidden_activation
         self.policy_only, self.double_Q, self.target = policy_only, double_Q, target
         self.tau, self.delay_update, self.action_range = tau, delay_update, action_range
@@ -60,7 +67,8 @@ class PolicyWithQs(object):
                              rew_shift=kwargs.get('rew_shift', 0.0), gamma=kwargs.get('gamma', 0.99),
                              policy_out_activation=policy_out_activation, action_range=action_range,
                              num_future_data=kwargs.get('num_future_data', 0), hidden=self.hidden,
-                             hidden_activation=self.hidden_activation, max_rows=max(rows, 64),
+                             hidden_activation=self.hidden_activation, hidden_layers=self.hidden_layers,
+                             max_rows=max(rows, 64),
                              max_horizon=max(lists + [1]), device=kwargs.get('device'), debug_lib=kwargs.get('debug_lib', False))
         # slot order == get_weights() order (policy.py:72-89)
         if policy_only:
@@ -81,8 +89,9 @@ class PolicyWithQs(object):
 
     def _init(self, rng, slot):
         if slot in (_lib.NET_POLICY, _lib.NET_POLICY_TARGET):
-            return make_mlp_weights(rng, self.obs_dim, self.hidden, 2 * self.act_dim, bias_scale=0.0)
-        return make_mlp_weights(rng, self.obs_dim + self.act_dim, self.hidden, 1, bias_scale=0.0)
+            return make_mlp_weights(rng, self.obs_dim, self.hidden, 2 * self.act_dim, bias_scale=0.0,
+                                    layers=self.hidden_layers)
+        return make_mlp_weights(rng, self.obs_dim + self.act_dim, self.hidden, 1, bias_scale=0.0, layers=self.hidden_layers)
 
     # -- weights --------------------------------------------------------------------------------
     def get_weights(self):
@@ -111,7 +120,7 @@ class PolicyWithQs(object):
         import os
         with np.load(os.path.join(load_dir, 'ckpt_ite%d.npz' % iteration)) as blob:
             for s in self.model_slots + self.target_slots:
-                self.engine.set_net_weights(s, [blob['net%d_w%d' % (s, i)] for i in range(6)])
+                self.engine.set_net_weights(s, [blob['net%d_w%d' % (s, i)] for i in range(2 * (self.hidden_layers + 1))])
             for s in self.model_slots:
                 self.engine.set_adam_state(s, blob['net%d_adam_m' % s], blob['net%d_adam_v' % s])
                 self.opt_iterations[s] = int(blob['net%d_opt_iterations' % s])
@@ -130,7 +139,7 @@ class PolicyWithQs(object):
 
     def apply_gradients(self, iteration, grads):
         """PolicyWithQs.apply_gradients (policy.py:123-156). `grads`: the list compute_gradient returns (numpy,
-        Q1[,Q2],policy x [W1,b1,W2,b2,W3,b3]) or one flat device tensor in the same order (no host round trip)."""
+        Q1[,Q2],policy x [W1,b1,W2,b2,W3,b3], 2 (L+1) arrays each) or one flat device tensor in the same order (no host round trip)."""
         e = self.engine
         if isinstance(grads, torch.Tensor):
             flat = grads.to(e.device, torch.float32).contiguous()

@@ -31,25 +31,25 @@ def orthogonal(rng, rows, cols, gain):
     return (gain * q[:rows, :cols]).astype(np.float32)
 
 
-def make_mlp_weights(rng, in_dim, hidden, out_dim, bias_scale=0.05):
-    """[W1,b1,W2,b2,W3,b3] with Keras (in,out) kernels, fp32 (model.py:20-43 order)."""
+def make_mlp_weights(rng, in_dim, hidden, out_dim, bias_scale=0.05, layers=2):
+    """[W1,b1,W2,b2,..,WL,bL,Wout,bout] (L = layers hidden layers) with Keras (in,out) kernels, fp32 (model.py:20-43
+    order).  The draws are made in list order, so at layers = 2 a seed gives the same weights it always gave."""
     g = np.sqrt(2.0)
-    return [
-        orthogonal(rng, in_dim, hidden, g), (bias_scale * rng.standard_normal(hidden)).astype(np.float32),
-        orthogonal(rng, hidden, hidden, g), (bias_scale * rng.standard_normal(hidden)).astype(np.float32),
-        orthogonal(rng, hidden, out_dim, 1.0), (bias_scale * rng.standard_normal(out_dim)).astype(np.float32),
-    ]
+    w = [orthogonal(rng, in_dim, hidden, g), (bias_scale * rng.standard_normal(hidden)).astype(np.float32)]
+    for _ in range(layers - 1):
+        w += [orthogonal(rng, hidden, hidden, g), (bias_scale * rng.standard_normal(hidden)).astype(np.float32)]
+    return w + [orthogonal(rng, hidden, out_dim, 1.0), (bias_scale * rng.standard_normal(out_dim)).astype(np.float32)]
 
 
-def make_policy_with_qs_weights(seed, obs_dim, act_dim, hidden=256, double_q=True):
+def make_policy_with_qs_weights(seed, obs_dim, act_dim, hidden=256, double_q=True, layers=2):
     """Weights in PolicyWithQs.get_weights() order: models + target_models (policy.py:72-89,112-121).
     double_q: [Q1,Q2,policy, Q1t,Q2t,policyt]; else [Q1,policy, Q1t,policyt]. Targets are
     independent draws (not copies) so that target-network paths are distinguishable in tests."""
     rng = np.random.default_rng(seed)
     def q():
-        return make_mlp_weights(rng, obs_dim + act_dim, hidden, 1)
+        return make_mlp_weights(rng, obs_dim + act_dim, hidden, 1, layers=layers)
     def pi():
-        return make_mlp_weights(rng, obs_dim, hidden, 2 * act_dim)
+        return make_mlp_weights(rng, obs_dim, hidden, 2 * act_dim, layers=layers)
     if double_q:
         return [q(), q(), pi(), q(), q(), pi()]
     return [q(), pi(), q(), pi()]

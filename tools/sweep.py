@@ -7,6 +7,8 @@ Prints one JSON line per case (device time by CUDA events, 3 warm-ups, median of
 and `flop_per_state_step`.  The algorithmic FLOP per state-step at that width (SURVEY.md 8(a)) is printed to stderr.
 --activation (elu, relu, tanh; default elu) sets the hidden activation of the policy and Q nets; the lines of a
 non-default activation carry `activation`.
+--layers L (1, 2, 3; default 2) sets the number of hidden layers of the policy and Q nets; the lines of L != 2 carry
+`hidden_layers` and `flop_per_state_step`.
 --env / --mode / --rows / --backend restrict the sweep to the matching cases."""
 import argparse
 import json
@@ -24,12 +26,13 @@ from mpg_b200.policy import PolicyWithQs  # noqa: E402
 N = 25
 
 
-def flop_per_state_step(mode, H, d_o, d_a, n=N):
-    """SURVEY.md 8(a) algorithmic work of one policy-gradient update per state-step (row x horizon step).
+def flop_per_state_step(mode, H, d_o, d_a, n=N, L=2):
+    """SURVEY.md 8(a) algorithmic work of one policy-gradient update per state-step (row x horizon step), L hidden layers.
     nadp: full BPTT, (n+1) F_pi fwd + n 2F_pi bwd + (2F_pi - 2 d_o H) at t=0 + 3 F_Q;
-    mpg: default MPG, (n+1) F_pi + n F_pi + (2F_pi - 2 d_o H) + 4 F_Q."""
-    f_pi = 2 * (d_o * H + H * H + H * 2 * d_a)
-    f_q = 2 * ((d_o + d_a) * H + H * H + H)
+    mpg: default MPG, (n+1) F_pi + n F_pi + (2F_pi - 2 d_o H) + 4 F_Q.
+    The h1 recompute of the L = 3 backward pass is not algorithmic work and is not counted."""
+    f_pi = 2 * (d_o * H + (L - 1) * H * H + H * 2 * d_a)
+    f_q = 2 * ((d_o + d_a) * H + (L - 1) * H * H + H)
     if mode == 'nadp':
         total = (n + 1) * f_pi + n * 2 * f_pi + (2 * f_pi - 2 * d_o * H) + 3 * f_q
     else:
@@ -37,12 +40,14 @@ def flop_per_state_step(mode, H, d_o, d_a, n=N):
     return total / n
 
 
-def run(env_id, mode, B, backend, H=256, act='elu'):
+def run(env_id, mode, B, backend, H=256, act='elu', L=2):
     args = default_args('NADP' if mode == 'nadp' else 'MPG-v2', env_id, replay_batch_size=B,
                         value_num_hidden_units=H, policy_num_hidden_units=H,
-                        value_hidden_activation=act, policy_hidden_activation=act)
+                        value_hidden_activation=act, policy_hidden_activation=act,
+                        value_num_hidden_layers=L, policy_num_hidden_layers=L)
     pol = PolicyWithQs(**vars(args))
-    pol.set_weights(synthetic.make_policy_with_qs_weights(1, args.obs_dim, args.act_dim, H, double_q=(mode != 'nadp')))
+    pol.set_weights(synthetic.make_policy_with_qs_weights(1, args.obs_dim, args.act_dim, H, double_q=(mode != 'nadp'),
+                                                          layers=L))
     e = pol.engine
     if backend == 'tc':
         if not e.tc_available():
@@ -63,8 +68,10 @@ def run(env_id, mode, B, backend, H=256, act='elu'):
             ts.append(a.elapsed_time(b))
     ms = float(np.median(ts))
     r = dict(env=env_id, mode=mode, rows=B, backend=backend, ms=ms, state_steps_per_s=B * N / (ms * 1e-3))
-    if H != 256:
-        r.update(hidden=H, flop_per_state_step=flop_per_state_step(mode, H, args.obs_dim, args.act_dim))
+    if H != 256 or L != 2:
+        r.update(hidden=H, flop_per_state_step=flop_per_state_step(mode, H, args.obs_dim, args.act_dim, L=L))
+    if L != 2:
+        r.update(hidden_layers=L)
     if act != 'elu':
         r.update(activation=act)
     return r
@@ -74,6 +81,7 @@ if __name__ == '__main__':
     ap = argparse.ArgumentParser()
     ap.add_argument('--hidden', type=int, default=256, choices=(64, 128, 256))
     ap.add_argument('--activation', default='elu', choices=('elu', 'relu', 'tanh'))
+    ap.add_argument('--layers', type=int, default=2, choices=(1, 2, 3))
     ap.add_argument('--env', default=None)
     ap.add_argument('--mode', default=None, choices=('nadp', 'mpg'))
     ap.add_argument('--rows', type=int, default=None)
@@ -81,8 +89,9 @@ if __name__ == '__main__':
     o = ap.parse_args()
     for env in ('PathTracking-v0', 'InvertedPendulumConti-v0', 'InvertedDoublePendulum-v2'):
         a = default_args('NADP', env)
-        print(json.dumps(dict(hidden=o.hidden, env=env, flop_per_state_step={
-            m: flop_per_state_step(m, o.hidden, a.obs_dim, a.act_dim) for m in ('nadp', 'mpg')})), file=sys.stderr)
+        print(json.dumps(dict(hidden=o.hidden, hidden_layers=o.layers, env=env, flop_per_state_step={
+            m: flop_per_state_step(m, o.hidden, a.obs_dim, a.act_dim, L=o.layers) for m in ('nadp', 'mpg')})),
+              file=sys.stderr)
     cases = [('PathTracking-v0', 'nadp', b) for b in (256, 4096, 65536, 262144)]
     cases += [('PathTracking-v0', 'mpg', b) for b in (256, 65536, 262144)]
     for env in ('InvertedPendulumConti-v0', 'InvertedDoublePendulum-v2'):
@@ -97,7 +106,7 @@ if __name__ == '__main__':
                 continue  # full-BPTT dW2 operand store is 53 KB per row: call in <= 256K-row chunks
             if backend == 'ffma' and B > 262144:
                 continue
-            r = run(env, mode, B, backend, o.hidden, o.activation)
+            r = run(env, mode, B, backend, o.hidden, o.activation, o.layers)
             if r:
                 print(json.dumps(r), flush=True)
             torch.cuda.empty_cache()
