@@ -51,6 +51,10 @@ enum { MPG_OK = 0, MPG_ERR_ARG = -1, MPG_ERR_CUDA = -2, MPG_ERR_UNSUPPORTED = -3
 
 #define MPG_MAX_OBS 16
 #define MPG_MAX_LIST 8
+/* longest rollout list of any call: lists of up to MPG_MAX_LIST entries fit mpg_rollout_params, longer ones are
+ * handed over with mpg_set_rollout_list and selected with n_list = MPG_LIST_FROM_HANDLE */
+#define MPG_MAX_LIST_LONG 64
+#define MPG_LIST_FROM_HANDLE (-1)
 
 /* What the learner constructors read from `args` (mpg_learner.py:30-58, nadp.py:29-47) that the
  * device path needs. */
@@ -75,7 +79,9 @@ typedef struct {
   int32_t rows;              /* B on this device (before M-tiling) */
   int32_t M;                 /* args.M: tf.tile factor */
   int32_t horizon;           /* n = max(rollout list) */
-  int32_t n_list;            /* len(num_rollout_list_*) <= MPG_MAX_LIST */
+  int32_t n_list;            /* len(num_rollout_list_*) <= MPG_MAX_LIST, or MPG_LIST_FROM_HANDLE: list and list_w are
+                              * ignored and the call uses the list of the last mpg_set_rollout_list (up to
+                              * MPG_MAX_LIST_LONG entries, with the same semantics) */
   int32_t list[MPG_MAX_LIST];   /* rollout indices k (each <= horizon), in any order; an index may repeat */
   float list_w[MPG_MAX_LIST];   /* loss weights w_k (rule_based_weights; 1 for NADP), any sign, zero allowed.  Entries
                                  * are independent terms of the loss, like the reference's tf.stack over the list:
@@ -110,6 +116,13 @@ int mpg_set_weights(mpg_ctx* ctx, int net, const float* const w[], void* stream)
 /* copy back in Keras layout (PolicyWithQs.get_weights, policy.py:112-114), the same 2(L+1) pointers */
 int mpg_get_weights(mpg_ctx* ctx, int net, float* const w[], void* stream);
 
+/* ---- rollout lists longer than mpg_rollout_params holds ---------------------------------- */
+/* Copies n <= MPG_MAX_LIST_LONG host entries (list_host: rollout indices, list_w_host: loss weights; the semantics of
+ * mpg_rollout_params.list / list_w) into the handle.  Calls whose params have n_list = MPG_LIST_FROM_HANDLE use them
+ * until the next mpg_set_rollout_list; the indices are checked against each call's horizon.  Host-side only: nothing is
+ * enqueued, so the list may change between calls on one stream.  n > MPG_MAX_LIST_LONG returns MPG_ERR_ARG. */
+int mpg_set_rollout_list(mpg_ctx* ctx, int n, const int32_t* list_host, const float* list_w_host);
+
 /* ---- policy gradient through the model rollout ------------------------------------------- */
 /* MPGLearner.policy_forward_and_backward (mpg_learner.py:356-365) /
  * NADPLearner.policy_forward_and_backward (nadp.py:186-194): forward rollout with per-step state
@@ -136,7 +149,8 @@ int mpg_rollout_forward(mpg_ctx* ctx, const mpg_rollout_params* p, const float* 
 /* mean over the M tiles, then sum / sum of squares over rows (mpg_learner.py:272-274):
  * out[0..n_list) = sum_i mean_m R_k ; out[n_list..2 n_list) = sum_i (mean_m R_k)^2 */
 int mpg_returns_stats(mpg_ctx* ctx, const float* returns, int n_list, int rows, int M, float* out, void* stream);
-/* tile mean only: out (n_list, rows) -- the stop_gradient targets of nadp.py:120-126 */
+/* ^ n_list <= MPG_MAX_LIST_LONG.  Tile mean only: out (n_list, rows) -- the stop_gradient targets of nadp.py:120-126; any
+ * n_list (it keeps no per-list workspace) */
 int mpg_returns_tile_mean(mpg_ctx* ctx, const float* returns, int n_list, int rows, int M, float* out, void* stream);
 
 /* ---- Q side ------------------------------------------------------------------------------- */

@@ -9,6 +9,7 @@ LIB_PATH = os.environ.get('MPG_B200_LIB', os.path.join(_HERE, 'libmpg_b200.so'))
 DEBUG_LIB_PATH = os.environ.get('MPG_B200_DBG_LIB', os.path.join(_HERE, 'libmpg_b200_dbg.so'))
 
 MAX_OBS, MAX_LIST = 16, 8
+MAX_LIST_LONG, LIST_FROM_HANDLE = 64, -1   # mpg_set_rollout_list: lists longer than the params struct holds
 ENV_IDS = {'PathTracking-v0': 0, 'InvertedPendulumConti-v0': 1, 'InvertedDoublePendulum-v2': 2,
            'PathTracking-v0-real': 3}   # the ground-truth PathTrackingEnv (forward only)
 NET_Q1, NET_Q2, NET_POLICY, NET_Q1_TARGET, NET_Q2_TARGET, NET_POLICY_TARGET = range(6)
@@ -26,7 +27,7 @@ SYMBOLS = [
     'mpg_set_adam_state', 'mpg_env_sample',
     'mpg_replay_create', 'mpg_replay_destroy', 'mpg_replay_last_error', 'mpg_replay_size', 'mpg_replay_add',
     'mpg_replay_sample', 'mpg_replay_update_priorities', 'mpg_replay_tree_stats', 'mpg_q_bootstrap', 'mpg_env_step',
-    'mpg_set_activation', 'mpg_get_activation', 'mpg_create_layers', 'mpg_hidden_layers',
+    'mpg_set_activation', 'mpg_get_activation', 'mpg_create_layers', 'mpg_hidden_layers', 'mpg_set_rollout_list',
 ]
 # exported by libmpg_b200_dbg.so only (include/mpg_b200.h, #ifdef MPG_DEBUG_PROBES)
 DEBUG_SYMBOLS = ['mpg_tc_selftest', 'mpg_set_profile_buffer']
@@ -78,6 +79,7 @@ def load(debug=False):
         'mpg_param_count': (i32, [vp, i32]),
         'mpg_set_weights': (i32, [vp, i32, P(vp), vp]),
         'mpg_get_weights': (i32, [vp, i32, P(vp), vp]),
+        'mpg_set_rollout_list': (i32, [vp, i32, P(ctypes.c_int32), P(ctypes.c_float)]),
         'mpg_policy_grad': (i32, [vp, P(RolloutParams), vp, vp, vp, vp, vp]),
         'mpg_rollout_forward': (i32, [vp, P(RolloutParams), vp, vp, vp, vp, vp, vp, vp, vp]),
         'mpg_returns_stats': (i32, [vp, vp, i32, i32, i32, vp, vp]),

@@ -53,7 +53,7 @@ struct mpg_ctx {
   float* ckpt = nullptr;
   float* partial = nullptr;
   float* loss_partial = nullptr;
-  float* stats_part = nullptr;   // [MPG_MAX_LIST][RS_BLOCKS][2]
+  float* stats_part = nullptr;   // [MPG_MAX_LIST_LONG][RS_BLOCKS][2]
   float* red_part = nullptr;     // [2][64] partial sums of the two-stage reductions (squared error, gradient norm)
   size_t partial_stride = 0;
   size_t ws_bytes = 0;
@@ -62,6 +62,11 @@ struct mpg_ctx {
   int act = MPG_ACT_ELU;                  // hidden activation of every net (MPG_ACT_*)
   int layers = 2;                         // hidden layers of every net (1..MAX_LAYERS)
   int timing = 0, timed = 0;
+  int long_n = -1;                        // list of mpg_set_rollout_list (n_list = MPG_LIST_FROM_HANDLE); -1: never set
+  int32_t long_list[MPG_MAX_LIST_LONG];
+  float long_w[MPG_MAX_LIST_LONG];
+  FarStep* far_steps = nullptr;          // the list at steps >= STEP_TAB of the last long-horizon rollout (grows)
+  size_t far_cap = 0;                     // steps
   long long* prof = nullptr;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   cudaStream_t aux = nullptr;             // side stream: weight-gradient GEMMs of finished waves run under the tail wave
@@ -251,19 +256,25 @@ int check_net(mpg_ctx* ctx, int net) {
 
 int fill_rollout_args(mpg_ctx* ctx, const mpg_rollout_params* p, RolloutArgs& a) {
   const mpg_config& c = ctx->cfg;
-  if (p->rows <= 0 || p->M <= 0 || p->horizon < 0 || p->n_list < 0 || p->n_list > MPG_MAX_LIST)
+  const bool from_handle = p->n_list == MPG_LIST_FROM_HANDLE;
+  if (p->rows <= 0 || p->M <= 0 || p->horizon < 0 || (!from_handle && (p->n_list < 0 || p->n_list > MPG_MAX_LIST)))
     return fail(ctx, MPG_ERR_ARG, "bad rollout params%s");
+  if (from_handle && ctx->long_n < 0)
+    return fail(ctx, MPG_ERR_STATE, "n_list = MPG_LIST_FROM_HANDLE but mpg_set_rollout_list was never called%s");
   if ((long long)p->rows * p->M > c.max_rows || p->horizon > c.max_horizon)
     return fail(ctx, MPG_ERR_ARG, "rollout exceeds the capacity given to mpg_create (max_rows / max_horizon)%s");
-  for (int k = 0; k < p->n_list; ++k)
-    if (p->list[k] < 0 || p->list[k] > p->horizon) return fail(ctx, MPG_ERR_ARG, "rollout index outside [0, horizon]%s");
+  const int n_list = from_handle ? ctx->long_n : p->n_list;
+  const int32_t* list = from_handle ? ctx->long_list : p->list;
+  const float* list_w = from_handle ? ctx->long_w : p->list_w;
+  for (int k = 0; k < n_list; ++k)
+    if (list[k] < 0 || list[k] > p->horizon) return fail(ctx, MPG_ERR_ARG, "rollout index outside [0, horizon]%s");
   memset(&a, 0, sizeof(a));
   a.obs_dim = c.obs_dim; a.act_dim = c.act_dim; a.nfd = c.num_future_data; a.policy_out_tanh = c.policy_out_tanh;
   a.action_range = c.action_range;
   for (int i = 0; i < MPG_MAX_OBS; ++i) a.obs_scale[i] = c.obs_scale[i];
   a.rew_scale = c.rew_scale; a.rew_shift = c.rew_shift; a.gamma = c.gamma;
-  a.rows = p->rows; a.M = p->M; a.horizon = p->horizon; a.n_list = p->n_list;
-  for (int k = 0; k < p->n_list; ++k) { a.list[k] = p->list[k]; a.list_w[k] = p->list_w[k]; }
+  a.rows = p->rows; a.M = p->M; a.horizon = p->horizon; a.n_list = n_list;
+  for (int k = 0; k < n_list; ++k) { a.list[k] = list[k]; a.list_w[k] = list_w[k]; }
   a.full_bptt = p->full_bptt;
   a.has_q = p->q_net >= 0;
   a.global_rows = p->global_rows > 0 ? p->global_rows : p->rows;
@@ -280,6 +291,30 @@ int fill_rollout_args(mpg_ctx* ctx, const mpg_rollout_params* p, RolloutArgs& a)
   a.ckpt = ctx->ckpt;
   a.partial = ctx->partial;
   a.partial_stride = (long long)ctx->partial_stride;
+  return MPG_OK;
+}
+
+// the list at steps [STEP_TAB, horizon] (StepTab serves the steps below from shared memory)
+__global__ void far_steps_kernel(const __grid_constant__ RolloutArgs a, FarStep* __restrict__ out) {
+  const int t = STEP_TAB + blockIdx.x * blockDim.x + threadIdx.x;
+  if (t <= a.horizon) out[t - STEP_TAB] = list_step(a.list, a.list_w, a.n_list, t);
+}
+
+// a.far_steps for a horizon that reaches past the shared-memory step tables; nothing to do for shorter ones
+int prepare_far_steps(mpg_ctx* ctx, RolloutArgs& a, cudaStream_t st) {
+  a.far_steps = nullptr;
+  if (a.horizon < STEP_TAB) return MPG_OK;
+  const size_t n = (size_t)(a.horizon + 1 - STEP_TAB);
+  if (n > ctx->far_cap) {
+    FarStep* p = nullptr;
+    CUDA_OK(ctx, cudaMalloc((void**)&p, n * sizeof(FarStep)));
+    cudaFree(ctx->far_steps);
+    ctx->far_steps = p; ctx->far_cap = n;
+  }
+  far_steps_kernel<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(a, ctx->far_steps);
+  ctx->launches++;
+  CUDA_OK(ctx, cudaGetLastError());
+  a.far_steps = ctx->far_steps;
   return MPG_OK;
 }
 
@@ -487,7 +522,7 @@ int mpg_create_layers(const mpg_config* cfg, int hidden_layers, mpg_ctx** out) {
   c->partial_stride = (maxP + 3) & ~size_t(3);
   ok = ok && alloc(&c->ckpt, (size_t)(cfg->max_horizon + 1) * cfg->max_rows * c->S)
        && alloc(&c->partial, (size_t)2 * c->sms * c->partial_stride) && alloc(&c->loss_partial, c->sms)
-       && alloc(&c->stats_part, (size_t)MPG_MAX_LIST * 64 * 2) && alloc(&c->red_part, 128);
+       && alloc(&c->stats_part, (size_t)MPG_MAX_LIST_LONG * RS_BLOCKS * 2) && alloc(&c->red_part, 128);
   if (ok) ok = tc_init(c->tc, c->cfg, hidden_layers, c->sms, c->ws_bytes);
   wait_dbg_init();   // best effort: without it a timed-out wait still traps, only the record is missing
   if (!ok) {
@@ -527,6 +562,7 @@ void mpg_destroy(mpg_ctx* c) {
     cudaFree(c->nets[n].adam_m); cudaFree(c->nets[n].adam_v);
   }
   cudaFree(c->ckpt); cudaFree(c->partial); cudaFree(c->loss_partial); cudaFree(c->stats_part); cudaFree(c->red_part);
+  cudaFree(c->far_steps);
   if (c->ev0) { cudaEventDestroy(c->ev0); cudaEventDestroy(c->ev1); }
   if (c->aux) { cudaStreamSynchronize(c->aux); cudaStreamDestroy(c->aux); }
   if (c->ev_wave) cudaEventDestroy(c->ev_wave);
@@ -660,6 +696,14 @@ int mpg_get_weights(mpg_ctx* ctx, int net, float* const w[], void* stream) {
   return MPG_OK;
 }
 
+int mpg_set_rollout_list(mpg_ctx* ctx, int n, const int32_t* list_host, const float* list_w_host) {
+  if (!ctx || n < 0 || (n > 0 && (!list_host || !list_w_host))) return fail(ctx, MPG_ERR_ARG, "bad argument to mpg_set_rollout_list%s");
+  if (n > MPG_MAX_LIST_LONG) return fail(ctx, MPG_ERR_ARG, "rollout list too long: at most 64 (MPG_MAX_LIST_LONG) entries%s");
+  for (int k = 0; k < n; ++k) { ctx->long_list[k] = list_host[k]; ctx->long_w[k] = list_w_host[k]; }
+  ctx->long_n = n;
+  return MPG_OK;
+}
+
 int mpg_policy_grad(mpg_ctx* ctx, const mpg_rollout_params* p, const float* obs, const float* noise, float* grad_out,
                     float* returns_out, void* stream) {
   if (!ctx || !p || !obs || !grad_out) return fail(ctx, MPG_ERR_ARG, "null argument to mpg_policy_grad%s");
@@ -670,11 +714,14 @@ int mpg_policy_grad(mpg_ctx* ctx, const mpg_rollout_params* p, const float* obs,
   if (rc) return rc;
   a.obs = obs; a.noise = noise; a.returns_out = returns_out;
   a.noise_mode = noise ? 1 : (p->use_philox ? 2 : 0);
+  if ((rc = prepare_far_steps(ctx, a, st))) return rc;
   const int MB = p->rows * p->M;
   if (ctx->backend == MPG_BACKEND_TC) {
     // tensor-core path: fused rollout + BPTT (dX chain), then the split-K weight-gradient GEMMs
     const int ntiles = (MB + tc::ACT_ROWS - 1) / tc::ACT_ROWS;
     const int grid = ntiles < ctx->sms ? ntiles : ctx->sms;
+    if (!tc_ensure_act_ckpt(ctx->tc, (size_t)a.n_list * MB * MAX_A * sizeof(float)))
+      return fail(ctx, MPG_ERR_CUDA, "cudaMalloc of the action checkpoints failed%s");
     tc::TcArgs ta = tc_args(ctx, a, p->policy_net, p->q_net);
     ta.store_steps = p->full_bptt ? p->horizon + 1 : 1;
     const size_t need = (size_t)ntiles * ta.store_steps * tc::SLOT_BYTES;
@@ -746,6 +793,7 @@ int mpg_rollout_forward(mpg_ctx* ctx, const mpg_rollout_params* p, const float* 
   a.start_actions = start_actions; a.use_start_actions = start_actions != nullptr;
   a.traj_obs = traj_obs; a.traj_rew = traj_rew; a.traj_act = traj_act;
   a.noise_mode = noise ? 1 : (p->use_philox ? 2 : 0);
+  if ((rc = prepare_far_steps(ctx, a, st))) return rc;
   const int MB = p->rows * p->M;
   int env = ctx->cfg.env;
   if (p->real_env) {
@@ -770,9 +818,9 @@ int mpg_rollout_forward(mpg_ctx* ctx, const mpg_rollout_params* p, const float* 
 
 int mpg_returns_stats(mpg_ctx* ctx, const float* returns, int n_list, int rows, int M, float* out, void* stream) {
   if (!ctx || !returns || !out || n_list <= 0) return fail(ctx, MPG_ERR_ARG, "bad argument to mpg_returns_stats%s");
-  if (n_list > MPG_MAX_LIST) return fail(ctx, MPG_ERR_ARG, "n_list too large%s");
+  if (n_list > MPG_MAX_LIST_LONG) return fail(ctx, MPG_ERR_ARG, "n_list too large: at most 64 (MPG_MAX_LIST_LONG)%s");
   returns_stats_kernel<<<dim3(n_list, RS_BLOCKS), 256, 0, (cudaStream_t)stream>>>(returns, n_list, rows, M, nullptr, ctx->stats_part);
-  returns_stats_final_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(ctx->stats_part, n_list, out);
+  returns_stats_final_kernel<<<1, MPG_MAX_LIST_LONG, 0, (cudaStream_t)stream>>>(ctx->stats_part, n_list, out);
   ctx->launches += 2;
   CUDA_OK(ctx, cudaGetLastError());
   return MPG_OK;
@@ -804,6 +852,8 @@ int mpg_q_grad(mpg_ctx* ctx, int net, int rows, int64_t global_rows, const float
     RolloutArgs a;
     if ((rc = fill_rollout_args(ctx, &p, a))) return rc;
     a.use_start_actions = 1; a.start_actions = act; a.obs = obs; a.returns_out = ctx->tc.qtmp;
+    if (!tc_ensure_act_ckpt(ctx->tc, (size_t)rows * MAX_A * sizeof(float)))
+      return fail(ctx, MPG_ERR_CUDA, "cudaMalloc of the action checkpoints failed%s");
     tc::TcArgs ta = tc_args(ctx, a, net, net);
     ta.q_regress = 1; ta.q_target = target; ta.q_inv_rows = 1.f / (float)a.global_rows;
     const int ntiles = (rows + tc::ACT_ROWS - 1) / tc::ACT_ROWS;

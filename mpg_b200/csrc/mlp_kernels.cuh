@@ -39,6 +39,7 @@ inline const MlpKernels& mlp_kernels(int hidden, int act) {
 template <int H, int ACT>
 struct MlpLaunch {
   static constexpr int SMEM = Smem<H>::FLOATS * 4, TC_SMEM = tc::SM_TOTAL + 1024;
+  static constexpr int ROLLOUT_SMEM = SMEM + (int)((sizeof(StepTab) + 15) / 16 * 16);   // + the list's step tables
 
   static cudaError_t set_smem() {
     cudaError_t e = cudaSuccess;
@@ -48,7 +49,7 @@ struct MlpLaunch {
     for_each_env([&](auto env, auto bwd) {
       constexpr int ENV = decltype(env)::value;
       constexpr bool BWD = decltype(bwd)::value;
-      set(rollout_kernel<H, ACT, ENV, BWD>, SMEM);
+      set(rollout_kernel<H, ACT, ENV, BWD>, ROLLOUT_SMEM);
       if constexpr (H == tc::H) set(tc::tc_rollout_kernel<ENV, BWD, ACT>, TC_SMEM);
     });
     set(q_grad_kernel<H, ACT>, SMEM);
@@ -58,7 +59,7 @@ struct MlpLaunch {
   }
   static bool rollout(int env, bool bwd, const RolloutArgs& a, int grid, cudaStream_t st) {
     return with_env(env, bwd, [&](auto e, auto b) {
-      rollout_kernel<H, ACT, decltype(e)::value, decltype(b)::value><<<grid, NT, SMEM, st>>>(a);
+      rollout_kernel<H, ACT, decltype(e)::value, decltype(b)::value><<<grid, NT, ROLLOUT_SMEM, st>>>(a);
     });
   }
   static void q_grad(const QGradArgs& a, int grid, cudaStream_t st) { q_grad_kernel<H, ACT><<<grid, NT, SMEM, st>>>(a); }

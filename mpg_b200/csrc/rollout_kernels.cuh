@@ -9,6 +9,8 @@
 
 namespace mpg {
 
+struct FarStep { float wq, wlater; int first, q; };   // one step of the rollout list, see list_step
+
 struct RolloutArgs {
   // learner config
   int obs_dim, act_dim, nfd, policy_out_tanh;
@@ -17,9 +19,10 @@ struct RolloutArgs {
   float rew_scale, rew_shift, gamma;
   // rollout
   int rows, M, horizon, n_list;
-  int list[MPG_MAX_LIST];
-  float list_w[MPG_MAX_LIST];
+  int list[MPG_MAX_LIST_LONG];
+  float list_w[MPG_MAX_LIST_LONG];
   int full_bptt, has_q, use_start_actions, noise_mode;  // noise_mode: 0 none, 1 tensor, 2 philox
+  const FarStep* far_steps;   // [horizon + 1 - STEP_TAB] the list at steps >= STEP_TAB (nullptr: the horizon stays below)
   long long global_rows, row_offset;
   unsigned long long seed;
   // pointers
@@ -35,6 +38,71 @@ struct RolloutArgs {
   long long partial_stride;   // floats, multiple of 4 (float4 accesses into the hidden -> hidden dW regions)
   NetDev pol, q;
 };
+
+// One step of the rollout list: the summed weight of the entries at step t (the upstream of Q(p_t, a_t)), the summed
+// weight of the entries at steps > t (the weight of the reward of step t), the first entry at t (-1: t is not in the list)
+// and whether some entry at t has a non-zero weight (step t has a Q part).  The sums run over the entries in list order.
+__device__ __forceinline__ FarStep list_step(const int* list, const float* list_w, int n, int t) {
+  FarStep r{0.f, 0.f, -1, 0};
+  for (int k = 0; k < n; ++k) {
+    const int l = list[k];
+    const float w = list_w[k];
+    if (l == t) {
+      r.wq += w;
+      if (r.first < 0) r.first = k;
+      if (w != 0.f) r.q = 1;
+    } else if (l > t) {
+      r.wlater += w;
+    }
+  }
+  return r;
+}
+
+// What the rollout list means at each step, built once per CTA so that no step scans the list (an indexed load of the list
+// from the kernel parameters costs ~1.5 K cycles on the row threads).  Steps [0, STEP_TAB) are tables in 3.1 KB of shared
+// memory (what the tensor-core kernel has left beside its 221 KB of images, DESIGN 4.2); a later step -- only horizons
+// beyond STEP_TAB reach one -- reads its FarStep from a global table the host side builds before the launch
+// (RolloutArgs::far_steps).  Either way a per-step question is one load.  Both kernels keep the tables behind their other
+// shared memory (ROLLOUT_SMEM, SM_TAB), which stays where it was.
+constexpr int STEP_TAB = 256;
+struct StepTab {
+  float wq_[STEP_TAB];
+  float wlater_[STEP_TAB];
+  int list[MPG_MAX_LIST_LONG];              // the list, staged for the build
+  float w[MPG_MAX_LIST_LONG];
+  const FarStep* far;                       // steps >= STEP_TAB
+  signed char first_[STEP_TAB];
+  signed char next[MPG_MAX_LIST_LONG];      // next entry at the step of entry k, -1: none
+  unsigned char q_[STEP_TAB];
+
+  __device__ __forceinline__ float wq(int t) const { return t < STEP_TAB ? wq_[t] : far[t - STEP_TAB].wq; }
+  __device__ __forceinline__ float wlater(int t) const { return t < STEP_TAB ? wlater_[t] : far[t - STEP_TAB].wlater; }
+  __device__ __forceinline__ int first(int t) const { return t < STEP_TAB ? first_[t] : far[t - STEP_TAB].first; }
+  __device__ __forceinline__ bool q_part(int t) const { return t < STEP_TAB ? q_[t] != 0 : far[t - STEP_TAB].q != 0; }
+};
+
+// every thread of the CTA takes part (contains __syncthreads()); the caller synchronises the CTA before the first read.
+// The list is staged in shared memory first: one parameter load per entry instead of one per entry and table step.
+__device__ __forceinline__ void build_step_tab(StepTab& T, const int* list, const float* list_w, int n, const FarStep* far,
+                                               int tid, int nthreads) {
+  for (int k = tid; k < MPG_MAX_LIST_LONG; k += nthreads) {
+    T.list[k] = k < n ? list[k] : -1;
+    T.w[k] = k < n ? list_w[k] : 0.f;
+  }
+  if (tid == 0) T.far = far;
+  __syncthreads();
+  for (int i = tid; i < STEP_TAB + MPG_MAX_LIST_LONG; i += nthreads) {
+    if (i < STEP_TAB) {
+      const FarStep r = list_step(T.list, T.w, n, i);
+      T.wq_[i] = r.wq; T.wlater_[i] = r.wlater; T.first_[i] = (signed char)r.first; T.q_[i] = (unsigned char)r.q;
+    } else {
+      const int k = i - STEP_TAB;
+      int nx = -1;
+      for (int j = n - 1; j > k; --j) if (T.list[j] == T.list[k]) nx = j;
+      T.next[k] = (signed char)nx;
+    }
+  }
+}
 
 // policy head (policy.py:193-199): z -> m = out_act(z) -> a = action_range * tanh(m) | m
 __device__ __forceinline__ float head_fwd(float z, int out_tanh, float range) {
@@ -60,9 +128,12 @@ template <int H, int ACT, int ENV, bool BWD>
 __global__ void __launch_bounds__(NT, 1) rollout_kernel(const __grid_constant__ RolloutArgs a) {
   extern __shared__ float4 smem_raw[];
   Smem<H> sm(reinterpret_cast<float*>(smem_raw));
+  StepTab& tab = *reinterpret_cast<StepTab*>(reinterpret_cast<float*>(smem_raw) + Smem<H>::FLOATS);   // behind the tiles
   using E = Env<ENV>;
   constexpr int S = E::S, A = E::A;
   const int tid = threadIdx.x;
+  build_step_tab(tab, a.list, a.list_w, a.n_list, a.far_steps, tid, blockDim.x);
+  __syncthreads();
   const int MB = a.rows * a.M;
   const int ntiles = (MB + TILE_R - 1) / TILE_R;
   const bool rowthread = tid < TILE_R;
@@ -115,9 +186,8 @@ __global__ void __launch_bounds__(NT, 1) rollout_kernel(const __grid_constant__ 
           if (a.traj_act && valid) a.traj_act[((size_t)t * MB + grow) * A + j] = act[j];
         }
       }
-      bool listed = false;
-      for (int k = 0; k < a.n_list; ++k) if (a.list[k] == t) listed = true;
-      if (listed) {
+      const int k0 = tab.first(t);
+      if (k0 >= 0) {
         float qv = 0.f;
         if (a.has_q) {
           __syncthreads();
@@ -126,8 +196,7 @@ __global__ void __launch_bounds__(NT, 1) rollout_kernel(const __grid_constant__ 
         }
         // every entry of step t gets its row, repeated entries included
         if (valid && a.returns_out)
-          for (int k = 0; k < a.n_list; ++k)
-            if (a.list[k] == t) a.returns_out[(size_t)k * MB + grow] = rsum + gpow * qv;
+          for (int k = k0; k >= 0; k = tab.next[k]) a.returns_out[(size_t)k * MB + grow] = rsum + gpow * qv;
       }
       if (t < a.horizon && rowthread && valid) {
         float eps = 0.f;
@@ -181,11 +250,8 @@ __global__ void __launch_bounds__(NT, 1) rollout_kernel(const __grid_constant__ 
           }
         }
         // Q part of step t: the summed weight of every entry at t; entries that all weigh zero are stats only
-        float w_t = 0.f;
-        bool q_part = false;
-        for (int k = 0; k < a.n_list; ++k)
-          if (a.list[k] == t) { w_t += a.list_w[k]; q_part = q_part || a.list_w[k] != 0.f; }
-        if (q_part && a.has_q) {
+        if (tab.q_part(t) && a.has_q) {
+          const float w_t = tab.wq(t);
           // Q input-gradient: upstream c w_t gamma^t on Q1(p_t, a_t)
           if (rowthread) {
 #pragma unroll
@@ -207,9 +273,7 @@ __global__ void __launch_bounds__(NT, 1) rollout_kernel(const __grid_constant__ 
           mlp_forward_tile<H, ACT>(a.pol, sm, A);   // the Q pass reused bufA/bufB: recompute every layer of the policy
         }
         if (t < a.horizon && rowthread && valid) {
-          float Wt = 0.f;
-          for (int k = 0; k < a.n_list; ++k) if (a.list[k] > t) Wt += a.list_w[k];
-          const float rc = cscale * Wt * gp * a.rew_scale;
+          const float rc = cscale * tab.wlater(t) * gp * a.rew_scale;
           env_step_bwd<ENV>(s, act, lam, rc, g_s, g_a, snext);
         }
         if (rowthread) {

@@ -46,7 +46,7 @@ constexpr size_t SLOT_BYTES = 270336;
 struct TcArgs {
   RolloutArgs r;            // config, lists, pointers (r.pol / r.q unused here)
   TcNet pol, q;
-  float* act_ckpt;          // [n_list][M*rows][A] actions at the list steps (for the Q input gradient)
+  float* act_ckpt;          // [n_list][M*rows][A] actions at the list steps, at the first entry of each (Q input gradient)
   float* z_ckpt;            // [horizon+1][M*rows][2A] action and head derivative d act / d z of every step (BPTT re-reads them)
   uint8_t* h2store;         // [tile][horizon+1][2*ACT_SPLIT] h2 images of the forward pass (BPTT loads them instead of
                             //    recomputing layer 2)
@@ -75,7 +75,9 @@ struct MiscF {
 static_assert(sizeof(MiscF) <= SmemMap::MISC_BYTES, "MISC region too small");
 
 constexpr int SM_D3IMG = SmemMap::TOTAL;          // delta3 image hi|lo (8 KB) appended after the base map
-constexpr int SM_TOTAL = SM_D3IMG + 8192;
+constexpr int SM_TAB = SM_D3IMG + 8192;           // StepTab of the rollout list
+constexpr int SM_TOTAL = SM_TAB + (int)((sizeof(StepTab) + 15) / 16 * 16);
+static_assert(SM_TOTAL + 1024 <= 227 * 1024, "the rollout kernel's shared memory (+ 1 KB of alignment slack) exceeds 227 KB");
 
 __device__ __forceinline__ void epi_bar() { asm volatile("bar.sync 1, %0;" ::"n"(EPI_THREADS) : "memory"); }
 __device__ __forceinline__ float elu_fast(float x) { return x > 0.f ? x : exp_fast(x) - 1.f; }
@@ -412,23 +414,7 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
 #endif
   };
 
-  // which steps are in the rollout list (bit t), and which of those carry a non-zero weight: looked up once per kernel
-  // instead of scanning the list several times in every step of every tile (steps >= 64 scan)
-  unsigned long long list_bits = 0ull, q_bits = 0ull;
-#pragma unroll
-  for (int k = 0; k < MPG_MAX_LIST; ++k)
-    if (k < a.n_list && a.list[k] < 64) {
-      list_bits |= 1ull << a.list[k];
-      if (a.list_w[k] != 0.f) q_bits |= 1ull << a.list[k];
-    }
-  auto list_index = [&](int tt) {       // position of step tt in the list, or -1
-    int kidx = -1;
-    if (tt >= 64 || ((list_bits >> tt) & 1ull)) {
-#pragma unroll
-      for (int k = 0; k < MPG_MAX_LIST; ++k) if (k < a.n_list && a.list[k] == tt) kidx = k;
-    }
-    return kidx;
-  };
+  const StepTab& tab = *reinterpret_cast<const StepTab*>(smem + SM_TAB);   // what the list means at each step
 
   const int tile_end = A.tile1 > 0 && A.tile1 < ntiles ? A.tile1 : ntiles;
   for (int tile = A.tile0 + blockIdx.x; tile < tile_end; tile += gridDim.x) {
@@ -598,7 +584,7 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
       if (valid && a.traj_act)
 #pragma unroll
         for (int j = 0; j < NA; ++j) a.traj_act[((size_t)t * MB + grow) * NA + j] = act[j];
-      const int kidx = list_index(t);   // fixed trip count inside: immediate constant-bank offsets (an indexed LDC is slow)
+      const int kidx = tab.first(t);   // the first entry at step t keys the action checkpoint of the step
       if (kidx >= 0) {
         float qv = 0.f;
         if (BWD && valid)
@@ -608,11 +594,9 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
           if (rowthread) write_pimg(s, act, true);
           qv = q_forward(false, nullptr);
         }
-        // every entry of step t gets its row, repeated entries included (kidx is the last of them)
+        // every entry of step t gets its row, repeated entries included
         if (valid && a.returns_out)
-#pragma unroll
-          for (int k = 0; k < MPG_MAX_LIST; ++k)
-            if (k < a.n_list && a.list[k] == t) a.returns_out[(size_t)k * MB + grow] = rsum + gpow * qv;
+          for (int k = kidx; k >= 0; k = tab.next[k]) a.returns_out[(size_t)k * MB + grow] = rsum + gpow * qv;
       }
       if (t < a.horizon && valid) {
         float eps = 0.f;
@@ -642,12 +626,7 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
 #pragma unroll
       for (int j = 0; j < 2 * NA; ++j)
         zpre_n[j] = (valid && !A.q_regress) ? A.z_ckpt[((size_t)a.horizon * MB + grow) * (2 * NA) + j] : 0.f;
-      float w_later = 0.f;     // sum of the list weights of the steps behind t (the reward of step t counts for those returns)
       for (int t = a.horizon; t >= 0; --t) {
-        if (t < a.horizon && list_index(t + 1) >= 0) {
-#pragma unroll
-          for (int k = 0; k < MPG_MAX_LIST; ++k) if (k < a.n_list && a.list[k] == t + 1) w_later += a.list_w[k];
-        }
         float gp = 1.f;
         for (int i = 0; i < t; ++i) gp *= a.gamma;
         const bool want_dw = a.full_bptt || t == 0;
@@ -675,27 +654,13 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
           }
         }
         if (ROLE == ROLE_ROW) stamp(4);
-        const int kidx = list_index(t);
+        const int kidx = tab.first(t);
         if (want_dw) any_dw = true;
         // ---- Q input gradient at the list steps: upstream c w_t gamma^t on Q1(p_t, a_t), w_t = the summed weight of
         // every entry at step t ----
-        float w_k = 0.f;
-        if (kidx >= 0) {
-#pragma unroll
-          for (int k = 0; k < MPG_MAX_LIST; ++k) if (k < a.n_list && a.list[k] == t) w_k += a.list_w[k];
-        }
         // does step tt start with a Q part (which uses the activation image before the policy part does)?  Yes when some
         // entry at tt has a non-zero weight: the h2 prefetch schedule below and the gate of the Q part both ask this
-        auto q_part_at = [&](int tt) {
-          bool q = false;
-          if (tt < 64) {
-            q = (q_bits >> tt) & 1ull;
-          } else {
-#pragma unroll
-            for (int k = 0; k < MPG_MAX_LIST; ++k) if (k < a.n_list && a.list[k] == tt && a.list_w[k] != 0.f) q = true;
-          }
-          return q && a.has_q;
-        };
+        auto q_part_at = [&](int tt) { return tab.q_part(tt) && a.has_q; };
         // early: the h2 image of this step was requested during the previous one; early_next: request the next one
         const bool early = t < a.horizon && !q_part_at(t);
         const bool early_next = t > 0 && !q_part_at(t - 1) && !A.q_regress;
@@ -736,8 +701,8 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
             mbar_arrive(&b->p_full);
           }
           if (rowthread) {
-            // upstream on Q: policy loss c w_k gamma^t, or the regression residual (Q - target) / B_global
-            const float up = !valid ? 0.f : (reg ? (qv - A.q_target[i_idx]) * A.q_inv_rows : cscale * w_k * gp);
+            // upstream on Q: policy loss c w_t gamma^t, or the regression residual (Q - target) / B_global
+            const float up = !valid ? 0.f : (reg ? (qv - A.q_target[i_idx]) * A.q_inv_rows : cscale * tab.wq(t) * gp);
             mf->d3s[row] = up;
             if (reg) {
               write_d3(d3_img, row, up, 0.f);
@@ -789,7 +754,7 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
           tc_fence_before();         // the g_p read of the previous step precedes the next g_p UMMAs (ordered through p_full)
           stamp(5);
           if (t < a.horizon && valid) {
-            env_step_bwd<ENV, true>(s, act, lam, cscale * w_later * gp * a.rew_scale, g_s, g_a, snext);
+            env_step_bwd<ENV, true>(s, act, lam, cscale * tab.wlater(t) * gp * a.rew_scale, g_s, g_a, snext);
           }
           stamp(14);
           float d3[2] = {0.f, 0.f};
@@ -958,6 +923,8 @@ __global__ void __launch_bounds__(ROLLOUT_THREADS, 1) tc_rollout_kernel(const __
     }
   }
   for (int i = threadIdx.x; i < 8192 / 16; i += blockDim.x) reinterpret_cast<uint4*>(smem + SM_D3IMG)[i] = make_uint4(0u, 0u, 0u, 0u);
+  build_step_tab(*reinterpret_cast<StepTab*>(smem + SM_TAB), A.r.list, A.r.list_w, A.r.n_list, A.r.far_steps, threadIdx.x,
+                 blockDim.x);
   if (threadIdx.x == 0) {
     mf->b3[0] = A.pol.b3[0];
     mf->b3[1] = Env<ENV>::A > 1 ? A.pol.b3[1] : 0.f;

@@ -171,7 +171,8 @@ struct TcState {
   bool ready = false;
   TcNetImages nets[MPG_NUM_NETS];
   uint8_t* scratch_img = nullptr;   // self-test image
-  float* act_ckpt = nullptr;        // [MPG_MAX_LIST][max_rows][MAX_A]
+  float* act_ckpt = nullptr;        // [n_list][max_rows][MAX_A]: MPG_MAX_LIST entries at creation, grows with longer lists
+  size_t act_ckpt_bytes = 0;
   float* qtmp = nullptr;            // [max_rows] Q values of the regression pass / of the target evaluations
   float* qtmp2 = nullptr;           // [max_rows] second Q value (double-Q minimum, TD error)
   float* z_ckpt = nullptr;          // [max_horizon+1][max_rows][2 MAX_A] action and head derivative of every step (BPTT)
@@ -196,7 +197,7 @@ inline bool tc_init(TcState& t, const mpg_config& cfg, int hidden_layers, int /*
     return true;
   };
   bool ok = alloc((void**)&t.scratch_img, tc::BIG_IMAGE_BYTES)
-            && alloc((void**)&t.act_ckpt, (size_t)MPG_MAX_LIST * cfg.max_rows * MAX_A * sizeof(float))
+            && alloc((void**)&t.act_ckpt, t.act_ckpt_bytes = (size_t)MPG_MAX_LIST * cfg.max_rows * MAX_A * sizeof(float))
             && alloc((void**)&t.z_ckpt, (size_t)(cfg.max_horizon + 1) * cfg.max_rows * 2 * MAX_A * sizeof(float))
             && alloc((void**)&t.qtmp, (size_t)cfg.max_rows * sizeof(float))
             && alloc((void**)&t.qtmp2, (size_t)cfg.max_rows * sizeof(float));
@@ -251,6 +252,15 @@ inline bool tc_ensure_buf(uint8_t*& buf, size_t& have, size_t bytes) {
 }
 inline bool tc_ensure_store(TcState& t, size_t bytes) { return tc_ensure_buf(t.store, t.store_bytes, bytes); }
 inline bool tc_ensure_h2store(TcState& t, size_t bytes) { return tc_ensure_buf(t.h2store, t.h2store_bytes, bytes); }
+// the old buffer stays when the larger one cannot be had
+inline bool tc_ensure_act_ckpt(TcState& t, size_t bytes) {
+  if (bytes <= t.act_ckpt_bytes) return true;
+  float* p = nullptr;
+  if (cudaMalloc((void**)&p, bytes) != cudaSuccess) { cudaGetLastError(); return false; }
+  cudaFree(t.act_ckpt);
+  t.act_ckpt = p; t.act_ckpt_bytes = bytes;
+  return true;
+}
 
 #ifdef MPG_DEBUG_PROBES
 // self test of one GEMM kind (see tc_gemm.cuh): W is fp32 [256 x 256] (kind 0), [16 x 256] (kinds 1, 2)

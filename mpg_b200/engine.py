@@ -22,6 +22,12 @@ def mlp_shapes(in_dim, hidden, out_dim, layers=2):
     return shapes + [(hidden, out_dim), (out_dim,)]
 
 
+def check_list_len(rollout_list):
+    """A rollout list has at most 64 entries (MPG_MAX_LIST_LONG); raises before anything reaches the device."""
+    if len(rollout_list) > _lib.MAX_LIST_LONG:
+        raise ValueError(f'rollout list has {len(rollout_list)} entries; at most {_lib.MAX_LIST_LONG} are supported')
+
+
 def _ptr(t):
     if t is None:
         return None
@@ -212,9 +218,15 @@ class Engine:
                 noise_seed, use_philox, real_env=False):
         p = RolloutParams()
         p.rows, p.M, p.horizon, p.n_list = int(rows), int(M), int(horizon), len(rollout_list)
-        for i, k in enumerate(rollout_list):
-            p.list[i] = int(k)
-            p.list_w[i] = float(list_w[i])
+        if len(rollout_list) <= _lib.MAX_LIST:
+            for i, k in enumerate(rollout_list):
+                p.list[i] = int(k)
+                p.list_w[i] = float(list_w[i])
+        else:   # longer lists are handed to the handle; the call selects them (the list was checked by the caller)
+            n = len(rollout_list)
+            self._check(self.lib.mpg_set_rollout_list(self.h, n, (ctypes.c_int32 * n)(*[int(k) for k in rollout_list]),
+                                                      (ctypes.c_float * n)(*[float(w) for w in list_w])))
+            p.n_list = _lib.LIST_FROM_HANDLE
         p.full_bptt, p.q_net, p.policy_net = int(full_bptt), int(q_net), int(policy_net)
         p.global_rows, p.row_offset = int(global_rows or rows), int(row_offset)
         p.noise_seed, p.use_philox, p.real_env = int(noise_seed), int(use_philox), int(bool(real_env))
@@ -222,7 +234,8 @@ class Engine:
 
     def policy_grad(self, obs, rollout_list, list_w, M=1, full_bptt=True, q_net=_lib.NET_Q1, policy_net=_lib.NET_POLICY,
                     noise=None, use_philox=False, noise_seed=0, global_rows=None, row_offset=0, want_returns=True):
-        """-> (flat unclipped gradient (P,), returns (n_list, M*rows) or None)."""
+        """-> (flat unclipped gradient (P,), returns (n_list, M*rows) or None).  Up to 64 list entries."""
+        check_list_len(rollout_list)
         rows, horizon = obs.shape[0], max(rollout_list)
         if self.backend == BACKEND_TC and full_bptt and rows * M > self.MAX_TC_FULL_BPTT_ROWS:
             return self._policy_grad_chunked(obs, rollout_list, list_w, M, q_net, policy_net, noise, use_philox,
@@ -265,6 +278,7 @@ class Engine:
     def rollout_forward(self, obs, rollout_list, M=1, q_net=_lib.NET_Q1, policy_net=_lib.NET_POLICY, start_actions=None,
                         noise=None, use_philox=False, noise_seed=0, global_rows=None, row_offset=0, want_traj=False,
                         horizon=None, real_env=False):
+        check_list_len(rollout_list)
         rows = obs.shape[0]
         horizon = max(rollout_list) if horizon is None else horizon
         self.ensure_capacity(rows * M, horizon)
@@ -287,12 +301,14 @@ class Engine:
 
     def returns_stats(self, returns, rows, M):
         n_list = returns.shape[0]
+        check_list_len(range(n_list))
         out = self.empty(2 * n_list)
         self._check(self.lib.mpg_returns_stats(self.h, _ptr(returns), n_list, rows, M, _ptr(out), self.stream))
         return out
 
     def returns_tile_mean(self, returns, rows, M):
         n_list = returns.shape[0]
+        check_list_len(range(n_list))
         out = self.empty(n_list, rows)
         self._check(self.lib.mpg_returns_tile_mean(self.h, _ptr(returns), n_list, rows, M, _ptr(out), self.stream))
         return out

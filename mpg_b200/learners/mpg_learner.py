@@ -12,6 +12,11 @@ from .base import LearnerBase, rule_based_weights
 
 class MPGLearner(LearnerBase):
     def __init__(self, policy_cls, args):
+        lst = list(args.num_rollout_list_for_policy_update)
+        n_run = len(lst) + (0 not in lst)   # policy_forward_and_backward adds step 0
+        if n_run > _lib.MAX_LIST_LONG:
+            raise ValueError(f'num_rollout_list_for_policy_update has {len(lst)} entries ({n_run} with the step 0 every '
+                             f'update adds for value_mean); at most {_lib.MAX_LIST_LONG} are supported')
         super().__init__(policy_cls, args)
         self.sample_num_in_learner = self.args.sample_num_in_learner
         n = len(self.num_rollout_list_for_policy_update)

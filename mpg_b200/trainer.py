@@ -1,7 +1,7 @@
 """Trainer (trainer.py:18-80) for the single-process topology: one worker, one replay buffer, one learner and one
 evaluator on one GPU, sharing ONE PolicyWithQs so that no weight ever crosses the host.
     python -m mpg_b200.trainer --alg MPG-v2 --iters 2000 [--hidden 64|128|256] [--activation elu|relu|tanh]
-    [--layers 1|2|3]"""
+    [--layers 1|2|3] [--rollout_list 1-25 | 0,25 | ...]"""
 import argparse
 import json
 import logging
@@ -42,6 +42,15 @@ class Trainer(object):
         return self.optimizer.eval_history
 
 
+def parse_rollout_list(text):
+    """'1-25' -> [1, .., 25]; '0,5,10-12' -> [0, 5, 10, 11, 12]"""
+    out = []
+    for part in text.split(','):
+        lo, _, hi = part.strip().partition('-')
+        out += list(range(int(lo), int(hi) + 1)) if hi else [int(lo)]
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--alg', default='MPG-v2')
@@ -51,6 +60,9 @@ def main():
     ap.add_argument('--activation', default='elu', choices=('elu', 'relu', 'tanh'),
                     help='hidden activation of the policy and Q nets')
     ap.add_argument('--layers', type=int, default=2, choices=(1, 2, 3), help='hidden layers of the policy and Q nets')
+    ap.add_argument('--rollout_list', default=None, type=parse_rollout_list,
+                    help='num_rollout_list_for_policy_update of MPG: comma-separated steps and ranges a-b, e.g. 1-25; '
+                         'up to 64 entries counting the step 0 MPG adds (default: the reference list)')
     ap.add_argument('--log_dir', default=None)
     o = ap.parse_args()
     logging.basicConfig(level=logging.INFO)
@@ -60,7 +72,8 @@ def main():
                         max_iter=o.iters, log_dir=o.log_dir, value_num_hidden_units=o.hidden,
                         policy_num_hidden_units=o.hidden, value_hidden_activation=o.activation,
                         policy_hidden_activation=o.activation, value_num_hidden_layers=o.layers,
-                        policy_num_hidden_layers=o.layers)
+                        policy_num_hidden_layers=o.layers,
+                        **({} if o.rollout_list is None else dict(num_rollout_list_for_policy_update=o.rollout_list)))
     import time
     trainer = Trainer(args)
     t0 = time.perf_counter()

@@ -9,10 +9,14 @@ and `flop_per_state_step`.  The algorithmic FLOP per state-step at that width (S
 non-default activation carry `activation`.
 --layers L (1, 2, 3; default 2) sets the number of hidden layers of the policy and Q nets; the lines of L != 2 carry
 `hidden_layers` and `flop_per_state_step`.
+--list dense runs MPG with the dense rollout list MPGLearner builds from num_rollout_list_for_policy_update = 1..25 (26
+entries with the step 0 it adds, rule_based_weights at iteration 0) instead of [0, 25]; every MPG line carries `list`.
+Every line carries the card's name and power limit.
 --env / --mode / --rows / --backend restrict the sweep to the matching cases."""
 import argparse
 import json
 import os
+import subprocess
 import sys
 
 import numpy as np
@@ -21,6 +25,7 @@ import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from mpg_b200 import synthetic  # noqa: E402
 from mpg_b200.config import default_args  # noqa: E402
+from mpg_b200.learners.base import rule_based_weights  # noqa: E402
 from mpg_b200.policy import PolicyWithQs  # noqa: E402
 
 N = 25
@@ -40,7 +45,27 @@ def flop_per_state_step(mode, H, d_o, d_a, n=N, L=2):
     return total / n
 
 
-def run(env_id, mode, B, backend, H=256, act='elu', L=2):
+def power_limit_w():
+    """the card's power limit: part of every number measured on it"""
+    try:
+        out = subprocess.run(['nvidia-smi', '--query-gpu=power.limit', '--format=csv,noheader,nounits', '-i',
+                              str(torch.cuda.current_device())], capture_output=True, text=True, timeout=30).stdout
+        return float(out.split()[0])
+    except (OSError, ValueError, IndexError, subprocess.SubprocessError):
+        return None
+
+
+def rollout_list(mode, dense):
+    """(list, weights, full BPTT) of one policy_grad call"""
+    if mode == 'nadp':
+        return [0, N], [0.0, 1.0], True
+    if dense:
+        ws = rule_based_weights(0, 9000, 0.1, list(range(1, N + 1)))
+        return list(range(N + 1)), [0.0] + [float(w) for w in ws], False
+    return [0, N], [0.42, 0.58], False
+
+
+def run(env_id, mode, B, backend, H=256, act='elu', L=2, dense=False):
     args = default_args('NADP' if mode == 'nadp' else 'MPG-v2', env_id, replay_batch_size=B,
                         value_num_hidden_units=H, policy_num_hidden_units=H,
                         value_hidden_activation=act, policy_hidden_activation=act,
@@ -56,7 +81,7 @@ def run(env_id, mode, B, backend, H=256, act='elu', L=2):
     else:
         e.set_backend(0)   # the handle defaults to the tensor-core backend wherever it covers the configuration
     obs = e.dev(synthetic.make_obs(np.random.default_rng(2), env_id, B))
-    lst, w, full = ([0, N], [0.0, 1.0], True) if mode == 'nadp' else ([0, N], [0.42, 0.58], False)
+    lst, w, full = rollout_list(mode, dense)
     ts = []
     for i in range(8):
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -74,6 +99,9 @@ def run(env_id, mode, B, backend, H=256, act='elu', L=2):
         r.update(hidden_layers=L)
     if act != 'elu':
         r.update(activation=act)
+    if mode == 'mpg':
+        r.update(list='dense 0..25' if dense else '[0, 25]')
+    r.update(gpu=torch.cuda.get_device_name(), power_limit_w=power_limit_w())
     return r
 
 
@@ -86,6 +114,7 @@ if __name__ == '__main__':
     ap.add_argument('--mode', default=None, choices=('nadp', 'mpg'))
     ap.add_argument('--rows', type=int, default=None)
     ap.add_argument('--backend', default=None, choices=('ffma', 'tc'))
+    ap.add_argument('--list', default='default', choices=('default', 'dense'))
     o = ap.parse_args()
     for env in ('PathTracking-v0', 'InvertedPendulumConti-v0', 'InvertedDoublePendulum-v2'):
         a = default_args('NADP', env)
@@ -106,7 +135,7 @@ if __name__ == '__main__':
                 continue  # full-BPTT dW2 operand store is 53 KB per row: call in <= 256K-row chunks
             if backend == 'ffma' and B > 262144:
                 continue
-            r = run(env, mode, B, backend, o.hidden, o.activation, o.layers)
+            r = run(env, mode, B, backend, o.hidden, o.activation, o.layers, o.list == 'dense')
             if r:
                 print(json.dumps(r), flush=True)
             torch.cuda.empty_cache()
