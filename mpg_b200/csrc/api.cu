@@ -19,8 +19,7 @@ struct NetStore {
   float* W1p = nullptr;
   float* Wp = nullptr;     // [L - 1][H][H]: the hidden -> hidden kernels W2..WL, packed columns (none at L = 1)
   float* WTp = nullptr;    // [L - 1][H][H]: their transposes, packed columns
-  float* adam_m = nullptr;   // Adam moments (allocated on the first optimiser step)
-  float* adam_v = nullptr;
+  DevBuf<float> adam_m, adam_v;   // Adam moments (allocated on the first optimiser step)
   int in_dim = 0, out_dim = 0;
   bool set = false;
 };
@@ -53,8 +52,9 @@ struct mpg_ctx {
   float* ckpt = nullptr;
   float* partial = nullptr;
   float* loss_partial = nullptr;
-  float* stats_part = nullptr;   // [MPG_MAX_LIST_LONG][RS_BLOCKS][2]
-  float* red_part = nullptr;     // [2][64] partial sums of the two-stage reductions (squared error, gradient norm)
+  float* stats_part = nullptr;   // [MPG_MAX_LIST_LONG][RED_BLOCKS][2]
+  float* red_part = nullptr;     // [2][RED_BLOCKS] partial sums of the two-stage reductions (squared error, gradient norm)
+  DevBuf<float> qtmp, qtmp2;     // [rows] Q values of the evaluations and of the tensor-core regression pass
   size_t partial_stride = 0;
   size_t ws_bytes = 0;
   uint64_t launches = 0;
@@ -65,8 +65,7 @@ struct mpg_ctx {
   int long_n = -1;                        // list of mpg_set_rollout_list (n_list = MPG_LIST_FROM_HANDLE); -1: never set
   int32_t long_list[MPG_MAX_LIST_LONG];
   float long_w[MPG_MAX_LIST_LONG];
-  FarStep* far_steps = nullptr;          // the list at steps >= STEP_TAB of the last long-horizon rollout (grows)
-  size_t far_cap = 0;                     // steps
+  DevBuf<FarStep> far_steps;             // the list at steps >= STEP_TAB of the last long-horizon rollout
   long long* prof = nullptr;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   cudaStream_t aux = nullptr;             // side stream: weight-gradient GEMMs of finished waves run under the tail wave
@@ -135,24 +134,16 @@ __global__ void adam_kernel(float* __restrict__ w, float* __restrict__ m, float*
   w[i] -= lr_t * mi / (sqrtf(vi) + eps);
 }
 
-// loss_sum = sum_i 0.5 (q_i - target_i)^2: CLIP_BLOCKS fixed slices, then their partial sums in index order
+// loss_sum = sum_i 0.5 (q_i - target_i)^2: RED_BLOCKS fixed slices, then their partial sums in index order
 __global__ void sq_err_partial_kernel(const float* __restrict__ q, const float* __restrict__ target, int n, float* __restrict__ part) {
-  __shared__ float red[256];
-  const int per = (n + 63) / 64, lo = blockIdx.x * per, hi = min(n, lo + per);
+  const int per = (n + RED_BLOCKS - 1) / RED_BLOCKS, lo = blockIdx.x * per, hi = min(n, lo + per);
   float s = 0.f;
   for (int i = lo + threadIdx.x; i < hi; i += blockDim.x) { const float d = q[i] - target[i]; s = fmaf(0.5f * d, d, s); }
-  red[threadIdx.x] = s;
-  __syncthreads();
-  for (int o = blockDim.x / 2; o > 0; o >>= 1) {
-    if (threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o];
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) part[blockIdx.x] = red[0];
+  s = block_sum(s);
+  if (threadIdx.x == 0) part[blockIdx.x] = s;
 }
-__global__ void sum_partials64_kernel(const float* __restrict__ part, float* __restrict__ out) {
-  float s = 0.f;
-  for (int b = 0; b < 64; ++b) s += part[b];
-  out[0] = s;
+__global__ void sum_partials_kernel(const float* __restrict__ part, float* __restrict__ out) {
+  out[0] = sum_in_order<RED_BLOCKS>(part);
 }
 
 __global__ void polyak_kernel(float* __restrict__ dst, const float* __restrict__ src, int n, float tau) {
@@ -176,66 +167,48 @@ __global__ void reduce_partials_kernel(const float* __restrict__ partial, size_t
   }
 }
 
-// tf.clip_by_global_norm in two stages (a single block needed 45 us for a 68K-float net: latency bound): CLIP_BLOCKS blocks
-// sum the squares of fixed slices, then every block adds the partial sums in index order (bit-reproducible) and scales
-// its slice.
-constexpr int CLIP_BLOCKS = 64;
+// tf.clip_by_global_norm in two stages (a single block needed 45 us for a 68K-float net: latency bound): RED_BLOCKS blocks
+// sum the squares of fixed slices, then every block adds the partial sums in index order and scales its slice.
 __global__ void sumsq_partial_kernel(const float* __restrict__ g, int n, float* __restrict__ part) {
-  __shared__ float red[256];
-  const int per = (n + CLIP_BLOCKS - 1) / CLIP_BLOCKS, lo = blockIdx.x * per, hi = min(n, lo + per);
+  const int per = (n + RED_BLOCKS - 1) / RED_BLOCKS, lo = blockIdx.x * per, hi = min(n, lo + per);
   float s = 0.f;
   for (int i = lo + threadIdx.x; i < hi; i += blockDim.x) s = fmaf(g[i], g[i], s);
-  red[threadIdx.x] = s;
-  __syncthreads();
-  for (int o = blockDim.x / 2; o > 0; o >>= 1) {
-    if (threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o];
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) part[blockIdx.x] = red[0];
+  s = block_sum(s);
+  if (threadIdx.x == 0) part[blockIdx.x] = s;
 }
 __global__ void clip_apply_kernel(float* __restrict__ g, int n, float clip, const float* __restrict__ part,
                                   float* __restrict__ norm_out) {
-  float tot = 0.f;
-  for (int b = 0; b < CLIP_BLOCKS; ++b) tot += part[b];
-  const float norm = sqrtf(tot);
+  const float norm = sqrtf(sum_in_order<RED_BLOCKS>(part));
   const float scale = clip * fminf(1.f / norm, 1.f / clip);   // tf.clip_by_global_norm
-  const int per = (n + CLIP_BLOCKS - 1) / CLIP_BLOCKS, lo = blockIdx.x * per, hi = min(n, lo + per);
+  const int per = (n + RED_BLOCKS - 1) / RED_BLOCKS, lo = blockIdx.x * per, hi = min(n, lo + per);
   if (scale != 1.f)
     for (int i = lo + threadIdx.x; i < hi; i += blockDim.x) g[i] *= scale;
   if (blockIdx.x == 0 && threadIdx.x == 0 && norm_out) norm_out[0] = norm;
 }
 
 // returns (n_list, M*rows) -> tile mean (n_list, rows) and/or sums over rows of mean, mean^2.
-// Two stages so that 64K-row batches do not serialise on one block: grid (n_list, RS_BLOCKS) partial sums in a
-// fixed slice order, then one block per k adds the RS_BLOCKS partials in index order (deterministic).
-constexpr int RS_BLOCKS = 64;
+// Two stages so that 64K-row batches do not serialise on one block: grid (n_list, RED_BLOCKS) partial sums of fixed
+// slices, then one thread per k adds the RED_BLOCKS partials in index order.
 __global__ void returns_stats_kernel(const float* __restrict__ ret, int n_list, int rows, int M,
                                      float* __restrict__ mean_out, float* __restrict__ part) {
-  __shared__ float red[2][256];
   const int k = blockIdx.x, blk = blockIdx.y;
-  const int per = (rows + RS_BLOCKS - 1) / RS_BLOCKS, lo = blk * per, hi = min(rows, lo + per);
-  float s1 = 0.f, s2 = 0.f;
+  const int per = (rows + RED_BLOCKS - 1) / RED_BLOCKS, lo = blk * per, hi = min(rows, lo + per);
+  float s[2] = {0.f, 0.f};
   for (int i = lo + threadIdx.x; i < hi; i += blockDim.x) {
     float m = 0.f;
     for (int t = 0; t < M; ++t) m += ret[(size_t)k * M * rows + (size_t)t * rows + i];
     m /= (float)M;
     if (mean_out) mean_out[(size_t)k * rows + i] = m;
-    s1 += m; s2 = fmaf(m, m, s2);
+    s[0] += m; s[1] = fmaf(m, m, s[1]);
   }
-  red[0][threadIdx.x] = s1; red[1][threadIdx.x] = s2;
-  __syncthreads();
-  for (int o = blockDim.x / 2; o > 0; o >>= 1) {
-    if (threadIdx.x < o) { red[0][threadIdx.x] += red[0][threadIdx.x + o]; red[1][threadIdx.x] += red[1][threadIdx.x + o]; }
-    __syncthreads();
-  }
-  if (threadIdx.x == 0 && part) { part[(k * RS_BLOCKS + blk) * 2] = red[0][0]; part[(k * RS_BLOCKS + blk) * 2 + 1] = red[1][0]; }
+  block_sum(s);
+  if (threadIdx.x == 0 && part) { part[(k * RED_BLOCKS + blk) * 2] = s[0]; part[(k * RED_BLOCKS + blk) * 2 + 1] = s[1]; }
 }
 __global__ void returns_stats_final_kernel(const float* __restrict__ part, int n_list, float* __restrict__ stats_out) {
   const int k = threadIdx.x;
   if (k >= n_list) return;
-  float s1 = 0.f, s2 = 0.f;
-  for (int b = 0; b < RS_BLOCKS; ++b) { s1 += part[(k * RS_BLOCKS + b) * 2]; s2 += part[(k * RS_BLOCKS + b) * 2 + 1]; }
-  stats_out[k] = s1; stats_out[n_list + k] = s2;
+  const float* pk = part + k * RED_BLOCKS * 2;
+  stats_out[k] = sum_in_order<RED_BLOCKS>(pk, 2); stats_out[n_list + k] = sum_in_order<RED_BLOCKS>(pk + 1, 2);
 }
 
 __global__ void philox_noise_kernel(unsigned long long seed, long long global_rows, long long row_offset, int rows,
@@ -305,17 +278,30 @@ int prepare_far_steps(mpg_ctx* ctx, RolloutArgs& a, cudaStream_t st) {
   a.far_steps = nullptr;
   if (a.horizon < STEP_TAB) return MPG_OK;
   const size_t n = (size_t)(a.horizon + 1 - STEP_TAB);
-  if (n > ctx->far_cap) {
-    FarStep* p = nullptr;
-    CUDA_OK(ctx, cudaMalloc((void**)&p, n * sizeof(FarStep)));
-    cudaFree(ctx->far_steps);
-    ctx->far_steps = p; ctx->far_cap = n;
-  }
-  far_steps_kernel<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(a, ctx->far_steps);
+  CUDA_OK(ctx, ctx->far_steps.grow(n));
+  far_steps_kernel<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(a, ctx->far_steps.p);
   ctx->launches++;
   CUDA_OK(ctx, cudaGetLastError());
-  a.far_steps = ctx->far_steps;
+  a.far_steps = ctx->far_steps.p;
   return MPG_OK;
+}
+
+// the Q scratch (ctx->qtmp, ctx->qtmp2) for `rows` rows
+int q_scratch(mpg_ctx* ctx, int rows) {
+  if (ctx->qtmp.grow(rows) != cudaSuccess || ctx->qtmp2.grow(rows) != cudaSuccess)
+    return fail(ctx, MPG_ERR_CUDA, "cudaMalloc of the Q scratch failed%s");
+  return MPG_OK;
+}
+
+// a rollout of horizon 0 over `rows` rows: the policy's action (or the given one) and, with q_net >= 0, the Q value of
+// that action as the returns row of the one-entry list {0}
+mpg_rollout_params horizon0_params(int rows, int policy_net, int q_net) {
+  mpg_rollout_params p;
+  memset(&p, 0, sizeof(p));
+  p.rows = rows; p.M = 1; p.horizon = 0;
+  p.n_list = q_net >= 0 ? 1 : 0; p.list[0] = 0; p.list_w[0] = 1.f;
+  p.q_net = q_net; p.policy_net = policy_net;
+  return p;
 }
 
 // dW2 = sum over (row, step) of h1^T delta2 is the only contraction of the path whose K is the batch.  With K in the
@@ -356,7 +342,7 @@ tc::TcArgs tc_args(const mpg_ctx* ctx, const RolloutArgs& a, int policy_net, int
   ta.r = a;
   ta.pol = tc_net(ctx->tc, policy_net, ctx->nets[policy_net].flat, a.pol.in_dim, a.pol.out_dim);
   if (a.has_q) ta.q = tc_net(ctx->tc, q_net, ctx->nets[q_net].flat, a.q.in_dim, a.q.out_dim);
-  ta.act_ckpt = ctx->tc.act_ckpt;
+  ta.act_ckpt = ctx->tc.act_ckpt.p;
   return ta;
 }
 
@@ -364,7 +350,7 @@ tc::TcArgs tc_args(const mpg_ctx* ctx, const RolloutArgs& a, int policy_net, int
 // part_row on: tc_dw_kernel, two CTAs per record, at most the even number of the `sms` SMs it may use
 void launch_dw(const mpg_ctx* ctx, const tc::TcArgs& ta, int tile0, int tiles, int part_row, int sms, cudaStream_t st) {
   tc::DwArgs da;
-  da.store = ctx->tc.store + (size_t)tile0 * ta.store_steps * tc::SLOT_BYTES;
+  da.store = ctx->tc.store.p + (size_t)tile0 * ta.store_steps * tc::SLOT_BYTES;
   da.nrecords = tiles * ta.store_steps;
   da.in_dim = ta.pol.in_dim; da.out_dim = ta.pol.out_dim;
   da.partial = ctx->partial + (size_t)part_row * ctx->partial_stride; da.partial_stride = (long long)ctx->partial_stride;
@@ -522,11 +508,17 @@ int mpg_create_layers(const mpg_config* cfg, int hidden_layers, mpg_ctx** out) {
   c->partial_stride = (maxP + 3) & ~size_t(3);
   ok = ok && alloc(&c->ckpt, (size_t)(cfg->max_horizon + 1) * cfg->max_rows * c->S)
        && alloc(&c->partial, (size_t)2 * c->sms * c->partial_stride) && alloc(&c->loss_partial, c->sms)
-       && alloc(&c->stats_part, (size_t)MPG_MAX_LIST_LONG * RS_BLOCKS * 2) && alloc(&c->red_part, 128);
+       && alloc(&c->stats_part, (size_t)MPG_MAX_LIST_LONG * RED_BLOCKS * 2) && alloc(&c->red_part, 2 * RED_BLOCKS);
   if (ok) ok = tc_init(c->tc, c->cfg, hidden_layers, c->sms, c->ws_bytes);
+  if (ok && c->tc.ready) {   // the tensor-core evaluations up to max_rows rows: their Q scratch is there from the start
+    ok = q_scratch(c, cfg->max_rows) == MPG_OK;
+    c->ws_bytes += 2 * (size_t)cfg->max_rows * sizeof(float);
+  }
   wait_dbg_init();   // best effort: without it a timed-out wait still traps, only the record is missing
   if (!ok) {
-    snprintf(g_create_err, 512, "cudaMalloc of the workspace failed: %s", cudaGetErrorString(cudaGetLastError()));
+    cudaError_t e = cudaGetLastError();   // a grow-only buffer has already taken its error off the record
+    snprintf(g_create_err, 512, "cudaMalloc of the workspace failed: %s",
+             cudaGetErrorString(e != cudaSuccess ? e : cudaErrorMemoryAllocation));
     mpg_destroy(c);
     return MPG_ERR_CUDA;
   }
@@ -559,10 +551,10 @@ void mpg_destroy(mpg_ctx* c) {
   if (!c) return;
   for (int n = 0; n < MPG_NUM_NETS; ++n) {
     cudaFree(c->nets[n].flat); cudaFree(c->nets[n].W1p); cudaFree(c->nets[n].Wp); cudaFree(c->nets[n].WTp);
-    cudaFree(c->nets[n].adam_m); cudaFree(c->nets[n].adam_v);
+    c->nets[n].adam_m.release(); c->nets[n].adam_v.release();
   }
   cudaFree(c->ckpt); cudaFree(c->partial); cudaFree(c->loss_partial); cudaFree(c->stats_part); cudaFree(c->red_part);
-  cudaFree(c->far_steps);
+  c->qtmp.release(); c->qtmp2.release(); c->far_steps.release();
   if (c->ev0) { cudaEventDestroy(c->ev0); cudaEventDestroy(c->ev1); }
   if (c->aux) { cudaStreamSynchronize(c->aux); cudaStreamDestroy(c->aux); }
   if (c->ev_wave) cudaEventDestroy(c->ev_wave);
@@ -618,11 +610,11 @@ static int repack(mpg_ctx* ctx, int net, cudaStream_t st) {
 }
 
 static int adam_alloc(mpg_ctx* ctx, NetStore& ns, int n, cudaStream_t st) {
-  if (ns.adam_m) return MPG_OK;
-  CUDA_OK(ctx, cudaMalloc(&ns.adam_m, n * sizeof(float)));
-  CUDA_OK(ctx, cudaMalloc(&ns.adam_v, n * sizeof(float)));
-  CUDA_OK(ctx, cudaMemsetAsync(ns.adam_m, 0, n * sizeof(float), st));
-  CUDA_OK(ctx, cudaMemsetAsync(ns.adam_v, 0, n * sizeof(float), st));
+  if (ns.adam_v.n >= (size_t)n) return MPG_OK;
+  CUDA_OK(ctx, ns.adam_m.grow(n));
+  CUDA_OK(ctx, ns.adam_v.grow(n));
+  CUDA_OK(ctx, cudaMemsetAsync(ns.adam_m.p, 0, n * sizeof(float), st));
+  CUDA_OK(ctx, cudaMemsetAsync(ns.adam_v.p, 0, n * sizeof(float), st));
   return MPG_OK;
 }
 
@@ -637,7 +629,7 @@ int mpg_adam_step(mpg_ctx* ctx, int net, const float* grad, float lr, int64_t st
   if ((rc = adam_alloc(ctx, ns, n, st))) return rc;
   const double t = (double)step;
   const float lr_t = (float)((double)lr * sqrt(1.0 - pow((double)beta2, t)) / (1.0 - pow((double)beta1, t)));
-  adam_kernel<<<(n + 255) / 256, 256, 0, st>>>(ns.flat, ns.adam_m, ns.adam_v, grad, n, lr_t, beta1, beta2, eps);
+  adam_kernel<<<(n + 255) / 256, 256, 0, st>>>(ns.flat, ns.adam_m.p, ns.adam_v.p, grad, n, lr_t, beta1, beta2, eps);
   ctx->launches++;
   CUDA_OK(ctx, cudaGetLastError());
   return repack(ctx, net, st);
@@ -651,8 +643,8 @@ int mpg_get_adam_state(mpg_ctx* ctx, int net, float* m, float* v, void* stream) 
   NetStore& ns = ctx->nets[net];
   const int n = layout(ctx, ns).total;
   if ((rc = adam_alloc(ctx, ns, n, st))) return rc;
-  CUDA_OK(ctx, cudaMemcpyAsync(m, ns.adam_m, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
-  CUDA_OK(ctx, cudaMemcpyAsync(v, ns.adam_v, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  CUDA_OK(ctx, cudaMemcpyAsync(m, ns.adam_m.p, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  CUDA_OK(ctx, cudaMemcpyAsync(v, ns.adam_v.p, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
   return MPG_OK;
 }
 
@@ -664,8 +656,8 @@ int mpg_set_adam_state(mpg_ctx* ctx, int net, const float* m, const float* v, vo
   NetStore& ns = ctx->nets[net];
   const int n = layout(ctx, ns).total;
   if ((rc = adam_alloc(ctx, ns, n, st))) return rc;
-  CUDA_OK(ctx, cudaMemcpyAsync(ns.adam_m, m, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
-  CUDA_OK(ctx, cudaMemcpyAsync(ns.adam_v, v, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  CUDA_OK(ctx, cudaMemcpyAsync(ns.adam_m.p, m, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  CUDA_OK(ctx, cudaMemcpyAsync(ns.adam_v.p, v, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
   return MPG_OK;
 }
 
@@ -720,17 +712,17 @@ int mpg_policy_grad(mpg_ctx* ctx, const mpg_rollout_params* p, const float* obs,
     // tensor-core path: fused rollout + BPTT (dX chain), then the split-K weight-gradient GEMMs
     const int ntiles = (MB + tc::ACT_ROWS - 1) / tc::ACT_ROWS;
     const int grid = ntiles < ctx->sms ? ntiles : ctx->sms;
-    if (!tc_ensure_act_ckpt(ctx->tc, (size_t)a.n_list * MB * MAX_A * sizeof(float)))
+    if (ctx->tc.act_ckpt.grow((size_t)a.n_list * MB * MAX_A) != cudaSuccess)
       return fail(ctx, MPG_ERR_CUDA, "cudaMalloc of the action checkpoints failed%s");
     tc::TcArgs ta = tc_args(ctx, a, p->policy_net, p->q_net);
     ta.store_steps = p->full_bptt ? p->horizon + 1 : 1;
     const size_t need = (size_t)ntiles * ta.store_steps * tc::SLOT_BYTES;
-    if (!tc_ensure_store(ctx->tc, need)) return fail(ctx, MPG_ERR_CUDA, "cudaMalloc of the dW operand store failed%s");
-    ta.store = ctx->tc.store;
+    if (ctx->tc.store.grow(need) != cudaSuccess) return fail(ctx, MPG_ERR_CUDA, "cudaMalloc of the dW operand store failed%s");
+    ta.store = ctx->tc.store.p;
     ta.rec_hi_only = rec_hi_only(ctx, (long long)MB * ta.store_steps);
-    if (!tc_ensure_h2store(ctx->tc, (size_t)ntiles * (p->horizon + 1) * 2 * tc::ACT_SPLIT))
+    if (ctx->tc.h2store.grow((size_t)ntiles * (p->horizon + 1) * 2 * tc::ACT_SPLIT) != cudaSuccess)
       return fail(ctx, MPG_ERR_CUDA, "cudaMalloc of the h2 image store failed%s");
-    ta.h2store = ctx->tc.h2store;
+    ta.h2store = ctx->tc.h2store.p;
     ta.z_ckpt = ctx->tc.z_ckpt;
     ta.prof = ctx->prof;
     // Wave-tail overlap: with ntiles = w * sms + tail the last wave leaves sms - tail SMs idle.  The full waves and
@@ -819,7 +811,7 @@ int mpg_rollout_forward(mpg_ctx* ctx, const mpg_rollout_params* p, const float* 
 int mpg_returns_stats(mpg_ctx* ctx, const float* returns, int n_list, int rows, int M, float* out, void* stream) {
   if (!ctx || !returns || !out || n_list <= 0) return fail(ctx, MPG_ERR_ARG, "bad argument to mpg_returns_stats%s");
   if (n_list > MPG_MAX_LIST_LONG) return fail(ctx, MPG_ERR_ARG, "n_list too large: at most 64 (MPG_MAX_LIST_LONG)%s");
-  returns_stats_kernel<<<dim3(n_list, RS_BLOCKS), 256, 0, (cudaStream_t)stream>>>(returns, n_list, rows, M, nullptr, ctx->stats_part);
+  returns_stats_kernel<<<dim3(n_list, RED_BLOCKS), 256, 0, (cudaStream_t)stream>>>(returns, n_list, rows, M, nullptr, ctx->stats_part);
   returns_stats_final_kernel<<<1, MPG_MAX_LIST_LONG, 0, (cudaStream_t)stream>>>(ctx->stats_part, n_list, out);
   ctx->launches += 2;
   CUDA_OK(ctx, cudaGetLastError());
@@ -828,7 +820,7 @@ int mpg_returns_stats(mpg_ctx* ctx, const float* returns, int n_list, int rows, 
 
 int mpg_returns_tile_mean(mpg_ctx* ctx, const float* returns, int n_list, int rows, int M, float* out, void* stream) {
   if (!ctx || !returns || !out || n_list <= 0) return fail(ctx, MPG_ERR_ARG, "bad argument to mpg_returns_tile_mean%s");
-  returns_stats_kernel<<<dim3(n_list, RS_BLOCKS), 256, 0, (cudaStream_t)stream>>>(returns, n_list, rows, M, out, nullptr);
+  returns_stats_kernel<<<dim3(n_list, RED_BLOCKS), 256, 0, (cudaStream_t)stream>>>(returns, n_list, rows, M, out, nullptr);
   ctx->launches++;
   CUDA_OK(ctx, cudaGetLastError());
   return MPG_OK;
@@ -843,24 +835,23 @@ int mpg_q_grad(mpg_ctx* ctx, int net, int rows, int64_t global_rows, const float
   if (ctx->backend == MPG_BACKEND_TC && rows <= ctx->cfg.max_rows) {
     // tensor-core path: the rollout kernel in regression mode (horizon 0, given actions) + the dW kernel
     const mpg_config& c = ctx->cfg;
-    mpg_rollout_params p;
-    memset(&p, 0, sizeof(p));
-    p.rows = rows; p.M = 1; p.horizon = 0; p.n_list = 1; p.list[0] = 0; p.list_w[0] = 1.f; p.full_bptt = 1;
+    // policy_net = net: unused in regression mode (actions are given, the policy part is skipped); fixes the gradient layout
+    mpg_rollout_params p = horizon0_params(rows, net, net);
+    p.full_bptt = 1;
     p.global_rows = global_rows;
-    p.q_net = net;
-    p.policy_net = net;   // unused in regression mode (actions are given, the policy part is skipped); fixes the gradient layout
     RolloutArgs a;
-    if ((rc = fill_rollout_args(ctx, &p, a))) return rc;
-    a.use_start_actions = 1; a.start_actions = act; a.obs = obs; a.returns_out = ctx->tc.qtmp;
-    if (!tc_ensure_act_ckpt(ctx->tc, (size_t)rows * MAX_A * sizeof(float)))
+    if ((rc = fill_rollout_args(ctx, &p, a)) || (rc = q_scratch(ctx, rows))) return rc;
+    a.use_start_actions = 1; a.start_actions = act; a.obs = obs; a.returns_out = ctx->qtmp.p;
+    if (ctx->tc.act_ckpt.grow((size_t)rows * MAX_A) != cudaSuccess)
       return fail(ctx, MPG_ERR_CUDA, "cudaMalloc of the action checkpoints failed%s");
     tc::TcArgs ta = tc_args(ctx, a, net, net);
     ta.q_regress = 1; ta.q_target = target; ta.q_inv_rows = 1.f / (float)a.global_rows;
     const int ntiles = (rows + tc::ACT_ROWS - 1) / tc::ACT_ROWS;
     const int grid = ntiles < ctx->sms ? ntiles : ctx->sms;
     ta.store_steps = 1;
-    if (!tc_ensure_store(ctx->tc, (size_t)ntiles * tc::SLOT_BYTES)) return fail(ctx, MPG_ERR_CUDA, "cudaMalloc of the dW operand store failed%s");
-    ta.store = ctx->tc.store;
+    if (ctx->tc.store.grow((size_t)ntiles * tc::SLOT_BYTES) != cudaSuccess)
+      return fail(ctx, MPG_ERR_CUDA, "cudaMalloc of the dW operand store failed%s");
+    ta.store = ctx->tc.store.p;
     // full hi + lo records always: a regression residual can be pure zero-mean noise (converged critic), the sum over the rows
     // then cancels to ~1/sqrt(rows) of its terms and the 2^-9 rounding of hi-only records would not average out relative
     // to it (measured 1.4e-3 at 262,144 rows); this GEMM is 0.04 ms, there is nothing to gain
@@ -870,8 +861,8 @@ int mpg_q_grad(mpg_ctx* ctx, int net, int rows, int64_t global_rows, const float
     launch_dw(ctx, ta, 0, ntiles, 0, ctx->sms, st);
     launch_reduce(ctx, net, ctx->sms, grad_out, nullptr, st);
     if (loss_sum_out) {
-      sq_err_partial_kernel<<<64, 256, 0, st>>>(ctx->tc.qtmp, target, rows, ctx->red_part);
-      sum_partials64_kernel<<<1, 1, 0, st>>>(ctx->red_part, loss_sum_out);
+      sq_err_partial_kernel<<<RED_BLOCKS, 256, 0, st>>>(ctx->qtmp.p, target, rows, ctx->red_part);
+      sum_partials_kernel<<<1, 1, 0, st>>>(ctx->red_part, loss_sum_out);
     }
     ctx->launches += 5;
     CUDA_OK(ctx, cudaGetLastError());
@@ -895,13 +886,21 @@ int mpg_q_grad(mpg_ctx* ctx, int net, int rows, int64_t global_rows, const float
   return MPG_OK;
 }
 
-static int launch_eval(mpg_ctx* ctx, EvalArgs& a, void* stream) {
+// the FFMA evaluation kernel over a replay batch: with q_net < 0 the actions pi_policy(sigma obs) into out, else
+// Q_q(sigma obs, a) into out and, with q2_net >= 0, Q_q2(sigma obs, a) into out2, a = act or pi_policy(sigma obs)
+static int ffma_eval(mpg_ctx* ctx, int policy_net, int rows, const float* obs, const float* act, int q_net, float* out,
+                     int q2_net, float* out2, void* stream) {
   const mpg_config& c = ctx->cfg;
-  a.obs_dim = c.obs_dim; a.act_dim = c.act_dim; a.policy_out_tanh = c.policy_out_tanh;
-  a.action_range = c.action_range; a.rew_scale = c.rew_scale; a.rew_shift = c.rew_shift;
-  if (a.mode != 4) a.gamma = c.gamma;   // mode 4 carries its own coefficient (gamma^T)
+  EvalArgs a;
+  memset(&a, 0, sizeof(a));
+  a.mode = q_net >= 0 ? 1 : 0; a.obs_dim = c.obs_dim; a.act_dim = c.act_dim; a.rows = rows;
+  a.policy_out_tanh = c.policy_out_tanh; a.action_range = c.action_range;
   for (int i = 0; i < MPG_MAX_OBS; ++i) a.obs_scale[i] = c.obs_scale[i];
-  const int ntiles = (a.rows + TILE_R - 1) / TILE_R;
+  a.obs = obs; a.act = act; a.out = out;
+  if (!act) a.pol = net_dev(ctx, policy_net);
+  if (q_net >= 0) a.q = net_dev(ctx, q_net);
+  if (q2_net >= 0) { a.q2 = net_dev(ctx, q2_net); a.out2 = out2; }
+  const int ntiles = (rows + TILE_R - 1) / TILE_R;
   const int grid = ntiles < ctx->sms ? ntiles : ctx->sms;
   mlp_kernels(c.hidden, ctx->act).eval(a, grid, (cudaStream_t)stream);
   ctx->launches++;
@@ -909,9 +908,32 @@ static int launch_eval(mpg_ctx* ctx, EvalArgs& a, void* stream) {
   return MPG_OK;
 }
 
-// ---- tensor-core evaluation of Q(sigma obs, a), a = given actions or pi(sigma obs): the forward rollout kernel with
-// horizon 0 (one policy forward + one Q forward per row) -- 0.07 ms per 65,536 rows instead of 0.4 ms per MLP on the
-// FFMA tile engine.  Used by the target / TD-error / bootstrap entry points when the handle runs the TC backend.
+static bool tc_eval_ok(const mpg_ctx* ctx, int rows) {
+  return ctx->backend == MPG_BACKEND_TC && ctx->tc.ready && rows <= ctx->cfg.max_rows;
+}
+
+// tensor-core evaluation of Q(sigma obs, a), a = given actions or pi(sigma obs): the forward rollout kernel with horizon 0
+// (one policy forward + one Q forward per row) -- 0.07 ms per 65,536 rows instead of 0.4 ms per MLP on the FFMA tile
+// engine.  Its step 0 observes get_obs(reset(obs)), as every rollout does.
+static int tc_q_eval(mpg_ctx* ctx, int q_net, int policy_net, int rows, const float* obs, const float* actions, float* out,
+                     void* stream) {
+  const mpg_rollout_params p = horizon0_params(rows, policy_net, q_net);
+  return mpg_rollout_forward(ctx, &p, obs, actions, nullptr, out, nullptr, nullptr, nullptr, stream);
+}
+
+// Q_q(sigma obs, a) into out and, with q2_net >= 0, Q_q2(sigma obs, a) into out2, a = act or pi_policy(sigma obs): the
+// evaluations of the target, TD-error and bootstrap entry points, on tensor cores where the handle runs them and the batch
+// fits its capacity, else on the FFMA kernel (both Q nets in one launch)
+static int eval_q(mpg_ctx* ctx, int policy_net, int rows, const float* obs, const float* act, int q_net, float* out,
+                  int q2_net, float* out2, void* stream) {
+  if (!tc_eval_ok(ctx, rows)) return ffma_eval(ctx, policy_net, rows, obs, act, q_net, out, q2_net, out2, stream);
+  int rc = tc_q_eval(ctx, q_net, policy_net, rows, obs, act, out, stream);
+  if (!rc && q2_net >= 0) rc = tc_q_eval(ctx, q2_net, policy_net, rows, obs, act, out2, stream);
+  return rc;
+}
+
+// out = (base + shift) scale + coef min(q1, q2) - sub, q2 and sub optional: the arithmetic of the Q target
+// (mpg_learner.py:126-134, 147-152), the TD error (136-144) and the n-step bootstrap (153-169)
 __global__ void affine_q_kernel(int n, const float* __restrict__ base, float shift, float scale, float coef,
                                 const float* __restrict__ q1, const float* __restrict__ q2, const float* __restrict__ sub,
                                 float* __restrict__ out) {
@@ -920,16 +942,12 @@ __global__ void affine_q_kernel(int n, const float* __restrict__ base, float shi
   const float q = q2 ? fminf(q1[i], q2[i]) : q1[i];
   out[i] = (base[i] + shift) * scale + coef * q - (sub ? sub[i] : 0.f);
 }
-static bool tc_eval_ok(const mpg_ctx* ctx, int rows) {
-  return ctx->backend == MPG_BACKEND_TC && ctx->tc.ready && rows <= ctx->cfg.max_rows;
-}
-static int tc_q_eval(mpg_ctx* ctx, int q_net, int policy_net, int rows, const float* obs, const float* actions, float* out,
-                     void* stream) {
-  mpg_rollout_params p;
-  memset(&p, 0, sizeof(p));
-  p.rows = rows; p.M = 1; p.horizon = 0; p.n_list = 1; p.list[0] = 0; p.list_w[0] = 1.f;
-  p.q_net = q_net; p.policy_net = policy_net;
-  return mpg_rollout_forward(ctx, &p, obs, actions, nullptr, out, nullptr, nullptr, nullptr, stream);
+static int affine_q(mpg_ctx* ctx, int rows, const float* base, float shift, float scale, float coef, const float* q2,
+                    const float* sub, float* out, void* stream) {
+  affine_q_kernel<<<(rows + 255) / 256, 256, 0, (cudaStream_t)stream>>>(rows, base, shift, scale, coef, ctx->qtmp.p, q2, sub, out);
+  ctx->launches++;
+  CUDA_OK(ctx, cudaGetLastError());
+  return MPG_OK;
 }
 
 int mpg_policy_forward(mpg_ctx* ctx, int net, int rows, const float* obs, float* act_out, void* stream) {
@@ -938,15 +956,10 @@ int mpg_policy_forward(mpg_ctx* ctx, int net, int rows, const float* obs, float*
   if (rc) return rc;
   if (tc_eval_ok(ctx, rows) && (net == MPG_NET_POLICY || net == MPG_NET_POLICY_TARGET)) {
     // tensor-core forward kernel, horizon 0, no Q: the action of step 0 is the output (traj_act)
-    mpg_rollout_params p;
-    memset(&p, 0, sizeof(p));
-    p.rows = rows; p.M = 1; p.horizon = 0; p.n_list = 0; p.q_net = -1; p.policy_net = net;
+    const mpg_rollout_params p = horizon0_params(rows, net, -1);
     return mpg_rollout_forward(ctx, &p, obs, nullptr, nullptr, nullptr, nullptr, nullptr, act_out, stream);
   }
-  EvalArgs a;
-  memset(&a, 0, sizeof(a));
-  a.mode = 0; a.rows = rows; a.obs = obs; a.out = act_out; a.net0 = net_dev(ctx, net);
-  return launch_eval(ctx, a, stream);
+  return ffma_eval(ctx, net, rows, obs, nullptr, -1, act_out, -1, nullptr, stream);
 }
 
 int mpg_q_forward(mpg_ctx* ctx, int net, int rows, const float* obs, const float* act, float* q_out, void* stream) {
@@ -955,10 +968,7 @@ int mpg_q_forward(mpg_ctx* ctx, int net, int rows, const float* obs, const float
   if (rc) return rc;
   if (tc_eval_ok(ctx, rows) && net != MPG_NET_POLICY && net != MPG_NET_POLICY_TARGET && ctx->nets[MPG_NET_POLICY].set)
     return tc_q_eval(ctx, net, MPG_NET_POLICY, rows, obs, act, q_out, stream);
-  EvalArgs a;
-  memset(&a, 0, sizeof(a));
-  a.mode = 1; a.rows = rows; a.obs = obs; a.act = act; a.out = q_out; a.net0 = net_dev(ctx, net);
-  return launch_eval(ctx, a, stream);
+  return ffma_eval(ctx, -1, rows, obs, act, net, q_out, -1, nullptr, stream);
 }
 
 int mpg_q_target(mpg_ctx* ctx, int double_q, int rows, const float* rew, const float* obs_tp1, float* target_out,
@@ -967,45 +977,23 @@ int mpg_q_target(mpg_ctx* ctx, int double_q, int rows, const float* rew, const f
   int rc = check_net(ctx, MPG_NET_POLICY_TARGET);
   if (!rc) rc = check_net(ctx, MPG_NET_Q1_TARGET);
   if (!rc && double_q) rc = check_net(ctx, MPG_NET_Q2_TARGET);
+  if (!rc) rc = q_scratch(ctx, rows);
+  if (!rc) rc = eval_q(ctx, MPG_NET_POLICY_TARGET, rows, obs_tp1, nullptr, MPG_NET_Q1_TARGET, ctx->qtmp.p,
+                       double_q ? MPG_NET_Q2_TARGET : -1, ctx->qtmp2.p, stream);
   if (rc) return rc;
-  if (tc_eval_ok(ctx, rows)) {
-    const mpg_config& c = ctx->cfg;
-    rc = tc_q_eval(ctx, MPG_NET_Q1_TARGET, MPG_NET_POLICY_TARGET, rows, obs_tp1, nullptr, ctx->tc.qtmp, stream);
-    if (!rc && double_q) rc = tc_q_eval(ctx, MPG_NET_Q2_TARGET, MPG_NET_POLICY_TARGET, rows, obs_tp1, nullptr, ctx->tc.qtmp2, stream);
-    if (rc) return rc;
-    affine_q_kernel<<<(rows + 255) / 256, 256, 0, (cudaStream_t)stream>>>(rows, rew, c.rew_shift, c.rew_scale, c.gamma, ctx->tc.qtmp,
-                                                                         double_q ? ctx->tc.qtmp2 : nullptr, nullptr, target_out);
-    ctx->launches++;
-    CUDA_OK(ctx, cudaGetLastError());
-    return MPG_OK;
-  }
-  EvalArgs a;
-  memset(&a, 0, sizeof(a));
-  a.mode = 2; a.rows = rows; a.obs = obs_tp1; a.rew = rew; a.out = target_out; a.n_q = double_q ? 2 : 1;
-  a.net0 = net_dev(ctx, MPG_NET_POLICY_TARGET); a.net1 = net_dev(ctx, MPG_NET_Q1_TARGET);
-  if (double_q) a.net2 = net_dev(ctx, MPG_NET_Q2_TARGET);
-  return launch_eval(ctx, a, stream);
+  const mpg_config& c = ctx->cfg;
+  return affine_q(ctx, rows, rew, c.rew_shift, c.rew_scale, c.gamma, double_q ? ctx->qtmp2.p : nullptr, nullptr,
+                  target_out, stream);
 }
 
 int mpg_q_bootstrap(mpg_ctx* ctx, int rows, const float* base, float coef, const float* obs, float* out, void* stream) {
   if (!ctx || !base || !obs || !out || rows <= 0) return fail(ctx, MPG_ERR_ARG, "bad argument to mpg_q_bootstrap%s");
   int rc = check_net(ctx, MPG_NET_POLICY_TARGET);
   if (!rc) rc = check_net(ctx, MPG_NET_Q1_TARGET);
+  if (!rc) rc = q_scratch(ctx, rows);
+  if (!rc) rc = eval_q(ctx, MPG_NET_POLICY_TARGET, rows, obs, nullptr, MPG_NET_Q1_TARGET, ctx->qtmp.p, -1, nullptr, stream);
   if (rc) return rc;
-  if (tc_eval_ok(ctx, rows)) {
-    rc = tc_q_eval(ctx, MPG_NET_Q1_TARGET, MPG_NET_POLICY_TARGET, rows, obs, nullptr, ctx->tc.qtmp, stream);
-    if (rc) return rc;
-    affine_q_kernel<<<(rows + 255) / 256, 256, 0, (cudaStream_t)stream>>>(rows, base, 0.f, 1.f, coef, ctx->tc.qtmp, nullptr, nullptr, out);
-    ctx->launches++;
-    CUDA_OK(ctx, cudaGetLastError());
-    return MPG_OK;
-  }
-  EvalArgs a;
-  memset(&a, 0, sizeof(a));
-  a.mode = 4; a.rows = rows; a.obs = obs; a.rew = base; a.out = out; a.gamma = coef;
-  a.net0 = net_dev(ctx, MPG_NET_POLICY_TARGET); a.net1 = net_dev(ctx, MPG_NET_Q1_TARGET);
-  rc = launch_eval(ctx, a, stream);
-  return rc;
+  return affine_q(ctx, rows, base, 0.f, 1.f, coef, nullptr, nullptr, out, stream);
 }
 
 int mpg_td_error(mpg_ctx* ctx, int rows, const float* obs, const float* act, const float* rew, const float* obs_tp1,
@@ -1014,23 +1002,13 @@ int mpg_td_error(mpg_ctx* ctx, int rows, const float* obs, const float* act, con
   int rc = check_net(ctx, MPG_NET_POLICY_TARGET);
   if (!rc) rc = check_net(ctx, MPG_NET_Q1_TARGET);
   if (!rc) rc = check_net(ctx, MPG_NET_Q1);
+  if (!rc) rc = q_scratch(ctx, rows);
+  if (!rc) rc = eval_q(ctx, MPG_NET_POLICY_TARGET, rows, obs_tp1, nullptr, MPG_NET_Q1_TARGET, ctx->qtmp.p, -1, nullptr, stream);
+  // the policy does not enter Q1(sigma obs, act); the tensor-core kernel takes the online policy's weight images
+  if (!rc) rc = eval_q(ctx, MPG_NET_POLICY, rows, obs, act, MPG_NET_Q1, ctx->qtmp2.p, -1, nullptr, stream);
   if (rc) return rc;
-  if (tc_eval_ok(ctx, rows)) {
-    const mpg_config& c = ctx->cfg;
-    rc = tc_q_eval(ctx, MPG_NET_Q1_TARGET, MPG_NET_POLICY_TARGET, rows, obs_tp1, nullptr, ctx->tc.qtmp, stream);
-    if (!rc) rc = tc_q_eval(ctx, MPG_NET_Q1, MPG_NET_POLICY, rows, obs, act, ctx->tc.qtmp2, stream);
-    if (rc) return rc;
-    affine_q_kernel<<<(rows + 255) / 256, 256, 0, (cudaStream_t)stream>>>(rows, rew, c.rew_shift, c.rew_scale, c.gamma, ctx->tc.qtmp,
-                                                                         nullptr, ctx->tc.qtmp2, td_out);
-    ctx->launches++;
-    CUDA_OK(ctx, cudaGetLastError());
-    return MPG_OK;
-  }
-  EvalArgs a;
-  memset(&a, 0, sizeof(a));
-  a.mode = 3; a.rows = rows; a.obs = obs; a.obs2 = obs_tp1; a.act = act; a.rew = rew; a.out = td_out;
-  a.net0 = net_dev(ctx, MPG_NET_POLICY_TARGET); a.net1 = net_dev(ctx, MPG_NET_Q1_TARGET); a.net2 = net_dev(ctx, MPG_NET_Q1);
-  return launch_eval(ctx, a, stream);
+  const mpg_config& c = ctx->cfg;
+  return affine_q(ctx, rows, rew, c.rew_shift, c.rew_scale, c.gamma, nullptr, ctx->qtmp2.p, td_out, stream);
 }
 
 int mpg_model_reset(mpg_ctx* ctx, int rows, const float* obs, float* state_out, void* stream) {
@@ -1126,8 +1104,8 @@ int mpg_compute_rewards(mpg_ctx* ctx, int rows, const float* state, const float*
 
 int mpg_clip_global_norm(mpg_ctx* ctx, float* grad, int n, float clip, float* norm_out, void* stream) {
   if (!ctx || !grad || n <= 0 || !(clip > 0.f)) return fail(ctx, MPG_ERR_ARG, "bad argument to mpg_clip_global_norm%s");
-  sumsq_partial_kernel<<<CLIP_BLOCKS, 256, 0, (cudaStream_t)stream>>>(grad, n, ctx->red_part + 64);
-  clip_apply_kernel<<<CLIP_BLOCKS, 256, 0, (cudaStream_t)stream>>>(grad, n, clip, ctx->red_part + 64, norm_out);
+  sumsq_partial_kernel<<<RED_BLOCKS, 256, 0, (cudaStream_t)stream>>>(grad, n, ctx->red_part + RED_BLOCKS);
+  clip_apply_kernel<<<RED_BLOCKS, 256, 0, (cudaStream_t)stream>>>(grad, n, clip, ctx->red_part + RED_BLOCKS, norm_out);
   ctx->launches += 2;
   CUDA_OK(ctx, cudaGetLastError());
   return MPG_OK;

@@ -76,4 +76,65 @@ __device__ __forceinline__ float philox_normal(uint64_t seed, uint64_t row, uint
   return sqrtf(-2.f * logf(u1)) * cospif(2.f * u2);
 }
 
+// ---------------------------------------------------------------------------------------------
+// Deterministic sums: every sum of the library runs in a fixed order, so that losses, norms and return statistics are
+// bit-reproducible.  A two-stage sum has RED_BLOCKS blocks each reduce a fixed slice with block_sum, then adds their
+// partials in index order with sum_in_order.
+// ---------------------------------------------------------------------------------------------
+constexpr int RED_BLOCKS = 64;
+
+// the sums over the block of each of v[0..N): a shared-memory tree (blockDim.x a power of two, at most 256); every
+// thread of the block calls it and gets the sums
+template <int N>
+__device__ __forceinline__ void block_sum(float (&v)[N]) {
+  __shared__ float red[N][256];
+#pragma unroll
+  for (int j = 0; j < N; ++j) red[j][threadIdx.x] = v[j];
+  __syncthreads();
+  for (int o = blockDim.x / 2; o > 0; o >>= 1) {
+    if (threadIdx.x < o) {
+#pragma unroll
+      for (int j = 0; j < N; ++j) red[j][threadIdx.x] += red[j][threadIdx.x + o];
+    }
+    __syncthreads();
+  }
+#pragma unroll
+  for (int j = 0; j < N; ++j) v[j] = red[j][0];
+}
+__device__ __forceinline__ float block_sum(float v) {
+  float s[1] = {v};
+  block_sum(s);
+  return s[0];
+}
+
+// p[0] + p[stride] + ... + p[(N - 1) stride], added in index order
+template <int N>
+__device__ __forceinline__ float sum_in_order(const float* p, int stride = 1) {
+  float s = 0.f;
+  for (int b = 0; b < N; ++b) s += p[b * stride];
+  return s;
+}
+
+// A device buffer that only grows.  grow() allocates the larger buffer before it frees the old one, so a growth that
+// fails leaves the old buffer in place; the contents are not carried over.
+template <typename T>
+struct DevBuf {
+  T* p = nullptr;
+  size_t n = 0;   // elements
+
+  cudaError_t grow(size_t want) {
+    if (want <= n) return cudaSuccess;
+    T* q = nullptr;
+    const cudaError_t e = cudaMalloc((void**)&q, want * sizeof(T));
+    if (e != cudaSuccess) {
+      cudaGetLastError();
+      return e;
+    }
+    cudaFree(p);
+    p = q; n = want;
+    return cudaSuccess;
+  }
+  void release() { cudaFree(p); p = nullptr; n = 0; }
+};
+
 }  // namespace mpg

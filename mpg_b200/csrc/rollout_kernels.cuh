@@ -350,33 +350,24 @@ __global__ void __launch_bounds__(NT, 1) q_grad_kernel(const __grid_constant__ Q
   flush_grad_acc(a.q, ga, partial);
   if (tid < TILE_R) red[tid] = loss;
   __syncthreads();
-  if (tid == 0) {
-    float sum = 0.f;
-    for (int i = 0; i < TILE_R; ++i) sum += red[i];
-    a.loss_partial[blockIdx.x] = sum;
-  }
+  if (tid == 0) a.loss_partial[blockIdx.x] = sum_in_order<TILE_R>(red);
 }
 
 // ---------------------------------------------------------------------------------------------
-// forward-only evaluations on a replay batch
-//   mode 0: act_out = pi_net0(sigma obs)                    (policy.py:193-212)
-//   mode 1: out = Q_net0(sigma obs, act)                    (policy.py:219-241)
-//   mode 2: out = rho(r+shift) + gamma min(Q_net1, Q_net2)(sigma o', pi_net0(sigma o'))  (mpg_learner.py:126-134);
-//           single-Q when n_q == 1 (mpg_learner.py:147-152)
-//   mode 3: out = rho(r+shift) + gamma Q_net1(sigma o', pi_net0(sigma o')) - Q_net2(sigma o, a)  (mpg_learner.py:136-144)
-//   mode 4: out = rew[row] + gamma * Q_net1(sigma o, pi_net0(sigma o))   (n-step bootstrap, mpg_learner.py:153-169;
-//           `rew` carries the partial return, `gamma` the coefficient gamma^T)
+// forward-only evaluations on a replay batch, a = act or, when act is null, pi_pol(sigma obs)
+//   mode 0: out = a = pi_pol(sigma obs)                                         (policy.py:193-212)
+//   mode 1: out = Q_q(sigma obs, a), and out2 = Q_q2(sigma obs, a) when out2 is set   (policy.py:219-241)
+// The Q targets, TD errors and bootstraps combine these values on the host side (api.cu: affine_q_kernel).
 // ---------------------------------------------------------------------------------------------
 struct EvalArgs {
-  int mode, obs_dim, act_dim, rows, n_q, policy_out_tanh;
-  float action_range, rew_scale, rew_shift, gamma;
+  int mode, obs_dim, act_dim, rows, policy_out_tanh;
+  float action_range;
   float obs_scale[MPG_MAX_OBS];
-  const float* obs;      // obs (modes 0,1,3) / obs_tp1 (mode 2)
-  const float* obs2;     // obs_tp1 (mode 3)
+  const float* obs;
   const float* act;
-  const float* rew;
   float* out;
-  NetDev net0, net1, net2;
+  float* out2;
+  NetDev pol, q, q2;
 };
 
 template <int H, int ACT>
@@ -388,58 +379,35 @@ __global__ void __launch_bounds__(NT, 1) eval_kernel(const __grid_constant__ Eva
   for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
     const int row = tile * TILE_R + tid;
     const bool rt = tid < TILE_R, valid = rt && row < a.rows;
-    auto load_obs = [&](const float* src) {
-      if (rt)
-        for (int i = 0; i < a.obs_dim; ++i)
-          sm.xin[i * RP + tid] = valid ? src[(size_t)row * a.obs_dim + i] * a.obs_scale[i] : 0.f;
-    };
-    auto load_act = [&]() {
+    if (rt)
+      for (int i = 0; i < a.obs_dim; ++i)
+        sm.xin[i * RP + tid] = valid ? a.obs[(size_t)row * a.obs_dim + i] * a.obs_scale[i] : 0.f;
+    if (a.act) {
       if (rt)
         for (int j = 0; j < a.act_dim; ++j)
           sm.xin[(a.obs_dim + j) * RP + tid] = valid ? a.act[(size_t)row * a.act_dim + j] : 0.f;
-    };
-    auto policy_to_xin = [&](const NetDev& net) {   // a = pi(xin obs rows) -> xin action rows
+    } else {   // a = pi(xin obs rows) -> xin action rows
       __syncthreads();
-      mlp_forward_tile<H, ACT>(net, sm, a.act_dim);
+      mlp_forward_tile<H, ACT>(a.pol, sm, a.act_dim);
       if (rt)
         for (int j = 0; j < a.act_dim; ++j)
           sm.xin[(a.obs_dim + j) * RP + tid] = head_fwd(sm.y3[j * RP + tid], a.policy_out_tanh, a.action_range);
-    };
+    }
     auto q_eval = [&](const NetDev& net) -> float {
       __syncthreads();
       mlp_forward_tile<H, ACT>(net, sm, 1);
       return rt ? sm.y3[tid] : 0.f;
     };
     if (a.mode == 0) {
-      load_obs(a.obs);
-      policy_to_xin(a.net0);
       if (valid)
         for (int j = 0; j < a.act_dim; ++j) a.out[(size_t)row * a.act_dim + j] = sm.xin[(a.obs_dim + j) * RP + tid];
-    } else if (a.mode == 1) {
-      load_obs(a.obs);
-      load_act();
-      float q = q_eval(a.net0);
-      if (valid) a.out[row] = q;
-    } else if (a.mode == 2) {
-      load_obs(a.obs);
-      policy_to_xin(a.net0);
-      float q = q_eval(a.net1);
-      if (a.n_q == 2) q = fminf(q, q_eval(a.net2));
-      if (valid) a.out[row] = (a.rew[row] + a.rew_shift) * a.rew_scale + a.gamma * q;
-    } else if (a.mode == 4) {
-      load_obs(a.obs);
-      policy_to_xin(a.net0);
-      float q = q_eval(a.net1);
-      if (valid) a.out[row] = a.rew[row] + a.gamma * q;
     } else {
-      load_obs(a.obs2);
-      policy_to_xin(a.net0);
-      float q1 = q_eval(a.net1);
-      __syncthreads();
-      load_obs(a.obs);
-      load_act();
-      float q0 = q_eval(a.net2);
-      if (valid) a.out[row] = (a.rew[row] + a.rew_shift) * a.rew_scale + a.gamma * q1 - q0;
+      const float q = q_eval(a.q);
+      if (valid) a.out[row] = q;
+      if (a.out2) {
+        const float q2 = q_eval(a.q2);
+        if (valid) a.out2[row] = q2;
+      }
     }
     __syncthreads();
   }

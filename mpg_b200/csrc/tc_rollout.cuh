@@ -171,15 +171,10 @@ struct TcState {
   bool ready = false;
   TcNetImages nets[MPG_NUM_NETS];
   uint8_t* scratch_img = nullptr;   // self-test image
-  float* act_ckpt = nullptr;        // [n_list][max_rows][MAX_A]: MPG_MAX_LIST entries at creation, grows with longer lists
-  size_t act_ckpt_bytes = 0;
-  float* qtmp = nullptr;            // [max_rows] Q values of the regression pass / of the target evaluations
-  float* qtmp2 = nullptr;           // [max_rows] second Q value (double-Q minimum, TD error)
+  DevBuf<float> act_ckpt;           // [n_list][max_rows][MAX_A]: MPG_MAX_LIST entries at creation, grows with longer lists
   float* z_ckpt = nullptr;          // [max_horizon+1][max_rows][2 MAX_A] action and head derivative of every step (BPTT)
-  uint8_t* store = nullptr;         // dW operand store (allocated on first use, grows)
-  size_t store_bytes = 0;
-  uint8_t* h2store = nullptr;       // h2 images of the forward pass, [tile][step][128 KB] (allocated on first use, grows)
-  size_t h2store_bytes = 0;
+  DevBuf<uint8_t> store;            // dW operand store (allocated on first use)
+  DevBuf<uint8_t> h2store;          // h2 images of the forward pass, [tile][step][128 KB] (allocated on first use)
 };
 
 template <typename K>
@@ -196,11 +191,10 @@ inline bool tc_init(TcState& t, const mpg_config& cfg, int hidden_layers, int /*
     ws_bytes += n;
     return true;
   };
-  bool ok = alloc((void**)&t.scratch_img, tc::BIG_IMAGE_BYTES)
-            && alloc((void**)&t.act_ckpt, t.act_ckpt_bytes = (size_t)MPG_MAX_LIST * cfg.max_rows * MAX_A * sizeof(float))
-            && alloc((void**)&t.z_ckpt, (size_t)(cfg.max_horizon + 1) * cfg.max_rows * 2 * MAX_A * sizeof(float))
-            && alloc((void**)&t.qtmp, (size_t)cfg.max_rows * sizeof(float))
-            && alloc((void**)&t.qtmp2, (size_t)cfg.max_rows * sizeof(float));
+  const size_t act_ckpt_n = (size_t)MPG_MAX_LIST * cfg.max_rows * MAX_A;
+  bool ok = alloc((void**)&t.scratch_img, tc::BIG_IMAGE_BYTES) && t.act_ckpt.grow(act_ckpt_n) == cudaSuccess
+            && alloc((void**)&t.z_ckpt, (size_t)(cfg.max_horizon + 1) * cfg.max_rows * 2 * MAX_A * sizeof(float));
+  if (ok) ws_bytes += act_ckpt_n * sizeof(float);
   for (int n = 0; n < MPG_NUM_NETS && ok; ++n)
     ok = alloc((void**)&t.nets[n].big_fwd, tc::BIG_IMAGE_BYTES) && alloc((void**)&t.nets[n].big_dx, tc::BIG_IMAGE_BYTES)
          && alloc((void**)&t.nets[n].l1, 16384) && alloc((void**)&t.nets[n].l1b, 16384) && alloc((void**)&t.nets[n].in, 16384);
@@ -215,7 +209,7 @@ inline bool tc_init(TcState& t, const mpg_config& cfg, int hidden_layers, int /*
 }
 
 inline void tc_destroy(TcState& t) {
-  cudaFree(t.scratch_img); cudaFree(t.act_ckpt); cudaFree(t.z_ckpt); cudaFree(t.h2store); cudaFree(t.qtmp); cudaFree(t.qtmp2); cudaFree(t.store);
+  cudaFree(t.scratch_img); t.act_ckpt.release(); cudaFree(t.z_ckpt); t.h2store.release(); t.store.release();
   for (int n = 0; n < MPG_NUM_NETS; ++n) {
     cudaFree(t.nets[n].big_fwd); cudaFree(t.nets[n].big_dx); cudaFree(t.nets[n].l1); cudaFree(t.nets[n].l1b); cudaFree(t.nets[n].in);
   }
@@ -240,26 +234,6 @@ inline tc::TcNet tc_net(const TcState& t, int net, const float* flat, int in_dim
   n.W3 = flat + L.oWout; n.b2 = flat + L.ob(2); n.b3 = flat + L.obout;
   n.in_dim = in_dim; n.out_dim = out_dim;
   return n;
-}
-
-inline bool tc_ensure_buf(uint8_t*& buf, size_t& have, size_t bytes) {
-  if (bytes <= have) return true;
-  cudaFree(buf);
-  buf = nullptr; have = 0;
-  if (cudaMalloc((void**)&buf, bytes) != cudaSuccess) { cudaGetLastError(); return false; }
-  have = bytes;
-  return true;
-}
-inline bool tc_ensure_store(TcState& t, size_t bytes) { return tc_ensure_buf(t.store, t.store_bytes, bytes); }
-inline bool tc_ensure_h2store(TcState& t, size_t bytes) { return tc_ensure_buf(t.h2store, t.h2store_bytes, bytes); }
-// the old buffer stays when the larger one cannot be had
-inline bool tc_ensure_act_ckpt(TcState& t, size_t bytes) {
-  if (bytes <= t.act_ckpt_bytes) return true;
-  float* p = nullptr;
-  if (cudaMalloc((void**)&p, bytes) != cudaSuccess) { cudaGetLastError(); return false; }
-  cudaFree(t.act_ckpt);
-  t.act_ckpt = p; t.act_ckpt_bytes = bytes;
-  return true;
 }
 
 #ifdef MPG_DEBUG_PROBES

@@ -302,16 +302,18 @@ def test_closed_loop_trajectories_vs_oracle(backend, H, act):
 # ------------------------------------------------------------------------------------------------
 @pytest.mark.gpu
 @pytest.mark.parametrize('act', ACTS)
-@pytest.mark.parametrize('backend,H', CONFIGS, ids=CONFIG_IDS)
-def test_forward_entry_points_vs_oracle(backend, H, act):
+@pytest.mark.parametrize('backend,H,cap', [c + (1000,) for c in CONFIGS] + [('tc', 256, 500)],
+                         ids=CONFIG_IDS + ['tc256_rows_over_capacity'])
+def test_forward_entry_points_vs_oracle(backend, H, act, cap):
     """compute_action / compute_Q1 (mpg_policy_forward / mpg_q_forward), mpg_q_target (double Q), mpg_td_error and
-    mpg_q_bootstrap against the oracle's networks."""
+    mpg_q_bootstrap against the oracle's networks.  A tensor-core handle evaluates a batch within its capacity on
+    tensor cores, and a larger one (cap < B: more rows than max_rows) on the FFMA kernel."""
     B = 1000
-    args = _args('MPG-v2', PT, H, act, replay_batch_size=B)   # capacity B: the tensor-core handle evaluates on tensor cores
+    args = _args('MPG-v2', PT, H, act, replay_batch_size=cap)
     w = synthetic.make_policy_with_qs_weights(3, args.obs_dim, args.act_dim, H, double_q=True)
     pol = _policy(args, w, backend)
     e = pol.engine
-    assert e.cfg.max_rows >= B
+    assert (e.cfg.max_rows >= B) == (cap >= B)
     rng = np.random.default_rng(4)
     obs, obs1 = synthetic.make_obs(rng, PT, B), synthetic.make_obs(rng, PT, B)
     sigma = np.asarray(args.obs_scale, np.float32)
