@@ -132,6 +132,9 @@ int mpg_set_rollout_list(mpg_ctx* ctx, int n, const int32_t* list_host, const fl
  *   grad_out   (param_count(policy)) UNCLIPPED d loss / d theta, loss = sum_k w_k * (-mean R_k),
  *              scaled by 1/(M*global_rows) so that per-rank results add up under all-reduce
  *   returns_out (n_list, M*rows) per-row R_k = sum_{t<k} gamma^t rho r_t + gamma^k Q(p_k, a_k)
+ * Step 0 observes obs as given (p_0 = sigma obs) while the model starts from reset(obs); a later step observes
+ * p_t = sigma get_obs(s_t).  obs need not lie on the model's observation map (real-environment future columns,
+ * double-pendulum constraint forces).  The same holds for mpg_rollout_forward and mpg_q_grad.
  */
 int mpg_policy_grad(mpg_ctx* ctx, const mpg_rollout_params* p, const float* obs, const float* noise,
                     float* grad_out, float* returns_out, void* stream);
@@ -141,7 +144,8 @@ int mpg_policy_grad(mpg_ctx* ctx, const mpg_rollout_params* p, const float* obs,
  *   start_actions (rows, act_dim) or NULL (a_0 = pi(p_0))
  *   returns_out (n_list, M*rows)
  *   traj_obs (horizon, M*rows, obs_dim) raw obs_{t+1};  traj_rew (horizon, M*rows) processed
- *   rewards;  traj_act (horizon+1, M*rows, act_dim) actions; each may be NULL */
+ *   rewards;  traj_act (horizon+1, M*rows, act_dim) actions; each may be NULL
+ * Step 0 observes obs as given, the model starts from reset(obs) (see mpg_policy_grad). */
 int mpg_rollout_forward(mpg_ctx* ctx, const mpg_rollout_params* p, const float* obs, const float* start_actions,
                         const float* noise, float* returns_out, float* traj_obs, float* traj_rew, float* traj_act,
                         void* stream);
@@ -155,7 +159,8 @@ int mpg_returns_tile_mean(mpg_ctx* ctx, const float* returns, int n_list, int ro
 
 /* ---- Q side ------------------------------------------------------------------------------- */
 /* q_forward_and_backward (mpg_learner.py:326-354, nadp.py:173-184): loss = 0.5 mean (Q(sigma o, a) - target)^2.
- *   grad_out (param_count(net)) scaled by 1/global_rows; loss_sum_out[0] = sum_i 0.5 (Q - target)^2 */
+ *   grad_out (param_count(net)) scaled by 1/global_rows; loss_sum_out[0] = sum_i 0.5 (Q - target)^2
+ * Q sees obs as given on both backends; on tensor cores this is step 0 of a horizon-0 rollout (see mpg_policy_grad). */
 int mpg_q_grad(mpg_ctx* ctx, int net, int rows, int64_t global_rows, const float* obs, const float* act,
                const float* target, float* grad_out, float* loss_sum_out, void* stream);
 /* compute_action / compute_target_action (policy.py:193-212) on RAW obs (scale applied inside) */

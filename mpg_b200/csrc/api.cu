@@ -914,7 +914,7 @@ static bool tc_eval_ok(const mpg_ctx* ctx, int rows) {
 
 // tensor-core evaluation of Q(sigma obs, a), a = given actions or pi(sigma obs): the forward rollout kernel with horizon 0
 // (one policy forward + one Q forward per row) -- 0.07 ms per 65,536 rows instead of 0.4 ms per MLP on the FFMA tile
-// engine.  Its step 0 observes get_obs(reset(obs)), as every rollout does.
+// engine.  Like every rollout, its step 0 feeds the nets sigma * obs as given, the same input eval_kernel reads.
 static int tc_q_eval(mpg_ctx* ctx, int q_net, int policy_net, int rows, const float* obs, const float* actions, float* out,
                      void* stream) {
   const mpg_rollout_params p = horizon0_params(rows, policy_net, q_net);

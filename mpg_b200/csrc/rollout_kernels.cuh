@@ -170,7 +170,10 @@ __global__ void __launch_bounds__(NT, 1) rollout_kernel(const __grid_constant__ 
             for (int j = 0; j < S; ++j) c[j] = s[j];
           }
         }
-        for (int i = 0; i < a.obs_dim; ++i) sm.xin[i * RP + tid] = valid ? o[i] * a.obs_scale[i] : 0.f;
+        // step 0 observes obs as given, re-read from global memory: replay data need not lie on the model's observation
+        // map (real path deltas in the future columns, constraint forces); a later step observes get_obs(s_t)
+        for (int i = 0; i < a.obs_dim; ++i)
+          sm.xin[i * RP + tid] = valid ? (t == 0 ? a.obs[(size_t)i_idx * a.obs_dim + i] : o[i]) * a.obs_scale[i] : 0.f;
       }
       const bool given = (t == 0 && a.use_start_actions);
       if (!given) {
@@ -233,7 +236,8 @@ __global__ void __launch_bounds__(NT, 1) rollout_kernel(const __grid_constant__ 
             for (int j = 0; j < S; ++j) s[j] = c[j];
             E::get_obs(s, o, a.nfd);
           }
-          for (int i = 0; i < a.obs_dim; ++i) sm.xin[i * RP + tid] = valid ? o[i] * a.obs_scale[i] : 0.f;
+          for (int i = 0; i < a.obs_dim; ++i)   // step 0: obs as given, as in the forward pass
+            sm.xin[i * RP + tid] = valid ? (t == 0 ? a.obs[(size_t)i_idx * a.obs_dim + i] : o[i]) * a.obs_scale[i] : 0.f;
         }
         __syncthreads();
         mlp_forward_tile<H, ACT>(a.pol, sm, A);

@@ -435,22 +435,23 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
     }
     float rsum = 0.f, gpow = 1.f;
 
-    // [sigma*obs(s) | act | 0.. | 1] -> p image (row warps)
+    // [sigma*obs_t | act | 0.. | 1] -> p image (row warps).  Step 0 observes the row of obs as given, re-read from global
+    // memory (replay data need not lie on the model's observation map); a later step observes get_obs(s_t).
     // f16: forward computations read the image as an fp16 pair; BPTT (first-layer recompute, D1, the db2 record) as bf16
-    auto write_pimg = [&](const float* st, const float* act_or_null, bool f16, uint8_t* gimg = nullptr) {
+    auto write_pimg = [&](int t, const float* act_or_null, bool f16, uint8_t* gimg = nullptr) {
       // every index below is a compile-time constant (fixed trip counts + predicates): o[] stays in registers, and the
       // image row is produced one 8-element chunk at a time
       float o[MPG_MAX_OBS];
 #pragma unroll
       for (int i = 0; i < MPG_MAX_OBS; ++i) o[i] = 0.f;
-      E::get_obs(st, o, a.nfd);
+      E::get_obs(s, o, a.nfd);
 #pragma unroll
       for (int kh = 0; kh < 2; ++kh) {
         float x[8];
 #pragma unroll
         for (int e = 0; e < 8; ++e) {
           const int i = kh * 8 + e;
-          float v = i < a.obs_dim ? o[i] * a.obs_scale[i] : 0.f;
+          float v = i < a.obs_dim ? (t == 0 ? a.obs[(size_t)i_idx * a.obs_dim + i] : o[i]) * a.obs_scale[i] : 0.f;
           if (act_or_null) {
 #pragma unroll
             for (int j = 0; j < NA; ++j)
@@ -560,7 +561,7 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
 #pragma unroll
           for (int j = 0; j < S; ++j) c[j] = s[j];
         }
-        if (!given) write_pimg(s, nullptr, true);
+        if (!given) write_pimg(t, nullptr, true);
       }
       if (!given) {
         float zpre[NA];
@@ -591,7 +592,7 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
 #pragma unroll
           for (int j = 0; j < NA; ++j) A.act_ckpt[((size_t)kidx * MB + grow) * NA + j] = act[j];
         if (a.has_q) {
-          if (rowthread) write_pimg(s, act, true);
+          if (rowthread) write_pimg(t, act, true);
           qv = q_forward(false, nullptr);
         }
         // every entry of step t gets its row, repeated entries included
@@ -687,7 +688,7 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
 #pragma unroll
             for (int j = 0; j < NA; ++j) ak[j] = valid ? A.act_ckpt[((size_t)kidx * MB + grow) * NA + j] : 0.f;
             acc_wait();
-            write_pimg(s, ak, true);
+            write_pimg(t, ak, true);
           }
           const float qv = q_forward(true, qslot);         // h2q image in ACT
           if (rowthread) {
@@ -696,7 +697,7 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
             float ak[NA];
 #pragma unroll
             for (int j = 0; j < NA; ++j) ak[j] = valid ? A.act_ckpt[((size_t)kidx * MB + grow) * NA + j] : 0.f;
-            write_pimg(s, ak, false, qslot ? qslot + SLOT_P : nullptr);
+            write_pimg(t, ak, false, qslot ? qslot + SLOT_P : nullptr);
             fence_proxy_async();
             mbar_arrive(&b->p_full);
           }
@@ -799,7 +800,7 @@ __device__ __forceinline__ void run_rollout(const TcArgs& A, uint8_t* smem, Bars
         if (rowthread) {
           acc_wait();
           stamp(12);
-          write_pimg(s, nullptr, false, rec ? slot + SLOT_P : nullptr);
+          write_pimg(t, nullptr, false, rec ? slot + SLOT_P : nullptr);
           fence_proxy_async();
           mbar_arrive(&b->p_full);
           stamp(13);

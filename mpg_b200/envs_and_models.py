@@ -126,7 +126,8 @@ class PathTrackingEnv(object):
     """The REAL PathTracking environment (path_tracking_env.py:356-487) batched on the GPU: reset(init_obs=obs) and
     step(action) -> (obs, reward, done, info) with the reference's 200 Hz x 20 sub-step simulation, reference-path
     projection and judge_done.  Used by the MPG-v1 n-step targets (through the fused rollout) and available to
-    workers / evaluators.  Random resets (`reset()` without init_obs) draw from the reset law in mpg_b200.synthetic."""
+    workers / evaluators.  Random resets (`reset()` without init_obs) draw the pose from the reset law in
+    mpg_b200.synthetic and observe it as the environment does, future columns against the reference path included."""
 
     def __init__(self, num_future_data=0, num_agent=1, **kwargs):
         self.num_future_data, self.num_agent = num_future_data, num_agent
@@ -142,9 +143,24 @@ class PathTrackingEnv(object):
             self.obs = self.engine.dev(kwargs['init_obs'])
         else:
             from .synthetic import make_obs
-            self.obs = self.engine.dev(make_obs(self._rng, 'PathTracking-v0', self.num_agent, self.num_future_data))
+            base = self.engine.dev(make_obs(self._rng, 'PathTracking-v0', self.num_agent))
+            # the future columns of the drawn pose, as the environment's own observation of it (not copies of delta_y)
+            fut = self._future_columns(base[:, 0] + 20.0, base[:, 3], base[:, 5])
+            self.obs = torch.stack([base[:, i] for i in range(6)] + fut, 1).contiguous()
         self.state = self.engine.model_reset(self.obs)
         return self.obs
+
+    def _future_columns(self, vx, dy, x):
+        """The future columns of _get_obs (path_tracking_env.py:384-402) at a reset pose: delta_y of the pose against the
+        reference path at x + k * v_x / 200 * 20 * 2, k = 1..num_future_data; at reset y = delta_y + path_y(x)."""
+        import math
+        path_y = lambda xs: (7.5 * torch.sin(xs * 2.0 * math.pi / 200.0) + 2.5 * torch.sin(xs * 2.0 * math.pi / 300.0)
+                             - 5.0 * torch.sin(xs * 2.0 * math.pi / 400.0))
+        y, xf, cols = dy + path_y(x), x.clone(), []
+        for _ in range(self.num_future_data):
+            xf = xf + vx * 1.0 / 200.0 * 20.0 * 2.0
+            cols.append(y - path_y(xf))
+        return cols
 
     def step(self, action):
         self.action = self.engine.dev(action)
@@ -167,15 +183,7 @@ class PathTrackingEnv(object):
         dy = z[0]
         x = 600.0 * u[0]
         cols = [vx - 20.0, vx * torch.tan(0.15 * z[2]), 0.3 * z[3], dy, (math.pi / 9) * z[1], x]
-        # future columns of _get_obs (path_tracking_env.py:384-402): delta_y of the pose against the reference path at
-        # x + k * v_x / 200 * 20 * 2; at reset y = delta_y + path_y(x)
-        path_y = lambda xs: (7.5 * torch.sin(xs * 2.0 * math.pi / 200.0) + 2.5 * torch.sin(xs * 2.0 * math.pi / 300.0)
-                             - 5.0 * torch.sin(xs * 2.0 * math.pi / 400.0))
-        y, xf = dy + path_y(x), x.clone()
-        for _ in range(self.num_future_data):
-            xf = xf + vx * 1.0 / 200.0 * 20.0 * 2.0
-            cols.append(y - path_y(xf))
-        return torch.stack(cols, 1).contiguous()
+        return torch.stack(cols + self._future_columns(vx, dy, x), 1).contiguous()
 
     def reset_done(self, fresh=None):
         """reset() of the reference without init_obs (path_tracking_env.py:422-454): agents whose `done` flag is set
