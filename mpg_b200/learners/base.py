@@ -58,6 +58,7 @@ class LearnerBase(object):
         self.policy_gradient_timer = CudaTimerStat()
         self.q_gradient_timer = CudaTimerStat()
         self.target_timer = CudaTimerStat()
+        self.allreduce_timer = CudaTimerStat()     # world_size > 1 only
         self.stats = {}
         self.info_for_buffer = {}
         # noise of the model rollout: None -> in-kernel Philox keyed by (seed, global row, step);
@@ -145,7 +146,10 @@ class LearnerBase(object):
         return parallel.shard_rows(self._dev['batch_obs'].shape[0], self.world_size, self.rank)[1]
 
     def _allreduce(self, flat):
-        return parallel.allreduce_flat(flat, self.world_size)
+        if self.world_size == 1:
+            return flat
+        with self.allreduce_timer:
+            return parallel.allreduce_flat(flat, self.world_size)
 
     def _to_host(self, dev):
         """The update's single device -> host copy: into a pinned staging buffer (a pageable destination makes the

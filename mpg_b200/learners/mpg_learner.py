@@ -133,6 +133,8 @@ class MPGLearner(LearnerBase):
             all_losses=list(all_losses),
             returns_var=[float(ret_sq[klist.index(k)] / B - (ret_sums[klist.index(k)] / B) ** 2) for k in lst],
         ))
+        if self.world_size > 1:
+            self.stats.update(allreduce_time=self.allreduce_timer.mean)
         if v2:
             self.stats.update(dict(q_loss2=np.float32(host[ng + 1] / B), q_gradient_norm2=np.float32(norm_vals[1])))
         self.flat_grad_device = flat[:ng]     # the same clipped gradients, still on the device (apply_gradients takes it)

@@ -94,5 +94,7 @@ class NADPLearner(LearnerBase):
             num_rollout_list_for_policy=self.num_rollout_list_for_policy_update,
             num_rollout_list_for_q=self.num_rollout_list_for_q_estimation,
         ))
+        if self.world_size > 1:
+            self.stats.update(allreduce_time=self.allreduce_timer.mean)
         self.flat_grad_device = flat[:ng]     # the same clipped gradients, still on the device (apply_gradients takes it)
         return self._split_to_numpy(host[:ng], ['q', 'pi'])

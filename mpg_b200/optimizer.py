@@ -1,12 +1,18 @@
 """SingleProcessOffPolicyOptimizer with the reference's interface (optimizer.py:286-397): the synchronous
 sample -> replay -> learn -> apply loop.  The asynchronous Ray variant (optimizer.py:127-280) is replaced by
-synchronous data parallelism inside the learner (one NCCL all-reduce of the flat gradient)."""
+synchronous data parallelism inside the learner (one NCCL all-reduce of the flat gradient).
+
+Under a process group every rank runs this loop on its own worker and replay buffer.  Every branch of step() is
+taken alike on every rank (the NaN check looks at the all-reduced gradient), so the replicas stay identical;
+the optimizer.jsonl log and the checkpoints are rank 0's, and the replicas are compared at every evaluation
+iteration and in stop()."""
 import json
 import logging
 import os
 
 import numpy as np
 
+from . import parallel
 from .utils.misc import TimerStat
 
 logger = logging.getLogger(__name__)
@@ -20,6 +26,7 @@ class SingleProcessOffPolicyOptimizer(object):
         self.stats, self.eval_history = {}, []
         self.log_dir = getattr(args, 'log_dir', None)
         self.shared = getattr(learner, 'policy_with_value', None) is getattr(worker, 'policy_with_value', object())
+        self.world_size, self.rank = parallel.dist_info()
         logger.info('start filling the replay')
         while not len(self.replay_buffer) >= self.args.replay_starts:
             self._sample()
@@ -28,7 +35,8 @@ class SingleProcessOffPolicyOptimizer(object):
 
     def _sample(self):
         batch = self.worker.sample_arrays()
-        self.num_sampled_steps += batch[0].shape[0]
+        # every rank samples as many steps on the same schedule: the count over all ranks
+        self.num_sampled_steps += batch[0].shape[0] * self.world_size
         self.replay_buffer.add_arrays(*batch)
 
     def get_stats(self):
@@ -61,22 +69,24 @@ class SingleProcessOffPolicyOptimizer(object):
             # one shared PolicyWithQs: hand over the flat device gradient, no host -> device copy of what just came back
             dev_grads = getattr(self.learner, 'flat_grad_device', None) if self.shared else None
             self.worker.apply_gradients(self.iteration, grads if dev_grads is None else dev_grads)
-        if self.log_dir and self.iteration % getattr(self.args, 'log_interval', 100) == 0:
+        if self.log_dir and self.rank == 0 and self.iteration % getattr(self.args, 'log_interval', 100) == 0:
             os.makedirs(self.log_dir, exist_ok=True)
             rec = {k: (v if not isinstance(v, (list, np.ndarray)) else [float(x) for x in v]) for k, v in learner_stats.items()}
             rec = {k: (float(v) if isinstance(v, (np.floating, np.integer)) else v) for k, v in rec.items()}
             with open(os.path.join(self.log_dir, 'optimizer.jsonl'), 'a') as f:
                 f.write(json.dumps(dict(rec, **self.get_stats())) + '\n')
+        if self.world_size > 1 and self.iteration % self.args.eval_interval == 0:
+            parallel.check_replicas(self.worker.policy_with_value, self.iteration)
         if self.evaluator is not None and self.iteration % self.args.eval_interval == 0:
             if not getattr(self.evaluator, 'policy_with_value', None) is self.worker.policy_with_value:
                 self.evaluator.set_weights(self.worker.get_weights())
             self.eval_history.append((self.iteration, self.evaluator.run_evaluation(self.iteration)))
         model_dir = getattr(self.args, 'model_dir', None)
-        if model_dir and self.iteration % getattr(self.args, 'save_interval', 3000) == 0:   # optimizer.py:389-391
+        if model_dir and self.rank == 0 and self.iteration % getattr(self.args, 'save_interval', 3000) == 0:   # optimizer.py:389-391
             self.worker.save_weights(model_dir, self.iteration)
             self.worker.save_ppc_params(model_dir)
         self.get_stats()
         self.iteration += 1
 
     def stop(self):
-        pass
+        parallel.check_replicas(self.worker.policy_with_value, self.iteration)

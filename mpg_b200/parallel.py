@@ -3,8 +3,14 @@ blocks), every rank produces SUMS already scaled by 1/B_global, and ONE all-redu
 flat buffer [grads of every net | scalar sums] makes all ranks hold the global-batch gradient; the per-net
 global-norm clip and the statistics are then computed redundantly on every rank.
 
+The data-parallel trainer keeps one replica of every net per rank: rank 0's weights are broadcast once at the
+start (broadcast_weights), after which every rank applies the same all-reduced gradient, and check_replicas
+compares a checksum of every rank's weights.
+
 Plumbing only (torch.distributed: NCCL over NVLink on GPUs, gloo in the CPU tests) -- no arithmetic of
 the hot path lives here."""
+import hashlib
+
 import numpy as np
 import torch
 
@@ -28,6 +34,55 @@ def allreduce_flat(flat, world_size):
     if world_size > 1:
         torch.distributed.all_reduce(flat, op=torch.distributed.ReduceOp.SUM)
     return flat
+
+
+def _collective_device():
+    """Where tensors of a collective live: the current GPU under NCCL, the host under gloo."""
+    if torch.distributed.get_backend() == 'nccl':
+        return torch.device('cuda', torch.cuda.current_device())
+    return torch.device('cpu')
+
+
+def broadcast_weights(policy, src=0):
+    """Overwrite every rank's nets (get_weights order: models, then targets) with those of rank `src`: one flat
+    fp32 broadcast.  The replicas start equal whatever seed each rank's nets were initialised with."""
+    nets = policy.get_weights()
+    flat = torch.from_numpy(np.concatenate([np.asarray(w, np.float32).ravel() for net in nets for w in net]))
+    flat = flat.to(_collective_device())
+    torch.distributed.broadcast(flat, src=src)
+    flat, pos, out = flat.cpu().numpy(), 0, []
+    for net in nets:
+        out.append([])
+        for w in net:
+            out[-1].append(flat[pos:pos + w.size].reshape(w.shape))
+            pos += w.size
+    policy.set_weights(out)
+
+
+def weights_checksum(nets):
+    """SHA-256 of the bytes of every weight array (get_weights order) -> 4 int64 words."""
+    h = hashlib.sha256()
+    for net in nets:
+        for w in net:
+            h.update(np.ascontiguousarray(w, np.float32).tobytes())
+    return torch.from_numpy(np.frombuffer(h.digest(), dtype=np.int64).copy())
+
+
+def check_replicas(policy, iteration):
+    """Fault detector of the data-parallel trainer: every rank all-gathers the checksum of every rank's weights and
+    raises if any differ.  Every rank sees the same gathered checksums, so every rank raises together and none is
+    left waiting in a later collective."""
+    world_size, rank = dist_info()
+    if world_size == 1:
+        return
+    mine = weights_checksum(policy.get_weights()).to(_collective_device())
+    every = [torch.empty_like(mine) for _ in range(world_size)]
+    torch.distributed.all_gather(every, mine)
+    every = [t.cpu() for t in every]
+    differ = [r for r in range(world_size) if not torch.equal(every[r], every[0])]
+    if differ:
+        raise RuntimeError(f'replica weights diverged at iteration {iteration}: ranks {differ} differ from rank 0 '
+                           f'(seen on rank {rank})')
 
 
 def net_shapes(obs_dim, act_dim, kind, hidden=256, layers=2):

@@ -1,4 +1,5 @@
-"""TimerStat with the reference's semantics (utils/misc.py:39-90): sliding window of 10, `.mean`.
+"""TimerStat with the reference's semantics (utils/misc.py:39-90): sliding window of 10, `.mean`; `.total` sums
+every sample, not only the window.
 
 CudaTimerStat keeps the interface but measures DEVICE time: the learners only enqueue kernels inside the `with` block,
 so a host clock would report launch overhead.  Events are recorded on the current stream around the section and read
@@ -15,6 +16,7 @@ class TimerStat:
         self._samples = []
         self._start_time = None
         self.count = 0
+        self._total = 0.0
 
     def __enter__(self):
         assert self._start_time is None, 'concurrent updates not supported'
@@ -29,10 +31,15 @@ class TimerStat:
         if len(self._samples) > self._window_size:
             self._samples.pop(0)
         self.count += 1
+        self._total += dt
 
     @property
     def mean(self):
         return float(np.mean(self._samples)) if self._samples else 0.0
+
+    @property
+    def total(self):
+        return self._total
 
 
 class CudaTimerStat(TimerStat):
@@ -65,3 +72,8 @@ class CudaTimerStat(TimerStat):
     def mean(self):
         self._resolve()
         return float(np.mean(self._samples)) if self._samples else 0.0
+
+    @property
+    def total(self):
+        self._resolve()
+        return self._total
